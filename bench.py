@@ -2,7 +2,7 @@
 """Benchmark of the GP+ hot path on B200: MLL + gradient evaluations per second at N=16384, D=10,
 Matern-5/2, FP64 (BASELINE.json configs[3]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n 16384]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n 16384] [--dump-outputs DIR]
 
 A *step* is one evaluation of the negative log marginal likelihood and its gradient w.r.t. all 13
 hyper-parameters on the full training set: fused covariance build, blocked DMMA Cholesky, triangular
@@ -49,6 +49,14 @@ def bench_config(n):
 def step_theta(thetas, k, rank=0):
     """theta of timed step k on ``rank``: prior draw 1 + (k + 8 rank) mod 65 (index 0 of ``thetas`` is theta_init)."""
     return thetas[1 + (k + 8 * rank) % W.N_PRIOR_DRAWS]
+
+
+def dump_outputs(dirname, arrays):
+    """``--dump-outputs``: every array of the last timed step as DIR/<name>.npy in float64, so that two builds can be
+    compared output for output (the inputs are seeded: the same arguments give the same inputs)."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.asarray(v, dtype=np.float64))
 
 
 class ClockSampler:
@@ -139,27 +147,23 @@ def oracle_full_size(n, theta_list, threads=None, warm=True):
 
 # ------------------------------------------------------------------------------------------------
 def run_reference(args):
-    """The reference arm: the reference's own CPU torch path for this workload.  The reference cannot be imported
-    on the GPU box (gpytorch / botorch are not installed anywhere, /root/reference does not travel), so the CPU
-    restatement in oracle/ -- pinned to the reference's own code by tests/test_reference_pin.py -- is timed (kind
-    "port") with every host thread, at the FULL size: ``steps`` in the line is the number of evaluations actually
-    run (bounded so that the arm ends within a few minutes; ``steps_requested`` keeps the driver's K)."""
+    """The reference arm: the reference's own CPU torch path for this workload.  The reference itself cannot be
+    imported where the benchmark runs (gpytorch / botorch are not installed, and the GP-Plus checkout is not part of
+    this repository), so the CPU restatement in oracle/ -- pinned to the reference's own code by
+    tests/test_reference_pin.py -- is timed (kind "port") with every host thread, at the FULL size, for exactly
+    ``--steps`` evaluations (about 25 s each at N=16384 on 16 cores)."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
     cores = os.cpu_count() or 1
     thetas = W.c4_theta_points(W.c4_model(256))
-    budget_s = float(os.environ.get("GPPLUS_REF_BUDGET_S", "150"))
-    run = []
     secs = []
-    t_begin = time.time()
-    for k in range(max(1, args.steps)):
-        s, _, threads = oracle_full_size(args.n, [step_theta(thetas, k)], cores, warm=(k == 0))
+    for k in range(args.steps):
+        s, outs, threads = oracle_full_size(args.n, [step_theta(thetas, k)], cores, warm=(k == 0))
         secs += s
-        run.append(k)
-        if time.time() - t_begin + max(secs) > budget_s:
-            break
     steps_run = len(secs)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs[0])
     rate = steps_run / sum(secs)
     line = {
         "impl": "reference", "metric": METRIC, "value": rate, "unit": "evals/s",
@@ -302,6 +306,9 @@ def run_ours(args):
     e2e_value = world * args.steps / float(e2e_elapsed)
     h2d = 8 * (eng.dq + eng.n_combo * eng.dz + eng.n_noise + eng.n_mean + 2)
     d2h = 8 * (4 + eng.dq + eng.n_noise + eng.n_mean) + 4
+    if args.dump_outputs and rank == 0:
+        # the last step of each timed arm: gpp_mll_grad's result dictionary, and (value, gradient) of the objective
+        dump_outputs(args.dump_outputs, dict(out, objective_value=f, objective_grad=g))
 
     # ---- the sharded workloads of the metric's second half, in the same torchrun world (every rank takes part) ----
     extra = {}
@@ -785,7 +792,14 @@ def main():
     ap.add_argument("--no-dmma-arm", action="store_true", help="mll workload: skip the exact-DMMA arm of the same evaluation")
     ap.add_argument("--no-prior-sweep", action="store_true",
                     help="mll workload: skip the untimed sweep over all 65 prior draws (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="mll workload: write what the last timed step computed to DIR/<name>.npy (float64, a few "
+                         "hundred bytes in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.workload != "mll":
+        ap.error("--dump-outputs applies to the mll workload only")
     if args.warmup < 3 and args.impl == "ours" and args.workload == "mll":
         args.warmup = 3
     if args.workload == "fit":

@@ -1,7 +1,9 @@
-"""Test-only import shim that lets the UNMODIFIED reference sources under /root/reference execute in this image.
+"""Test-only import shim that lets the UNMODIFIED reference sources (a checkout of Bostanabad-Research-Group/GP-Plus,
+not part of this repository) execute without gpytorch / botorch.  The checkout is looked for in ``$GPPLUS_REFERENCE``,
+else in ``oracle/_ref`` (git-ignored); without one the live tests skip and the stored fixtures stand in for it.
 
 TEST INFRASTRUCTURE -- only ``tests/`` and ``tests/golden/make_reference_fixtures.py`` use it; the product package
-never imports it, and nothing under /root/reference is copied: ``install()`` registers a package called ``gpplus``
+never imports it, and nothing of the reference is copied: ``install()`` registers a package called ``gpplus``
 whose ``__path__`` is the reference checkout itself, so ``import gpplus.models`` runs the reference's own files where
 they lie.
 
@@ -26,7 +28,7 @@ import sys
 import types
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REFERENCE = os.environ.get("GPPLUS_REFERENCE", "/root/reference")
+REFERENCE = os.environ.get("GPPLUS_REFERENCE", os.path.join(os.path.dirname(HERE), "_ref"))
 
 
 def available() -> bool:
@@ -44,7 +46,7 @@ def install():
         pkg.__path__ = [REFERENCE]
         pkg.__spec__ = importlib.machinery.ModuleSpec("gpplus", None, is_package=True)
         pkg.__spec__.submodule_search_locations = [REFERENCE]
-        sys.dont_write_bytecode = True  # /root/reference is read-only
+        sys.dont_write_bytecode = True  # leave the reference checkout as it is
         sys.modules["gpplus"] = pkg
     import gpytorch  # noqa: F401  (the shim)
     return sys.modules["gpplus"]

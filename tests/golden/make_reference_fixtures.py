@@ -1,8 +1,8 @@
-"""Generate fixtures FROM THE REFERENCE ITSELF: /root/reference's own, unmodified Python files are imported through
+"""Generate fixtures FROM THE REFERENCE ITSELF: a GP-Plus checkout's own, unmodified Python files are imported through
 the test-only shim (oracle/_ref_shim: a fake ``gpplus`` package pointing at the checkout plus a dense-torch
 re-statement of the gpytorch API the reference calls) and their outputs are stored next to this script.
 
-    python tests/golden/make_reference_fixtures.py        # needs /root/reference; ~1 min on CPU
+    GPPLUS_REFERENCE=<GP-Plus checkout> python tests/golden/make_reference_fixtures.py   # ~1 min on CPU
 
 What the fixtures pin (every number below is produced by the reference's code, not by this repo's):
   * model construction: parameter names / shapes / order (``named_parameters``), prior names / order

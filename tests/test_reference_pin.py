@@ -1,6 +1,6 @@
 """Parity pinned to the REFERENCE'S OWN CODE (SURVEY 8c).
 
-``tests/golden/ref_*.npz`` are outputs of the unmodified files under /root/reference, executed through the test-only
+``tests/golden/ref_*.npz`` are outputs of the unmodified files of a GP-Plus checkout, executed through the test-only
 import shim ``oracle/_ref_shim`` by ``tests/golden/make_reference_fixtures.py``.  Here (CPU):
 
   * the CPU oracle (oracle/gpplus_oracle.py) is checked against those outputs -- this is what moves the oracle off
@@ -8,8 +8,8 @@ import shim ``oracle/_ref_shim`` by ``tests/golden/make_reference_fixtures.py``.
     means, noise model, priors, MLLObjective packing);
   * the product's host-side logic (parameter / prior order, ``pack_parameters``, ``get_bounds``,
     ``_sample_from_prior``, priors, acquisition formulas, preprocessing, test functions) is checked against them;
-  * when /root/reference is present (this container, not the GPU box) the reference functions are additionally
-    called LIVE on fresh random inputs.
+  * when a GP-Plus checkout is present (``$GPPLUS_REFERENCE`` or ``oracle/_ref``; it is not part of this repository)
+    the reference functions are additionally called LIVE on fresh random inputs.
 
 The GPU half (engine vs the same fixtures through the C ABI) is tests/test_reference_pin_gpu.py.
 """
@@ -218,11 +218,11 @@ def test_misc_helpers_match_the_reference_fixtures():
 
 
 # ------------------------------------------------------------------------------------------------
-# live comparison with the reference (this container only)
+# live comparison with the reference (only where a GP-Plus checkout is present: GPPLUS_REFERENCE or oracle/_ref)
 def _live():
     from oracle import _ref_shim
     if not _ref_shim.available():
-        pytest.skip("/root/reference is not present on this machine (fixtures cover the GPU box)")
+        pytest.skip("no GP-Plus reference checkout to call live (set GPPLUS_REFERENCE or place one at oracle/_ref)")
     _ref_shim.install()
 
 
