@@ -817,7 +817,9 @@ struct CholLookahead {
         GPP_TRY(cudaMalloc(&blk_flags, 256 * sizeof(int)));
         GPP_TRY(cudaMemset(blk_flags, 0, 256 * sizeof(int)));
         if (getenv("GPP_BLOCK_CTAS")) blk_ctas = atoi(getenv("GPP_BLOCK_CTAS"));
-        panels = (T + PANEL_BLOCKS - 1) / PANEL_BLOCKS;
+        // one set of panel events per tile column: enough for every panel width the schedules accept (GPP_PANEL,
+        // GPP_OZ_LAZY_PB down to 2; sizing by PANEL_BLOCKS made narrower panels fail with cudaErrorInvalidValue)
+        panels = T;
         ev_pf.resize(panels);
         ev_tu.resize(panels);
         ev_m1.resize(panels);

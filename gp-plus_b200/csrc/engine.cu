@@ -48,6 +48,16 @@ static void set_err(const char* what, cudaError_t e) {
 
 enum { EV_START = 0, EV_COV, EV_CHOL, EV_TRTRI, EV_SOLVE, EV_LAUUM, EV_GRAD, EV_END, EV_COUNT };
 
+// Everything gpp_create decides besides the problem's shape: the arithmetic of the O(N^3) stages (gpp_set_fp64_mode,
+// GPP_FP64) and the development switches, per handle and process-wide (int fields only: compared with memcmp).
+// A parked handle is handed back only when the configuration in force now equals the one it was built under.
+struct CreateConfig {
+    int lookahead, graph, early_out, small_block;                                    // per handle
+    int panel_blocks, overlap_inverse, gemm_bm, gemm_stagger, oz_items_per_cta;       // process globals
+    int int8;                                                                         // INT8-sliced O(N^3) stages
+    int oz_min_trail, oz_min_level, oz_next, oz_inner, oz_lazy, oz_kinv_levels, oz_lazy_min, oz_lazy_pb, oz_stagger;
+};
+
 struct gpp_handle {
     int device = 0;
     cudaStream_t st = nullptr;
@@ -112,6 +122,7 @@ struct gpp_handle {
     cudaEvent_t ev_info = nullptr;                 // factorisation status available (jitter-ladder early-out)
     ThetaLayout layout;                            // optional: O(p) host side of MLLObjective.fun
     std::vector<double> g_w, g_z, g_noise, g_beta;  // gradient scratch of gpp_objective
+    CreateConfig cfg;                              // configuration the handle was created under
 };
 
 static const double* hyp_w(const gpp_handle* h) { return h->hyp; }
@@ -188,8 +199,96 @@ static const size_t kPoolMaxHandleBytes = 192ull << 20;  // handles up to Np = 2
 static const size_t kPoolMaxBytes = 6ull << 30;
 static const size_t kPoolMaxHandles = 160;
 
-static bool same_shape(const gpp_handle* h, const gpp_problem* p, int device) {
-    return h->device == device && h->n == p->n && h->dq == p->dq && h->dz == p->dz &&
+// the configuration a handle with T tile rows gets when it is created now (defaults are the production configuration;
+// the process globals keep the value an earlier gpp_create gave them unless the environment sets them again)
+static CreateConfig read_config(int T) {
+    CreateConfig c;
+    memset(&c, 0, sizeof(c));
+    const char* e;
+    c.lookahead = 1;
+    if ((e = getenv("GPP_CHOL")) != nullptr) c.lookahead = strcmp(e, "blocked") != 0;
+    c.graph = T <= 16;  // N <= 2048: an evaluation is a chain of ~25-100 tiny launches
+    if ((e = getenv("GPP_GRAPH")) != nullptr) c.graph = atoi(e) != 0;
+    c.early_out = 1;
+    if ((e = getenv("GPP_EARLY_OUT")) != nullptr) c.early_out = atoi(e) != 0;
+    c.small_block = 0;
+    if ((e = getenv("GPP_SMALL_BLOCK")) != nullptr) c.small_block = atoi(e);
+    c.panel_blocks = g_panel_blocks;
+    if ((e = getenv("GPP_PANEL")) != nullptr) c.panel_blocks = atoi(e);
+    c.overlap_inverse = g_overlap_inverse;
+    if ((e = getenv("GPP_OVERLAP_INV")) != nullptr) c.overlap_inverse = atoi(e);
+    c.gemm_bm = g_gemm_bm;
+    if ((e = getenv("GPP_GEMM_BM")) != nullptr) c.gemm_bm = atoi(e) == 64 ? 64 : 128;
+    c.gemm_stagger = g_gemm_stagger;
+    if ((e = getenv("GPP_STAGGER")) != nullptr) c.gemm_stagger = atoi(e);
+    {
+        // FP64 work of the O(N^3) stages: exact integer GEMMs on the INT8 tcgen05 tensor cores from Np = 3072 up
+        // (measured: 3.08 vs 3.42 ms at N = 3072, 14.8 vs 22.0 at 8192, 28.8 vs 63.5 at 12288; below that an evaluation
+        // is a CUDA-graph replay of latency-bound launches); GPP_FP64=dmma keeps everything on DMMA
+        e = getenv("GPP_FP64");
+        bool int8 = T >= 24;
+        const int mode = g_fp64_mode.load();
+        if (mode == GPP_FP64_DMMA) int8 = false;
+        if (mode == GPP_FP64_INT8) int8 = T >= 8;   // forced: the stages still pick DMMA for shapes that are too small
+        if (e && mode < 0) int8 = int8 && strcmp(e, "dmma") != 0;
+        c.int8 = int8;
+    }
+    c.oz_items_per_cta = g_oz_items_per_cta;
+    OzCtx d;   // defaults only (init() allocates)
+    c.oz_min_trail = d.min_trailing_tiles;
+    c.oz_min_level = d.min_level_tiles;
+    c.oz_next = d.next_on_oz;
+    c.oz_inner = d.inner_min_k;
+    c.oz_lazy = d.lazy;
+    c.oz_kinv_levels = d.kinv_levels;
+    c.oz_lazy_min = d.lazy_min_tiles;
+    c.oz_lazy_pb = d.lazy_pb;
+    c.oz_stagger = d.stagger;
+    if (c.int8) {
+        if ((e = getenv("GPP_OZ_IPC")) != nullptr) c.oz_items_per_cta = atoi(e) > 0 ? atoi(e) : 2;
+        if ((e = getenv("GPP_OZ_MIN_TRAIL")) != nullptr) c.oz_min_trail = atoi(e);
+        if ((e = getenv("GPP_OZ_MIN_LEVEL")) != nullptr) c.oz_min_level = atoi(e);
+        if ((e = getenv("GPP_OZ_NEXT")) != nullptr) c.oz_next = atoi(e);
+        if ((e = getenv("GPP_OZ_INNER")) != nullptr) c.oz_inner = atoi(e);
+        if ((e = getenv("GPP_OZ_LAZY")) != nullptr) c.oz_lazy = atoi(e);
+        if ((e = getenv("GPP_OZ_KINV_LEVELS")) != nullptr) c.oz_kinv_levels = atoi(e);
+        if ((e = getenv("GPP_OZ_LAZY_MIN")) != nullptr) c.oz_lazy_min = atoi(e);
+        if ((e = getenv("GPP_OZ_LAZY_PB")) != nullptr) c.oz_lazy_pb = std::min(std::max(atoi(e), 2), OzCtx::LAZY_PB);
+        if ((e = getenv("GPP_OZ_STAGGER")) != nullptr) c.oz_stagger = atoi(e);
+    }
+    return c;
+}
+
+static void apply_globals(const CreateConfig& c) {
+    g_panel_blocks = c.panel_blocks;
+    g_overlap_inverse = c.overlap_inverse;
+    g_gemm_bm = c.gemm_bm;
+    g_gemm_stagger = c.gemm_stagger;
+    g_oz_items_per_cta = c.oz_items_per_cta;
+}
+
+// per-handle switches (h->oz, when the handle has one, must exist already)
+static void apply_handle_config(gpp_handle* h, const CreateConfig& c) {
+    h->cfg = c;
+    h->use_lookahead = c.lookahead != 0;
+    h->use_graph = c.graph != 0;
+    h->early_out = c.early_out != 0;
+    h->small_block = c.small_block;
+    if (h->oz) {
+        h->oz->min_trailing_tiles = c.oz_min_trail;
+        h->oz->min_level_tiles = c.oz_min_level;
+        h->oz->next_on_oz = c.oz_next;
+        h->oz->inner_min_k = c.oz_inner;
+        h->oz->lazy = c.oz_lazy;
+        h->oz->kinv_levels = c.oz_kinv_levels;
+        h->oz->lazy_min_tiles = c.oz_lazy_min;
+        h->oz->lazy_pb = c.oz_lazy_pb;
+        h->oz->stagger = c.oz_stagger;
+    }
+}
+
+static bool same_shape(const gpp_handle* h, const gpp_problem* p, int device, const CreateConfig& cfg) {
+    return memcmp(&h->cfg, &cfg, sizeof(cfg)) == 0 && h->device == device && h->n == p->n && h->dq == p->dq && h->dz == p->dz &&
            h->n_combo == (p->dz > 0 ? p->n_combo : 0) && h->n_noise == p->n_noise && h->n_mean == p->n_mean &&
            h->kernel == p->kernel && h->n_pass == (p->n_pass > 1 ? p->n_pass : 1) && (h->level_idx != nullptr) == (p->dz > 0 && p->level_idx != nullptr) &&
            (h->noise_idx != nullptr) == (p->noise_idx != nullptr) && (h->mean_idx != nullptr) == (p->mean_idx != nullptr);
@@ -301,13 +400,15 @@ extern "C" int gpp_create(const gpp_problem* p, int device, gpp_handle** out) {
         return GPP_ERR_CUDA;
     }
 
+    const CreateConfig cfg = read_config((int)((p->n + 127) / 128));
+    apply_globals(cfg);
     {
-        // a parked handle of the same shape on this device: re-upload the data, keep everything else
+        // a parked handle of the same shape and configuration on this device: re-upload the data, keep everything else
         gpp_handle* reuse = nullptr;
         {
             std::lock_guard<std::mutex> lk(g_pool_mu);
             for (size_t i = 0; i < g_pool.size(); i++)
-                if (same_shape(g_pool[i], p, device)) {
+                if (same_shape(g_pool[i], p, device, cfg)) {
                     reuse = g_pool[i];
                     g_pool_bytes -= reuse->slab_bytes;
                     g_pool.erase(g_pool.begin() + (long)i);
@@ -316,6 +417,7 @@ extern "C" int gpp_create(const gpp_problem* p, int device, gpp_handle** out) {
         }
         if (reuse) {
             memset(&reuse->stats, 0, sizeof(reuse->stats));
+            apply_handle_config(reuse, cfg);   // (a failed graph capture may have switched the replay off)
             int rc = upload_problem(reuse, p);
             if (rc != GPP_OK) {
                 destroy_now(reuse);
@@ -382,54 +484,21 @@ extern "C" int gpp_create(const gpp_problem* p, int device, gpp_handle** out) {
             if (device < 64) done[device] = true;
         }
     }
-    {
-        // development switches (defaults are the production configuration)
-        const char* e;
-        if ((e = getenv("GPP_CHOL")) != nullptr) h->use_lookahead = strcmp(e, "blocked") != 0;
-        if ((e = getenv("GPP_PANEL")) != nullptr) g_panel_blocks = atoi(e);
-        if ((e = getenv("GPP_OVERLAP_INV")) != nullptr) g_overlap_inverse = atoi(e);
-        if ((e = getenv("GPP_GEMM_BM")) != nullptr) g_gemm_bm = atoi(e) == 64 ? 64 : 128;
-        if ((e = getenv("GPP_STAGGER")) != nullptr) g_gemm_stagger = atoi(e);
-        h->use_graph = h->T <= 16;  // N <= 2048: an evaluation is a chain of ~25-100 tiny launches
-        if ((e = getenv("GPP_GRAPH")) != nullptr) h->use_graph = atoi(e) != 0;
-        if ((e = getenv("GPP_EARLY_OUT")) != nullptr) h->early_out = atoi(e) != 0;
-        if ((e = getenv("GPP_SMALL_BLOCK")) != nullptr) h->small_block = atoi(e);
-    }
     CKH(h->la.init(h->T));
-    {
-        // FP64 work of the O(N^3) stages: exact integer GEMMs on the INT8 tcgen05 tensor cores from Np = 3072 up
-        // (measured: 3.08 vs 3.42 ms at N = 3072, 14.8 vs 22.0 at 8192, 28.8 vs 63.5 at 12288; below that an evaluation
-        // is a CUDA-graph replay of latency-bound launches); GPP_FP64=dmma keeps everything on DMMA
-        const char* e = getenv("GPP_FP64");
-        bool int8 = h->T >= 24;
-        const int mode = g_fp64_mode.load();
-        if (mode == GPP_FP64_DMMA) int8 = false;
-        if (mode == GPP_FP64_INT8) int8 = h->T >= 8;   // forced: the stages still pick DMMA for shapes that are too small
-        if (e && mode < 0) int8 = int8 && strcmp(e, "dmma") != 0;
-        if (int8) {
-            h->oz = new OzCtx();
-            if ((e = getenv("GPP_OZ_MIN_TRAIL")) != nullptr) h->oz->min_trailing_tiles = atoi(e);
-            if ((e = getenv("GPP_OZ_MIN_LEVEL")) != nullptr) h->oz->min_level_tiles = atoi(e);
-            if ((e = getenv("GPP_OZ_IPC")) != nullptr) g_oz_items_per_cta = atoi(e) > 0 ? atoi(e) : 2;
-            if ((e = getenv("GPP_OZ_NEXT")) != nullptr) h->oz->next_on_oz = atoi(e);
-            if ((e = getenv("GPP_OZ_INNER")) != nullptr) h->oz->inner_min_k = atoi(e);
-            if ((e = getenv("GPP_OZ_LAZY")) != nullptr) h->oz->lazy = atoi(e);
-            if ((e = getenv("GPP_OZ_KINV_LEVELS")) != nullptr) h->oz->kinv_levels = atoi(e);
-            if ((e = getenv("GPP_OZ_LAZY_MIN")) != nullptr) h->oz->lazy_min_tiles = atoi(e);
-            if ((e = getenv("GPP_OZ_LAZY_PB")) != nullptr) h->oz->lazy_pb = std::min(std::max(atoi(e), 2), OzCtx::LAZY_PB);
-            if ((e = getenv("GPP_OZ_STAGGER")) != nullptr) h->oz->stagger = atoi(e);
-            cudaError_t oe = h->oz->init((int)h->np);
-            if (oe == cudaErrorMemoryAllocation) {
-                // the digit planes (3 x 7 Np^2 bytes) do not fit next to the FP64 work matrices: stay on DMMA
-                cudaGetLastError();
-                h->oz->destroy();
-                delete h->oz;
-                h->oz = nullptr;
-            } else {
-                CKH(oe);
-            }
+    if (cfg.int8) {
+        h->oz = new OzCtx();
+        cudaError_t oe = h->oz->init((int)h->np);
+        if (oe == cudaErrorMemoryAllocation) {
+            // the digit planes (3 x 7 Np^2 bytes) do not fit next to the FP64 work matrices: stay on DMMA
+            cudaGetLastError();
+            h->oz->destroy();
+            delete h->oz;
+            h->oz = nullptr;
+        } else {
+            CKH(oe);
         }
     }
+    apply_handle_config(h, cfg);
 
     h->hyp_len = h->dq + h->n_pass * h->n_combo * h->dz + h->n_noise + h->n_mean + 2;
     h->res_len = 4 + h->dq + h->n_noise + h->n_mean;

@@ -16,20 +16,24 @@
 
 namespace gpp {
 
-__device__ __forceinline__ double oz_scale_from_max(double amax, double& inv56) {
-    // amax = m 2^ex (m in [0.5,1)): scale = 2^(ex+2); inv56 = 2^56 / scale.  Zero rows: scale 1, digits 0.
+__device__ __forceinline__ double oz_scale_from_max(double amax, double2& inv56) {
+    // amax = m 2^ex (m in [0.5,1)): scale = 2^(ex+2); x * 2^56 / scale = (x * inv56.x) * inv56.y with
+    // inv56.x * inv56.y = 2^(54-ex).  That power of two overflows a double for rows with a maximum below 2^-970, so it
+    // is applied as two exact multiplications there (inv56.y = 2^512); for every other row inv56.y = 1.
+    // Zero rows: scale 1, digits 0.
     if (!(amax > 0.0) || !(amax < 1.0e300)) {  // zero, NaN or infinite rows: keep them finite, the caller's status flags the NaN
-        inv56 = 0.0;
+        inv56 = make_double2(0.0, 0.0);
         return 1.0;
     }
     int ex;
     frexp(amax, &ex);
-    inv56 = ldexp(1.0, 56 - (ex + 2));
+    const int e56 = 56 - (ex + 2);
+    inv56 = e56 <= 1023 ? make_double2(ldexp(1.0, e56), 1.0) : make_double2(ldexp(1.0, e56 - 512), ldexp(1.0, 512));
     return ldexp(1.0, ex + 2);
 }
 
-__device__ __forceinline__ void oz_digits(double x, double inv56, int8_t (&d)[OZ_S]) {
-    long long v = __double2ll_rd(x * inv56);
+__device__ __forceinline__ void oz_digits(double x, double2 inv56, int8_t (&d)[OZ_S]) {
+    long long v = __double2ll_rd((x * inv56.x) * inv56.y);
 #pragma unroll
     for (int p = OZ_S - 1; p >= 0; p--) {
         const long long lo = (long long)(int8_t)(v & 0xff);
@@ -61,7 +65,7 @@ __global__ void __launch_bounds__(256) oz_split_rows_kernel(const double* __rest
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) amax = fmax(amax, __shfl_xor_sync(0xffffffffu, amax, o));
-    double inv56;
+    double2 inv56;
     const double sc = oz_scale_from_max(amax, inv56);
     if (lane == 0) scale[(long long)z * sc_zs + r] = sc;
     int8_t* out = planes + (long long)z * pl_zs + (long long)r * pitch;
@@ -119,7 +123,7 @@ __global__ void __launch_bounds__(256) oz_split_cols_kernel(const double* __rest
                                                             long long plane_stride, long long pl_zs,
                                                             double* __restrict__ scale, long long sc_zs) {
     __shared__ __align__(16) int8_t sm[OZ_S][64][OZ_TP];
-    __shared__ double s_inv[64];
+    __shared__ double2 s_inv[64];
     const int z = blockIdx.z;
     const int nk = (z == (int)gridDim.z - 1) ? krows_last : krows;
     const int c0 = blockIdx.x * 64, k0 = blockIdx.y * 64;
@@ -128,7 +132,7 @@ __global__ void __launch_bounds__(256) oz_split_cols_kernel(const double* __rest
     const int tid = threadIdx.x;
     if (tid < 64) {
         const double amax = __longlong_as_double((long long)colmax[(long long)z * cm_zs + c0 + tid]);
-        double inv56;
+        double2 inv56;
         const double sc = oz_scale_from_max(amax, inv56);
         s_inv[tid] = inv56;
         const int kfirst = lower ? (c0 / 128) * 128 : 0;
@@ -140,7 +144,7 @@ __global__ void __launch_bounds__(256) oz_split_cols_kernel(const double* __rest
     // (plane, column) instead of eight byte stores
     const int cp = (tid & 31) * 2;
     const int kb = (tid >> 5) * 8;
-    const double i0 = s_inv[cp], i1 = s_inv[cp + 1];
+    const double2 i0 = s_inv[cp], i1 = s_inv[cp + 1];
     unsigned long long w0[OZ_S], w1[OZ_S];
 #pragma unroll
     for (int p = 0; p < OZ_S; p++) { w0[p] = 0ull; w1[p] = 0ull; }

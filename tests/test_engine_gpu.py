@@ -249,7 +249,9 @@ def test_schedule_variants_are_bitwise_identical(n, monkeypatch):
     from gpplus_b200 import _engine as E
     p = make_problem(n, 5, 2, dz=2, n_combo=7, n_noise=2, seed=31)
     h = make_hyper(p, seed=13)
-    results = []
+    results, launches = [], []
+    # every configuration gets a handle built under its own settings: a parked handle of the same shape is only
+    # handed back under the configuration it was created with (gpp_create compares them)
     for env in ({"GPP_OVERLAP_INV": "1", "GPP_GRAPH": "1"}, {"GPP_OVERLAP_INV": "0", "GPP_GRAPH": "0"},
                 {"GPP_OVERLAP_INV": "1", "GPP_GRAPH": "0"}, {"GPP_CHOL": "blocked", "GPP_GRAPH": "0"}):
         for k in ("GPP_OVERLAP_INV", "GPP_GRAPH", "GPP_CHOL"):
@@ -258,12 +260,19 @@ def test_schedule_variants_are_bitwise_identical(n, monkeypatch):
             monkeypatch.setenv(k, v)
         eng = E.Engine(**engine_kwargs(p))
         try:
+            assert eng.fp64_mode() == E.FP64_DMMA
             out = eng.mll_grad(h, want_grad=True)
+            before = E.launch_count()
             out2 = eng.mll_grad(h, want_grad=True)  # second call replays the captured graph
+            launches.append(E.launch_count() - before)
             assert out["nll"] == out2["nll"] and np.array_equal(out["d_w"], out2["d_w"])
             results.append((out, eng.fetch("Linv"), eng.fetch("Kinv")))
         finally:
             eng.close()
+    # the blocked factorisation is a different chain of launches than the look-ahead schedule (same GPP_GRAPH=0);
+    # at T = 5 (n = 513) both happen to issue 29 launches per evaluation
+    if n > 640:
+        assert launches[3] != launches[2], launches
     ref = results[0]
     for out, li, ki in results[1:3]:
         assert out["nll"] == ref[0]["nll"]
@@ -306,6 +315,57 @@ def test_recycled_handles_give_the_results_of_fresh_ones():
     again.close()
     fresh_b.close()
     E.pool_clear()
+
+
+def test_pooled_handles_follow_the_settings_in_force(monkeypatch):
+    """A handle parked under one configuration is not handed back under another: set_fp64_mode ("for engines created
+    afterwards") and the per-handle switches read by gpp_create apply to the next create of the same shape, in both
+    orders.  N = 1100 (T = 9) is pooled and small enough for the forced INT8-sliced arithmetic (T >= 8)."""
+    from gpplus_b200 import _engine as E
+    p = make_problem(1100, 5, 2, dz=1, n_combo=4, seed=46)
+    h = make_hyper(p, seed=47)
+    want = {-1: E.FP64_DMMA, E.FP64_INT8: E.FP64_INT8}   # by size, T = 9 < 24: DMMA
+    E.pool_clear()
+    prev = E.set_fp64_mode(-1)
+    try:
+        for order in ((-1, E.FP64_INT8), (E.FP64_INT8, -1)):
+            nll = []
+            for mode in order:
+                E.set_fp64_mode(mode)
+                eng = E.Engine(**engine_kwargs(p))   # the second create finds the first handle parked
+                try:
+                    assert eng.fp64_mode() == want[mode], (order, mode)
+                    nll.append(eng.mll_grad(h, want_grad=True)["nll"])
+                finally:
+                    eng.close()
+            assert abs(nll[0] - nll[1]) <= 1e-11 * abs(nll[1]), nll
+        E.set_fp64_mode(-1)
+
+        def launches_per_evaluation(chol, fresh):
+            if fresh:
+                E.pool_clear()
+            if chol is None:
+                monkeypatch.delenv("GPP_CHOL", raising=False)
+            else:
+                monkeypatch.setenv("GPP_CHOL", chol)
+            eng = E.Engine(**engine_kwargs(p))
+            try:
+                eng.mll_grad(h, want_grad=True)
+                before = E.launch_count()
+                eng.mll_grad(h, want_grad=True)
+                return E.launch_count() - before
+            finally:
+                eng.close()
+
+        fresh = {c: launches_per_evaluation(c, True) for c in (None, "blocked")}
+        assert fresh[None] != fresh["blocked"], fresh
+        for order in ((None, "blocked"), ("blocked", None)):
+            E.pool_clear()
+            for c in order:
+                assert launches_per_evaluation(c, False) == fresh[c], (order, c)
+    finally:
+        E.set_fp64_mode(prev)
+        E.pool_clear()
 
 
 @pytest.mark.parametrize("kernel,n,n_pass", [(0, 300, 3), (2, 517, 5), (1, 130, 2)])

@@ -1,9 +1,18 @@
 // Development bench for the INT8-sliced FP64 GEMM (oz_gemm.cuh / oz_split.cuh); not part of the product library.
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -o tools/oz_lab tools/oz_lab.cu
-//   ./tools/oz_lab [check|perf|all]
+//   ./tools/oz_lab [check|ragged|maps|segments|limits|exponents|perf|all]
 // check: digit planes against a host re-computation, the integer GEMM against an exact host sum over the planes,
 //        the scaled result against a long-double product, transposed split against the row split, the
 //        lower-triangular K-range map (K^-1 = M^T M shape) and the batched form.
+// The check groups below print one line per check (observed error, its bound) and "<group>: ok" or "<group>: FAILED":
+//   ragged     the batched inverse levels of oz_trtri_level with a short last group (tiles_m_last = 1 and hb - 1)
+//   maps       oz_update_region with lower_off > 0 (filtered tiles untouched), oz_panel_solve (KSEL_TJ upper bound,
+//              B planes of LAZY_PB * 128 rows)
+//   segments   a K range of 2 * 128 + 10 blocks accumulated in k_min / k_max segments, items with empty ranges
+//   limits     digit planes written directly: the largest int32 accumulation (K = 16384, every pair product
+//              positive) in closed form, random digits against int64 host sums at 7, 6 and 5 levels
+//   exponents  split_rows / split_cols of rows with maxima from 2^-1074 to 2^996, NaN / Inf / zero rows, and the
+//              product of such rows
 // perf:  timings of square / SYRK / LAUUM shapes against the DMMA kernel.
 #include <cuda_runtime.h>
 #include <math.h>
@@ -11,9 +20,10 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <vector>
 
-#include "../gp-plus_b200/csrc/oz_split.cuh"
+#include "../gp-plus_b200/csrc/oz_chol.cuh"
 
 using namespace gpp;
 
@@ -342,6 +352,562 @@ static int check_batched() {
     return fails;
 }
 
+// ---- check groups ---------------------------------------------------------------------------------------------
+// Operand entries of the product checks have magnitudes in [0.5, 1] (random sign), so that even a one-term sum is far
+// above the representation error of its row: every product check can then use 1e-15 of sum |a||b| (plus |beta C|).
+static double mag_rand(unsigned long long& s) {
+    const double u = urand(s);
+    return (u < 0.0 ? -1.0 : 1.0) * (0.5 + 0.5 * fabs(u));
+}
+// C outside the live region of a launch is filled with this NaN bit pattern and must come back bit for bit
+static const unsigned long long kSentinel = 0x7ff4deadbeef0001ull;
+static double sentinel() {
+    double d;
+    memcpy(&d, &kSentinel, sizeof(d));
+    return d;
+}
+static bool same_bits(double a, double b) { return memcmp(&a, &b, sizeof(double)) == 0; }
+
+static int report(const char* group, const char* what, double err, double bound) {
+    const bool ok = err <= bound;   // a NaN error fails
+    printf("%s %s: error %.3e bound %.3e %s\n", group, what, err, bound, ok ? "ok" : "FAILED");
+    fflush(stdout);
+    return ok ? 0 : 1;
+}
+static int report_count(const char* group, const char* what, long long bad) {
+    printf("%s %s: %lld (bound 0) %s\n", group, what, bad, bad ? "FAILED" : "ok");
+    fflush(stdout);
+    return bad ? 1 : 0;
+}
+static int group_end(const char* group, int fails) {
+    printf("%s: %s (%d failing checks)\n", group, fails ? "FAILED" : "ok", fails);
+    fflush(stdout);
+    return fails;
+}
+
+template <typename Tv>
+static Tv* dev_upload(const std::vector<Tv>& h) {
+    Tv* d;
+    CHECK(cudaMalloc(&d, sizeof(Tv) * h.size()));
+    CHECK(cudaMemcpy(d, h.data(), sizeof(Tv) * h.size(), cudaMemcpyHostToDevice));
+    return d;
+}
+template <typename Tv>
+static void dev_download(std::vector<Tv>& h, const Tv* d) {
+    CHECK(cudaMemcpy(h.data(), d, sizeof(Tv) * h.size(), cudaMemcpyDeviceToHost));
+}
+
+// plane buffers of a context hold stale digits of earlier launches in practice: a K range that reaches past the
+// region a launch split would pick these up
+static void poison_planes(OzCtx& oz) {
+    for (OzPlanes* P : {&oz.PP, &oz.PA, &oz.PB, &oz.PW[0], &oz.PW[1]})
+        CHECK(cudaMemset(P->planes, 0x3c, (size_t)OZ_S * P->rows * P->pitch));
+}
+
+// one level of the recursive-doubling inverse (oz_trtri_level), nb = 3 groups, the last with last_s2 tile rows.
+// M is lower triangular by element inside its diagonal tiles and carries data of the same magnitude in the tiles
+// above the diagonal, which the K ranges (KSEL_TJ lower bound of part 1, KSEL_TI upper bound of part 2) must exclude.
+static int ragged_case(int hb, int T) {
+    const char* G = "ragged";
+    int fails = 0;
+    const int n = T * TILE, h = hb * TILE;
+    int nb = 0, last_s2 = 0;
+    for (int g = 0;; g++) {   // groups with a non-empty second half (trtri_level)
+        int s2 = T - (g * 2 * hb + hb);
+        if (s2 <= 0) break;
+        nb++;
+        last_s2 = s2 < hb ? s2 : hb;
+    }
+    std::vector<double> L((size_t)n * n), M((size_t)n * n), X((size_t)n * n, sentinel());
+    unsigned long long seed = 4242 + T;
+    for (auto& v : L) v = mag_rand(seed);
+    for (int r = 0; r < n; r++)
+        for (int c = 0; c < n; c++) M[(size_t)r * n + c] = (r / TILE == c / TILE && c > r) ? 0.0 : mag_rand(seed);
+    double *dL = dev_upload(L), *dM = dev_upload(M), *dX = dev_upload(X);
+    OzCtx oz;
+    CHECK(oz.init(n));
+    poison_planes(oz);
+    CHECK(oz_trtri_level(oz, dL, dM, dX, n, hb, 0, nb, last_s2, 1, 0));
+    CHECK(cudaDeviceSynchronize());
+    std::vector<double> Xg((size_t)n * n), Mg((size_t)n * n);
+    dev_download(Xg, dX);
+    // part 1: X21 = L21 M11, k blocks [tj, hb) of the group
+    double worst = 0.0;
+    long long touched = 0;
+    std::vector<char> live((size_t)n * n, 0);
+    for (int z = 0; z < nb; z++) {
+        const int g0 = z * 2 * h, rows = (z == nb - 1 ? last_s2 : hb) * TILE;
+        for (int i = g0 + h; i < g0 + h + rows; i++)
+            for (int j = g0; j < g0 + h; j++) {
+                live[(size_t)i * n + j] = 1;
+                long double acc = 0.0L, mag = 0.0L;
+                for (int k = g0 + ((j - g0) / TILE) * TILE; k < g0 + h; k++) {
+                    const long double t = (long double)L[(size_t)i * n + k] * M[(size_t)k * n + j];
+                    acc += t;
+                    mag += fabsl(t);
+                }
+                worst = fmax(worst, (double)(fabsl(Xg[(size_t)i * n + j] - acc) / mag));
+            }
+    }
+    for (size_t e = 0; e < X.size(); e++)
+        if (!live[e] && !same_bits(Xg[e], X[e])) touched++;
+    char what[160];
+    snprintf(what, sizeof(what), "hb=%d T=%d nb=%d last=%d part 1 (X21 = L21 M11) / sum|a||b|", hb, T, nb, last_s2);
+    fails += report(G, what, worst, 1e-15);
+    snprintf(what, sizeof(what), "hb=%d T=%d part 1 entries changed outside the live X21 blocks", hb, T);
+    fails += report_count(G, what, touched);
+    // part 2: M21 = -M22 X21, k blocks [0, ti] of the group's second half (X21 as computed above).  X21 is a computed
+    // operand: its entries cancel to far below their column maximum, which sets the column's scale, so the error is
+    // measured against sum_k |M22[i,k]| max_k' |X21[k',j]| (the representation error of a column is <= its scale 2^-56)
+    CHECK(oz_trtri_level(oz, dL, dM, dX, n, hb, 0, nb, last_s2, 2, 0));
+    CHECK(cudaDeviceSynchronize());
+    dev_download(Mg, dM);
+    worst = 0.0;
+    touched = 0;
+    for (int z = 0; z < nb; z++) {
+        const int g0 = z * 2 * h, rows = (z == nb - 1 ? last_s2 : hb) * TILE;
+        std::vector<double> colmax(h, 0.0);
+        for (int k = g0 + h; k < g0 + h + rows; k++)
+            for (int j = g0; j < g0 + h; j++) colmax[j - g0] = fmax(colmax[j - g0], fabs(Xg[(size_t)k * n + j]));
+        for (int i = g0 + h; i < g0 + h + rows; i++)
+            for (int j = g0; j < g0 + h; j++) {
+                long double acc = 0.0L, mag = 0.0L;
+                const int kend = g0 + h + ((i - g0 - h) / TILE + 1) * TILE;
+                for (int k = g0 + h; k < kend; k++) {
+                    acc -= (long double)M[(size_t)i * n + k] * Xg[(size_t)k * n + j];
+                    mag += fabsl((long double)M[(size_t)i * n + k]) * colmax[j - g0];
+                }
+                worst = fmax(worst, (double)(fabsl(Mg[(size_t)i * n + j] - acc) / mag));
+            }
+    }
+    for (size_t e = 0; e < M.size(); e++)
+        if (!live[e] && !same_bits(Mg[e], M[e])) touched++;
+    snprintf(what, sizeof(what), "hb=%d T=%d nb=%d last=%d part 2 (M21 = -M22 X21) / sum|a| max|b|", hb, T, nb, last_s2);
+    fails += report(G, what, worst, 1e-15);
+    snprintf(what, sizeof(what), "hb=%d T=%d part 2 entries of M changed outside the live M21 blocks", hb, T);
+    fails += report_count(G, what, touched);
+    oz.destroy();
+    cudaFree(dL); cudaFree(dM); cudaFree(dX);
+    return fails;
+}
+
+static int check_ragged() {
+    int fails = 0;
+    fails += ragged_case(4, 21);   // groups of 8 tiles: 2 full, the last with 1 tile row
+    fails += ragged_case(4, 23);   // the last with hb - 1 = 3 tile rows
+    return group_end("ragged", fails);
+}
+
+static int check_maps() {
+    const char* G = "maps";
+    int fails = 0;
+    const int T = 10, n = T * TILE;
+    unsigned long long seed = 515;
+    OzCtx oz;
+    CHECK(oz.init(n));
+    poison_planes(oz);
+    {
+        // C[i,j] -= sum_{k in panel [0,2)} A[i,k] A[j,k] on tile rows [4,10) x tile columns [2,8), i >= j:
+        // lower_filter with lower_off = 2 (tiles (4,5..7), (5,6..7), (6,7) are filtered out)
+        const int p0 = 0, pend = 2, r0 = 4, r1 = 10, c0 = 2, c1 = 8;
+        std::vector<double> A((size_t)n * n);
+        for (auto& v : A) v = mag_rand(seed);
+        double* dA = dev_upload(A);
+        CHECK(oz_split_panel_rows(oz, dA, n, p0, pend, c0, r1, 0, 0));
+        CHECK(oz_update_region(oz, dA, n, p0, pend, r0, r1, c0, c1, 0, 0));
+        CHECK(cudaDeviceSynchronize());
+        std::vector<double> Ag((size_t)n * n);
+        dev_download(Ag, dA);
+        double worst = 0.0;
+        long long touched = 0;
+        for (int i = 0; i < n; i++)
+            for (int j = 0; j < n; j++) {
+                const int ti = i / TILE, tj = j / TILE;
+                const bool in = ti >= r0 && ti < r1 && tj >= c0 && tj < c1 && ti >= tj;
+                if (!in) {
+                    if (!same_bits(Ag[(size_t)i * n + j], A[(size_t)i * n + j])) touched++;
+                    continue;
+                }
+                long double acc = A[(size_t)i * n + j], mag = fabs(A[(size_t)i * n + j]);
+                for (int k = p0 * TILE; k < pend * TILE; k++) {
+                    const long double t = (long double)A[(size_t)i * n + k] * A[(size_t)j * n + k];
+                    acc -= t;
+                    mag += fabsl(t);
+                }
+                worst = fmax(worst, (double)(fabsl(Ag[(size_t)i * n + j] - acc) / mag));
+            }
+        fails += report(G, "oz_update_region rows [4,10) x cols [2,8) lower_off 2, alpha -1 beta 1 / (|C| + sum|a||b|)",
+                        worst, 1e-15);
+        fails += report_count(G, "oz_update_region entries changed outside the live tiles (filtered tiles included)", touched);
+        cudaFree(dA);
+    }
+    {
+        // lazy panel solve X = A W^T in place on rows [5,10) x panel columns [2,5): k blocks [0, tj]; W lower triangular
+        // by element in its diagonal tiles, data of the same magnitude in the tiles above (excluded by KSEL_TJ)
+        const int p0 = 2, pend = 5, pw = pend - p0, r0 = 5, r1 = 10;
+        std::vector<double> A((size_t)n * n), W((size_t)n * n, 0.0);
+        for (auto& v : A) v = mag_rand(seed);
+        for (int r = 0; r < pw * TILE; r++)
+            for (int c = 0; c < pw * TILE; c++)
+                W[(size_t)r * n + c] = (r / TILE == c / TILE && c > r) ? 0.0 : mag_rand(seed);
+        double *dA = dev_upload(A), *dW = dev_upload(W);
+        CHECK(oz_split_w(oz, dW, n, pw, 1, 0));
+        CHECK(oz_panel_solve(oz, dA, n, p0, pend, r0, r1, 1, 4, 0));
+        CHECK(cudaDeviceSynchronize());
+        std::vector<double> Ag((size_t)n * n);
+        dev_download(Ag, dA);
+        double worst = 0.0;
+        long long touched = 0;
+        for (int i = 0; i < n; i++)
+            for (int j = 0; j < n; j++) {
+                const int ti = i / TILE, tj = j / TILE;
+                if (!(ti >= r0 && ti < r1 && tj >= p0 && tj < pend)) {
+                    if (!same_bits(Ag[(size_t)i * n + j], A[(size_t)i * n + j])) touched++;
+                    continue;
+                }
+                const int c = j - p0 * TILE;
+                long double acc = 0.0L, mag = 0.0L;
+                for (int k = 0; k < (c / TILE + 1) * TILE; k++) {
+                    const long double t = (long double)A[(size_t)i * n + p0 * TILE + k] * W[(size_t)c * n + k];
+                    acc += t;
+                    mag += fabsl(t);
+                }
+                worst = fmax(worst, (double)(fabsl(Ag[(size_t)i * n + j] - acc) / mag));
+            }
+        fails += report(G, "oz_panel_solve rows [5,10) x panel [2,5), B planes of LAZY_PB*128 rows / sum|a||b|", worst, 1e-15);
+        fails += report_count(G, "oz_panel_solve entries changed outside the panel rows", touched);
+        cudaFree(dA);
+        cudaFree(dW);
+    }
+    oz.destroy();
+    return group_end(G, fails);
+}
+
+// K range of S = 2 * 128 + 10 blocks cut into k_min / k_max segments of <= 128 blocks (beta 0, then 1), as oz_lauum
+// does for N > 16384.  Item (ti, tj) accumulates k blocks [127 + ti, 255 + tj): item row 1 has an empty range in the
+// first segment (C <- 0 C), item columns 0 and 1 in the last (C <- C).
+static int check_segments() {
+    const char* G = "segments";
+    int fails = 0;
+    const int S = 2 * 128 + 10, K = S * TILE, m = 2 * TILE, nc = 3 * TILE;
+    unsigned long long seed = 266;
+    std::vector<double> A((size_t)m * K), B((size_t)nc * K);
+    for (auto& v : A) v = mag_rand(seed);
+    for (auto& v : B) v = mag_rand(seed);
+    double *dA = dev_upload(A), *dB = dev_upload(B);
+    std::vector<double> C((size_t)m * nc, sentinel());
+    double* dC = dev_upload(C);
+    OzPlanes PA = alloc_planes(m, K), PB = alloc_planes(nc, K);
+    CHECK(oz_split_rows(dA, K, 0, m, m, K, PA, 0, 0, 0, 0, 1, 0));
+    CHECK(oz_split_rows(dB, K, 0, nc, nc, K, PB, 0, 0, 0, 0, 1, 0));
+    CUtensorMap tmA, tmB;
+    CHECK(oz_make_map(&tmA, PA.planes, K, (long long)OZ_S * m, K, OZ_BM));
+    CHECK(oz_make_map(&tmB, PB.planes, K, (long long)OZ_S * nc, K, OZ_BN));
+    OzGemmOp op = oz_default();
+    op.a_plane_rows = m;
+    op.b_plane_rows = nc;
+    op.a_scale = PA.scale;
+    op.b_scale = PB.scale;
+    op.C = dC;
+    op.ldc = nc;
+    op.tiles_m = op.tiles_m_last = m / TILE;
+    op.tiles_n = nc / TILE;
+    op.klo_sel = KSEL_TI;
+    op.klo_c = 127;
+    op.khi_sel = KSEL_TJ;
+    op.khi_c = 255;
+    for (int k0 = 0; k0 < S; k0 += 128) {
+        op.k_min = k0;
+        op.k_max = std::min(k0 + 128, S);
+        op.beta = k0 == 0 ? 0.0 : 1.0;
+        CHECK(launch_oz_gemm(tmA, tmB, op, 1, 0));
+    }
+    CHECK(cudaDeviceSynchronize());
+    dev_download(C, dC);
+    double worst = 0.0;
+    long long nonfinite = 0;
+    for (int i = 0; i < m; i++)
+        for (int j = 0; j < nc; j++) {
+            if (!isfinite(C[(size_t)i * nc + j])) {   // e.g. the sentinel carried through the C <- 0 C path
+                nonfinite++;
+                continue;
+            }
+            long double acc = 0.0L, mag = 0.0L;
+            for (int k = (127 + i / TILE) * TILE; k < (255 + j / TILE) * TILE; k++) {
+                const long double t = (long double)A[(size_t)i * K + k] * B[(size_t)j * K + k];
+                acc += t;
+                mag += fabsl(t);
+            }
+            worst = fmax(worst, (double)(fabsl(C[(size_t)i * nc + j] - acc) / mag));
+        }
+    // ~17000 terms of random sign per entry: representation errors and FP64 roundings average out (observed ~5e-18 of
+    // sum |a||b|), so the bound is 1e-16 here; with 6 instead of 7 significance levels the error is ~8e-16
+    fails += report(G, "K range of 266 blocks in 3 segments (empty ranges included) / sum|a||b|", worst, 1e-16);
+    fails += report_count(G, "non-finite entries of C (sentinel NaN before the first segment)", nonfinite);
+    cudaFree(dA); cudaFree(dB); cudaFree(dC);
+    free_planes(PA); free_planes(PB);
+    return group_end(G, fails);
+}
+
+// digit planes written directly (not through a split): K = 16384 (128 blocks, the longest single accumulation)
+static int check_limits() {
+    const char* G = "limits";
+    int fails = 0;
+    const int K = 128 * TILE;
+    {
+        // d_0 = -64, d_1..6 = -128 in both operands: every pair product is positive; level 6 sums
+        // 2 * 64 * 128 + 5 * 128 * 128 = 98304 per k, 1.61e9 over K (int32 limit 2.15e9)
+        const int m = TILE;
+        OzPlanes PA = alloc_planes(m, K), PB = alloc_planes(m, K);
+        for (OzPlanes* P : {&PA, &PB}) {
+            CHECK(cudaMemset(P->planes, 0xc0, (size_t)m * K));                        // plane 0: -64
+            CHECK(cudaMemset(P->planes + (size_t)m * K, 0x80, (size_t)(OZ_S - 1) * m * K));   // planes 1..6: -128
+            std::vector<double> one(m, 1.0);
+            CHECK(cudaMemcpy(P->scale, one.data(), sizeof(double) * m, cudaMemcpyHostToDevice));
+        }
+        double* dC;
+        CHECK(cudaMalloc(&dC, sizeof(double) * m * m));
+        CUtensorMap tmA, tmB;
+        CHECK(oz_make_map(&tmA, PA.planes, K, (long long)OZ_S * m, K, OZ_BM));
+        CHECK(oz_make_map(&tmB, PB.planes, K, (long long)OZ_S * m, K, OZ_BN));
+        OzGemmOp op = oz_default();
+        op.a_plane_rows = op.b_plane_rows = m;
+        op.a_scale = PA.scale;
+        op.b_scale = PB.scale;
+        op.C = dC;
+        op.ldc = m;
+        op.tiles_m = op.tiles_m_last = 1;
+        op.tiles_n = 1;
+        op.khi_c = 128;
+        CHECK(launch_oz_gemm(tmA, tmB, op, 1, 0));
+        CHECK(cudaDeviceSynchronize());
+        std::vector<double> C((size_t)m * m);
+        dev_download(C, dC);
+        const long long d[OZ_S] = {-64, -128, -128, -128, -128, -128, -128};
+        long long lv[OZ_S] = {0};
+        for (int i = 0; i < OZ_S; i++)
+            for (int j = 0; i + j < OZ_S; j++) lv[i + j] += d[i] * d[j] * (long long)K;
+        long double want = 0.0L;
+        for (int l = OZ_S - 1; l >= 0; l--) want = want / 256.0L + (long double)lv[l];
+        want /= 65536.0L;
+        double worst = 0.0;
+        for (double v : C) worst = fmax(worst, (double)(fabsl(v - want) / want));
+        printf("%s largest accumulation: level 6 sums %lld (int32 limit %d)\n", G, lv[OZ_S - 1], 2147483647);
+        fails += report(G, "extreme digits, K = 16384, against the closed form / value", worst, ldexp(1.0, -52));
+        cudaFree(dC);
+        free_planes(PA); free_planes(PB);
+    }
+    {
+        // random digits (|d_0| <= 64) and power-of-two scales, 7 / 6 / 5 levels against int64 host sums over the
+        // same levels at 400 sampled entries
+        const int m = 2 * TILE;
+        std::vector<int8_t> a((size_t)OZ_S * m * K), b((size_t)OZ_S * m * K);
+        std::vector<double> sa(m), sb(m);
+        unsigned long long seed = 16384;
+        for (auto* v : {&a, &b})
+            for (size_t e = 0; e < v->size(); e++) {
+                seed = seed * 6364136223846793005ull + 1442695040888963407ull;
+                const int r = (int)(seed >> 33);
+                (*v)[e] = e < (size_t)m * K ? (int8_t)(r % 129 - 64) : (int8_t)(r & 0xff);
+            }
+        for (int r = 0; r < m; r++) {
+            sa[r] = ldexp(1.0, (int)(8.0 * urand(seed)));
+            sb[r] = ldexp(1.0, (int)(8.0 * urand(seed)));
+        }
+        OzPlanes PA = alloc_planes(m, K), PB = alloc_planes(m, K);
+        CHECK(cudaMemcpy(PA.planes, a.data(), a.size(), cudaMemcpyHostToDevice));
+        CHECK(cudaMemcpy(PB.planes, b.data(), b.size(), cudaMemcpyHostToDevice));
+        CHECK(cudaMemcpy(PA.scale, sa.data(), sizeof(double) * m, cudaMemcpyHostToDevice));
+        CHECK(cudaMemcpy(PB.scale, sb.data(), sizeof(double) * m, cudaMemcpyHostToDevice));
+        double* dC;
+        CHECK(cudaMalloc(&dC, sizeof(double) * m * m));
+        CUtensorMap tmA, tmB;
+        CHECK(oz_make_map(&tmA, PA.planes, K, (long long)OZ_S * m, K, OZ_BM));
+        CHECK(oz_make_map(&tmB, PB.planes, K, (long long)OZ_S * m, K, OZ_BN));
+        const int ns = 400;
+        std::vector<int> si(ns), sj(ns);
+        std::vector<long long> lv((size_t)ns * OZ_S, 0);
+        for (int s = 0; s < ns; s++) {
+            si[s] = (int)((urand(seed) * 0.5 + 0.5) * m) % m;
+            sj[s] = (int)((urand(seed) * 0.5 + 0.5) * m) % m;
+            for (int i = 0; i < OZ_S; i++)
+                for (int j = 0; i + j < OZ_S; j++) {
+                    const int8_t* pa = &a[((size_t)i * m + si[s]) * K];
+                    const int8_t* pb = &b[((size_t)j * m + sj[s]) * K];
+                    long long acc = 0;
+                    for (int k = 0; k < K; k++) acc += (long long)pa[k] * pb[k];
+                    lv[(size_t)s * OZ_S + i + j] += acc;
+                }
+        }
+        std::vector<double> C((size_t)m * m);
+        for (int levels : {7, 6, 5}) {
+            OzGemmOp op = oz_default();
+            op.a_plane_rows = op.b_plane_rows = m;
+            op.a_scale = PA.scale;
+            op.b_scale = PB.scale;
+            op.C = dC;
+            op.ldc = m;
+            op.tiles_m = op.tiles_m_last = m / TILE;
+            op.tiles_n = m / TILE;
+            op.khi_c = 128;
+            op.levels = levels == 7 ? 0 : levels;
+            CHECK(launch_oz_gemm(tmA, tmB, op, 1, 0));
+            CHECK(cudaDeviceSynchronize());
+            dev_download(C, dC);
+            double worst = 0.0;
+            for (int s = 0; s < ns; s++) {
+                long double want = 0.0L, mag = 0.0L;
+                for (int l = levels - 1; l >= 0; l--) {
+                    want = want / 256.0L + (long double)lv[(size_t)s * OZ_S + l];
+                    mag = mag / 256.0L + fabsl((long double)lv[(size_t)s * OZ_S + l]);
+                }
+                const long double sc = (long double)sa[si[s]] * sb[sj[s]] / 65536.0L;
+                worst = fmax(worst, (double)(fabsl(C[(size_t)si[s] * m + sj[s]] - want * sc) / (mag * sc)));
+            }
+            char what[160];
+            snprintf(what, sizeof(what), "random digits, K = 16384, %d levels, 400 entries against int64 sums / magnitude", levels);
+            fails += report(G, what, worst, ldexp(1.0, -52));
+        }
+        cudaFree(dC);
+        free_planes(PA); free_planes(PB);
+    }
+    return group_end(G, fails);
+}
+
+// the documented split of one row: scale 2^(ex+2) for a finite non-zero maximum below 1e300, else scale 1 and zero digits
+static double host_scale(double amax, bool& zero_digits) {
+    zero_digits = !(amax > 0.0) || !(amax < 1.0e300);
+    if (zero_digits) return 1.0;
+    int ex;
+    frexp(amax, &ex);
+    return ldexp(1.0, ex + 2);
+}
+
+static int check_exponents() {
+    const char* G = "exponents";
+    int fails = 0;
+    const int R = 256, K = 128, NB = 128;
+    std::vector<double> X((size_t)R * K, 0.0);
+    unsigned long long seed = 1074;
+    auto row = [&](int r) { return &X[(size_t)r * K]; };
+    // rows 1..199: maxima swept over 2^-1074 .. 2^996 (entries of magnitude [0.5, 1] x 2^e and some smaller)
+    for (int r = 1; r < 200; r++) {
+        const int e = -1074 + (int)((long long)(r - 1) * (996 + 1074) / 198);
+        for (int k = 0; k < K; k++) row(r)[k] = ldexp(mag_rand(seed) * ((k % 5 == 0) ? 1e-3 : 1.0), e);
+    }
+    // rows 200..223: exact powers of two of both signs, around the 2^-970 boundary and at both ends
+    const int pw[12] = {-1074, -1073, -1060, -1022, -1000, -971, -970, -969, -500, 0, 995, 996};
+    for (int q = 0; q < 24; q++) {
+        const int r = 200 + q, e = pw[q % 12];
+        for (int k = 0; k < K; k++) row(r)[k] = ldexp((q < 12) == (k % 2 == 0) ? 1.0 : -1.0, e - (k % 3));
+    }
+    // rows 224..235: a single non-zero entry
+    for (int q = 0; q < 12; q++) row(224 + q)[(q * 37) % K] = ldexp(mag_rand(seed), pw[q]);
+    // rows 236..247: subnormal entries next to normal maxima (and one all-subnormal row)
+    for (int q = 0; q < 12; q++) {
+        const int r = 236 + q, e = q == 11 ? -1040 : -1022 + 6 * q;
+        for (int k = 0; k < K; k++) row(r)[k] = ldexp(mag_rand(seed), k == 3 ? e : -1050 - (k % 20));
+    }
+    // rows 248..251 NaN (every entry), 252 / 253 one +Inf / -Inf entry, 0 and 254..255 zero
+    for (int r = 248; r < 252; r++)
+        for (int k = 0; k < K; k++) row(r)[k] = nan("");
+    row(252)[5] = INFINITY;
+    row(253)[77] = -INFINITY;
+    std::vector<double> Xt((size_t)K * R);
+    for (int r = 0; r < R; r++)
+        for (int k = 0; k < K; k++) Xt[(size_t)k * R + r] = X[(size_t)r * K + k];
+    double *dX = dev_upload(X), *dXt = dev_upload(Xt);
+    OzPlanes PR = alloc_planes(R, K), PC = alloc_planes(R, K);
+    CHECK(oz_split_rows(dX, K, 0, R, R, K, PR, 0, 0, 0, 0, 1, 0));
+    CHECK(oz_split_cols(dXt, R, 0, K, K, R, 0, PC, 0, 0, 0, 0, 1, 0));
+    CHECK(cudaDeviceSynchronize());
+    std::vector<int8_t> hr((size_t)OZ_S * R * K), hc((size_t)OZ_S * R * K);
+    std::vector<double> sr(R), sc(R);
+    dev_download(hr, PR.planes);
+    dev_download(hc, PC.planes);
+    dev_download(sr, PR.scale);
+    dev_download(sc, PC.scale);
+    long long bad_rows = 0, bad_cols = 0, bad_tiny = 0;
+    double worst_rep = 0.0;
+    for (int r = 0; r < R; r++) {
+        double amax = 0.0;
+        for (int k = 0; k < K; k++) amax = fmax(amax, fabs(row(r)[k]));   // fmax drops NaN, as on the device
+        bool zero;
+        const double s = host_scale(amax, zero);
+        bool row_bad = !same_bits(sr[r], s), col_bad = !same_bits(sc[r], s);
+        for (int k = 0; k < K; k++) {
+            int8_t d[OZ_S] = {0, 0, 0, 0, 0, 0, 0};
+            if (!zero) host_digits(row(r)[k], s, d);
+            long double rep = 0.0L;
+            for (int p = 0; p < OZ_S; p++) {
+                const int8_t g = hr[((size_t)p * R + r) * K + k];
+                row_bad |= g != d[p];
+                col_bad |= hc[((size_t)p * R + r) * K + k] != d[p];
+                rep += (long double)g * powl(256.0L, -(p + 1));
+            }
+            if (!zero) {
+                // documented: x = scale * sum_p d_p 256^-(p+1) + t, 0 <= t < scale 2^-56
+                const long double t = ((long double)row(r)[k] - rep * s) / s;
+                worst_rep = fmax(worst_rep, t < 0 ? 1.0 : (double)t);
+            }
+        }
+        bad_rows += row_bad;
+        bad_cols += col_bad;
+        if ((row_bad || col_bad) && amax > 0.0 && amax < ldexp(1.0, -970)) bad_tiny++;
+    }
+    printf("%s rows with a maximum below 2^-970 among the mismatching rows: %lld\n", G, bad_tiny);
+    fails += report_count(G, "split_rows rows whose scale or digits differ from the documented split", bad_rows);
+    fails += report_count(G, "split_cols rows whose scale or digits differ from the documented split", bad_cols);
+    fails += report(G, "representation t / scale on every finite row (bound 2^-56, t >= 0)", worst_rep, ldexp(1.0, -56));
+    // product of these rows with moderate ones: 1e-15 of sum |a||b| plus an absolute floor (the scale products of the
+    // smallest rows are subnormal or zero); NaN / Inf rows are excluded (their planes are zero by contract)
+    std::vector<double> B((size_t)NB * K);
+    for (int c = 0; c < NB; c++) {
+        const int e = -(int)(20.0 * (urand(seed) * 0.5 + 0.5));
+        for (int k = 0; k < K; k++) B[(size_t)c * K + k] = ldexp(mag_rand(seed), e);
+    }
+    double* dB = dev_upload(B);
+    OzPlanes PB = alloc_planes(NB, K);
+    CHECK(oz_split_rows(dB, K, 0, NB, NB, K, PB, 0, 0, 0, 0, 1, 0));
+    double* dC;
+    CHECK(cudaMalloc(&dC, sizeof(double) * R * NB));
+    CUtensorMap tmA, tmB;
+    CHECK(oz_make_map(&tmA, PR.planes, K, (long long)OZ_S * R, K, OZ_BM));
+    CHECK(oz_make_map(&tmB, PB.planes, K, (long long)OZ_S * NB, K, OZ_BN));
+    OzGemmOp op = oz_default();
+    op.a_plane_rows = R;
+    op.b_plane_rows = NB;
+    op.a_scale = PR.scale;
+    op.b_scale = PB.scale;
+    op.C = dC;
+    op.ldc = NB;
+    op.tiles_m = op.tiles_m_last = R / TILE;
+    op.tiles_n = NB / TILE;
+    op.khi_c = K / TILE;
+    CHECK(launch_oz_gemm(tmA, tmB, op, 1, 0));
+    CHECK(cudaDeviceSynchronize());
+    std::vector<double> C((size_t)R * NB);
+    dev_download(C, dC);
+    const double floor_abs = ldexp(1.0, -1000);
+    double worst = 0.0;
+    for (int r = 0; r < R; r++) {
+        if (r >= 248 && r <= 253) continue;
+        for (int c = 0; c < NB; c++) {
+            long double acc = 0.0L, mag = 0.0L;
+            for (int k = 0; k < K; k++) {
+                const long double t = (long double)row(r)[k] * B[(size_t)c * K + k];
+                acc += t;
+                mag += fabsl(t);
+            }
+            worst = fmax(worst, (double)(fabsl(C[(size_t)r * NB + c] - acc) / (1e-15L * mag + floor_abs)));
+        }
+    }
+    fails += report(G, "product of the finite rows, |error| / (1e-15 sum|a||b| + 2^-1000)", worst, 1.0);
+    cudaFree(dX); cudaFree(dXt); cudaFree(dB); cudaFree(dC);
+    free_planes(PR); free_planes(PC); free_planes(PB);
+    return group_end(G, fails);
+}
+
 __global__ void fill_rand(double* A, long long n, unsigned seed) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
@@ -542,6 +1108,11 @@ int main(int argc, char** argv) {
         mma_rate<128, 32>(7, 7);
         return 0;
     }
+    const struct { const char* name; int (*fn)(); } groups[] = {
+        {"ragged", check_ragged}, {"maps", check_maps}, {"segments", check_segments}, {"limits", check_limits},
+        {"exponents", check_exponents}};
+    for (const auto& g : groups)
+        if (!strcmp(what, g.name)) return g.fn() ? 1 : 0;
     if (!strcmp(what, "check") || !strcmp(what, "all")) {
         fails += check_small();
         fails += check_lauum(512);
