@@ -40,7 +40,6 @@ constexpr int LLD = 132;   // smem leading dimension: 132 = 4 (mod 16) keeps eve
 constexpr int TLD = 36;    // per-warp scratch leading dimension (same residue)
 constexpr int PANEL_BLOCKS = 4;   // leaf-level panel: in-panel updates run at K = 128
 constexpr int PANEL_BASE = 2;      // widest piece factored with K = 128 in-panel updates (the recursion stops here)
-inline int g_panel_blocks = 0;     // look-ahead panel width in 128-columns; 0 = by size (12 from N = 12288, else 4)
 constexpr unsigned FULL = 0xffffffffu;
 
 // C(32x32) += A(32x32) * B(32x32) by one warp on DMMA; A(r,k) and B(k,n) are element getters.
@@ -714,73 +713,17 @@ inline cudaError_t launch_leaf(double* A, int ld, int col, double* M, double* lo
         if (_e != cudaSuccess) return _e; \
     } while (0)
 
-// A (lower) -> L in place; diagonal blocks of M <- inverse of the diagonal blocks of L.
-inline cudaError_t potrf_blocked(double* A, double* M, int ld, int T, double* logdet_part, int* info,
-                                 cudaStream_t st) {
-    for (int p0 = 0; p0 < T; p0 += PANEL_BLOCKS) {
-        const int pw = (T - p0 < PANEL_BLOCKS) ? (T - p0) : PANEL_BLOCKS;
-        const int pend = p0 + pw;
-        for (int col = p0; col < pend; col++) {
-            GPP_TRY(launch_leaf(A, ld, col, M, logdet_part, info, st));
-            const int below = T - col - 1;
-            if (below <= 0) continue;
-            {   // TRSM: A[i,col] <- A[i,col] * Linv_col^T   (in place; a CTA only reads its own rows)
-                GemmOp op = gemm_default();
-                op.A = A + (long long)(col + 1) * TILE * ld + (long long)col * TILE;
-                op.lda = ld;
-                op.B = M + (long long)col * TILE * ld + (long long)col * TILE;
-                op.ldb = ld;
-                op.C = const_cast<double*>(op.A);
-                op.ldc = ld;
-                op.tiles_m = op.tiles_m_last = below;
-                op.tiles_n = 1;
-                op.klo_c = 0;
-                op.khi_c = 1;
-                GPP_TRY(launch_gemm(op, true, true, 1, st));
-            }
-            const int pc = pend - col - 1;  // panel columns still to update
-            if (pc > 0) {
-                // A[i,j] -= A[i,col] * A[j,col]^T  for col < j < pend, i >= j
-                GemmOp op = gemm_default();
-                op.A = A + (long long)(col + 1) * TILE * ld + (long long)col * TILE;
-                op.lda = ld;
-                op.B = op.A;
-                op.ldb = ld;
-                op.C = A + (long long)(col + 1) * TILE * ld + (long long)(col + 1) * TILE;
-                op.ldc = ld;
-                op.tiles_m = op.tiles_m_last = below;
-                op.tiles_n = pc;
-                op.lower_filter = 1;
-                op.lower_off = 0;
-                op.klo_c = 0;
-                op.khi_c = 1;
-                op.alpha = -1.0;
-                op.beta = 1.0;
-                GPP_TRY(launch_gemm(op, true, true, 1, st));
-            }
-        }
-        const int rest = T - pend;
-        if (rest > 0) {
-            // trailing SYRK: A[i,j] -= sum_{k in panel} A[i,k] A[j,k]^T , i >= j >= pend
-            GemmOp op = gemm_default();
-            op.A = A + (long long)pend * TILE * ld + (long long)p0 * TILE;
-            op.lda = ld;
-            op.B = op.A;
-            op.ldb = ld;
-            op.C = A + (long long)pend * TILE * ld + (long long)pend * TILE;
-            op.ldc = ld;
-            op.map = MAP_TRI;
-            op.tiles_m = op.tiles_m_last = rest;
-            op.tiles_n = rest;
-            op.klo_c = 0;
-            op.khi_c = pw;
-            op.alpha = -1.0;
-            op.beta = 1.0;
-            GPP_TRY(launch_gemm(op, true, true, 1, st));
-        }
-    }
-    return cudaSuccess;
-}
+// ---------------------------------------------------------------------------------------------
+// Schedule settings of one handle's factorisation (int fields only: gpp_create compares configurations with memcmp).
+// The member initialisers are the production configuration.
+struct CholSchedule {
+    int panel_blocks = 0;     // look-ahead panel width in 128-columns (GPP_PANEL); 0 = by size (12 from N = 12288, else 4)
+    int overlap_inverse = 1;  // start the early part of L^-1 (trtri_early) as soon as its columns of L are final
+                              // (GPP_OVERLAP_INV)
+    int block_ctas = 24;      // CTAs of one diagonal-block launch of potrf_lazy (GPP_BLOCK_CTAS; 0 = the launch-per-step
+                              // chain)
+    int timeline = 0;         // GPP_TIMELINE=1 (development): timing-enabled panel events, dumped by dump_timeline()
+};
 
 // ---------------------------------------------------------------------------------------------
 // Look-ahead variant.  The panel factorisation (leaf / TRSM / in-panel update: a chain of small, latency-bound
@@ -802,11 +745,9 @@ struct CholLookahead {
 
     int* blk_flags = nullptr;   // tile flags of block_potrf_kernel (256 ints), epoch = launch counter
     int blk_epoch = 0;
-    int blk_ctas = 24;          // CTAs of one diagonal-block launch (GPP_BLOCK_CTAS; 0 = the launch-per-step chain)
-    bool timeline = false;   // GPP_TIMELINE=1 (development): timing-enabled panel events, dumped by dump_timeline()
+    CholSchedule sched;         // set before init(): the timeline setting picks the event flags
     cudaError_t init(int T) {
-        timeline = getenv("GPP_TIMELINE") != nullptr && atoi(getenv("GPP_TIMELINE")) != 0;
-        const unsigned evf = timeline ? cudaEventDefault : cudaEventDisableTiming;
+        const unsigned evf = sched.timeline ? cudaEventDefault : cudaEventDisableTiming;
         int lo = 0, hi = 0;
         GPP_TRY(cudaDeviceGetStreamPriorityRange(&lo, &hi));
         GPP_TRY(cudaStreamCreateWithPriority(&side, cudaStreamNonBlocking, hi));
@@ -816,7 +757,6 @@ struct CholLookahead {
         GPP_TRY(cudaEventCreateWithFlags(&inv_done, cudaEventDisableTiming));
         GPP_TRY(cudaMalloc(&blk_flags, 256 * sizeof(int)));
         GPP_TRY(cudaMemset(blk_flags, 0, 256 * sizeof(int)));
-        if (getenv("GPP_BLOCK_CTAS")) blk_ctas = atoi(getenv("GPP_BLOCK_CTAS"));
         // one set of panel events per tile column: enough for every panel width the schedules accept (GPP_PANEL,
         // GPP_OZ_LAZY_PB down to 2; sizing by PANEL_BLOCKS made narrower panels fail with cudaErrorInvalidValue)
         panels = T;
@@ -834,7 +774,7 @@ struct CholLookahead {
     }
     // ms since the fork of the last factorisation at which each panel event completed (call after a synchronise)
     void dump_timeline(int np) const {
-        if (!timeline) return;
+        if (!sched.timeline) return;
         for (int p = 0; p < np && p < panels; p++) {
             float a = -1.f, b = -1.f, c = -1.f, d = -1.f;
             if (cudaEventElapsedTime(&a, fork, ev_pf[p]) != cudaSuccess) a = -1.f;
@@ -938,6 +878,18 @@ inline cudaError_t trailing_update(double* A, int ld, int T, int p0, int pend, i
     return launch_gemm(op, true, true, 1, st);
 }
 
+// A (lower) -> L in place; diagonal blocks of M <- inverse of the diagonal blocks of L.  One stream: each panel of
+// PANEL_BLOCKS tile columns, then the whole trailing SYRK with it.
+inline cudaError_t potrf_blocked(double* A, double* M, int ld, int T, double* logdet_part, int* info,
+                                 cudaStream_t st) {
+    for (int p0 = 0; p0 < T; p0 += PANEL_BLOCKS) {
+        const int pend = (T - p0 < PANEL_BLOCKS) ? T : p0 + PANEL_BLOCKS;
+        GPP_TRY(panel_factor_base(A, M, ld, T, p0, pend, logdet_part, info, st));
+        GPP_TRY(trailing_update(A, ld, T, p0, pend, pend, T, st));
+    }
+    return cudaSuccess;
+}
+
 // panels wider than PANEL_BLOCKS are factored recursively: left half, update of the right half with the left
 // (one DMMA GEMM at K = width/2), right half -- so that only PANEL_BLOCKS-wide pieces run at K = 128
 inline cudaError_t panel_factor(double* A, double* M, int ld, int T, int p0, int pend, double* logdet_part, int* info,
@@ -948,7 +900,7 @@ inline cudaError_t panel_factor(double* A, double* M, int ld, int T, int p0, int
     while (half * 2 < w) half *= 2;
     const int mid = p0 + half;
     GPP_TRY(panel_factor(A, M, ld, T, p0, mid, logdet_part, info, st, oz));
-    if (oz && oz->ready && oz->inner_min_k > 0 && half >= oz->inner_min_k && oz_use_trailing(oz, T, mid)) {
+    if (oz && oz->ready && oz->sched.inner_min_k > 0 && half >= oz->sched.inner_min_k && oz_use_trailing(oz, T, mid)) {
         // wide in-panel update on the INT8-sliced GEMM (planes of the left half, rows mid..T; scale slot 4)
         GPP_TRY(oz_split_panel(*oz, A, ld, T, p0, mid, mid, 4, st));
         GPP_TRY(oz_trailing_update(*oz, A, ld, T, p0, mid, mid, pend, 4, st));
@@ -957,10 +909,6 @@ inline cudaError_t panel_factor(double* A, double* M, int ld, int T, int p0, int
     }
     return panel_factor(A, M, ld, T, mid, pend, logdet_part, info, st, oz);
 }
-
-inline int g_lookahead_depth = 2;  // 1: the next panel waits for the whole previous trailing update; 2: see below
-
-inline int g_overlap_inverse = 1;   // start the early part of L^-1 (trtri_early) as soon as its columns of L are final
 
 // defined below; X is the scratch of the triangular inverse (may be null: no overlap)
 inline int trtri_split_point(int T);
@@ -972,12 +920,11 @@ inline cudaError_t potrf_lookahead(double* A, double* M, int ld, int T, double* 
     // K of the trailing update: wide panels only pay off when the trailing matrix is large (measured:
     // N = 16384 59.0 -> 56.6 ms with 8, N = 8192 12.3 -> 12.8 ms; round 2, whole evaluation at N = 16384:
     // 139.3 ms with 8, 138.4 with 12, 138.6 with 16)
-    const int PB = g_panel_blocks > 0 ? g_panel_blocks : (T >= 96 ? 12 : 4);
+    const int PB = la.sched.panel_blocks > 0 ? la.sched.panel_blocks : (T >= 96 ? 12 : 4);
     const int NP = (T + PB - 1) / PB;
     if (NP > la.panels) return cudaErrorInvalidValue;
-    const bool deep = g_lookahead_depth >= 2;
     const int H = trtri_split_point(T);
-    const bool overlap = g_overlap_inverse && X != nullptr && H > 0 && NP > 1;
+    const bool overlap = la.sched.overlap_inverse && X != nullptr && H > 0 && NP > 1;
     la.inv_pending = false;
     GPP_TRY(cudaEventRecord(la.fork, st));
     GPP_TRY(cudaStreamWaitEvent(la.side, la.fork, 0));
@@ -986,14 +933,14 @@ inline cudaError_t potrf_lookahead(double* A, double* M, int ld, int T, double* 
     //   main:  [wait PF(0)] U(0,2) U(0,3..) [wait PF(1)] U(1,3) U(1,4..) ...
     // The side chain only waits for U(p-1,p+1), which the main stream issues BEFORE the bulk U(p-1,p+2..), so it can
     // run one panel further ahead than with a single trailing launch per panel (depth 1).
-    int last_ev = -1;  // last panel with a recorded ev_tu (U(p,p+2) at depth 2, the whole trailing update at depth 1)
+    int last_ev = -1;  // last panel with a recorded ev_tu (U(p,p+2))
     for (int p = 0; p < NP; p++) {
         const int p0 = p * PB;
         const int pend = (p0 + PB < T) ? p0 + PB : T;
         GPP_TRY(panel_factor(A, M, ld, T, p0, pend, logdet_part, info, la.side, oz));
         // with U(p,p+1) on the INT8-sliced GEMM the digit planes of the whole panel (rows pend..T) are cut here, on the
         // side stream, and the main stream's updates reuse them
-        const bool ozp = oz && oz->next_on_oz && oz_use_trailing(oz, T, pend);
+        const bool ozp = oz && oz->sched.next_on_oz && oz_use_trailing(oz, T, pend);
         if (ozp) GPP_TRY(oz_split_panel(*oz, A, ld, T, p0, pend, pend, p & 3, la.side));
         GPP_TRY(cudaEventRecord(la.ev_pf[p], la.side));
         if (pend >= T) break;
@@ -1010,22 +957,18 @@ inline cudaError_t potrf_lookahead(double* A, double* M, int ld, int T, double* 
         else GPP_TRY(trailing_update(A, ld, T, p0, pend, pend, nend, la.side));
         if (nend < T) {
             GPP_TRY(cudaStreamWaitEvent(st, la.ev_pf[p], 0));
+            const int n2end = (nend + PB < T) ? nend + PB : T;
             if (oz_use_trailing(oz, T, nend)) {
                 // the bulk of the trailing update on the INT8-sliced GEMM: digit planes of the panel rows nend..T once,
                 // then U(p,p+2) and U(p,p+3..) as integer GEMMs
                 if (!ozp) GPP_TRY(oz_split_panel(*oz, A, ld, T, p0, pend, nend, p & 3, st));
-                const int n2end = (deep && nend + PB < T) ? nend + PB : T;
                 GPP_TRY(oz_trailing_update(*oz, A, ld, T, p0, pend, nend, n2end, p & 3, st));
                 GPP_TRY(cudaEventRecord(la.ev_tu[p], st));
                 if (n2end < T) GPP_TRY(oz_trailing_update(*oz, A, ld, T, p0, pend, n2end, T, p & 3, st));
-            } else if (deep) {
-                const int n2end = (nend + PB < T) ? nend + PB : T;
+            } else {
                 GPP_TRY(trailing_update(A, ld, T, p0, pend, nend, n2end, st));  // U(p,p+2)
                 GPP_TRY(cudaEventRecord(la.ev_tu[p], st));
                 GPP_TRY(trailing_update(A, ld, T, p0, pend, n2end, T, st));  // U(p,p+3..)
-            } else {
-                GPP_TRY(trailing_update(A, ld, T, p0, pend, nend, T, st));
-                GPP_TRY(cudaEventRecord(la.ev_tu[p], st));
             }
             last_ev = p;
         }
@@ -1156,11 +1099,11 @@ inline cudaError_t trtri_late(const double* L, double* M, double* X, int ld, int
 //   m3(p)  update of everything to the right of block p+3, issued after the urgent pieces of panel p+1
 inline cudaError_t potrf_lazy(double* A, double* M, int ld, int T, double* logdet_part, int* info, cudaStream_t st,
                               CholLookahead& la, double* X, OzCtx& oz) {
-    const int PB = oz.lazy_pb;
+    const int PB = oz.sched.lazy_pb;
     const int NP = (T + PB - 1) / PB;
     if (NP > la.panels || PB > OzCtx::LAZY_PB || PB < 2) return cudaErrorInvalidValue;
     const int H = trtri_split_point(T);
-    const bool overlap = g_overlap_inverse && X != nullptr && H > 0 && NP > 1;
+    const bool overlap = la.sched.overlap_inverse && X != nullptr && H > 0 && NP > 1;
     la.inv_pending = false;
     GPP_TRY(cudaEventRecord(la.fork, st));
     GPP_TRY(cudaStreamWaitEvent(la.side, la.fork, 0));
@@ -1172,9 +1115,9 @@ inline cudaError_t potrf_lazy(double* A, double* M, int ld, int T, double* logde
         const int n2end = (nend + PB < T) ? nend + PB : T;
         const int buf = p & 1, slot = p & 3;
         // ---- B(p): diagonal block on the chain: one dataflow launch (or the launch-per-step chain with row limit pend) ----
-        if (la.blk_ctas > 0 && pend - p0 <= 16)
-            GPP_TRY(launch_block_potrf(A, M, ld, p0, pend - p0, logdet_part, info, la.blk_flags, ++la.blk_epoch, la.blk_ctas,
-                                       la.side));
+        if (la.sched.block_ctas > 0 && pend - p0 <= 16)
+            GPP_TRY(launch_block_potrf(A, M, ld, p0, pend - p0, logdet_part, info, la.blk_flags, ++la.blk_epoch,
+                                       la.sched.block_ctas, la.side));
         else
             GPP_TRY(panel_factor(A, M, ld, pend, p0, pend, logdet_part, info, la.side, nullptr));
         if (pend < T) {

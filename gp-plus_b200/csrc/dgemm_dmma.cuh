@@ -48,13 +48,11 @@ struct GemmCfg {
     static constexpr int SMEM_BYTES = STAGES * (A_STAGE + B_STAGE) * 8;
     static constexpr int MIN_CTAS = (BM == 128) ? 1 : 2;
 };
-constexpr int GEMM_SMEM_BYTES = GemmCfg<128>::SMEM_BYTES;  // 163840
 
-// CTA shape used by launch_gemm (process-wide; 128 or 64)
-inline int g_gemm_bm = 64;
+constexpr int GEMM_BM = 64;         // CTA shape of launch_gemm
 constexpr int GEMM_NUM_SMS = 148;   // B200
-inline int g_gemm_stagger = 10;     // phase shift of the two resident CTAs of an SM in tenths of half a tile time
-                                    // (GPP_STAGGER; 0 = off): potrf alone 53.4 -> 52.4 ms at N = 16384
+constexpr int GEMM_STAGGER = 10;    // phase shift of the two resident CTAs of an SM in tenths of half a tile time:
+                                    // potrf alone 53.4 -> 52.4 ms at N = 16384
 
 enum KSel { KSEL_CONST = 0, KSEL_TI = 1, KSEL_TJ = 2 };
 enum TileMap { MAP_RECT = 0, MAP_TRI = 1 };
@@ -330,15 +328,14 @@ inline cudaError_t launch_gemm(const GemmOp& op, bool a_kc, bool b_kc, int nbatc
     else nt = op.tiles_m * op.tiles_n;
     if (nt <= 0 || nbatch <= 0) return cudaSuccess;
     count_launch();
-    if (g_gemm_bm == 64 && g_gemm_stagger > 0 && nbatch == 1 && op.klo_sel == KSEL_CONST && op.khi_sel == KSEL_CONST &&
-        2 * nt >= 16 * GEMM_NUM_SMS && op.max_ctas == 0) {
+    if (nbatch == 1 && op.klo_sel == KSEL_CONST && op.khi_sel == KSEL_CONST && 2 * nt >= 16 * GEMM_NUM_SMS &&
+        op.max_ctas == 0) {
         // uniform K, at least eight waves: half a tile time = (khi - klo) * 8 chunks * ~2.2 us per chunk / 2
         GemmOp o2 = op;
-        o2.stagger_ns = (op.khi_c - op.klo_c) * 8 * 11 * g_gemm_stagger * 10;
-        return launch_gemm_bm<64>(o2, a_kc, b_kc, nt, nbatch, st);
+        o2.stagger_ns = (op.khi_c - op.klo_c) * 8 * 11 * GEMM_STAGGER * 10;
+        return launch_gemm_bm<GEMM_BM>(o2, a_kc, b_kc, nt, nbatch, st);
     }
-    if (g_gemm_bm == 64) return launch_gemm_bm<64>(op, a_kc, b_kc, nt, nbatch, st);
-    return launch_gemm_bm<128>(op, a_kc, b_kc, nt, nbatch, st);
+    return launch_gemm_bm<GEMM_BM>(op, a_kc, b_kc, nt, nbatch, st);
 }
 
 template <int BM>
@@ -355,11 +352,7 @@ inline cudaError_t gemm_set_attributes_bm() {
     return e;
 }
 
-inline cudaError_t gemm_set_attributes() {
-    cudaError_t e = gemm_set_attributes_bm<128>();
-    if (e != cudaSuccess) return e;
-    return gemm_set_attributes_bm<64>();
-}
+inline cudaError_t gemm_set_attributes() { return gemm_set_attributes_bm<GEMM_BM>(); }
 
 inline GemmOp gemm_default() {
     GemmOp op{};

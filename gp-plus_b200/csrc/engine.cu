@@ -49,13 +49,15 @@ static void set_err(const char* what, cudaError_t e) {
 enum { EV_START = 0, EV_COV, EV_CHOL, EV_TRTRI, EV_SOLVE, EV_LAUUM, EV_GRAD, EV_END, EV_COUNT };
 
 // Everything gpp_create decides besides the problem's shape: the arithmetic of the O(N^3) stages (gpp_set_fp64_mode,
-// GPP_FP64) and the development switches, per handle and process-wide (int fields only: compared with memcmp).
-// A parked handle is handed back only when the configuration in force now equals the one it was built under.
+// GPP_FP64) and the schedule switches of the handle (int fields only: compared with memcmp).  A parked handle is
+// handed back only when the configuration in force now equals the one it was built under.
 struct CreateConfig {
-    int lookahead, graph, early_out, small_block;                                    // per handle
-    int panel_blocks, overlap_inverse, gemm_bm, gemm_stagger, oz_items_per_cta;       // process globals
-    int int8;                                                                         // INT8-sliced O(N^3) stages
-    int oz_min_trail, oz_min_level, oz_next, oz_inner, oz_lazy, oz_kinv_levels, oz_lazy_min, oz_lazy_pb, oz_stagger;
+    int lookahead = 1;     // look-ahead / lazy-panel factorisation; GPP_CHOL=blocked: potrf_blocked
+    int graph = 0;         // CUDA-graph replay of a whole evaluation (GPP_GRAPH)
+    int small_block = 0;   // T <= 16: CTAs of the one-launch factorisation (GPP_SMALL_BLOCK; 0 = launch chain)
+    int int8 = 0;          // INT8-sliced O(N^3) stages
+    CholSchedule chol;
+    OzSchedule oz;         // used when the handle carries an OzCtx
 };
 
 struct gpp_handle {
@@ -103,14 +105,11 @@ struct gpp_handle {
     bool ev_valid[EV_COUNT];
     gpp_timings tm;
     CholLookahead la;
-    bool use_lookahead = true;
-    int small_block = 0;     // T <= 16: CTAs of the one-launch factorisation (GPP_SMALL_BLOCK; 0 = launch chain)
     OzCtx* oz = nullptr;     // INT8-sliced tcgen05 path of the O(N^3) stages (large problems; GPP_FP64=dmma turns it off)
     // CUDA-graph replay of one whole evaluation (small problems are launch-bound): [want_grad]
     cudaGraphExec_t graph_exec[2] = {nullptr, nullptr};
     long long graph_kernels[2] = {0, 0};
-    bool use_graph = false;
-    bool early_out = true;   // read the factorisation status before enqueueing the rest (non-graph path)
+    bool use_graph = false;  // cfg.graph until a capture fails
     bool capturing = false;
     bool pending = false;    // gpp_objective_enqueue issued, gpp_objective_collect not yet called
     int pending_grad = 0;
@@ -199,28 +198,19 @@ static const size_t kPoolMaxHandleBytes = 192ull << 20;  // handles up to Np = 2
 static const size_t kPoolMaxBytes = 6ull << 30;
 static const size_t kPoolMaxHandles = 160;
 
-// the configuration a handle with T tile rows gets when it is created now (defaults are the production configuration;
-// the process globals keep the value an earlier gpp_create gave them unless the environment sets them again)
+// the configuration a handle with T tile rows gets when it is created now: the production configuration, changed
+// only by the environment variables set at this moment
 static CreateConfig read_config(int T) {
     CreateConfig c;
-    memset(&c, 0, sizeof(c));
     const char* e;
-    c.lookahead = 1;
     if ((e = getenv("GPP_CHOL")) != nullptr) c.lookahead = strcmp(e, "blocked") != 0;
     c.graph = T <= 16;  // N <= 2048: an evaluation is a chain of ~25-100 tiny launches
     if ((e = getenv("GPP_GRAPH")) != nullptr) c.graph = atoi(e) != 0;
-    c.early_out = 1;
-    if ((e = getenv("GPP_EARLY_OUT")) != nullptr) c.early_out = atoi(e) != 0;
-    c.small_block = 0;
     if ((e = getenv("GPP_SMALL_BLOCK")) != nullptr) c.small_block = atoi(e);
-    c.panel_blocks = g_panel_blocks;
-    if ((e = getenv("GPP_PANEL")) != nullptr) c.panel_blocks = atoi(e);
-    c.overlap_inverse = g_overlap_inverse;
-    if ((e = getenv("GPP_OVERLAP_INV")) != nullptr) c.overlap_inverse = atoi(e);
-    c.gemm_bm = g_gemm_bm;
-    if ((e = getenv("GPP_GEMM_BM")) != nullptr) c.gemm_bm = atoi(e) == 64 ? 64 : 128;
-    c.gemm_stagger = g_gemm_stagger;
-    if ((e = getenv("GPP_STAGGER")) != nullptr) c.gemm_stagger = atoi(e);
+    if ((e = getenv("GPP_PANEL")) != nullptr) c.chol.panel_blocks = atoi(e);
+    if ((e = getenv("GPP_OVERLAP_INV")) != nullptr) c.chol.overlap_inverse = atoi(e);
+    if ((e = getenv("GPP_BLOCK_CTAS")) != nullptr) c.chol.block_ctas = atoi(e);
+    if ((e = getenv("GPP_TIMELINE")) != nullptr) c.chol.timeline = atoi(e) != 0;
     {
         // FP64 work of the O(N^3) stages: exact integer GEMMs on the INT8 tcgen05 tensor cores from Np = 3072 up
         // (measured: 3.08 vs 3.42 ms at N = 3072, 14.8 vs 22.0 at 8192, 28.8 vs 63.5 at 12288; below that an evaluation
@@ -233,58 +223,17 @@ static CreateConfig read_config(int T) {
         if (e && mode < 0) int8 = int8 && strcmp(e, "dmma") != 0;
         c.int8 = int8;
     }
-    c.oz_items_per_cta = g_oz_items_per_cta;
-    OzCtx d;   // defaults only (init() allocates)
-    c.oz_min_trail = d.min_trailing_tiles;
-    c.oz_min_level = d.min_level_tiles;
-    c.oz_next = d.next_on_oz;
-    c.oz_inner = d.inner_min_k;
-    c.oz_lazy = d.lazy;
-    c.oz_kinv_levels = d.kinv_levels;
-    c.oz_lazy_min = d.lazy_min_tiles;
-    c.oz_lazy_pb = d.lazy_pb;
-    c.oz_stagger = d.stagger;
     if (c.int8) {
-        if ((e = getenv("GPP_OZ_IPC")) != nullptr) c.oz_items_per_cta = atoi(e) > 0 ? atoi(e) : 2;
-        if ((e = getenv("GPP_OZ_MIN_TRAIL")) != nullptr) c.oz_min_trail = atoi(e);
-        if ((e = getenv("GPP_OZ_MIN_LEVEL")) != nullptr) c.oz_min_level = atoi(e);
-        if ((e = getenv("GPP_OZ_NEXT")) != nullptr) c.oz_next = atoi(e);
-        if ((e = getenv("GPP_OZ_INNER")) != nullptr) c.oz_inner = atoi(e);
-        if ((e = getenv("GPP_OZ_LAZY")) != nullptr) c.oz_lazy = atoi(e);
-        if ((e = getenv("GPP_OZ_KINV_LEVELS")) != nullptr) c.oz_kinv_levels = atoi(e);
-        if ((e = getenv("GPP_OZ_LAZY_MIN")) != nullptr) c.oz_lazy_min = atoi(e);
-        if ((e = getenv("GPP_OZ_LAZY_PB")) != nullptr) c.oz_lazy_pb = std::min(std::max(atoi(e), 2), OzCtx::LAZY_PB);
-        if ((e = getenv("GPP_OZ_STAGGER")) != nullptr) c.oz_stagger = atoi(e);
+        if ((e = getenv("GPP_OZ_MIN_TRAIL")) != nullptr) c.oz.min_trailing_tiles = atoi(e);
+        if ((e = getenv("GPP_OZ_MIN_LEVEL")) != nullptr) c.oz.min_level_tiles = atoi(e);
+        if ((e = getenv("GPP_OZ_NEXT")) != nullptr) c.oz.next_on_oz = atoi(e);
+        if ((e = getenv("GPP_OZ_INNER")) != nullptr) c.oz.inner_min_k = atoi(e);
+        if ((e = getenv("GPP_OZ_KINV_LEVELS")) != nullptr) c.oz.kinv_levels = atoi(e);
+        if ((e = getenv("GPP_OZ_LAZY_MIN")) != nullptr) c.oz.lazy_min_tiles = atoi(e);
+        if ((e = getenv("GPP_OZ_LAZY_PB")) != nullptr) c.oz.lazy_pb = std::min(std::max(atoi(e), 2), OzCtx::LAZY_PB);
+        if ((e = getenv("GPP_OZ_STAGGER")) != nullptr) c.oz.stagger = atoi(e);
     }
     return c;
-}
-
-static void apply_globals(const CreateConfig& c) {
-    g_panel_blocks = c.panel_blocks;
-    g_overlap_inverse = c.overlap_inverse;
-    g_gemm_bm = c.gemm_bm;
-    g_gemm_stagger = c.gemm_stagger;
-    g_oz_items_per_cta = c.oz_items_per_cta;
-}
-
-// per-handle switches (h->oz, when the handle has one, must exist already)
-static void apply_handle_config(gpp_handle* h, const CreateConfig& c) {
-    h->cfg = c;
-    h->use_lookahead = c.lookahead != 0;
-    h->use_graph = c.graph != 0;
-    h->early_out = c.early_out != 0;
-    h->small_block = c.small_block;
-    if (h->oz) {
-        h->oz->min_trailing_tiles = c.oz_min_trail;
-        h->oz->min_level_tiles = c.oz_min_level;
-        h->oz->next_on_oz = c.oz_next;
-        h->oz->inner_min_k = c.oz_inner;
-        h->oz->lazy = c.oz_lazy;
-        h->oz->kinv_levels = c.oz_kinv_levels;
-        h->oz->lazy_min_tiles = c.oz_lazy_min;
-        h->oz->lazy_pb = c.oz_lazy_pb;
-        h->oz->stagger = c.oz_stagger;
-    }
 }
 
 static bool same_shape(const gpp_handle* h, const gpp_problem* p, int device, const CreateConfig& cfg) {
@@ -401,7 +350,6 @@ extern "C" int gpp_create(const gpp_problem* p, int device, gpp_handle** out) {
     }
 
     const CreateConfig cfg = read_config((int)((p->n + 127) / 128));
-    apply_globals(cfg);
     {
         // a parked handle of the same shape and configuration on this device: re-upload the data, keep everything else
         gpp_handle* reuse = nullptr;
@@ -417,7 +365,7 @@ extern "C" int gpp_create(const gpp_problem* p, int device, gpp_handle** out) {
         }
         if (reuse) {
             memset(&reuse->stats, 0, sizeof(reuse->stats));
-            apply_handle_config(reuse, cfg);   // (a failed graph capture may have switched the replay off)
+            reuse->use_graph = cfg.graph != 0;   // (a failed graph capture may have switched the replay off)
             int rc = upload_problem(reuse, p);
             if (rc != GPP_OK) {
                 destroy_now(reuse);
@@ -429,6 +377,8 @@ extern "C" int gpp_create(const gpp_problem* p, int device, gpp_handle** out) {
     }
 
     gpp_handle* h = new gpp_handle();
+    h->cfg = cfg;
+    h->use_graph = cfg.graph != 0;
     memset(&h->tm, 0, sizeof(h->tm));
     memset(&h->stats, 0, sizeof(h->stats));
     for (int i = 0; i < EV_COUNT; i++) h->ev_valid[i] = false;
@@ -484,9 +434,11 @@ extern "C" int gpp_create(const gpp_problem* p, int device, gpp_handle** out) {
             if (device < 64) done[device] = true;
         }
     }
+    h->la.sched = cfg.chol;
     CKH(h->la.init(h->T));
     if (cfg.int8) {
         h->oz = new OzCtx();
+        h->oz->sched = cfg.oz;
         cudaError_t oe = h->oz->init((int)h->np);
         if (oe == cudaErrorMemoryAllocation) {
             // the digit planes (3 x 7 Np^2 bytes) do not fit next to the FP64 work matrices: stay on DMMA
@@ -498,7 +450,6 @@ extern "C" int gpp_create(const gpp_problem* p, int device, gpp_handle** out) {
             CKH(oe);
         }
     }
-    apply_handle_config(h, cfg);
 
     h->hyp_len = h->dq + h->n_pass * h->n_combo * h->dz + h->n_noise + h->n_mean + 2;
     h->res_len = 4 + h->dq + h->n_noise + h->n_mean;
@@ -680,16 +631,16 @@ static int stage_factor(gpp_handle* h) {
         CK(launch_cov(ca, h->kernel, h->st));
     }
     mark(h, EV_COV);
-    if (h->small_block > 0 && h->T <= 16) {
+    if (h->cfg.small_block > 0 && h->T <= 16) {
         // small problems: the whole factorisation is one dataflow launch (block_potrf_kernel) instead of a chain of
         // T leaf / TRSM / update launches.  Inside a captured graph the launch arguments are frozen, so the tile flags
         // are cleared by a memset node and the epoch is constant.
         CK(cudaMemsetAsync(h->la.blk_flags, 0, 256 * sizeof(int), h->st));
-        CK(launch_block_potrf(h->A, h->M, (int)h->np, 0, h->T, h->logdet_part, h->info, h->la.blk_flags, 1, h->small_block,
-                              h->st));
-    } else if (h->use_lookahead && h->oz && h->oz->ready && h->oz->lazy && h->T >= h->oz->lazy_min_tiles)
+        CK(launch_block_potrf(h->A, h->M, (int)h->np, 0, h->T, h->logdet_part, h->info, h->la.blk_flags, 1,
+                              h->cfg.small_block, h->st));
+    } else if (h->cfg.lookahead && h->oz && h->oz->ready && h->T >= h->oz->sched.lazy_min_tiles)
         CK(potrf_lazy(h->A, h->M, (int)h->np, h->T, h->logdet_part, h->info, h->st, h->la, h->S, *h->oz));
-    else if (h->use_lookahead)
+    else if (h->cfg.lookahead)
         CK(potrf_lookahead(h->A, h->M, (int)h->np, h->T, h->logdet_part, h->info, h->st, h->la, h->S, h->oz));
     else
         CK(potrf_blocked(h->A, h->M, (int)h->np, h->T, h->logdet_part, h->info, h->st));
@@ -699,7 +650,7 @@ static int stage_factor(gpp_handle* h) {
 
 // M <- L^-1, v = M r, alpha = M^T v
 static int stage_inverse_solve(gpp_handle* h) {
-    if (h->use_lookahead && h->la.inv_pending) {
+    if (h->cfg.lookahead && h->la.inv_pending) {
         // the leading part of L^-1 was started behind the factorisation (trtri_early): join it, finish the rest
         CK(cudaStreamWaitEvent(h->st, h->la.inv_done, 0));
         h->la.inv_pending = false;
@@ -851,7 +802,7 @@ static int enqueue_eval_early_out(gpp_handle* h, int want_grad, int* failed) {
     CK(cudaEventSynchronize(h->ev_info));
     if (*h->info_host != 0) {
         *failed = *h->info_host;
-        if (h->use_lookahead && h->la.inv_pending) {
+        if (h->cfg.lookahead && h->la.inv_pending) {
             // the leading part of L^-1 was started behind the factorisation: let it drain before A / M are reused
             CK(cudaStreamWaitEvent(h->st, h->la.inv_done, 0));
             h->la.inv_pending = false;
@@ -881,20 +832,15 @@ static int run_eval(gpp_handle* h, const gpp_hyper* hy, int want_grad, int first
             mark(h, EV_END);
             CK(cudaStreamSynchronize(h->st));
             info = (int)h->res_host[2];
-        } else if (h->early_out) {
+        } else {
             int failed = 0;
             int rc = enqueue_eval_early_out(h, want_grad, &failed);
             if (rc != GPP_OK) return rc;
             mark(h, EV_END);
             CK(cudaStreamSynchronize(h->st));
-            if (h->la.timeline) h->la.dump_timeline(h->oz ? (h->T + h->oz->lazy_pb - 1) / h->oz->lazy_pb : h->la.panels);
+            if (h->la.sched.timeline)
+                h->la.dump_timeline(h->oz ? (h->T + h->oz->sched.lazy_pb - 1) / h->oz->sched.lazy_pb : h->la.panels);
             info = failed ? failed : (int)h->res_host[2];
-        } else {
-            int rc = enqueue_eval(h, want_grad);
-            if (rc != GPP_OK) return rc;
-            mark(h, EV_END);
-            CK(cudaStreamSynchronize(h->st));
-            info = (int)h->res_host[2];
         }
         if (info & 2) {
             g_err = "NaN encountered while factorising K_y";

@@ -14,6 +14,28 @@
 
 namespace gpp {
 
+// Which work of the three stages runs on the INT8-sliced GEMM, and how (int fields only: gpp_create compares
+// configurations with memcmp).  The member initialisers are the production configuration.
+struct OzSchedule {
+    int min_trailing_tiles = 12;   // smaller trailing matrices stay on DMMA (too few 128x64 items for 148 SMs)
+                                   // (GPP_OZ_MIN_TRAIL)
+    int min_level_tiles = 4;       // inverse levels below this half-width stay on DMMA (K < 512) (GPP_OZ_MIN_LEVEL)
+    int next_on_oz = 1;            // U(p,p+1), the update of the next panel's own columns, also runs here (GPP_OZ_NEXT)
+    int inner_min_k = 4;           // in-panel (recursive) updates with K >= this many tiles run here; 0 = never
+                                   // (GPP_OZ_INNER)
+    int kinv_levels = 7;           // significance levels of K^-1 = M^T M (GPP_OZ_KINV_LEVELS).  Its only consumer is the
+                                   // gradient trace (tolerance 1e-8 of the gradient's max-norm): with 6 levels (21 of 28
+                                   // plane pairs) the product takes 11.1 instead of 13.4 ms at N = 16384 and the gradient
+                                   // moves by 6.6e-11 instead of 2.9e-13.  Default 7: both arithmetics then agree at the
+                                   // FP64 rounding level and multi-start fits follow the same L-BFGS-B paths
+    int lazy_min_tiles = 96;       // lazy panels (potrf_lazy) from N = 12288 (GPP_OZ_LAZY_MIN); below, 512-column panels
+                                   // of the look-ahead schedule keep the chain shorter (measured: N = 8192 12.7 vs 14.0 ms,
+                                   // N = 12288 28.5 vs 27.9, N = 16384 55.3 vs 54.4)
+    int lazy_pb = 12;              // lazy panel width in 128-tiles, 2 .. OzCtx::LAZY_PB (GPP_OZ_LAZY_PB)
+    int stagger = 6000;            // ns per 128-block of K: estimated duration of one 128x128 item, see OzGemmOp.stagger_ns
+                                   // (GPP_OZ_STAGGER)
+};
+
 struct OzCtx {
     bool ready = false;
     int np = 0, T = 0;
@@ -24,23 +46,10 @@ struct OzCtx {
     // lazy panels: only the diagonal block of a panel is factored on the latency-bound chain; the rows below are solved
     // against its explicit inverse W = L_pp^-1 by one integer GEMM.  W's digit planes, double-buffered by panel parity:
     static constexpr int LAZY_PB = 16;     // widest panel in 128-tiles (sizes the W planes)
-    int lazy_pb = 12;                      // panel width used (GPP_OZ_LAZY_PB)
-    int lazy = 1;
-    int kinv_levels = 7;           // significance levels of K^-1 = M^T M (GPP_OZ_KINV_LEVELS).  Its only consumer is the
-                                   // gradient trace (tolerance 1e-8 of the gradient's max-norm): with 6 levels (21 of 28
-                                   // plane pairs) the product takes 11.1 instead of 13.4 ms at N = 16384 and the gradient
-                                   // moves by 6.6e-11 instead of 2.9e-13.  Default 7: both arithmetics then agree at the
-                                   // FP64 rounding level and multi-start fits follow the same L-BFGS-B paths
-    int lazy_min_tiles = 96;       // from N = 12288; below, 512-column panels of the look-ahead schedule keep the chain
-                                   // shorter (measured: N = 8192 12.7 vs 14.0 ms, N = 12288 28.5 vs 27.9, N = 16384 55.3 vs 54.4)
-    int stagger = 6000;            // ns per 128-block of K: estimated duration of one 128x128 item, see OzGemmOp.stagger_ns
     OzPlanes PW[2];
     CUtensorMap mPW_b[2];
-    int next_on_oz = 1;            // U(p,p+1), the update of the next panel's own columns, also runs here
-    int inner_min_k = 4;           // in-panel (recursive) updates with K >= this many tiles run here; 0 = never
     CUtensorMap mPP_a, mPP_b, mPA_a, mPB_a, mPB_b;
-    int min_trailing_tiles = 12;   // smaller trailing matrices stay on DMMA (too few 128x64 items for 148 SMs)
-    int min_level_tiles = 4;       // inverse levels below this half-width stay on DMMA (K < 512)
+    OzSchedule sched;
     size_t bytes = 0;
 
     static cudaError_t alloc_planes(OzPlanes& P, long long np, size_t& bytes) {
@@ -114,7 +123,7 @@ inline cudaError_t oz_split_panel(OzCtx& oz, const double* A, int ld, int T, int
                          (long long)r0 * TILE, (long long)p0 * TILE, 0, 0, 1, st);
 }
 
-inline bool oz_use_trailing(const OzCtx* oz, int T, int c0) { return oz && oz->ready && (T - c0) >= oz->min_trailing_tiles; }
+inline bool oz_use_trailing(const OzCtx* oz, int T, int c0) { return oz && oz->ready && (T - c0) >= oz->sched.min_trailing_tiles; }
 
 // C[i,j] -= sum_{k in [p0,pend)} L[i,k] L[j,k] for tile rows i >= c0, tile columns j in [c0, c1), i >= j
 inline cudaError_t oz_trailing_update(OzCtx& oz, double* A, int ld, int T, int p0, int pend, int c0, int c1, int slot,
@@ -140,7 +149,7 @@ inline cudaError_t oz_trailing_update(OzCtx& oz, double* A, int ld, int T, int p
         op.lower_filter = 1;
         op.lower_off = 0;
     }
-    op.stagger_ns = oz.stagger * (pend - p0);
+    op.stagger_ns = oz.sched.stagger * (pend - p0);
     return launch_oz_gemm(oz.mPP_a, oz.mPP_b, op, 1, st);
 }
 
@@ -169,7 +178,7 @@ inline cudaError_t oz_update_region(OzCtx& oz, double* A, int ld, int p0, int pe
         op.lower_filter = 1;
         op.lower_off = r0 - c0;
     }
-    if (stagger) op.stagger_ns = oz.stagger * (pend - p0);
+    if (stagger) op.stagger_ns = oz.sched.stagger * (pend - p0);
     return launch_oz_gemm(oz.mPP_a, oz.mPP_b, op, 1, st);
 }
 
@@ -206,7 +215,7 @@ inline cudaError_t oz_panel_solve(OzCtx& oz, double* A, int ld, int p0, int pend
     op.klo_c = 0;
     op.khi_sel = KSEL_TJ;
     op.khi_c = 1;
-    if (stagger) op.stagger_ns = oz.stagger * (pend - p0) / 2;
+    if (stagger) op.stagger_ns = oz.sched.stagger * (pend - p0) / 2;
     return launch_oz_gemm(oz.mPP_a, oz.mPW_b[buf], op, 1, st);
 }
 
@@ -221,7 +230,7 @@ inline cudaError_t oz_split_panel_rows(OzCtx& oz, const double* A, int ld, int p
                          (long long)r0 * TILE, (long long)p0 * TILE, 0, 0, 1, st);
 }
 
-inline bool oz_use_level(const OzCtx* oz, int hb) { return oz && oz->ready && hb >= oz->min_level_tiles && hb <= 128; }
+inline bool oz_use_level(const OzCtx* oz, int hb) { return oz && oz->ready && hb >= oz->sched.min_level_tiles && hb <= 128; }
 
 // one level of the recursive doubling (see trtri_level in chol.cuh): X21 = L21 * M11 (part & 1), M21 = -M22 * X21 (part & 2)
 inline cudaError_t oz_trtri_level(OzCtx& oz, const double* L, double* M, double* X, int ld, int hb, int g_lo, int nb,
@@ -309,7 +318,7 @@ inline cudaError_t oz_lauum(OzCtx& oz, const double* M, double* Kinv, int ld, in
     op.klo_c = 0;
     op.khi_sel = KSEL_CONST;
     op.khi_c = T;
-    op.levels = oz.kinv_levels;
+    op.levels = oz.sched.kinv_levels;
     // K ranges longer than 128 blocks (N > 16384) are accumulated in segments: |digit| <= 128, so 16384 products per
     // int32 accumulation cannot overflow
     for (int k0 = 0; k0 < T; k0 += 128) {

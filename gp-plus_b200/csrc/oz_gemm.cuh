@@ -491,17 +491,14 @@ inline cudaError_t oz_set_attributes() {
 
 // items_per_cta: CTAs are NOT persistent over the whole launch -- each handles about this many 128x128 tiles
 // (grid-stride), so that SMs are handed back every few items and higher-priority streams (the panel chain of the
-// factorisation) get in; the hardware block scheduler does the load balancing.
-inline int g_oz_items_per_cta = 1;
-
+// factorisation) get in; the hardware block scheduler does the load balancing (two per CTA: DESIGN.md section 7).
 inline cudaError_t launch_oz_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, const OzGemmOp& op_in, int nbatch,
-                                  cudaStream_t st, int items_per_cta = 0) {
+                                  cudaStream_t st, int items_per_cta = 1) {
     OzGemmOp op = op_in;
     if (op.map == MAP_TRI) op.n_tiles = op.tiles_m * (op.tiles_m + 1) / 2;
     else op.n_tiles = op.tiles_m * op.tiles_n;
     if (op.n_tiles <= 0 || nbatch <= 0) return cudaSuccess;
-    const int ipc = items_per_cta > 0 ? items_per_cta : g_oz_items_per_cta;
-    int gx = (op.n_tiles + ipc - 1) / ipc;
+    int gx = (op.n_tiles + items_per_cta - 1) / items_per_cta;
     if (gx < 1) gx = 1;
     count_launch();
     oz_gemm_kernel<<<dim3(gx, nbatch), OZ_THREADS, OZ_SMEM_BYTES, st>>>(tmA, tmB, op);

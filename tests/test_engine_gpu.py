@@ -368,6 +368,45 @@ def test_pooled_handles_follow_the_settings_in_force(monkeypatch):
         E.pool_clear()
 
 
+def test_schedule_settings_stay_with_the_handle_created_under_them(monkeypatch):
+    """A schedule switch belongs to the handle created under it: creating another handle with GPP_OVERLAP_INV=0
+    changes neither the launches nor the likelihood of a handle that exists already, and once the variable is unset
+    the next handle gets the default schedule again.  N = 2300 (T = 18) evaluates as a chain of launches (no graph
+    replay), so the overlapped inverse changes the launches per evaluation."""
+    from gpplus_b200 import _engine as E
+    p = make_problem(2300, 5, 2, dz=2, n_combo=7, n_noise=2, seed=31)
+    h = make_hyper(p, seed=13)
+
+    def evaluate(eng):
+        eng.mll_grad(h, want_grad=True)
+        before = E.launch_count()
+        nll = eng.mll_grad(h, want_grad=True)["nll"]
+        return E.launch_count() - before, nll
+
+    E.pool_clear()
+    monkeypatch.delenv("GPP_OVERLAP_INV", raising=False)
+    a = E.Engine(**engine_kwargs(p))
+    try:
+        count_a, nll_a = evaluate(a)
+        monkeypatch.setenv("GPP_OVERLAP_INV", "0")
+        b = E.Engine(**engine_kwargs(p))
+        try:
+            count_b = evaluate(b)[0]
+        finally:
+            b.close()   # parked under GPP_OVERLAP_INV=0
+        assert count_b != count_a, count_a
+        assert evaluate(a) == (count_a, nll_a)
+        monkeypatch.delenv("GPP_OVERLAP_INV")
+        c = E.Engine(**engine_kwargs(p))
+        try:
+            assert evaluate(c)[0] == count_a
+        finally:
+            c.close()
+    finally:
+        a.close()
+        E.pool_clear()
+
+
 @pytest.mark.parametrize("kernel,n,n_pass", [(0, 300, 3), (2, 517, 5), (1, 130, 2)])
 def test_multi_pass_ensemble_covariance_matches_oracle(kernel, n, n_pass):
     """Multi-pass ensemble covariance of the probabilistic embedding (gp_plus.py:387-399, 474-482):

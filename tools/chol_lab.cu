@@ -1,7 +1,7 @@
 // Development bench for the factorisation kernels (not part of the product library).
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -o tools/chol_lab tools/chol_lab.cu
 //   ./tools/chol_lab [N ...]
-// Times the leaf kernels (with clock64 phase stamps), the DMMA GEMM CTA shapes and the blocked / look-ahead
+// Times the leaf kernels (with clock64 phase stamps), DMMA GEMM shapes and the blocked / look-ahead
 // Cholesky drivers on a Kac-Murdock-Szego test matrix, and cross-checks every variant against the first one.
 #include <cuda_runtime.h>
 #include <math.h>
@@ -277,46 +277,42 @@ static void gemm_lab(cudaStream_t st) {
     fill_kms<<<(int)(((long long)n * n + 255) / 256), 256, 0, st>>>(A, n, n, 0.99, 0.0);
     fill_kms<<<(int)(((long long)n * n + 255) / 256), 256, 0, st>>>(B, n, n, 0.98, 0.0);
     Timer tm;
-    for (int bm : {128, 64}) {
-        g_gemm_bm = bm;
-        // full GEMM 8192^3
-        GemmOp op = gemm_default();
-        op.A = A; op.lda = n; op.B = B; op.ldb = n; op.C = C; op.ldc = n;
-        op.tiles_m = op.tiles_m_last = n / 128; op.tiles_n = n / 128; op.khi_c = n / 128;
-        for (int kc = 0; kc < 2; kc++) {
-            bool akc = kc == 0, bkc = kc == 0;
-            CHECK(launch_gemm(op, akc, bkc, 1, st));
-            tm.start(st);
-            for (int i = 0; i < 3; i++) CHECK(launch_gemm(op, akc, bkc, 1, st));
-            float ms = tm.stop(st) / 3;
-            printf("gemm bm=%d layout=%s 8192^3: %.3f ms  %.2f TFLOP/s\n", bm, kc == 0 ? "kc,kc" : "ks,ks", ms,
-                   2.0 * n * (double)n * n / (ms * 1e-3) / 1e12);
-        }
-        // SYRK-shaped trailing update: 60x60 lower tiles, K = 512
-        for (int kblocks : {2, 4, 8}) {
-            GemmOp s = gemm_default();
-            s.A = A; s.lda = n; s.B = A; s.ldb = n; s.C = C; s.ldc = n;
-            s.map = MAP_TRI; s.tiles_m = s.tiles_m_last = 60; s.tiles_n = 60; s.khi_c = kblocks; s.alpha = -1.0; s.beta = 1.0;
-            CHECK(launch_gemm(s, true, true, 1, st));
-            tm.start(st);
-            for (int i = 0; i < 5; i++) CHECK(launch_gemm(s, true, true, 1, st));
-            float ms = tm.stop(st) / 5;
-            double fl = 60.0 * 61.0 / 2 * 2.0 * 128 * 128 * 128 * kblocks;
-            printf("syrk bm=%d 60x60 tri tiles K=%d: %.3f ms  %.2f TFLOP/s\n", bm, kblocks * 128, ms, fl / (ms * 1e-3) / 1e12);
-        }
-        // TRSM-shaped: 100 x 1 tiles, K = 128; panel update: 100 x 3 tiles K = 128
-        for (int tn : {1, 3}) {
-            GemmOp s = gemm_default();
-            s.A = A; s.lda = n; s.B = B; s.ldb = n; s.C = C; s.ldc = n;
-            s.tiles_m = s.tiles_m_last = 60; s.tiles_n = tn; s.khi_c = 1;
-            CHECK(launch_gemm(s, true, true, 1, st));
-            tm.start(st);
-            for (int i = 0; i < 10; i++) CHECK(launch_gemm(s, true, true, 1, st));
-            float ms = tm.stop(st) / 10;
-            printf("small bm=%d 60x%d tiles K=128: %.1f us per launch (back to back)\n", bm, tn, ms * 1e3);
-        }
+    // full GEMM 8192^3
+    GemmOp op = gemm_default();
+    op.A = A; op.lda = n; op.B = B; op.ldb = n; op.C = C; op.ldc = n;
+    op.tiles_m = op.tiles_m_last = n / 128; op.tiles_n = n / 128; op.khi_c = n / 128;
+    for (int kc = 0; kc < 2; kc++) {
+        bool akc = kc == 0, bkc = kc == 0;
+        CHECK(launch_gemm(op, akc, bkc, 1, st));
+        tm.start(st);
+        for (int i = 0; i < 3; i++) CHECK(launch_gemm(op, akc, bkc, 1, st));
+        float ms = tm.stop(st) / 3;
+        printf("gemm layout=%s 8192^3: %.3f ms  %.2f TFLOP/s\n", kc == 0 ? "kc,kc" : "ks,ks", ms,
+               2.0 * n * (double)n * n / (ms * 1e-3) / 1e12);
     }
-    g_gemm_bm = 128;
+    // SYRK-shaped trailing update: 60x60 lower tiles, K = 512
+    for (int kblocks : {2, 4, 8}) {
+        GemmOp s = gemm_default();
+        s.A = A; s.lda = n; s.B = A; s.ldb = n; s.C = C; s.ldc = n;
+        s.map = MAP_TRI; s.tiles_m = s.tiles_m_last = 60; s.tiles_n = 60; s.khi_c = kblocks; s.alpha = -1.0; s.beta = 1.0;
+        CHECK(launch_gemm(s, true, true, 1, st));
+        tm.start(st);
+        for (int i = 0; i < 5; i++) CHECK(launch_gemm(s, true, true, 1, st));
+        float ms = tm.stop(st) / 5;
+        double fl = 60.0 * 61.0 / 2 * 2.0 * 128 * 128 * 128 * kblocks;
+        printf("syrk 60x60 tri tiles K=%d: %.3f ms  %.2f TFLOP/s\n", kblocks * 128, ms, fl / (ms * 1e-3) / 1e12);
+    }
+    // TRSM-shaped: 100 x 1 tiles, K = 128; panel update: 100 x 3 tiles K = 128
+    for (int tn : {1, 3}) {
+        GemmOp s = gemm_default();
+        s.A = A; s.lda = n; s.B = B; s.ldb = n; s.C = C; s.ldc = n;
+        s.tiles_m = s.tiles_m_last = 60; s.tiles_n = tn; s.khi_c = 1;
+        CHECK(launch_gemm(s, true, true, 1, st));
+        tm.start(st);
+        for (int i = 0; i < 10; i++) CHECK(launch_gemm(s, true, true, 1, st));
+        float ms = tm.stop(st) / 10;
+        printf("small 60x%d tiles K=128: %.1f us per launch (back to back)\n", tn, ms * 1e3);
+    }
     cudaFree(A); cudaFree(B); cudaFree(C);
 }
 
@@ -339,15 +335,12 @@ static void potrf_lab(int n, cudaStream_t st) {
     CholLookahead la;
     CHECK(la.init(T));
     Timer tm;
-    struct Var { const char* name; int bm, look, pb, depth; };
-    const Var vars[] = {{"blocked   P4        ", 64, 0, 4, 1}, {"lookahead P8 depth 1", 64, 1, 8, 1},
-                        {"lookahead P8 depth 2", 64, 1, 8, 2}, {"lookahead P4 depth 2", 64, 1, 4, 2},
-                        {"lookahead P8 bm128  ", 128, 1, 8, 2}};
+    struct Var { const char* name; int look, pb; };
+    const Var vars[] = {{"blocked   P4", 0, 4}, {"lookahead P8", 1, 8}, {"lookahead P4", 1, 4}};
+    const int nvars = (int)(sizeof(vars) / sizeof(vars[0]));
     const int nblk = (int)((ld * ld + 255) / 256);
-    for (int v = 0; v < 5; v++) {
-        g_gemm_bm = vars[v].bm;
-        g_panel_blocks = vars[v].pb;
-        g_lookahead_depth = vars[v].depth;
+    for (int v = 0; v < nvars; v++) {
+        la.sched.panel_blocks = vars[v].pb;
         float best = 1e9f;
         for (int it = 0; it < 3; it++) {
             CHECK(cudaMemcpyAsync(A, A0, (size_t)ld * ld * 8, cudaMemcpyDeviceToDevice, st));
@@ -380,9 +373,6 @@ static void potrf_lab(int n, cudaStream_t st) {
                n, vars[v].name, best, (double)n * n * n / 3.0 / (best * 1e-3) / 1e12, hinfo, logdet, res, invres, dl);
         fflush(stdout);
     }
-    g_gemm_bm = 64;
-    g_panel_blocks = 0;
-    g_lookahead_depth = 2;
     la.destroy();
     cudaFree(A0); cudaFree(A); cudaFree(M); cudaFree(Lref); cudaFree(ldp); cudaFree(mx); cudaFree(info);
 }

@@ -14,4 +14,4 @@ for l in sys.stdin:
 }
 run lazy X=1
 run lazy_noverlap GPP_OVERLAP_INV=0
-run nolazy GPP_OZ_LAZY=0
+run nolazy GPP_OZ_LAZY_MIN=100000

@@ -2,9 +2,9 @@
 # INT8-sliced vs DMMA at mid sizes (which arithmetic should be the default where), lazy panels on / off
 mkdir -p gpurun_out
 for n in 3072 4096 6144 8192 12288; do
-for cfg in "1 1" "1 0" "0 1"; do
+for cfg in "1 0" "1 100000" "0 0"; do
   set -- $cfg
-  GPP_OZ_LAZY=$2 python - <<PY 2>&1 | tail -1
+  GPP_OZ_LAZY_MIN=$2 python - <<PY 2>&1 | tail -1
 import sys, time
 sys.path[:0] = ['.', 'gp-plus_b200']
 import numpy as np
@@ -22,7 +22,7 @@ for k in range(6):
     t = eng.timings()
     if k >= 2: outs.append(t)
 tot = np.median([t['total'] for t in outs])
-print("n=%5d fp64_mode %d lazy $2: total %.3f ms  chol %.3f trtri %.3f lauum %.3f  nll %.12e" % (n, eng.fp64_mode(), tot, outs[-1]['cholesky'], outs[-1]['trtri'], outs[-1]['lauum'], o['nll']))
+print("n=%5d fp64_mode %d lazy_min $2: total %.3f ms  chol %.3f trtri %.3f lauum %.3f  nll %.12e" % (n, eng.fp64_mode(), tot, outs[-1]['cholesky'], outs[-1]['trtri'], outs[-1]['lauum'], o['nll']))
 eng.close()
 PY
 done
