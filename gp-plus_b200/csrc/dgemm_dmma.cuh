@@ -56,7 +56,9 @@ constexpr int GEMM_STAGGER = 10;    // phase shift of the two resident CTAs of a
 
 enum KSel { KSEL_CONST = 0, KSEL_TI = 1, KSEL_TJ = 2 };
 enum TileMap { MAP_RECT = 0, MAP_TRI = 1 };
-enum Epilogue { EPI_STORE = 0, EPI_ROWSQ = 2 };
+// EPI_STORE_ROWSQ: the EPI_ROWSQ row sums (same values, bit for bit) and the plain EPI_STORE tile (alpha = 1, beta = 0
+// assumed by the caller), for prediction gradients that need U = K* L^-T itself
+enum Epilogue { EPI_STORE = 0, EPI_ROWSQ = 2, EPI_STORE_ROWSQ = 3 };
 
 struct GemmOp {
     const double* A;
@@ -254,7 +256,8 @@ __global__ void __launch_bounds__(GemmCfg<BM>::THREADS, GemmCfg<BM>::MIN_CTAS) d
     __syncthreads();  // every operand read of this CTA is complete (C may alias A)
 
     const double alpha = op.alpha, beta = op.beta;
-    if (op.epilogue == EPI_ROWSQ) {
+    constexpr bool STORE_ROWSQ = A_KC && B_KC;  // EPI_STORE_ROWSQ exists in the K* L^-T instantiation only
+    if (op.epilogue == EPI_ROWSQ || (STORE_ROWSQ && op.epilogue == EPI_STORE_ROWSQ)) {
         // rowsq[tj][row] = sum over the tile's 128 columns of (alpha*acc)^2 ; reduce t-lanes then the 2 N-warps
         double* red = smem;  // [2][BM]
 #pragma unroll
@@ -276,7 +279,7 @@ __global__ void __launch_bounds__(GemmCfg<BM>::THREADS, GemmCfg<BM>::MIN_CTAS) d
             op.rowsq[(long long)tj * op.rowsq_ld + (long long)z * op.c_zs + (long long)ti * TILE + r0 + tid] = s;
         }
         __syncthreads();  // `red` aliases the first pipeline stage of the next work item
-        continue;
+        if (!STORE_ROWSQ || op.epilogue == EPI_ROWSQ) continue;
     }
 
     double* Cg = op.C + (long long)z * op.c_zs + ((long long)ti * TILE + r0) * op.ldc + (long long)tj * TILE;

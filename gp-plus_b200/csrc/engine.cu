@@ -19,6 +19,7 @@
 #include "cov.cuh"
 #include "objective.h"
 #include "predict.cuh"
+#include "predict_grad.cuh"
 #include "solve.cuh"
 
 using namespace gpp;
@@ -96,6 +97,10 @@ struct gpp_handle {
     double *c_mean_part = nullptr, *c_rowsq = nullptr, *c_mu = nullptr, *c_var = nullptr, *c_score = nullptr;
     double* c_blk_best = nullptr;
     long long* c_blk_idx = nullptr;
+    // prediction-gradient buffers (gpp_predict_grad only; allocated on its first call)
+    long long g_alloc = 0;  // mc_alloc they were sized for
+    long long g_step = 0;   // candidates per chunk on that path
+    double *g_U = nullptr, *g_part_m = nullptr, *g_part_v = nullptr, *g_dmean = nullptr, *g_dvar = nullptr;
     double* acq_par = nullptr;  // [cost n_cost | best_f n_cost]
     int* acq_kind = nullptr;
     int acq_cap = 0;
@@ -133,7 +138,7 @@ static const double* hyp_beta(const gpp_handle* h) { return h->hyp + h->dq + zta
 static const double* hyp_sf2(const gpp_handle* h) { return hyp_beta(h) + h->n_mean; }
 static const double* hyp_jitter(const gpp_handle* h) { return hyp_beta(h) + h->n_mean + 1; }
 
-extern "C" int gpp_version(void) { return 106; }
+extern "C" int gpp_version(void) { return 107; }
 
 // process-wide default for handles created afterwards: -1 = by size (INT8-sliced from Np = 4096), 0 = DMMA, 1 = INT8
 static std::atomic<int> g_fp64_mode{-1};
@@ -167,7 +172,8 @@ static void destroy_now(gpp_handle* h) {
     if (h->st) cudaStreamSynchronize(h->st);
     void* dptrs[] = {h->slab, h->c_xq, h->c_xs, h->c_nrm, h->c_zpt, h->c_K, h->c_lvl,
                      h->c_noise, h->c_mean, h->c_cost, h->c_mean_part, h->c_rowsq, h->c_mu, h->c_var, h->c_score,
-                     h->c_blk_best, h->c_blk_idx, h->acq_par, h->acq_kind};
+                     h->c_blk_best, h->c_blk_idx, h->acq_par, h->acq_kind, h->g_U, h->g_part_m, h->g_part_v,
+                     h->g_dmean, h->g_dvar};
     for (void* p : dptrs)
         if (p) cudaFree(p);
     if (h->pinned_slab) cudaFreeHost(h->pinned_slab);
@@ -1164,6 +1170,29 @@ static int ensure_chunk_buffers(gpp_handle* h, long long m) {
     return GPP_OK;
 }
 
+// U = K* L^-T of one chunk, the per-column-tile gradient partials and the chunk's gradients (gpp_predict_grad).  The
+// partials take T*dq doubles per candidate each, so this path caps its chunk at 2^24 / (T*dq) candidates (128 MiB per
+// partial buffer; 4096 candidates at N = 16384, dq = 32); mean and variance do not depend on the chunking.
+static int ensure_grad_buffers(gpp_handle* h) {
+    if (h->g_alloc == h->mc_alloc) return GPP_OK;
+    void* olds[] = {h->g_U, h->g_part_m, h->g_part_v, h->g_dmean, h->g_dvar};
+    for (void* p : olds)
+        if (p) cudaFree(p);
+    h->g_U = h->g_part_m = h->g_part_v = h->g_dmean = h->g_dvar = nullptr;
+    h->g_alloc = h->g_step = 0;
+    long long step = ((1LL << 24) / ((long long)h->T * std::max(h->dq, 1))) / 128 * 128;
+    step = std::min(std::max(step, 128LL), h->mc_alloc);
+    const size_t sc = (size_t)step;
+    CK(dev_alloc(&h->g_U, sc * (size_t)h->np));
+    CK(dev_alloc(&h->g_part_m, sc * (size_t)h->T * h->dq));
+    CK(dev_alloc(&h->g_part_v, sc * (size_t)h->T * h->dq));
+    CK(dev_alloc(&h->g_dmean, sc * h->dq));
+    CK(dev_alloc(&h->g_dvar, sc * h->dq));
+    h->g_alloc = h->mc_alloc;
+    h->g_step = step;
+    return GPP_OK;
+}
+
 struct AcqSpec {
     const int32_t* cost_idx = nullptr;
     int n_cost = 0;
@@ -1179,7 +1208,8 @@ struct AcqSpec {
 
 static int predict_impl(gpp_handle* h, long long m, const double* xq, const int32_t* level_idx,
                         const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, double min_var,
-                        double* mean, double* var, AcqSpec* acq) {
+                        double* mean, double* var, AcqSpec* acq, bool grad = false, double* d_mean = nullptr,
+                        double* d_var = nullptr) {
     if (!h->factorized) ARG_FAIL("predict: call gpp_factorize (or gpp_mll_grad) first");
     if (m <= 0) return GPP_OK;
     if (h->dq > 0 && !xq) ARG_FAIL("predict: xq missing");
@@ -1187,6 +1217,10 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
     CK(cudaSetDevice(h->device));
     int rc = ensure_chunk_buffers(h, m);
     if (rc != GPP_OK) return rc;
+    if (grad) {
+        rc = ensure_grad_buffers(h);
+        if (rc != GPP_OK) return rc;
+    }
     if (acq) {
         if (acq->n_cost <= 0 || !acq->cost || !acq->kind_by_cost || !acq->best_f) ARG_FAIL("acq: cost tables missing");
         if (acq->n_cost > h->acq_cap) {
@@ -1205,9 +1239,10 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
     }
     std::vector<double> hb;
     std::vector<long long> hi;
-    const long long MC = h->mc_alloc;
-    for (long long base = 0; base < m; base += MC) {
-        const long long mc = std::min(MC, m - base);
+    const long long MC = h->mc_alloc;  // leading dimension of the chunk buffers
+    const long long step = grad ? h->g_step : MC;
+    for (long long base = 0; base < m; base += step) {
+        const long long mc = std::min(step, m - base);
         const long long mcp = (mc + 127) / 128 * 128;
         const int tiles_r = (int)(mcp / 128);
         if (h->dq > 0)
@@ -1281,6 +1316,11 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
         op.epilogue = EPI_ROWSQ;
         op.rowsq = h->c_rowsq;
         op.rowsq_ld = (int)MC;
+        if (grad) {  // the gradient pass needs U = K* L^-T itself; the row sums come out bitwise the same
+            op.epilogue = EPI_STORE_ROWSQ;
+            op.C = h->g_U;
+            op.ldc = (int)h->np;
+        }
         CK(launch_gemm(op, true, true, 1, h->st));
 
         PredFinishArgs fa;
@@ -1320,6 +1360,70 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
         predict_finish_kernel<<<nblk, 256, 0, h->st>>>(fa);
         CK(cudaGetLastError());
     count_launch();
+        if (grad) {
+            // V = U L^-1 = K* K_y^-1 over the K* chunk, which is not read again: B(tj, k) = L^-1[k, tj], k in [tj, T)
+            GemmOp vo = gemm_default();
+            vo.A = h->g_U;
+            vo.lda = (int)h->np;
+            vo.B = h->M;
+            vo.ldb = (int)h->np;
+            vo.C = h->c_K;
+            vo.ldc = (int)h->np;
+            vo.tiles_m = vo.tiles_m_last = tiles_r;
+            vo.tiles_n = h->T;
+            vo.klo_sel = KSEL_TJ;
+            vo.klo_c = 0;
+            vo.khi_c = h->T;
+            CK(launch_gemm(vo, true, false, 1, h->st));
+
+            PredGradArgs ga;
+            memset(&ga, 0, sizeof(ga));
+            ga.xs_r = h->c_xs;
+            ga.zpt_r = h->c_zpt;
+            ga.zs_r = mcp * ZP;
+            ga.xs_c = h->xs;
+            ga.zpt_c = h->zpt;
+            ga.zs_c = h->np * ZP;
+            ga.alpha = h->alpha;
+            ga.V = h->c_K;
+            ga.ldv = h->np;
+            ga.n_r = (int)mc;
+            ga.n_c = (int)h->n;
+            ga.dq = h->dq;
+            ga.dqp = h->dqp;
+            ga.dz = h->dz;
+            ga.n_pass = h->n_pass;
+            ga.part_m = h->g_part_m;
+            ga.part_v = h->g_part_v;
+            ga.ldp = step;
+            CK(launch_predict_grad(ga, h->kernel, tiles_r, h->T, h->st));
+
+            PredGradFinishArgs gf;
+            memset(&gf, 0, sizeof(gf));
+            gf.part_m = h->g_part_m;
+            gf.part_v = h->g_part_v;
+            gf.ldp = step;
+            gf.rowsq = h->c_rowsq;
+            gf.ldr = MC;
+            gf.tiles_c = h->T;
+            gf.m = (int)mc;
+            gf.dq = h->dq;
+            gf.w = hyp_w(h);
+            gf.sf2 = h->sf2;
+            gf.noise_idx = noise_idx ? h->c_noise : nullptr;
+            gf.noise = hyp_noise(h);
+            gf.n_noise = h->n_noise;
+            gf.include_noise = include_noise;
+            gf.min_var = min_var;
+            gf.d_mean = h->g_dmean;
+            gf.d_var = h->g_dvar;
+            predict_grad_finish_kernel<<<nblk, 256, 0, h->st>>>(gf);
+            CK(cudaGetLastError());
+            count_launch();
+            const size_t gb = sizeof(double) * (size_t)mc * h->dq;
+            if (d_mean) CK(cudaMemcpyAsync(d_mean + base * h->dq, h->g_dmean, gb, cudaMemcpyDefault, h->st));
+            if (d_var) CK(cudaMemcpyAsync(d_var + base * h->dq, h->g_dvar, gb, cudaMemcpyDefault, h->st));
+        }
         if (mean) CK(cudaMemcpyAsync(mean + base, h->c_mu, sizeof(double) * mc, cudaMemcpyDefault, h->st));
         if (var) CK(cudaMemcpyAsync(var + base, h->c_var, sizeof(double) * mc, cudaMemcpyDefault, h->st));
         if (acq) {
@@ -1349,6 +1453,16 @@ extern "C" int gpp_predict(gpp_handle* h, int64_t m, const double* xq, const int
                            double* mean, double* var) {
     if (!h) ARG_FAIL("gpp_predict: null handle");
     return predict_impl(h, m, xq, level_idx, noise_idx, mean_idx, include_noise, min_var, mean, var, nullptr);
+}
+
+extern "C" int gpp_predict_grad(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
+                                const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, double min_var,
+                                double* mean, double* var, double* d_mean, double* d_var) {
+    if (!h) ARG_FAIL("gpp_predict_grad: null handle");
+    // no quantitative input (or no gradient asked for): nothing to differentiate, the gpp_predict sequence
+    const bool grad = h->dq > 0 && (d_mean || d_var);
+    return predict_impl(h, m, xq, level_idx, noise_idx, mean_idx, include_noise, min_var, mean, var, nullptr, grad,
+                        d_mean, d_var);
 }
 
 extern "C" int gpp_acq_argmax(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,

@@ -22,7 +22,8 @@ LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libg
 EXPORTS = (
     "gpp_version", "gpp_device_count", "gpp_last_error", "gpp_launch_count", "gpp_create", "gpp_destroy", "gpp_pool_clear",
     "gpp_mll_grad",
-    "gpp_get_timings", "gpp_get_stats", "gpp_covariance", "gpp_fetch", "gpp_factorize", "gpp_predict", "gpp_acq_argmax",
+    "gpp_get_timings", "gpp_get_stats", "gpp_covariance", "gpp_fetch", "gpp_factorize", "gpp_predict", "gpp_predict_grad",
+    "gpp_acq_argmax",
     "gpp_probe_dgemm", "gpp_probe_i8", "gpp_set_fp64_mode", "gpp_get_fp64_mode", "gpp_set_theta_layout", "gpp_objective", "gpp_objective_enqueue", "gpp_objective_collect",
 )
 
@@ -123,6 +124,9 @@ def load_library():
         lib.gpp_predict.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                     C.c_double, C.c_void_p, C.c_void_p]
         lib.gpp_predict.restype = C.c_int
+        lib.gpp_predict_grad.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.gpp_predict_grad.restype = C.c_int
         lib.gpp_acq_argmax.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_double,
                                        C.c_double, C.c_double, C.c_double, C.c_void_p, _dp, C.POINTER(C.c_int64)]
@@ -426,6 +430,28 @@ class Engine:
         if rc != GPP_OK:
             _raise(rc, "gpp_predict")
         return mean, var
+
+    def predict_grad(self, xq, level_idx=None, noise_idx=None, mean_idx=None, include_noise: bool = False,
+                     min_var: float = 1e-10, out_mean=None, out_var=None, out_d_mean=None, out_d_var=None):
+        """``predict`` plus the derivatives of the scaled mean and of the clamped variance with respect to the
+        quantitative inputs: returns ``(mean [m], var [m], d_mean [m, dq], d_var [m, dq])``.  Inputs and output
+        buffers as for ``predict``."""
+        if isinstance(xq, np.ndarray) or not hasattr(xq, "data_ptr"):
+            xq = _f64(xq)
+            m = xq.shape[0] if xq.ndim == 2 else (xq.size // max(self.dq, 1))
+            level_idx, noise_idx, mean_idx = _i32(level_idx, m), _i32(noise_idx, m), _i32(mean_idx, m)
+        else:
+            m = int(xq.shape[0])
+        mean = np.empty(m) if out_mean is None else out_mean
+        var = np.empty(m) if out_var is None else out_var
+        d_mean = np.empty((m, self.dq)) if out_d_mean is None else out_d_mean
+        d_var = np.empty((m, self.dq)) if out_d_var is None else out_d_var
+        rc = self._lib.gpp_predict_grad(self._h, m, _ptr(xq), _ptr(level_idx), _ptr(noise_idx), _ptr(mean_idx),
+                                        1 if include_noise else 0, float(min_var), _ptr(mean), _ptr(var),
+                                        _ptr(d_mean), _ptr(d_var))
+        if rc != GPP_OK:
+            _raise(rc, "gpp_predict_grad")
+        return mean, var, d_mean, d_var
 
     def acq_argmax(self, xq, cost_idx, cost: Sequence[float], kind_by_cost: Sequence[int], best_f: Sequence[float],
                    level_idx=None, mean_idx=None, maximize: bool = True, si: float = 0.0, y_min: float = 0.0,

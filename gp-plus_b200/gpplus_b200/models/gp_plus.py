@@ -458,15 +458,11 @@ class GP_Plus(GPR):
             return super().predict(Xtest, return_std=return_std, include_noise=include_noise)
 
     def predict_with_grad(self, Xtest, return_std=True, include_noise=True):
-        """Reference: ``predict`` without ``torch.no_grad()`` (gp_plus.py:626-628), i.e. mean / std that carry an
-        autograd graph back to ``Xtest`` and the parameters.  The engine returns plain numbers (host buffers filled
-        by the device), so there is no graph to return: asking for one is refused instead of silently handing back
-        detached tensors; inputs that do not require a gradient are served like ``predict``."""
+        """Reference: ``predict`` without ``torch.no_grad()`` (gp_plus.py:626-628).  When ``Xtest`` requires a gradient
+        the mean and std carry an autograd graph back to ``Xtest`` only: the derivatives w.r.t. its quantitative
+        columns come from the engine (gpp_predict_grad), its categorical and source columns get zero, and the graph
+        does not reach the model's parameters.  First derivatives only.  The values equal ``predict``'s."""
         Xtest = data_type_check(Xtest)
-        if torch.is_tensor(Xtest) and Xtest.requires_grad:
-            raise NotImplementedError(
-                "predict_with_grad: the B200 engine does not provide d(mean, std)/d(Xtest); use predict() for values "
-                "(finite differences over predict() cost one batched kernel pass per perturbation)")
         return super().predict(Xtest, return_std=return_std, include_noise=include_noise)
 
     def noise_value(self):

@@ -16,6 +16,7 @@ from typing import List, Optional, Tuple, Union
 
 import numpy as np
 import torch
+from torch.autograd.function import once_differentiable
 
 from .. import _engine, kernels
 from .._compat import (ConstantMean, GaussianLikelihood, GreaterThan, Kernel, LogNormalPrior, Module,
@@ -70,6 +71,35 @@ class _EngineLogProb(torch.autograd.Function):
         g = g.to(torch.float64)
         return (None, (g * gw).to(gw.dtype), (g * gz).to(gz.dtype), (g * gs).to(gs.dtype), (g * gn).to(gn.dtype),
                 (g * gb).to(gb.dtype))
+
+
+class _EnginePrediction(torch.autograd.Function):
+    """Scaled predictive mean and clamped variance at the rows of ``x`` (gpp_predict_grad), differentiable w.r.t. the
+    quantitative columns of ``x``: the graph the reference's ``GPR.predict`` keeps when its inputs require a gradient
+    (models/gpregression.py:122-149, reached through GP_Plus.predict_with_grad, models/gp_plus.py:626-628).
+    Categorical and source columns get a zero gradient (the reference turns them into integer indices), the
+    hyper-parameters none.  First derivatives only: differentiating the backward raises."""
+
+    @staticmethod
+    def forward(ctx, x, eng, xq, cols, kwargs):
+        mean, var, d_mean, d_var = eng.predict_grad(xq, **kwargs)
+        mean, var = torch.from_numpy(np.asarray(mean)), torch.from_numpy(np.asarray(var))
+        ctx.x_meta = (x.shape, x.dtype, x.device)
+        ctx.cols = cols
+        ctx.d_mean = torch.as_tensor(np.asarray(d_mean), dtype=torch.float64).reshape(len(mean), len(cols))
+        # a variance at min_var was clamped there: no gradient, as through torch's clamp_min
+        d_var = torch.as_tensor(np.asarray(d_var), dtype=torch.float64).reshape(len(var), len(cols))
+        ctx.d_var = torch.where((var > kwargs["min_var"])[:, None], d_var, torch.zeros_like(d_var))
+        return mean, var
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_mean, g_var):
+        shape, dtype, device = ctx.x_meta
+        gq = g_mean.double()[:, None] * ctx.d_mean + g_var.double()[:, None] * ctx.d_var
+        gx = torch.zeros(shape, dtype=dtype, device=device)
+        gx[:, ctx.cols] = gq.to(dtype=dtype, device=device)
+        return gx, None, None, None, None
 
 
 class GPR(Module):
@@ -323,7 +353,10 @@ class GPR(Module):
 
     def predict(self, x: torch.Tensor, return_std: bool = False, include_noise: bool = False
                 ) -> Union[torch.Tensor, Tuple[torch.Tensor]]:
-        """Posterior mean (and standard deviation) in the original y units (gpregression.py:122-149)."""
+        """Posterior mean (and standard deviation) in the original y units (gpregression.py:122-149).
+
+        When gradients are enabled and ``x`` requires one, the outputs carry a graph back to the quantitative columns
+        of ``x`` (gpp_predict_grad; the values are bitwise those of the plain call); otherwise they carry none."""
         self.eval()
         with settings.fast_computations(log_prob=False):
             if self.train_targets.ndim != 1:
@@ -341,22 +374,25 @@ class GPR(Module):
             levels = self._level_index(xc, False)
             if levels is not None:
                 self._check_combos_seen(levels)
-            mean_sc, var_sc = eng.predict(
-                np.ascontiguousarray(xq), level_idx=levels,
-                noise_idx=self._noise_index(xc) if add_noise else None, mean_idx=self._mean_index(xc),
-                include_noise=add_noise, min_var=settings.min_variance)
+            kwargs = dict(level_idx=levels, noise_idx=self._noise_index(xc) if add_noise else None,
+                          mean_idx=self._mean_index(xc), include_noise=add_noise, min_var=settings.min_variance)
+            if torch.is_grad_enabled() and x.requires_grad:
+                mean_sc, var_sc = _EnginePrediction.apply(x, eng, np.ascontiguousarray(xq), cols, kwargs)
+            else:
+                mean_sc, var_sc = (torch.from_numpy(a) for a in eng.predict(np.ascontiguousarray(xq), **kwargs))
             dtype = self.y_std.dtype if self.y_std.dtype.is_floating_point else torch.float64
-            out_mean = self.y_min + self.y_std * torch.from_numpy(mean_sc).to(dtype)
+            out_mean = self.y_min + self.y_std * mean_sc.to(dtype)
             if return_std:
-                out_std = torch.from_numpy(var_sc).to(dtype).sqrt() * self.y_std
+                out_std = var_sc.to(dtype).sqrt() * self.y_std
                 return out_mean, out_std
             return out_mean
 
     def posterior(self, X, output_indices=None, observation_noise=True, posterior_transform=None, **kwargs):
-        """Predictive distribution at X in SCALED units (botorch posterior stand-in: mean + marginal variance)."""
+        """Predictive distribution at X in SCALED units (botorch posterior stand-in: mean + marginal variance);
+        differentiable in X when X requires a gradient (GPR.predict, which subclasses' no_grad predict wraps)."""
         self.eval()
         X = X.double()
-        mean, std = self.predict(X, return_std=True, include_noise=bool(observation_noise))
+        mean, std = GPR.predict(self, X, return_std=True, include_noise=bool(observation_noise))
         mu = (mean - self.y_min) / self.y_std
         var = (std / self.y_std) ** 2
         return MultivariateNormal(mu, torch.diag(var))

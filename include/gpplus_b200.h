@@ -9,6 +9,7 @@
  *       (forward:  models/gp_plus.py:386-484, likelihood: likelihoods_noise/multifidelity.py:63-136,
  *        log_prob: optim/mll_scipy.py:37-39, backward: optim/mll_scipy.py:123)
  *   - GPR.predict                 models/gpregression.py:122-149 -> gpp_factorize + gpp_predict
+ *   - GP_Plus.predict_with_grad   models/gp_plus.py:626-628      -> gpp_factorize + gpp_predict_grad
  *   - AF_*_Engineering + argmax   bayesian_optimizations/AFs.py:102-159,
  *                                 bayesian_optimizations/BO_GP_plus.py:183-194 -> gpp_acq_argmax
  *   - covar_module(x).evaluate()  models/gp_plus.py:472-474      -> gpp_covariance
@@ -163,6 +164,14 @@ int gpp_factorize(gpp_handle* h, const gpp_hyper* hyper);
 int gpp_predict(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
                 const int32_t* noise_idx, const int32_t* mean_idx, int include_noise,
                 double min_var, double* mean, double* var);
+
+/* GP_Plus.predict_with_grad (models/gp_plus.py:626-628): gpp_predict plus, per candidate, the derivatives of the
+ * scaled mean and of the clamped variance w.r.t. its quantitative inputs xq; d_mean, d_var are [m*dq] row-major,
+ * either may be NULL.  mean/var are bitwise those of gpp_predict.  Same pointer conventions as gpp_predict.
+ * d_var is 0 where the variance was clamped at min_var; categorical / source inputs have no derivative. */
+int gpp_predict_grad(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
+                     const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, double min_var,
+                     double* mean, double* var, double* d_mean, double* d_var);
 
 /* fused predict + acquisition + argmax over m candidates (BO_GP_plus.py:183-194).
  * y_min/y_std undo the target scaling; cost_idx[m] selects cost[n_cost]; kind_by_cost[n_cost]
