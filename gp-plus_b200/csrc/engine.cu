@@ -17,6 +17,7 @@
 
 #include "chol.cuh"
 #include "cov.cuh"
+#include "joint.cuh"
 #include "objective.h"
 #include "predict.cuh"
 #include "predict_grad.cuh"
@@ -101,6 +102,14 @@ struct gpp_handle {
     long long g_alloc = 0;  // mc_alloc they were sized for
     long long g_step = 0;   // candidates per chunk on that path
     double *g_U = nullptr, *g_part_m = nullptr, *g_part_v = nullptr, *g_dmean = nullptr, *g_dvar = nullptr;
+    // joint-posterior buffers (gpp_predict_joint / gpp_sample_posterior only; allocated on their first call, they only
+    // grow).  Candidate rows are padded to j_mp; the diagonal-block inverses of L* take a full [j_mp x j_mp] matrix
+    // because potrf_blocked addresses them with the leading dimension of Sigma*.
+    long long j_mp = 0;  // candidate rows the buffers below hold
+    long long j_draw_cap = 0;  // doubles in each of the base-sample / draw chunk buffers (j_E, j_Y)
+    double *j_xq = nullptr, *j_xs = nullptr, *j_nrm = nullptr, *j_zpt = nullptr, *j_U = nullptr, *j_S = nullptr;
+    double *j_Minv = nullptr, *j_diag = nullptr, *j_mu = nullptr, *j_logdet = nullptr, *j_E = nullptr, *j_Y = nullptr;
+    int *j_lvl = nullptr, *j_noise = nullptr, *j_info = nullptr;
     double* acq_par = nullptr;  // [cost n_cost | best_f n_cost]
     int* acq_kind = nullptr;
     int acq_cap = 0;
@@ -138,7 +147,7 @@ static const double* hyp_beta(const gpp_handle* h) { return h->hyp + h->dq + zta
 static const double* hyp_sf2(const gpp_handle* h) { return hyp_beta(h) + h->n_mean; }
 static const double* hyp_jitter(const gpp_handle* h) { return hyp_beta(h) + h->n_mean + 1; }
 
-extern "C" int gpp_version(void) { return 107; }
+extern "C" int gpp_version(void) { return 108; }
 
 // process-wide default for handles created afterwards: -1 = by size (INT8-sliced from Np = 4096), 0 = DMMA, 1 = INT8
 static std::atomic<int> g_fp64_mode{-1};
@@ -173,7 +182,8 @@ static void destroy_now(gpp_handle* h) {
     void* dptrs[] = {h->slab, h->c_xq, h->c_xs, h->c_nrm, h->c_zpt, h->c_K, h->c_lvl,
                      h->c_noise, h->c_mean, h->c_cost, h->c_mean_part, h->c_rowsq, h->c_mu, h->c_var, h->c_score,
                      h->c_blk_best, h->c_blk_idx, h->acq_par, h->acq_kind, h->g_U, h->g_part_m, h->g_part_v,
-                     h->g_dmean, h->g_dvar};
+                     h->g_dmean, h->g_dvar, h->j_xq, h->j_xs, h->j_nrm, h->j_zpt, h->j_U, h->j_S, h->j_Minv,
+                     h->j_diag, h->j_mu, h->j_logdet, h->j_E, h->j_Y, h->j_lvl, h->j_noise, h->j_info};
     for (void* p : dptrs)
         if (p) cudaFree(p);
     if (h->pinned_slab) cudaFreeHost(h->pinned_slab);
@@ -263,7 +273,8 @@ extern "C" void gpp_destroy(gpp_handle* h) {
     if (!h) return;
     const char* e = getenv("GPP_POOL");
     const bool pooling = !(e && atoi(e) == 0);
-    if (pooling && h->slab_bytes <= kPoolMaxHandleBytes && h->mc_alloc == 0) {
+    // a handle that has predicted (chunk or joint buffers allocated) is never parked
+    if (pooling && h->slab_bytes <= kPoolMaxHandleBytes && h->mc_alloc == 0 && h->j_mp == 0) {
         cudaSetDevice(h->device);
         if (h->st) cudaStreamSynchronize(h->st);
         std::lock_guard<std::mutex> lk(g_pool_mu);
@@ -1206,10 +1217,17 @@ struct AcqSpec {
     long long best_index = -1;
 };
 
+// gpp_predict_joint: point panels of all m candidates, prepared once (ld mp), and the destination of U = K* L^-T
+struct JointDest {
+    const double *xs, *nrm, *zpt;  // [mp*dqp], [mp], [n_pass][mp*ZP]
+    long long mp;
+    double* U;                     // [mp x Np]
+};
+
 static int predict_impl(gpp_handle* h, long long m, const double* xq, const int32_t* level_idx,
                         const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, double min_var,
                         double* mean, double* var, AcqSpec* acq, bool grad = false, double* d_mean = nullptr,
-                        double* d_var = nullptr) {
+                        double* d_var = nullptr, const JointDest* jd = nullptr) {
     if (!h->factorized) ARG_FAIL("predict: call gpp_factorize (or gpp_mll_grad) first");
     if (m <= 0) return GPP_OK;
     if (h->dq > 0 && !xq) ARG_FAIL("predict: xq missing");
@@ -1245,9 +1263,9 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
         const long long mc = std::min(step, m - base);
         const long long mcp = (mc + 127) / 128 * 128;
         const int tiles_r = (int)(mcp / 128);
-        if (h->dq > 0)
+        if (h->dq > 0 && !jd)
             CK(cudaMemcpyAsync(h->c_xq, xq + base * h->dq, sizeof(double) * mc * h->dq, cudaMemcpyDefault, h->st));
-        if (h->dz > 0)
+        if (h->dz > 0 && !jd)
             CK(cudaMemcpyAsync(h->c_lvl, level_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
         if (noise_idx) CK(cudaMemcpyAsync(h->c_noise, noise_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
         if (mean_idx) CK(cudaMemcpyAsync(h->c_mean, mean_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
@@ -1270,14 +1288,16 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
         pa.xst = nullptr;
         pa.nrm = h->c_nrm;
         pa.zpt = h->c_zpt;
-        prep_points_kernel<<<(int)((mcp + 255) / 256), 256, 0, h->st>>>(pa);
-        CK(cudaGetLastError());
-    count_launch();
+        if (!jd) {
+            prep_points_kernel<<<(int)((mcp + 255) / 256), 256, 0, h->st>>>(pa);
+            CK(cudaGetLastError());
+            count_launch();
+        }
 
         CovArgs ca;
         memset(&ca, 0, sizeof(ca));
-        ca.xs_r = h->c_xs;
-        ca.nrm_r = h->c_nrm;
+        ca.xs_r = jd ? jd->xs + base * h->dqp : h->c_xs;
+        ca.nrm_r = jd ? jd->nrm + base : h->c_nrm;
         ca.xs_c = h->xs;
         ca.nrm_c = h->nrm;
         ca.out = h->c_K;
@@ -1294,7 +1314,7 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
         ca.ld_part = MC;
         ca.scale = 1.0 / (double)h->n_pass;
         for (int p = 0; p < h->n_pass; p++) {
-            ca.zpt_r = h->c_zpt + (size_t)p * mcp * ZP;
+            ca.zpt_r = jd ? jd->zpt + ((size_t)p * jd->mp + base) * ZP : h->c_zpt + (size_t)p * mcp * ZP;
             ca.zpt_c = h->zpt + (size_t)p * h->np * ZP;
             ca.accum = p > 0;
             ca.last = p == h->n_pass - 1;
@@ -1319,6 +1339,11 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
         if (grad) {  // the gradient pass needs U = K* L^-T itself; the row sums come out bitwise the same
             op.epilogue = EPI_STORE_ROWSQ;
             op.C = h->g_U;
+            op.ldc = (int)h->np;
+        }
+        if (jd) {  // the joint covariance keeps U of every candidate (rows base .. base + mcp of jd->U)
+            op.epilogue = EPI_STORE_ROWSQ;
+            op.C = jd->U + base * h->np;
             op.ldc = (int)h->np;
         }
         CK(launch_gemm(op, true, true, 1, h->st));
@@ -1487,6 +1512,286 @@ extern "C" int gpp_acq_argmax(gpp_handle* h, int64_t m, const double* xq, const 
     if (rc != GPP_OK) return rc;
     if (best_score) *best_score = a.best_score;
     if (best_index) *best_index = a.best_index;
+    return GPP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Joint posterior over m candidates: Sigma* = K** - K* K_y^-1 K*^T = K** - U U^T with U = K* L^-T, and draws
+// mu + E L*^T with L* L*^T = Sigma* + jitter I.  Stages (all on h->st, none of them touches A, M, S, alpha or the
+// captured graphs):
+//   J1  panels of all candidates once, then the gpp_predict chunk loop with U stored (mean bitwise gpp_predict's)
+//   J2  K** on the lower tiles (+ noise, + jitter), then Sigma* -= U U^T over K range [0, T)  (one DMMA SYRK)
+//   J3  potrf_blocked(Sigma*) in DMMA arithmetic whatever the handle's FP64 mode, psd_safe_cholesky ladder
+//   J4  per chunk of base samples: Y = mu + E L*^T  (one triangular DMMA GEMM)
+static long long round128(long long x) { return (x + 127) / 128 * 128; }
+
+static int ensure_joint_buffers(gpp_handle* h, long long mp) {
+    if (mp <= h->j_mp) return GPP_OK;
+    void* olds[] = {h->j_xq, h->j_xs, h->j_nrm, h->j_zpt, h->j_U, h->j_S, h->j_Minv, h->j_diag, h->j_mu, h->j_logdet,
+                    h->j_lvl, h->j_noise, h->j_info, h->j_E, h->j_Y};
+    CK(cudaStreamSynchronize(h->st));
+    for (void* p : olds)
+        if (p) cudaFree(p);
+    h->j_xq = h->j_xs = h->j_nrm = h->j_zpt = h->j_U = h->j_S = h->j_Minv = h->j_diag = h->j_mu = h->j_logdet = nullptr;
+    h->j_lvl = h->j_noise = h->j_info = nullptr;
+    h->j_E = h->j_Y = nullptr;  // the draw chunk is reallocated by the next gpp_sample_posterior
+    h->j_draw_cap = 0;
+    h->j_mp = 0;
+    const size_t n = (size_t)mp;
+    CK(dev_alloc(&h->j_xq, n * std::max(h->dq, 1)));
+    CK(dev_alloc(&h->j_xs, n * h->dqp));
+    CK(dev_alloc(&h->j_nrm, n));
+    CK(dev_alloc(&h->j_zpt, n * ZP * h->n_pass));
+    CK(dev_alloc(&h->j_U, n * (size_t)h->np));
+    CK(dev_alloc(&h->j_S, n * n));
+    CK(dev_alloc(&h->j_Minv, n * n));
+    CK(dev_alloc(&h->j_diag, n));
+    CK(dev_alloc(&h->j_mu, n));
+    CK(dev_alloc(&h->j_logdet, n / 128));
+    CK(dev_alloc(&h->j_lvl, n));
+    CK(dev_alloc(&h->j_noise, n));
+    CK(dev_alloc(&h->j_info, 1));
+    CK(cudaMemsetAsync(h->j_mu, 0, sizeof(double) * n, h->st));
+    h->j_mp = mp;
+    return GPP_OK;
+}
+
+// base samples and draws of one chunk, `elems` doubles each (rows x mp of the current call)
+static int ensure_draw_buffers(gpp_handle* h, long long elems) {
+    if (elems <= h->j_draw_cap) return GPP_OK;
+    CK(cudaStreamSynchronize(h->st));
+    if (h->j_E) cudaFree(h->j_E);
+    if (h->j_Y) cudaFree(h->j_Y);
+    h->j_E = h->j_Y = nullptr;
+    h->j_draw_cap = 0;
+    CK(dev_alloc(&h->j_E, (size_t)elems));
+    CK(dev_alloc(&h->j_Y, (size_t)elems));
+    CK(cudaMemsetAsync(h->j_E, 0, sizeof(double) * elems, h->st));
+    h->j_draw_cap = elems;
+    return GPP_OK;
+}
+
+static int joint_check(gpp_handle* h, long long m, const double* xq, const int32_t* level_idx, const char* name) {
+    if (!h) {
+        g_err = std::string(name) + ": null handle";
+        return GPP_ERR_ARG;
+    }
+    if (!h->factorized) {
+        g_err = std::string(name) + ": call gpp_factorize (or gpp_mll_grad) first";
+        return GPP_ERR_ARG;
+    }
+    if (m < 0 || m > GPP_MAX_JOINT) {
+        g_err = std::string(name) + ": m must be in [0, GPP_MAX_JOINT]";
+        return GPP_ERR_ARG;
+    }
+    if (m > 0 && h->dq > 0 && !xq) {
+        g_err = std::string(name) + ": xq missing";
+        return GPP_ERR_ARG;
+    }
+    if (m > 0 && h->dz > 0 && !level_idx) {
+        g_err = std::string(name) + ": level_idx missing";
+        return GPP_ERR_ARG;
+    }
+    return GPP_OK;
+}
+
+// J1: candidate panels, U = K* L^-T of every candidate into j_U, the predictive mean into j_mu
+static int joint_stage_u(gpp_handle* h, long long m, const double* xq, const int32_t* level_idx,
+                         const int32_t* noise_idx, const int32_t* mean_idx, int include_noise) {
+    CK(cudaSetDevice(h->device));
+    const long long mp = round128(m);
+    int rc = ensure_chunk_buffers(h, m);  // before the joint buffers: a handle holding them has mc_alloc > 0
+    if (rc != GPP_OK) return rc;
+    if ((rc = ensure_joint_buffers(h, mp)) != GPP_OK) return rc;
+    if (h->dq > 0) CK(cudaMemcpyAsync(h->j_xq, xq, sizeof(double) * m * h->dq, cudaMemcpyDefault, h->st));
+    if (h->dz > 0) CK(cudaMemcpyAsync(h->j_lvl, level_idx, sizeof(int) * m, cudaMemcpyDefault, h->st));
+    if (include_noise && noise_idx)
+        CK(cudaMemcpyAsync(h->j_noise, noise_idx, sizeof(int) * m, cudaMemcpyDefault, h->st));
+    PrepArgs pa;
+    pa.xq = h->j_xq;
+    pa.level_idx = h->dz > 0 ? h->j_lvl : nullptr;
+    pa.w = hyp_w(h);
+    pa.centre = h->centre;
+    pa.ztab = hyp_z(h);
+    pa.n = (int)m;
+    pa.np = (int)mp;
+    pa.dq = h->dq;
+    pa.dqp = h->dqp;
+    pa.dz = h->dz;
+    pa.n_combo = h->n_combo;
+    pa.n_pass = h->n_pass;
+    pa.xs = h->j_xs;
+    pa.xst = nullptr;
+    pa.nrm = h->j_nrm;
+    pa.zpt = h->j_zpt;
+    prep_points_kernel<<<(int)((mp + 255) / 256), 256, 0, h->st>>>(pa);
+    CK(cudaGetLastError());
+    count_launch();
+    JointDest jd;
+    jd.xs = h->j_xs;
+    jd.nrm = h->j_nrm;
+    jd.zpt = h->j_zpt;
+    jd.mp = mp;
+    jd.U = h->j_U;
+    rc = predict_impl(h, m, xq, level_idx, noise_idx, mean_idx, include_noise, 0.0, h->j_mu, nullptr, nullptr, false,
+                      nullptr, nullptr, &jd);
+    if (rc != GPP_OK) return rc;
+    // Columns n .. Np of U are K* L^-T against the identity padding of K_y, i.e. zero in exact arithmetic; clear them
+    // so that the SYRK, which runs over whole 128-blocks of K, never depends on how L^-1's padding was produced.
+    if (h->np > h->n)
+        CK(cudaMemset2DAsync(h->j_U + h->n, sizeof(double) * h->np, 0, sizeof(double) * (h->np - h->n), (size_t)mp,
+                             h->st));
+    return GPP_OK;
+}
+
+// J2: Sigma* (lower tiles) = K** + diag(noise + jitter) - U U^T into j_S
+static int joint_stage_sigma(gpp_handle* h, long long m, const int32_t* noise_idx, int include_noise, double jitter) {
+    const long long mp = round128(m);
+    const int mt = (int)(mp / 128);
+    joint_diag_kernel<<<(int)((mp + 255) / 256), 256, 0, h->st>>>(noise_idx ? h->j_noise : nullptr, hyp_noise(h),
+                                                                 h->n_noise, include_noise, jitter, (int)m, (int)mp,
+                                                                 h->j_diag);
+    CK(cudaGetLastError());
+    count_launch();
+    CovArgs ca;
+    memset(&ca, 0, sizeof(ca));
+    ca.xs_r = ca.xs_c = h->j_xs;
+    ca.nrm_r = ca.nrm_c = h->j_nrm;
+    ca.out = h->j_S;
+    ca.ld = mp;
+    ca.n_r = ca.n_c = (int)m;
+    ca.tiles_r = ca.tiles_c = mt;
+    ca.tri = 1;
+    ca.same = 1;
+    ca.pad_identity = 1;
+    ca.dqp = h->dqp;
+    ca.dz = h->dz;
+    ca.sf2 = h->sf2;
+    ca.diag_add = h->j_diag;
+    ca.scale = 1.0 / (double)h->n_pass;
+    for (int p = 0; p < h->n_pass; p++) {
+        ca.zpt_r = ca.zpt_c = h->j_zpt + (size_t)p * mp * ZP;
+        ca.accum = p > 0;
+        ca.last = p == h->n_pass - 1;
+        CK(launch_cov(ca, h->kernel, h->st));
+    }
+    GemmOp op = gemm_default();  // Sigma* -= U U^T on the lower tiles (the trailing_update op shape)
+    op.A = h->j_U;
+    op.lda = (int)h->np;
+    op.B = h->j_U;
+    op.ldb = (int)h->np;
+    op.C = h->j_S;
+    op.ldc = (int)mp;
+    op.map = MAP_TRI;
+    op.tiles_m = op.tiles_m_last = mt;
+    op.tiles_n = mt;
+    op.klo_c = 0;
+    op.khi_c = h->T;
+    op.alpha = -1.0;
+    op.beta = 1.0;
+    CK(launch_gemm(op, true, true, 1, h->st));
+    return GPP_OK;
+}
+
+extern "C" int gpp_predict_joint(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
+                                 const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, double* mean,
+                                 double* cov) {
+    int rc = joint_check(h, m, xq, level_idx, "gpp_predict_joint");
+    if (rc != GPP_OK || m == 0) return rc;
+    if ((rc = joint_stage_u(h, m, xq, level_idx, noise_idx, mean_idx, include_noise)) != GPP_OK) return rc;
+    if ((rc = joint_stage_sigma(h, m, noise_idx, include_noise, 0.0)) != GPP_OK) return rc;
+    const long long mp = round128(m);
+    const int nb = (int)(mp / 32);
+    mirror_lower_kernel<<<dim3(nb, nb), dim3(32, 8), 0, h->st>>>(h->j_S, mp);
+    CK(cudaGetLastError());
+    count_launch();
+    if (mean) CK(cudaMemcpyAsync(mean, h->j_mu, sizeof(double) * m, cudaMemcpyDefault, h->st));
+    if (cov)
+        CK(cudaMemcpy2DAsync(cov, sizeof(double) * m, h->j_S, sizeof(double) * mp, sizeof(double) * m, (size_t)m,
+                             cudaMemcpyDefault, h->st));
+    CK(cudaStreamSynchronize(h->st));
+    return GPP_OK;
+}
+
+extern "C" int gpp_sample_posterior(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
+                                    const int32_t* noise_idx, const int32_t* mean_idx, int include_noise,
+                                    int64_t n_samples, const double* base_samples, double* samples, double* jitter) {
+    int rc = joint_check(h, m, xq, level_idx, "gpp_sample_posterior");
+    if (rc != GPP_OK) return rc;
+    if (n_samples < 0) ARG_FAIL("gpp_sample_posterior: n_samples must be >= 0");
+    if (m > 0 && n_samples > 0 && (!base_samples || !samples)) ARG_FAIL("gpp_sample_posterior: samples missing");
+    if (m == 0) {
+        if (jitter) *jitter = 0.0;
+        return GPP_OK;
+    }
+    if ((rc = joint_stage_u(h, m, xq, level_idx, noise_idx, mean_idx, include_noise)) != GPP_OK) return rc;
+    const long long mp = round128(m);
+    const int mt = (int)(mp / 128);
+    // The leaf writes only the lower 32 x 32 sub-blocks of each diagonal block of L*^-1, and the TRSM reads the whole
+    // block, so the [mp x mp] matrix potrf_blocked addresses must start at zero.  A previous call with a larger mp
+    // left inverse entries there at another leading dimension: clear it on every call.
+    CK(cudaMemsetAsync(h->j_Minv, 0, sizeof(double) * mp * mp, h->st));
+    int a = 0;
+    for (;; a++) {
+        if (a == 4) {
+            g_err = "gpp_sample_posterior: the joint posterior covariance is not positive definite after adding "
+                    "jitter up to 1e-6";
+            return GPP_ERR_NOT_PD;
+        }
+        if ((rc = joint_stage_sigma(h, m, noise_idx, include_noise, kJitter[a])) != GPP_OK) return rc;
+        CK(cudaMemsetAsync(h->j_info, 0, sizeof(int), h->st));
+        CK(potrf_blocked(h->j_S, h->j_Minv, (int)mp, mt, h->j_logdet, h->j_info, h->st));
+        int info = 0;
+        CK(cudaMemcpyAsync(&info, h->j_info, sizeof(int), cudaMemcpyDeviceToHost, h->st));
+        CK(cudaStreamSynchronize(h->st));
+        if (info & 2) {
+            g_err = "gpp_sample_posterior: NaN encountered while factorising the joint posterior covariance";
+            return GPP_ERR_NAN;
+        }
+        if (info == 0) break;
+    }
+    if (jitter) *jitter = kJitter[a];
+    zero_diag_upper_kernel<<<mt, 256, 0, h->st>>>(h->j_S, mp);
+    CK(cudaGetLastError());
+    count_launch();
+    if (n_samples == 0) {
+        CK(cudaStreamSynchronize(h->st));
+        return GPP_OK;
+    }
+    long long cap = ((1LL << 27) / mp) / 128 * 128;
+    if (cap < 128) cap = 128;
+    const long long sc = std::min(round128(n_samples), cap);
+    if ((rc = ensure_draw_buffers(h, sc * mp)) != GPP_OK) return rc;
+    for (long long s0 = 0; s0 < n_samples; s0 += sc) {
+        const long long rows = std::min(sc, n_samples - s0);
+        const long long rp = round128(rows);
+        CK(cudaMemcpy2DAsync(h->j_E, sizeof(double) * mp, base_samples + s0 * m, sizeof(double) * m,
+                             sizeof(double) * m, (size_t)rows, cudaMemcpyDefault, h->st));
+        if (mp > m)  // padding columns of E meet only zeros of L*, but must not be stale non-finite values
+            CK(cudaMemset2DAsync(h->j_E + m, sizeof(double) * mp, 0, sizeof(double) * (mp - m), (size_t)rp, h->st));
+        const long long total = rp * mp;
+        fill_rows_kernel<<<(int)std::min<long long>((total + 255) / 256, 4096), 256, 0, h->st>>>(h->j_Y, h->j_mu, mp,
+                                                                                                total);
+        CK(cudaGetLastError());
+        count_launch();
+        GemmOp op = gemm_default();  // Y += E L*^T: B(tj, kb) = L*[tj, kb], kb in [0, tj]
+        op.A = h->j_E;
+        op.lda = (int)mp;
+        op.B = h->j_S;
+        op.ldb = (int)mp;
+        op.C = h->j_Y;
+        op.ldc = (int)mp;
+        op.tiles_m = op.tiles_m_last = (int)(rp / 128);
+        op.tiles_n = mt;
+        op.klo_c = 0;
+        op.khi_sel = KSEL_TJ;
+        op.khi_c = 1;
+        op.beta = 1.0;
+        CK(launch_gemm(op, true, true, 1, h->st));
+        CK(cudaMemcpy2DAsync(samples + s0 * m, sizeof(double) * m, h->j_Y, sizeof(double) * mp, sizeof(double) * m,
+                             (size_t)rows, cudaMemcpyDefault, h->st));
+    }
+    CK(cudaStreamSynchronize(h->st));
     return GPP_OK;
 }
 

@@ -26,6 +26,10 @@ NotPSDError = _engine.NotPSDError
 NanError = _engine.NanError
 
 
+class NumericalWarning(RuntimeWarning):
+    """gpytorch.utils.warnings.NumericalWarning: jitter was added to make a covariance positive definite."""
+
+
 class _Flag:
     """Context manager stand-in for gpytorch.settings.fast_computations: the engine always uses the
     exact Cholesky path, so the flag is accepted and ignored."""

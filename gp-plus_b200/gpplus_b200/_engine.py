@@ -16,6 +16,7 @@ GPP_OK, GPP_ERR_NOT_PD, GPP_ERR_NAN, GPP_ERR_ARG, GPP_ERR_CUDA = 0, 1, 2, 3, -1
 KERNEL_EXPSQ, KERNEL_MATERN32, KERNEL_MATERN52 = 0, 1, 2
 ACQ_HF, ACQ_LF, ACQ_EI = 0, 1, 2
 MAX_DQ, MAX_DZ = 32, 4
+MAX_JOINT = 16384  # GPP_MAX_JOINT: candidates of one gpp_predict_joint / gpp_sample_posterior call
 
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libgpplus_b200.so")
 
@@ -23,7 +24,7 @@ EXPORTS = (
     "gpp_version", "gpp_device_count", "gpp_last_error", "gpp_launch_count", "gpp_create", "gpp_destroy", "gpp_pool_clear",
     "gpp_mll_grad",
     "gpp_get_timings", "gpp_get_stats", "gpp_covariance", "gpp_fetch", "gpp_factorize", "gpp_predict", "gpp_predict_grad",
-    "gpp_acq_argmax",
+    "gpp_predict_joint", "gpp_sample_posterior", "gpp_acq_argmax",
     "gpp_probe_dgemm", "gpp_probe_i8", "gpp_set_fp64_mode", "gpp_get_fp64_mode", "gpp_set_theta_layout", "gpp_objective", "gpp_objective_enqueue", "gpp_objective_collect",
 )
 
@@ -127,6 +128,12 @@ def load_library():
         lib.gpp_predict_grad.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                          C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.gpp_predict_grad.restype = C.c_int
+        lib.gpp_predict_joint.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_int, C.c_void_p, C.c_void_p]
+        lib.gpp_predict_joint.restype = C.c_int
+        lib.gpp_sample_posterior.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.POINTER(C.c_double)]
+        lib.gpp_sample_posterior.restype = C.c_int
         lib.gpp_acq_argmax.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_double,
                                        C.c_double, C.c_double, C.c_double, C.c_void_p, _dp, C.POINTER(C.c_int64)]
@@ -452,6 +459,47 @@ class Engine:
         if rc != GPP_OK:
             _raise(rc, "gpp_predict_grad")
         return mean, var, d_mean, d_var
+
+    def _candidates(self, xq, level_idx, noise_idx, mean_idx):
+        if isinstance(xq, np.ndarray) or not hasattr(xq, "data_ptr"):
+            xq = _f64(xq)
+            m = xq.shape[0] if xq.ndim == 2 else (xq.size // max(self.dq, 1))
+            return xq, m, _i32(level_idx, m), _i32(noise_idx, m), _i32(mean_idx, m)
+        return xq, int(xq.shape[0]), level_idx, noise_idx, mean_idx
+
+    def predict_joint(self, xq, level_idx=None, noise_idx=None, mean_idx=None, include_noise: bool = False,
+                      out_mean=None, out_cov=None):
+        """Predictive mean [m] (bitwise ``predict``'s) and the full, unclamped predictive covariance [m, m] in scaled y
+        units (gpp_predict_joint).  Inputs and output buffers as for ``predict``; m <= MAX_JOINT."""
+        xq, m, level_idx, noise_idx, mean_idx = self._candidates(xq, level_idx, noise_idx, mean_idx)
+        mean = np.empty(m) if out_mean is None else out_mean
+        cov = np.empty((m, m)) if out_cov is None else out_cov
+        rc = self._lib.gpp_predict_joint(self._h, m, _ptr(xq), _ptr(level_idx), _ptr(noise_idx), _ptr(mean_idx),
+                                         1 if include_noise else 0, _ptr(mean), _ptr(cov))
+        if rc != GPP_OK:
+            _raise(rc, "gpp_predict_joint")
+        return mean, cov
+
+    def sample_posterior(self, xq, base_samples, level_idx=None, noise_idx=None, mean_idx=None,
+                         include_noise: bool = False, out=None):
+        """Draws ``mean + base_samples L^T`` from the joint posterior with ``L L^T = cov + jitter I``
+        (gpp_sample_posterior): returns ``(samples [S, m], jitter)``.  ``base_samples`` [S, m] may live on the host or
+        on this engine's GPU, like the other inputs."""
+        xq, m, level_idx, noise_idx, mean_idx = self._candidates(xq, level_idx, noise_idx, mean_idx)
+        if isinstance(base_samples, np.ndarray) or not hasattr(base_samples, "data_ptr"):
+            base_samples = _f64(base_samples)
+        if len(base_samples.shape) != 2 or int(base_samples.shape[1]) != m:
+            raise ValueError("sample_posterior: base_samples must have shape [S, %d], got %s"
+                             % (m, tuple(base_samples.shape)))
+        s = int(base_samples.shape[0])
+        samples = np.empty((s, m)) if out is None else out
+        jit = C.c_double(0.0)
+        rc = self._lib.gpp_sample_posterior(self._h, m, _ptr(xq), _ptr(level_idx), _ptr(noise_idx), _ptr(mean_idx),
+                                            1 if include_noise else 0, s, _ptr(base_samples), _ptr(samples),
+                                            C.byref(jit))
+        if rc != GPP_OK:
+            _raise(rc, "gpp_sample_posterior")
+        return samples, float(jit.value)
 
     def acq_argmax(self, xq, cost_idx, cost: Sequence[float], kind_by_cost: Sequence[int], best_f: Sequence[float],
                    level_idx=None, mean_idx=None, maximize: bool = True, si: float = 0.0, y_min: float = 0.0,

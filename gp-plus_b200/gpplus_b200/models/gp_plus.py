@@ -465,6 +465,19 @@ class GP_Plus(GPR):
         Xtest = data_type_check(Xtest)
         return super().predict(Xtest, return_std=return_std, include_noise=include_noise)
 
+    def predict_joint(self, Xtest, include_noise=False):
+        """Posterior mean [M] and full covariance [M, M] at ``Xtest`` in the original y units (GPR.predict_joint)."""
+        Xtest = data_type_check(Xtest)
+        with torch.no_grad():
+            return super().predict_joint(Xtest, include_noise=include_noise)
+
+    def sample_posterior(self, Xtest, num_samples=1, include_noise=False, base_samples=None, generator=None):
+        """``num_samples`` joint posterior draws [S, M] at ``Xtest`` in the original y units (GPR.sample_posterior)."""
+        Xtest = data_type_check(Xtest)
+        with torch.no_grad():
+            return super().sample_posterior(Xtest, num_samples=num_samples, include_noise=include_noise,
+                                            base_samples=base_samples, generator=generator)
+
     def noise_value(self):
         return self.likelihood.noise_covar.noise.detach() * self.y_std ** 2
 

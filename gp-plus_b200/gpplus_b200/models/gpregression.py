@@ -12,6 +12,7 @@ import contextlib
 
 import math
 import threading
+import warnings
 from typing import List, Optional, Tuple, Union
 
 import numpy as np
@@ -20,7 +21,7 @@ from torch.autograd.function import once_differentiable
 
 from .. import _engine, kernels
 from .._compat import (ConstantMean, GaussianLikelihood, GreaterThan, Kernel, LogNormalPrior, Module,
-                       MultivariateNormal, Positive, ZeroMean, settings)
+                       MultivariateNormal, NumericalWarning, Positive, ZeroMean, settings)
 from ..likelihoods_noise.multifidelity import Multifidelity_likelihood
 from ..priors import LogHalfHorseshoePrior, MollifiedUniformPrior
 from ..utils.transforms import inv_softplus, softplus
@@ -386,6 +387,65 @@ class GPR(Module):
                 out_std = var_sc.to(dtype).sqrt() * self.y_std
                 return out_mean, out_std
             return out_mean
+
+    def _joint_request(self, x: torch.Tensor, include_noise: bool):
+        """Engine (factorised for the current hyper-parameters), quantitative inputs and index arguments of a joint
+        posterior call at the rows of ``x``: levels, noise groups and means exactly as ``predict`` gathers them."""
+        self.eval()
+        if self.train_targets.ndim != 1:
+            raise NotImplementedError("batched GPs are not supported by the engine")
+        if x.dim() != 2:
+            raise ValueError("expected a 2-D tensor of inputs")
+        eng = self._ensure_factor()
+        xc = x.detach().cpu()
+        cols = self._quant_columns()
+        xq = xc[:, cols].double().numpy() if len(cols) > 0 else np.zeros((xc.shape[0], 0))
+        levels = self._level_index(xc, False)
+        if levels is not None:
+            self._check_combos_seen(levels)
+        kwargs = dict(level_idx=levels, noise_idx=self._noise_index(xc) if include_noise else None,
+                      mean_idx=self._mean_index(xc), include_noise=bool(include_noise))
+        return eng, np.ascontiguousarray(xq), kwargs
+
+    def _out_dtype(self):
+        return self.y_std.dtype if self.y_std.dtype.is_floating_point else torch.float64
+
+    def predict_joint(self, x: torch.Tensor, include_noise: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Posterior mean [M] and full covariance [M, M] at the rows of ``x`` in the original y units: the joint
+        structure that the reference's ``posterior`` carries (gpregression.py:151-166).  The mean equals ``predict``'s;
+        the covariance is exactly symmetric and not clamped.  ``include_noise`` adds each row's observation noise on
+        the diagonal.  No autograd graph; M is at most ``_engine.MAX_JOINT``."""
+        with torch.no_grad():
+            eng, xq, kwargs = self._joint_request(x, include_noise)
+            mean_sc, cov_sc = eng.predict_joint(xq, **kwargs)
+            dtype = self._out_dtype()
+            mean = self.y_min + self.y_std * torch.as_tensor(np.asarray(mean_sc)).to(dtype)
+            cov = (self.y_std * self.y_std) * torch.as_tensor(np.asarray(cov_sc)).to(dtype)
+        return mean, cov
+
+    def sample_posterior(self, x: torch.Tensor, num_samples: int = 1, include_noise: bool = False,
+                         base_samples: Optional[torch.Tensor] = None, generator: Optional[torch.Generator] = None
+                         ) -> torch.Tensor:
+        """``num_samples`` draws [S, M] from the joint posterior at the rows of ``x``, in the original y units
+        (gpytorch ``MultivariateNormal.rsample``): ``mean + base_samples L^T`` with ``L`` the Cholesky factor of the
+        posterior covariance.  The default base samples are ``torch.randn(S, M, generator=generator)`` in float64 on
+        the CPU, as gpytorch draws them; a singular covariance gets the psd_safe_cholesky jitter and a warning."""
+        with torch.no_grad():
+            eng, xq, kwargs = self._joint_request(x, include_noise)
+            m = xq.shape[0]
+            if base_samples is None:
+                base_samples = torch.randn(int(num_samples), m, generator=generator, dtype=torch.float64)
+            else:
+                base_samples = torch.as_tensor(base_samples)
+            if tuple(base_samples.shape) != (int(num_samples), m):
+                raise ValueError("base_samples must have shape %s, got %s"
+                                 % ((int(num_samples), m), tuple(base_samples.shape)))
+            base = np.ascontiguousarray(base_samples.detach().to(device="cpu", dtype=torch.float64).numpy())
+            samples_sc, jitter = eng.sample_posterior(xq, base, **kwargs)
+            if jitter > 0:
+                warnings.warn("A not p.d., added jitter of %.1e to the diagonal" % jitter, NumericalWarning)
+            dtype = self._out_dtype()
+            return self.y_min + self.y_std * torch.as_tensor(np.asarray(samples_sc)).to(dtype)
 
     def posterior(self, X, output_indices=None, observation_noise=True, posterior_transform=None, **kwargs):
         """Predictive distribution at X in SCALED units (botorch posterior stand-in: mean + marginal variance);

@@ -10,6 +10,8 @@
  *        log_prob: optim/mll_scipy.py:37-39, backward: optim/mll_scipy.py:123)
  *   - GPR.predict                 models/gpregression.py:122-149 -> gpp_factorize + gpp_predict
  *   - GP_Plus.predict_with_grad   models/gp_plus.py:626-628      -> gpp_factorize + gpp_predict_grad
+ *   - GPR.posterior (joint), MultivariateNormal.rsample
+ *                                 models/gpregression.py:151-166 -> gpp_predict_joint, gpp_sample_posterior
  *   - AF_*_Engineering + argmax   bayesian_optimizations/AFs.py:102-159,
  *                                 bayesian_optimizations/BO_GP_plus.py:183-194 -> gpp_acq_argmax
  *   - covar_module(x).evaluate()  models/gp_plus.py:472-474      -> gpp_covariance
@@ -172,6 +174,31 @@ int gpp_predict(gpp_handle* h, int64_t m, const double* xq, const int32_t* level
 int gpp_predict_grad(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
                      const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, double min_var,
                      double* mean, double* var, double* d_mean, double* d_var);
+
+/* Joint posterior over m <= GPP_MAX_JOINT candidates: the full predictive covariance
+ *   Sigma* = K** - K* K_y^-1 K*^T  (+ noise of each candidate's group on the diagonal when include_noise)
+ * and draws from N(mean, Sigma*).  Replace GPR.posterior's joint GPyTorchPosterior (gpregression.py:151-166) and
+ * the MultivariateNormal.rsample of gpytorch that its fantasize / samplers call (gpregression.py:177-221).
+ * Same pointer conventions as gpp_predict (host or device, cudaMemcpyDefault).  Neither call changes the factor of
+ * K_y, alpha, gpp_get_stats or gpp_get_timings: gpp_predict / gpp_fetch return bitwise the same afterwards.  The
+ * candidate buffers (about 6 GiB at m = N = 16384) are allocated on the first call and freed with the handle;
+ * gpp_sample_posterior adds one chunk of base samples and one of draws, min(n_samples, 2^27/m) rows each (up to
+ * 2 x 1 GiB), so up to about 8 GiB at m = N = 16384.  m > GPP_MAX_JOINT returns GPP_ERR_ARG before any
+ * allocation. */
+#define GPP_MAX_JOINT 16384
+
+/* mean[m] (bitwise gpp_predict's), cov[m*m] row-major, exactly symmetric, scaled y units, NOT clamped.
+ * Either output may be NULL. */
+int gpp_predict_joint(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
+                      const int32_t* noise_idx, const int32_t* mean_idx, int include_noise,
+                      double* mean, double* cov);
+
+/* samples[s*m+i] = mean_i + sum_j L[i,j] base_samples[s*m+j],  L L^T = cov + jitter*I (psd_safe_cholesky ladder:
+ * jitter 0, 1e-8, 1e-7, 1e-6; the one that succeeded is written to *jitter, GPP_ERR_NOT_PD when none does).
+ * base_samples and samples are [n_samples*m] row-major; with base_samples = I_m the draws are mean + L^T rows. */
+int gpp_sample_posterior(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
+                         const int32_t* noise_idx, const int32_t* mean_idx, int include_noise,
+                         int64_t n_samples, const double* base_samples, double* samples, double* jitter);
 
 /* fused predict + acquisition + argmax over m candidates (BO_GP_plus.py:183-194).
  * y_min/y_std undo the target scaling; cost_idx[m] selects cost[n_cost]; kind_by_cost[n_cost]
