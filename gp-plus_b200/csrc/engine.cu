@@ -21,6 +21,7 @@
 #include "objective.h"
 #include "predict.cuh"
 #include "predict_grad.cuh"
+#include "qbatch.cuh"
 #include "solve.cuh"
 
 using namespace gpp;
@@ -110,6 +111,11 @@ struct gpp_handle {
     double *j_xq = nullptr, *j_xs = nullptr, *j_nrm = nullptr, *j_zpt = nullptr, *j_U = nullptr, *j_S = nullptr;
     double *j_Minv = nullptr, *j_diag = nullptr, *j_mu = nullptr, *j_logdet = nullptr, *j_E = nullptr, *j_Y = nullptr;
     int *j_lvl = nullptr, *j_noise = nullptr, *j_info = nullptr;
+    // t-batch posterior buffers (gpp_posterior_qbatch[_grad] only; allocated on their first call): one chunk's q x q
+    // blocks (Sigma out, or the upstream gradient G in) and its upstream mean gradient in the tile layout
+    long long q_rows = 0;  // g_step they were sized for
+    long long q_cap = 0;   // doubles in q_buf
+    double *q_buf = nullptr, *q_gm = nullptr;
     double* acq_par = nullptr;  // [cost n_cost | best_f n_cost]
     int* acq_kind = nullptr;
     int acq_cap = 0;
@@ -147,7 +153,7 @@ static const double* hyp_beta(const gpp_handle* h) { return h->hyp + h->dq + zta
 static const double* hyp_sf2(const gpp_handle* h) { return hyp_beta(h) + h->n_mean; }
 static const double* hyp_jitter(const gpp_handle* h) { return hyp_beta(h) + h->n_mean + 1; }
 
-extern "C" int gpp_version(void) { return 108; }
+extern "C" int gpp_version(void) { return 109; }
 
 // process-wide default for handles created afterwards: -1 = by size (INT8-sliced from Np = 4096), 0 = DMMA, 1 = INT8
 static std::atomic<int> g_fp64_mode{-1};
@@ -183,7 +189,8 @@ static void destroy_now(gpp_handle* h) {
                      h->c_noise, h->c_mean, h->c_cost, h->c_mean_part, h->c_rowsq, h->c_mu, h->c_var, h->c_score,
                      h->c_blk_best, h->c_blk_idx, h->acq_par, h->acq_kind, h->g_U, h->g_part_m, h->g_part_v,
                      h->g_dmean, h->g_dvar, h->j_xq, h->j_xs, h->j_nrm, h->j_zpt, h->j_U, h->j_S, h->j_Minv,
-                     h->j_diag, h->j_mu, h->j_logdet, h->j_E, h->j_Y, h->j_lvl, h->j_noise, h->j_info};
+                     h->j_diag, h->j_mu, h->j_logdet, h->j_E, h->j_Y, h->j_lvl, h->j_noise, h->j_info,
+                     h->q_buf, h->q_gm};
     for (void* p : dptrs)
         if (p) cudaFree(p);
     if (h->pinned_slab) cudaFreeHost(h->pinned_slab);
@@ -1224,10 +1231,55 @@ struct JointDest {
     double* U;                     // [mp x Np]
 };
 
+// gpp_posterior_qbatch[_grad]: b t-batches of q rows.  Every 128-row tile of the chunk buffers holds qpt = 128 / q whole
+// t-batches followed by padding rows, so chunks (multiples of 128 rows) hold whole t-batches.
+struct QBatchSpec {
+    long long b;
+    int q, qpt;
+    double* cov;           // forward: [b*q*q] or NULL
+    const double* g_mean;  // backward: [b*q] or NULL
+    const double* g_cov;   // backward: [b*q*q] or NULL
+    double* d_xq;          // backward: [b*q*dq]
+};
+
+// rows of nbat t-batches, from t-batch bt0 of a compact [b*q rows] array, to (into_tiles) or from their tile slots in
+// a chunk buffer: one pitched copy for the full tiles, one plain copy for the last, partly filled one
+static cudaError_t qb_copy_rows(const QBatchSpec* qb, void* dst, const void* src, size_t row_bytes, long long bt0,
+                                long long nbat, bool into_tiles, cudaStream_t st) {
+    if (row_bytes == 0 || nbat <= 0) return cudaSuccess;
+    const size_t run = (size_t)qb->qpt * qb->q * row_bytes, tile = (size_t)CT * row_bytes;
+    const size_t off = (size_t)bt0 * qb->q * row_bytes;
+    char* d = (char*)dst + (into_tiles ? 0 : off);
+    const char* s = (const char*)src + (into_tiles ? off : 0);
+    const size_t dp = into_tiles ? tile : run, sp = into_tiles ? run : tile;
+    const long long full = nbat / qb->qpt, rest = nbat % qb->qpt;
+    if (full > 0) {
+        cudaError_t e = cudaMemcpy2DAsync(d, dp, s, sp, run, (size_t)full, cudaMemcpyDefault, st);
+        if (e != cudaSuccess) return e;
+    }
+    if (rest > 0)
+        return cudaMemcpyAsync(d + full * dp, s + full * sp, (size_t)rest * qb->q * row_bytes, cudaMemcpyDefault, st);
+    return cudaSuccess;
+}
+
+static int ensure_qbatch_buffers(gpp_handle* h, int q) {
+    const long long cap = h->g_step * q;
+    if (h->q_rows == h->g_step && cap <= h->q_cap) return GPP_OK;
+    if (h->q_buf) cudaFree(h->q_buf);
+    if (h->q_gm) cudaFree(h->q_gm);
+    h->q_buf = h->q_gm = nullptr;
+    h->q_rows = h->q_cap = 0;
+    CK(dev_alloc(&h->q_buf, (size_t)cap));
+    CK(dev_alloc(&h->q_gm, (size_t)h->g_step));
+    h->q_rows = h->g_step;
+    h->q_cap = cap;
+    return GPP_OK;
+}
+
 static int predict_impl(gpp_handle* h, long long m, const double* xq, const int32_t* level_idx,
                         const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, double min_var,
                         double* mean, double* var, AcqSpec* acq, bool grad = false, double* d_mean = nullptr,
-                        double* d_var = nullptr, const JointDest* jd = nullptr) {
+                        double* d_var = nullptr, const JointDest* jd = nullptr, const QBatchSpec* qb = nullptr) {
     if (!h->factorized) ARG_FAIL("predict: call gpp_factorize (or gpp_mll_grad) first");
     if (m <= 0) return GPP_OK;
     if (h->dq > 0 && !xq) ARG_FAIL("predict: xq missing");
@@ -1235,10 +1287,12 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
     CK(cudaSetDevice(h->device));
     int rc = ensure_chunk_buffers(h, m);
     if (rc != GPP_OK) return rc;
-    if (grad) {
+    const bool keep_u = grad || qb;  // U = K* L^-T stored per chunk, in chunks of the gradient path
+    if (keep_u) {
         rc = ensure_grad_buffers(h);
         if (rc != GPP_OK) return rc;
     }
+    if (qb && (rc = ensure_qbatch_buffers(h, qb->q)) != GPP_OK) return rc;
     if (acq) {
         if (acq->n_cost <= 0 || !acq->cost || !acq->kind_by_cost || !acq->best_f) ARG_FAIL("acq: cost tables missing");
         if (acq->n_cost > h->acq_cap) {
@@ -1258,17 +1312,32 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
     std::vector<double> hb;
     std::vector<long long> hi;
     const long long MC = h->mc_alloc;  // leading dimension of the chunk buffers
-    const long long step = grad ? h->g_step : MC;
+    const long long step = keep_u ? h->g_step : MC;
     for (long long base = 0; base < m; base += step) {
         const long long mc = std::min(step, m - base);
         const long long mcp = (mc + 127) / 128 * 128;
         const int tiles_r = (int)(mcp / 128);
-        if (h->dq > 0 && !jd)
-            CK(cudaMemcpyAsync(h->c_xq, xq + base * h->dq, sizeof(double) * mc * h->dq, cudaMemcpyDefault, h->st));
-        if (h->dz > 0 && !jd)
-            CK(cudaMemcpyAsync(h->c_lvl, level_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
-        if (noise_idx) CK(cudaMemcpyAsync(h->c_noise, noise_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
-        if (mean_idx) CK(cudaMemcpyAsync(h->c_mean, mean_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
+        // t-batches of this chunk (t-batch path): [bt0, bt0 + nbc)
+        const long long bt0 = qb ? base / CT * qb->qpt : 0;
+        const long long nbc = qb ? std::min(qb->b, bt0 + (long long)tiles_r * qb->qpt) - bt0 : 0;
+        if (qb) {  // scatter the rows into their tile slots; padding rows are zero points of level, group and mean 0
+            CK(cudaMemsetAsync(h->c_xq, 0, sizeof(double) * mcp * h->dq, h->st));
+            CK(cudaMemsetAsync(h->c_lvl, 0, sizeof(int) * mcp, h->st));
+            CK(cudaMemsetAsync(h->c_noise, 0, sizeof(int) * mcp, h->st));
+            CK(cudaMemsetAsync(h->c_mean, 0, sizeof(int) * mcp, h->st));
+            CK(qb_copy_rows(qb, h->c_xq, xq, sizeof(double) * h->dq, bt0, nbc, true, h->st));
+            if (h->dz > 0) CK(qb_copy_rows(qb, h->c_lvl, level_idx, sizeof(int), bt0, nbc, true, h->st));
+            if (noise_idx) CK(qb_copy_rows(qb, h->c_noise, noise_idx, sizeof(int), bt0, nbc, true, h->st));
+            if (mean_idx) CK(qb_copy_rows(qb, h->c_mean, mean_idx, sizeof(int), bt0, nbc, true, h->st));
+        } else {
+            if (h->dq > 0 && !jd)
+                CK(cudaMemcpyAsync(h->c_xq, xq + base * h->dq, sizeof(double) * mc * h->dq, cudaMemcpyDefault, h->st));
+            if (h->dz > 0 && !jd)
+                CK(cudaMemcpyAsync(h->c_lvl, level_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
+            if (noise_idx)
+                CK(cudaMemcpyAsync(h->c_noise, noise_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
+            if (mean_idx) CK(cudaMemcpyAsync(h->c_mean, mean_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
+        }
         if (acq && acq->cost_idx)
             CK(cudaMemcpyAsync(h->c_cost, acq->cost_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
         PrepArgs pa;
@@ -1336,7 +1405,7 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
         op.epilogue = EPI_ROWSQ;
         op.rowsq = h->c_rowsq;
         op.rowsq_ld = (int)MC;
-        if (grad) {  // the gradient pass needs U = K* L^-T itself; the row sums come out bitwise the same
+        if (keep_u) {  // the gradient and t-batch passes need U = K* L^-T itself; the row sums come out bitwise the same
             op.epilogue = EPI_STORE_ROWSQ;
             op.C = h->g_U;
             op.ldc = (int)h->np;
@@ -1385,6 +1454,35 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
         predict_finish_kernel<<<nblk, 256, 0, h->st>>>(fa);
         CK(cudaGetLastError());
     count_launch();
+        if (qb && !grad && qb->cov) {  // Sigma_t = K**_t - U_t U_t^T of the chunk's t-batches into q_buf
+            QSyrkArgs sa;
+            memset(&sa, 0, sizeof(sa));
+            sa.U = h->g_U;
+            sa.ldu = h->np;
+            sa.kcols = (int)h->n;
+            sa.rowsq = h->c_rowsq;
+            sa.ldr = MC;
+            sa.tiles_c = h->T;
+            sa.xs = h->c_xs;
+            sa.zpt = h->c_zpt;
+            sa.zs = mcp * ZP;
+            sa.dq = h->dq;
+            sa.dqp = h->dqp;
+            sa.dz = h->dz;
+            sa.n_pass = h->n_pass;
+            sa.sf2 = h->sf2;
+            sa.noise_idx = noise_idx ? h->c_noise : nullptr;
+            sa.noise = hyp_noise(h);
+            sa.n_noise = h->n_noise;
+            sa.include_noise = include_noise;
+            sa.q = qb->q;
+            sa.qpt = qb->qpt;
+            sa.nb = nbc;
+            sa.cov = h->q_buf;
+            CK(launch_qbatch_syrk(sa, h->kernel, tiles_r, h->st));
+            const size_t qq = (size_t)qb->q * qb->q;
+            CK(cudaMemcpyAsync(qb->cov + bt0 * qq, h->q_buf, sizeof(double) * nbc * qq, cudaMemcpyDefault, h->st));
+        }
         if (grad) {
             // V = U L^-1 = K* K_y^-1 over the K* chunk, which is not read again: B(tj, k) = L^-1[k, tj], k in [tj, T)
             GemmOp vo = gemm_default();
@@ -1400,6 +1498,30 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             vo.klo_c = 0;
             vo.khi_c = h->T;
             CK(launch_gemm(vo, true, false, 1, h->st));
+            if (qb) {  // W = blockdiag(G + G^T) V into g_U (U is not read again), the upstream mean gradient into q_gm
+                const size_t qq = (size_t)qb->q * qb->q;
+                if (qb->g_cov)
+                    CK(cudaMemcpyAsync(h->q_buf, qb->g_cov + bt0 * qq, sizeof(double) * nbc * qq, cudaMemcpyDefault,
+                                       h->st));
+                else
+                    CK(cudaMemsetAsync(h->q_buf, 0, sizeof(double) * nbc * qq, h->st));
+                if (qb->g_mean) {
+                    CK(cudaMemsetAsync(h->q_gm, 0, sizeof(double) * mcp, h->st));
+                    CK(qb_copy_rows(qb, h->q_gm, qb->g_mean, sizeof(double), bt0, nbc, true, h->st));
+                }
+                QWArgs wa;
+                wa.V = h->c_K;
+                wa.ldv = h->np;
+                wa.G = h->q_buf;
+                wa.q = qb->q;
+                wa.qpt = qb->qpt;
+                wa.nb = nbc;
+                wa.W = h->g_U;
+                wa.ldw = h->np;
+                qbatch_w_kernel<<<dim3((unsigned)(h->np / QB_KC), (unsigned)tiles_r), QB_THREADS, 0, h->st>>>(wa);
+                CK(cudaGetLastError());
+                count_launch();
+            }
 
             PredGradArgs ga;
             memset(&ga, 0, sizeof(ga));
@@ -1410,7 +1532,7 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             ga.zpt_c = h->zpt;
             ga.zs_c = h->np * ZP;
             ga.alpha = h->alpha;
-            ga.V = h->c_K;
+            ga.V = qb ? h->g_U : h->c_K;
             ga.ldv = h->np;
             ga.n_r = (int)mc;
             ga.n_c = (int)h->n;
@@ -1422,7 +1544,40 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             ga.part_v = h->g_part_v;
             ga.ldp = step;
             CK(launch_predict_grad(ga, h->kernel, tiles_r, h->T, h->st));
-
+        }
+        if (grad && qb) {  // the K**_t term, then d_xq of the chunk's rows (tile layout in g_dvar)
+            QInArgs ia;
+            ia.xs = h->c_xs;
+            ia.zpt = h->c_zpt;
+            ia.zs = mcp * ZP;
+            ia.dq = h->dq;
+            ia.dqp = h->dqp;
+            ia.dz = h->dz;
+            ia.n_pass = h->n_pass;
+            ia.G = h->q_buf;
+            ia.q = qb->q;
+            ia.qpt = qb->qpt;
+            ia.nb = nbc;
+            ia.rows = (int)mcp;
+            ia.part_k = h->g_dmean;
+            CK(launch_qbatch_inbatch_grad(ia, h->kernel, h->st));
+            QFinishArgs qf;
+            qf.part_m = h->g_part_m;
+            qf.part_v = h->g_part_v;
+            qf.ldp = step;
+            qf.tiles_c = h->T;
+            qf.part_k = h->g_dmean;
+            qf.g_mean = qb->g_mean ? h->q_gm : nullptr;
+            qf.m = (int)mcp;
+            qf.dq = h->dq;
+            qf.w = hyp_w(h);
+            qf.sf2 = h->sf2;
+            qf.d_x = h->g_dvar;
+            qbatch_grad_finish_kernel<<<(int)((mcp + 255) / 256), 256, 0, h->st>>>(qf);
+            CK(cudaGetLastError());
+            count_launch();
+            CK(qb_copy_rows(qb, qb->d_xq, h->g_dvar, sizeof(double) * h->dq, bt0, nbc, false, h->st));
+        } else if (grad) {
             PredGradFinishArgs gf;
             memset(&gf, 0, sizeof(gf));
             gf.part_m = h->g_part_m;
@@ -1449,7 +1604,8 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             if (d_mean) CK(cudaMemcpyAsync(d_mean + base * h->dq, h->g_dmean, gb, cudaMemcpyDefault, h->st));
             if (d_var) CK(cudaMemcpyAsync(d_var + base * h->dq, h->g_dvar, gb, cudaMemcpyDefault, h->st));
         }
-        if (mean) CK(cudaMemcpyAsync(mean + base, h->c_mu, sizeof(double) * mc, cudaMemcpyDefault, h->st));
+        if (mean && qb) CK(qb_copy_rows(qb, mean, h->c_mu, sizeof(double), bt0, nbc, false, h->st));
+        else if (mean) CK(cudaMemcpyAsync(mean + base, h->c_mu, sizeof(double) * mc, cudaMemcpyDefault, h->st));
         if (var) CK(cudaMemcpyAsync(var + base, h->c_var, sizeof(double) * mc, cudaMemcpyDefault, h->st));
         if (acq) {
             if (acq->scores)
@@ -1793,6 +1949,61 @@ extern "C" int gpp_sample_posterior(gpp_handle* h, int64_t m, const double* xq, 
     }
     CK(cudaStreamSynchronize(h->st));
     return GPP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Joint posteriors of b independent t-batches of q candidates (qbatch.cuh): the gpp_predict chunk loop on the tile
+// layout of QBatchSpec with U stored, then only the q x q diagonal blocks.  Nothing is kept between the two calls.
+static int qbatch_check(gpp_handle* h, long long b, int q, const double* xq, const int32_t* level_idx,
+                        const char* name) {
+    const char* why = nullptr;
+    if (!h) why = "null handle";
+    else if (!h->factorized) why = "call gpp_factorize (or gpp_mll_grad) first";
+    else if (q < 1 || q > GPP_MAX_QBATCH) why = "q must be in [1, GPP_MAX_QBATCH]";
+    else if (b < 0) why = "b must be >= 0";
+    else if (h->dq > GPP_MAX_DQ) why = "at most GPP_MAX_DQ quantitative inputs";
+    else if (b > 0 && h->dq > 0 && !xq) why = "xq missing";
+    else if (b > 0 && h->dz > 0 && !level_idx) why = "level_idx missing";
+    if (!why) return GPP_OK;
+    g_err = std::string(name) + ": " + why;
+    return GPP_ERR_ARG;
+}
+
+static QBatchSpec qbatch_spec(long long b, int q) {
+    QBatchSpec s;
+    memset(&s, 0, sizeof(s));
+    s.b = b;
+    s.q = q;
+    s.qpt = CT / q;
+    return s;
+}
+
+static long long qbatch_rows(const QBatchSpec& s) { return (s.b + s.qpt - 1) / s.qpt * CT; }
+
+extern "C" int gpp_posterior_qbatch(gpp_handle* h, int64_t b, int32_t q, const double* xq, const int32_t* level_idx,
+                                    const int32_t* noise_idx, const int32_t* mean_idx, int include_noise,
+                                    double* mean, double* cov) {
+    int rc = qbatch_check(h, b, q, xq, level_idx, "gpp_posterior_qbatch");
+    if (rc != GPP_OK || b == 0) return rc;
+    QBatchSpec s = qbatch_spec(b, q);
+    s.cov = cov;
+    return predict_impl(h, qbatch_rows(s), xq, level_idx, noise_idx, mean_idx, include_noise, 0.0, mean, nullptr,
+                        nullptr, false, nullptr, nullptr, nullptr, &s);
+}
+
+extern "C" int gpp_posterior_qbatch_grad(gpp_handle* h, int64_t b, int32_t q, const double* xq,
+                                         const int32_t* level_idx, const int32_t* noise_idx, const int32_t* mean_idx,
+                                         int include_noise, const double* g_mean, const double* g_cov, double* d_xq) {
+    int rc = qbatch_check(h, b, q, xq, level_idx, "gpp_posterior_qbatch_grad");
+    if (rc != GPP_OK) return rc;
+    if (b > 0 && h->dq > 0 && !d_xq) ARG_FAIL("gpp_posterior_qbatch_grad: d_xq missing");
+    if (b == 0 || h->dq == 0) return GPP_OK;  // no quantitative input: d_xq is empty
+    QBatchSpec s = qbatch_spec(b, q);
+    s.g_mean = g_mean;
+    s.g_cov = g_cov;
+    s.d_xq = d_xq;
+    return predict_impl(h, qbatch_rows(s), xq, level_idx, noise_idx, mean_idx, include_noise, 0.0, nullptr, nullptr,
+                        nullptr, true, nullptr, nullptr, nullptr, &s);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -10,6 +10,7 @@ sm_100a kernel family evaluates them.  No covariance arithmetic happens in Pytho
 from __future__ import annotations
 
 import math
+import warnings
 from collections import OrderedDict
 from typing import Callable, Iterator, Optional, Tuple
 
@@ -456,3 +457,35 @@ class MultivariateNormal:
     @property
     def stddev(self):
         return self.variance.sqrt()
+
+    def rsample(self, sample_shape=torch.Size(), base_samples=None):
+        """Draws [*sample_shape, *batch, q]: mean + L e with L the Cholesky factor of each q x q covariance block
+        (gpytorch's MultivariateNormal.rsample).  ``base_samples`` e defaults to standard normal draws; a block that is
+        not positive definite gets the psd_safe_cholesky jitter (1e-8, 1e-7, 1e-6) and a NumericalWarning, the other
+        blocks none."""
+        shape = torch.Size(sample_shape) + self.mean.shape
+        if base_samples is None:
+            base_samples = torch.randn(shape, dtype=self.mean.dtype, device=self.mean.device)
+        elif tuple(base_samples.shape) != tuple(shape):
+            raise ValueError("base_samples must have shape %s, got %s" % (tuple(shape), tuple(base_samples.shape)))
+        L = _psd_safe_cholesky(self._covar)
+        return self.mean + (L @ base_samples.to(self.mean.dtype).unsqueeze(-1)).squeeze(-1)
+
+
+def _psd_safe_cholesky(A):
+    """Batched Cholesky factor; blocks that fail get the smallest jitter of the ladder that lets them factor."""
+    L, info = torch.linalg.cholesky_ex(A)
+    bad = info != 0
+    if not bool(bad.any()):
+        return L
+    eye = torch.eye(A.shape[-1], dtype=A.dtype, device=A.device)
+    for jitter in (1e-8, 1e-7, 1e-6):
+        Lj, info_j = torch.linalg.cholesky_ex(A + jitter * eye)
+        fix = bad & (info_j == 0)
+        if bool(fix.any()):
+            warnings.warn("A not p.d., added jitter of %.1e to the diagonal" % jitter, NumericalWarning)
+            L = torch.where(fix[..., None, None], Lj, L)
+            bad = bad & ~fix
+        if not bool(bad.any()):
+            return L
+    raise NotPSDError("Matrix not positive definite after repeatedly adding jitter up to 1.0e-06.")

@@ -17,6 +17,7 @@ KERNEL_EXPSQ, KERNEL_MATERN32, KERNEL_MATERN52 = 0, 1, 2
 ACQ_HF, ACQ_LF, ACQ_EI = 0, 1, 2
 MAX_DQ, MAX_DZ = 32, 4
 MAX_JOINT = 16384  # GPP_MAX_JOINT: candidates of one gpp_predict_joint / gpp_sample_posterior call
+MAX_QBATCH = 128  # GPP_MAX_QBATCH: points per t-batch of gpp_posterior_qbatch / gpp_posterior_qbatch_grad
 
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libgpplus_b200.so")
 
@@ -24,7 +25,7 @@ EXPORTS = (
     "gpp_version", "gpp_device_count", "gpp_last_error", "gpp_launch_count", "gpp_create", "gpp_destroy", "gpp_pool_clear",
     "gpp_mll_grad",
     "gpp_get_timings", "gpp_get_stats", "gpp_covariance", "gpp_fetch", "gpp_factorize", "gpp_predict", "gpp_predict_grad",
-    "gpp_predict_joint", "gpp_sample_posterior", "gpp_acq_argmax",
+    "gpp_predict_joint", "gpp_sample_posterior", "gpp_posterior_qbatch", "gpp_posterior_qbatch_grad", "gpp_acq_argmax",
     "gpp_probe_dgemm", "gpp_probe_i8", "gpp_set_fp64_mode", "gpp_get_fp64_mode", "gpp_set_theta_layout", "gpp_objective", "gpp_objective_enqueue", "gpp_objective_collect",
 )
 
@@ -134,6 +135,12 @@ def load_library():
         lib.gpp_sample_posterior.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                              C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.POINTER(C.c_double)]
         lib.gpp_sample_posterior.restype = C.c_int
+        lib.gpp_posterior_qbatch.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+        lib.gpp_posterior_qbatch.restype = C.c_int
+        lib.gpp_posterior_qbatch_grad.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p,
+                                                  C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.gpp_posterior_qbatch_grad.restype = C.c_int
         lib.gpp_acq_argmax.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_double,
                                        C.c_double, C.c_double, C.c_double, C.c_void_p, _dp, C.POINTER(C.c_int64)]
@@ -500,6 +507,49 @@ class Engine:
         if rc != GPP_OK:
             _raise(rc, "gpp_sample_posterior")
         return samples, float(jit.value)
+
+    def _qbatch(self, xq, q, level_idx, noise_idx, mean_idx):
+        xq, m, level_idx, noise_idx, mean_idx = self._candidates(xq, level_idx, noise_idx, mean_idx)
+        q = int(q)
+        if q < 1 or m % q:
+            raise ValueError("posterior_qbatch: %d rows do not split into t-batches of q = %d" % (m, q))
+        return xq, m // q, q, level_idx, noise_idx, mean_idx
+
+    def posterior_qbatch(self, xq, q, level_idx=None, noise_idx=None, mean_idx=None, include_noise: bool = False,
+                         out_mean=None, out_cov=None):
+        """Mean [b, q] (bitwise ``predict``'s) and joint covariance [b, q, q] of b t-batches of q consecutive rows of
+        ``xq`` in scaled y units (gpp_posterior_qbatch): each block exactly symmetric and not clamped.  Inputs and
+        output buffers as for ``predict``; q <= MAX_QBATCH."""
+        xq, b, q, level_idx, noise_idx, mean_idx = self._qbatch(xq, q, level_idx, noise_idx, mean_idx)
+        mean = np.empty((b, q)) if out_mean is None else out_mean
+        cov = np.empty((b, q, q)) if out_cov is None else out_cov
+        rc = self._lib.gpp_posterior_qbatch(self._h, b, q, _ptr(xq), _ptr(level_idx), _ptr(noise_idx), _ptr(mean_idx),
+                                            1 if include_noise else 0, _ptr(mean), _ptr(cov))
+        if rc != GPP_OK:
+            _raise(rc, "gpp_posterior_qbatch")
+        return mean, cov
+
+    def posterior_qbatch_grad(self, xq, q, g_mean, g_cov, level_idx=None, noise_idx=None, mean_idx=None,
+                              include_noise: bool = False, out=None):
+        """d_xq [b*q, dq] = d/d xq of sum(g_mean * mean) + sum(g_cov * cov) of ``posterior_qbatch`` at the same
+        arguments (gpp_posterior_qbatch_grad).  ``g_mean`` [b, q] and ``g_cov`` [b, q, q] may be None (zero) and live
+        on the host or on this engine's GPU, like the other inputs."""
+        xq, b, q, level_idx, noise_idx, mean_idx = self._qbatch(xq, q, level_idx, noise_idx, mean_idx)
+        g = []
+        for a, n in ((g_mean, b * q), (g_cov, b * q * q)):
+            if a is not None and (isinstance(a, np.ndarray) or not hasattr(a, "data_ptr")):
+                a = _f64(a)
+            if a is not None and int(np.prod(a.shape)) != n:
+                raise ValueError("posterior_qbatch_grad: upstream gradient of %d entries, expected %d"
+                                 % (int(np.prod(a.shape)), n))
+            g.append(a)
+        d_xq = np.empty((b * q, self.dq)) if out is None else out
+        rc = self._lib.gpp_posterior_qbatch_grad(self._h, b, q, _ptr(xq), _ptr(level_idx), _ptr(noise_idx),
+                                                 _ptr(mean_idx), 1 if include_noise else 0, _ptr(g[0]), _ptr(g[1]),
+                                                 _ptr(d_xq))
+        if rc != GPP_OK:
+            _raise(rc, "gpp_posterior_qbatch_grad")
+        return d_xq
 
     def acq_argmax(self, xq, cost_idx, cost: Sequence[float], kind_by_cost: Sequence[int], best_f: Sequence[float],
                    level_idx=None, mean_idx=None, maximize: bool = True, si: float = 0.0, y_min: float = 0.0,

@@ -103,6 +103,40 @@ class _EnginePrediction(torch.autograd.Function):
         return gx, None, None, None, None
 
 
+class _EngineQBatchPosterior(torch.autograd.Function):
+    """Scaled means [b, q] and joint covariances [b, q, q] of b t-batches of q consecutive rows of ``x``
+    (gpp_posterior_qbatch), differentiable w.r.t. the quantitative columns of ``x``: the backward runs
+    gpp_posterior_qbatch_grad at the same rows with the hyper-parameters of the forward.  Categorical and source
+    columns get a zero gradient, the hyper-parameters none.  First derivatives only: differentiating the backward
+    raises."""
+
+    @staticmethod
+    def forward(ctx, x, model, eng, xq, q, kwargs):
+        mean, cov = eng.posterior_qbatch(xq, q, **kwargs)
+        ctx.set_materialize_grads(False)
+        ctx.x_meta = (x.shape, x.dtype, x.device)
+        ctx.request = (model, eng, model._factor_key, model._hyper_numpy(), xq, q, kwargs)
+        return torch.from_numpy(np.asarray(mean)), torch.from_numpy(np.asarray(cov))
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_mean, g_cov):
+        shape, dtype, device = ctx.x_meta
+        model, eng, key, hyper, xq, q, kwargs = ctx.request
+        gx = torch.zeros(shape, dtype=dtype, device=device)
+        cols = model._quant_columns()
+        if len(cols) == 0 or (g_mean is None and g_cov is None):
+            return gx, None, None, None, None, None
+        if model._factor_key != key:  # the engine was refactorised since the forward: restore its hyper-parameters
+            eng.factorize(hyper)
+            model._factor_key = key
+        gm, gc = (None if g is None else np.ascontiguousarray(g.detach().double().cpu().numpy()) for g in (g_mean, g_cov))
+        d_xq = eng.posterior_qbatch_grad(xq, q, gm, gc, **kwargs)
+        gx[:, cols] = torch.as_tensor(np.asarray(d_xq), dtype=torch.float64).reshape(-1, len(cols)).to(dtype=dtype,
+                                                                                                     device=device)
+        return gx, None, None, None, None, None
+
+
 class GPR(Module):
     def __init__(
         self,
@@ -448,14 +482,31 @@ class GPR(Module):
             return self.y_min + self.y_std * torch.as_tensor(np.asarray(samples_sc)).to(dtype)
 
     def posterior(self, X, output_indices=None, observation_noise=True, posterior_transform=None, **kwargs):
-        """Predictive distribution at X in SCALED units (botorch posterior stand-in: mean + marginal variance);
-        differentiable in X when X requires a gradient (GPR.predict, which subclasses' no_grad predict wraps)."""
+        """Predictive distribution at X in SCALED units (botorch posterior stand-in); differentiable in X when X
+        requires a gradient.  A 2-D X [m, d] gives the mean and the marginal variances (GPR.predict, which subclasses'
+        no_grad predict wraps).  X [..., q, d] gives the joint distribution of every t-batch of q points, mean
+        [..., q] and covariance [..., q, q], the input of Monte-Carlo batch acquisition (qEI, qNEI, qUCB, qKG)."""
         self.eval()
         X = X.double()
+        if X.dim() >= 3:
+            return self._posterior_qbatch(X, bool(observation_noise))
         mean, std = GPR.predict(self, X, return_std=True, include_noise=bool(observation_noise))
         mu = (mean - self.y_min) / self.y_std
         var = (std / self.y_std) ** 2
         return MultivariateNormal(mu, torch.diag(var))
+
+    def _posterior_qbatch(self, X: torch.Tensor, include_noise: bool) -> MultivariateNormal:
+        """Joint posterior of the t-batches of X [..., q, d] (gpp_posterior_qbatch): the leading dimensions are
+        flattened into b t-batches, whose rows are gathered as ``predict`` gathers one 2-D batch (categorical columns
+        ranked against the training inputs and all rows of X)."""
+        batch, q = X.shape[:-2], int(X.shape[-2])
+        x = X.reshape(-1, X.shape[-1])
+        eng, xq, kwargs = self._joint_request(x, include_noise)
+        if torch.is_grad_enabled() and X.requires_grad:
+            mean, cov = _EngineQBatchPosterior.apply(x, self, eng, xq, q, kwargs)
+        else:
+            mean, cov = (torch.from_numpy(np.asarray(a)) for a in eng.posterior_qbatch(xq, q, **kwargs))
+        return MultivariateNormal(mean.reshape(*batch, q), cov.reshape(*batch, q, q))
 
     def reset_parameters(self) -> None:
         """Reset parameters by sampling from the priors (gpregression.py:168-174)."""

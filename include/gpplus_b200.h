@@ -12,6 +12,8 @@
  *   - GP_Plus.predict_with_grad   models/gp_plus.py:626-628      -> gpp_factorize + gpp_predict_grad
  *   - GPR.posterior (joint), MultivariateNormal.rsample
  *                                 models/gpregression.py:151-166 -> gpp_predict_joint, gpp_sample_posterior
+ *   - GPR.posterior on [..., q, d] (botorch's posterior(X) for q-batch acquisition) and its backward
+ *                                 models/gpregression.py:151-166 -> gpp_posterior_qbatch, gpp_posterior_qbatch_grad
  *   - AF_*_Engineering + argmax   bayesian_optimizations/AFs.py:102-159,
  *                                 bayesian_optimizations/BO_GP_plus.py:183-194 -> gpp_acq_argmax
  *   - covar_module(x).evaluate()  models/gp_plus.py:472-474      -> gpp_covariance
@@ -199,6 +201,34 @@ int gpp_predict_joint(gpp_handle* h, int64_t m, const double* xq, const int32_t*
 int gpp_sample_posterior(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
                          const int32_t* noise_idx, const int32_t* mean_idx, int include_noise,
                          int64_t n_samples, const double* base_samples, double* samples, double* jitter);
+
+/* Joint posteriors of b independent t-batches of q candidates each (Monte-Carlo batch acquisition: qEI, qNEI, qUCB
+ * and qKG call posterior on a [b, q, d] batch).  Same pointer conventions as gpp_predict (host or device,
+ * cudaMemcpyDefault).  Only the q x q diagonal blocks are formed, so the cost over gpp_predict at the same b*q rows is
+ * about q/N for the covariance and the same for its gradient over gpp_predict_grad.  Neither call changes the factor
+ * of K_y, alpha, gpp_get_stats or gpp_get_timings.  The chunk buffers are those of gpp_predict_grad plus one chunk's
+ * q x q blocks, allocated on the first call and freed with the handle.  q > GPP_MAX_QBATCH, q < 1, b < 0 or dq > 32
+ * return GPP_ERR_ARG before any allocation. */
+#define GPP_MAX_QBATCH 128   /* q: points per t-batch, at most one 128-row tile */
+
+/* Mean and joint covariance of each of b independent t-batches of q candidates.
+ * Candidate rows are t-batch-major: xq is [b*q*dq], and level_idx / noise_idx / mean_idx are [b*q].
+ * Outputs, in scaled units:
+ *   mean [b*q]    bitwise gpp_predict's at the same rows
+ *   cov  [b*q*q]  Sigma_t = K**_t - K*_t K_y^-1 K*_t^T (+ each row's noise when include_noise)
+ * cov is exactly symmetric and not clamped. Its diagonal is bitwise the unclamped variance that gpp_predict forms
+ * from the same row sums, sf2 - sum_t rowsq[t][i] (+ noise_i), before the min_var clamp.  A t-batch's outputs do not
+ * depend on the other t-batches of the call.  Either output may be NULL. */
+int gpp_posterior_qbatch(gpp_handle* h, int64_t b, int32_t q, const double* xq, const int32_t* level_idx,
+                         const int32_t* noise_idx, const int32_t* mean_idx, int include_noise,
+                         double* mean, double* cov);
+
+/* Vector-Jacobian product of gpp_posterior_qbatch at the same arguments.
+ * Inputs:  g_mean [b*q], g_cov [b*q*q], both upstream gradients; either may be NULL (zero).
+ * Output:  d_xq [b*q*dq] = d/d xq of ( sum g_mean*mean + sum g_cov*cov ), quantitative inputs only. */
+int gpp_posterior_qbatch_grad(gpp_handle* h, int64_t b, int32_t q, const double* xq, const int32_t* level_idx,
+                              const int32_t* noise_idx, const int32_t* mean_idx, int include_noise,
+                              const double* g_mean, const double* g_cov, double* d_xq);
 
 /* fused predict + acquisition + argmax over m candidates (BO_GP_plus.py:183-194).
  * y_min/y_std undo the target scaling; cost_idx[m] selects cost[n_cost]; kind_by_cost[n_cost]
