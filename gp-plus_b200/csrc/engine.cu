@@ -21,6 +21,7 @@
 #include "objective.h"
 #include "predict.cuh"
 #include "predict_grad.cuh"
+#include "qacq.cuh"
 #include "qbatch.cuh"
 #include "solve.cuh"
 
@@ -116,6 +117,11 @@ struct gpp_handle {
     long long q_rows = 0;  // g_step they were sized for
     long long q_cap = 0;   // doubles in q_buf
     double *q_buf = nullptr, *q_gm = nullptr;
+    // Monte-Carlo acquisition buffers (gpp_acq_qbatch only; allocated on its first call, they only grow): the base
+    // samples of the call, one chunk's values and jitters, and the status word of the call
+    long long a_e_cap = 0, a_chunk_cap = 0;
+    double *a_E = nullptr, *a_val = nullptr, *a_jit = nullptr;
+    int* a_info = nullptr;
     double* acq_par = nullptr;  // [cost n_cost | best_f n_cost]
     int* acq_kind = nullptr;
     int acq_cap = 0;
@@ -153,7 +159,7 @@ static const double* hyp_beta(const gpp_handle* h) { return h->hyp + h->dq + zta
 static const double* hyp_sf2(const gpp_handle* h) { return hyp_beta(h) + h->n_mean; }
 static const double* hyp_jitter(const gpp_handle* h) { return hyp_beta(h) + h->n_mean + 1; }
 
-extern "C" int gpp_version(void) { return 109; }
+extern "C" int gpp_version(void) { return 110; }
 
 // process-wide default for handles created afterwards: -1 = by size (INT8-sliced from Np = 4096), 0 = DMMA, 1 = INT8
 static std::atomic<int> g_fp64_mode{-1};
@@ -190,7 +196,7 @@ static void destroy_now(gpp_handle* h) {
                      h->c_blk_best, h->c_blk_idx, h->acq_par, h->acq_kind, h->g_U, h->g_part_m, h->g_part_v,
                      h->g_dmean, h->g_dvar, h->j_xq, h->j_xs, h->j_nrm, h->j_zpt, h->j_U, h->j_S, h->j_Minv,
                      h->j_diag, h->j_mu, h->j_logdet, h->j_E, h->j_Y, h->j_lvl, h->j_noise, h->j_info,
-                     h->q_buf, h->q_gm};
+                     h->q_buf, h->q_gm, h->a_E, h->a_val, h->a_jit, h->a_info};
     for (void* p : dptrs)
         if (p) cudaFree(p);
     if (h->pinned_slab) cudaFreeHost(h->pinned_slab);
@@ -1231,6 +1237,16 @@ struct JointDest {
     double* U;                     // [mp x Np]
 };
 
+// gpp_acq_qbatch: the utility, its parameters in scaled units and the per-t-batch outputs
+struct QAcqSpec {
+    int kind, n_base, maximize;
+    double best_f, cbeta;
+    long long S;
+    const double* E;  // [S*q] caller's base samples
+    double* values;   // [b]
+    double* jitter;   // [b] or NULL
+};
+
 // gpp_posterior_qbatch[_grad]: b t-batches of q rows.  Every 128-row tile of the chunk buffers holds qpt = 128 / q whole
 // t-batches followed by padding rows, so chunks (multiples of 128 rows) hold whole t-batches.
 struct QBatchSpec {
@@ -1240,6 +1256,7 @@ struct QBatchSpec {
     const double* g_mean;  // backward: [b*q] or NULL
     const double* g_cov;   // backward: [b*q*q] or NULL
     double* d_xq;          // backward: [b*q*dq]
+    const QAcqSpec* acq;   // gpp_acq_qbatch: Monte-Carlo acquisition of every t-batch, or NULL
 };
 
 // rows of nbat t-batches, from t-batch bt0 of a compact [b*q rows] array, to (into_tiles) or from their tile slots in
@@ -1276,6 +1293,27 @@ static int ensure_qbatch_buffers(gpp_handle* h, int q) {
     return GPP_OK;
 }
 
+static int ensure_acq_buffers(gpp_handle* h, long long e_elems) {
+    if (!h->a_info) CK(dev_alloc(&h->a_info, 1));
+    if (e_elems > h->a_e_cap) {
+        if (h->a_E) cudaFree(h->a_E);
+        h->a_E = nullptr;
+        h->a_e_cap = 0;
+        CK(dev_alloc(&h->a_E, (size_t)e_elems));
+        h->a_e_cap = e_elems;
+    }
+    if (h->g_step > h->a_chunk_cap) {  // a chunk holds at most g_step t-batches
+        if (h->a_val) cudaFree(h->a_val);
+        if (h->a_jit) cudaFree(h->a_jit);
+        h->a_val = h->a_jit = nullptr;
+        h->a_chunk_cap = 0;
+        CK(dev_alloc(&h->a_val, (size_t)h->g_step));
+        CK(dev_alloc(&h->a_jit, (size_t)h->g_step));
+        h->a_chunk_cap = h->g_step;
+    }
+    return GPP_OK;
+}
+
 static int predict_impl(gpp_handle* h, long long m, const double* xq, const int32_t* level_idx,
                         const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, double min_var,
                         double* mean, double* var, AcqSpec* acq, bool grad = false, double* d_mean = nullptr,
@@ -1293,6 +1331,12 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
         if (rc != GPP_OK) return rc;
     }
     if (qb && (rc = ensure_qbatch_buffers(h, qb->q)) != GPP_OK) return rc;
+    const QAcqSpec* qa = qb ? qb->acq : nullptr;
+    if (qa) {
+        if ((rc = ensure_acq_buffers(h, qa->S * qb->q)) != GPP_OK) return rc;
+        CK(cudaMemcpyAsync(h->a_E, qa->E, sizeof(double) * qa->S * qb->q, cudaMemcpyDefault, h->st));
+        CK(cudaMemsetAsync(h->a_info, 0, sizeof(int), h->st));
+    }
     if (acq) {
         if (acq->n_cost <= 0 || !acq->cost || !acq->kind_by_cost || !acq->best_f) ARG_FAIL("acq: cost tables missing");
         if (acq->n_cost > h->acq_cap) {
@@ -1454,7 +1498,7 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
         predict_finish_kernel<<<nblk, 256, 0, h->st>>>(fa);
         CK(cudaGetLastError());
     count_launch();
-        if (qb && !grad && qb->cov) {  // Sigma_t = K**_t - U_t U_t^T of the chunk's t-batches into q_buf
+        if (qb && (qa || (!grad && qb->cov))) {  // Sigma_t = K**_t - U_t U_t^T of the chunk's t-batches into q_buf
             QSyrkArgs sa;
             memset(&sa, 0, sizeof(sa));
             sa.U = h->g_U;
@@ -1481,7 +1525,33 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             sa.cov = h->q_buf;
             CK(launch_qbatch_syrk(sa, h->kernel, tiles_r, h->st));
             const size_t qq = (size_t)qb->q * qb->q;
-            CK(cudaMemcpyAsync(qb->cov + bt0 * qq, h->q_buf, sizeof(double) * nbc * qq, cudaMemcpyDefault, h->st));
+            if (qb->cov)
+                CK(cudaMemcpyAsync(qb->cov + bt0 * qq, h->q_buf, sizeof(double) * nbc * qq, cudaMemcpyDefault, h->st));
+        }
+        if (qa) {  // values and jitters; with the gradient, G_t over Sigma_t in q_buf and mu_bar into q_gm
+            if (grad) CK(cudaMemsetAsync(h->q_gm, 0, sizeof(double) * mcp, h->st));
+            QAcqArgs aa;
+            memset(&aa, 0, sizeof(aa));
+            aa.blk = h->q_buf;
+            aa.mu = h->c_mu;
+            aa.gm = h->q_gm;
+            aa.E = h->a_E;
+            aa.S = qa->S;
+            aa.q = qb->q;
+            aa.qpt = qb->qpt;
+            aa.n_base = qa->n_base;
+            aa.nb = nbc;
+            aa.sgn = qa->maximize ? 1.0 : -1.0;
+            aa.best_f = qa->best_f;
+            aa.cbeta = qa->cbeta;
+            aa.grad = grad ? 1 : 0;
+            aa.value = h->a_val;
+            aa.jitter = h->a_jit;
+            aa.info = h->a_info;
+            CK(launch_qacq(aa, qa->kind, h->st));
+            CK(cudaMemcpyAsync(qa->values + bt0, h->a_val, sizeof(double) * nbc, cudaMemcpyDefault, h->st));
+            if (qa->jitter)
+                CK(cudaMemcpyAsync(qa->jitter + bt0, h->a_jit, sizeof(double) * nbc, cudaMemcpyDefault, h->st));
         }
         if (grad) {
             // V = U L^-1 = K* K_y^-1 over the K* chunk, which is not read again: B(tj, k) = L^-1[k, tj], k in [tj, T)
@@ -1500,12 +1570,12 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             CK(launch_gemm(vo, true, false, 1, h->st));
             if (qb) {  // W = blockdiag(G + G^T) V into g_U (U is not read again), the upstream mean gradient into q_gm
                 const size_t qq = (size_t)qb->q * qb->q;
-                if (qb->g_cov)
+                if (qb->g_cov)  // (the acquisition path has G_t in q_buf and mu_bar in q_gm already)
                     CK(cudaMemcpyAsync(h->q_buf, qb->g_cov + bt0 * qq, sizeof(double) * nbc * qq, cudaMemcpyDefault,
                                        h->st));
-                else
+                else if (!qa)
                     CK(cudaMemsetAsync(h->q_buf, 0, sizeof(double) * nbc * qq, h->st));
-                if (qb->g_mean) {
+                if (qb->g_mean && !qa) {
                     CK(cudaMemsetAsync(h->q_gm, 0, sizeof(double) * mcp, h->st));
                     CK(qb_copy_rows(qb, h->q_gm, qb->g_mean, sizeof(double), bt0, nbc, true, h->st));
                 }
@@ -1567,7 +1637,7 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             qf.ldp = step;
             qf.tiles_c = h->T;
             qf.part_k = h->g_dmean;
-            qf.g_mean = qb->g_mean ? h->q_gm : nullptr;
+            qf.g_mean = (qb->g_mean || qa) ? h->q_gm : nullptr;
             qf.m = (int)mcp;
             qf.dq = h->dq;
             qf.w = hyp_w(h);
@@ -1615,7 +1685,18 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             CK(cudaMemcpyAsync(hb.data(), h->c_blk_best, sizeof(double) * nblk, cudaMemcpyDeviceToHost, h->st));
             CK(cudaMemcpyAsync(hi.data(), h->c_blk_idx, sizeof(long long) * nblk, cudaMemcpyDeviceToHost, h->st));
         }
+        int qa_info = 0;
+        if (qa) CK(cudaMemcpyAsync(&qa_info, h->a_info, sizeof(int), cudaMemcpyDeviceToHost, h->st));
         CK(cudaStreamSynchronize(h->st));
+        if (qa_info & 2) {
+            g_err = "gpp_acq_qbatch: NaN in a t-batch posterior or its samples";
+            return GPP_ERR_NAN;
+        }
+        if (qa_info & 1) {
+            g_err = "gpp_acq_qbatch: a t-batch posterior covariance is not positive definite after adding jitter up to "
+                    "1e-6";
+            return GPP_ERR_NOT_PD;
+        }
         if (acq) {
             for (int b = 0; b < nblk; b++) {
                 if (acq->best_index < 0 || hb[b] > acq->best_score ||
@@ -2004,6 +2085,44 @@ extern "C" int gpp_posterior_qbatch_grad(gpp_handle* h, int64_t b, int32_t q, co
     s.d_xq = d_xq;
     return predict_impl(h, qbatch_rows(s), xq, level_idx, noise_idx, mean_idx, include_noise, 0.0, nullptr, nullptr,
                         nullptr, true, nullptr, nullptr, nullptr, &s);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Monte-Carlo batch acquisition (qacq.cuh): the gpp_posterior_qbatch chunk loop, then per t-batch the factor, the
+// samples and the utility in one CTA; with d_xq, the utility's adjoint (G_t, mu_bar) feeds the q-batch backward in the
+// same chunk, so no block leaves the device.
+extern "C" int gpp_acq_qbatch(gpp_handle* h, int64_t b, int32_t q_tot, const double* xq, const int32_t* level_idx,
+                              const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, int kind,
+                              int32_t n_baseline, double best_f, double beta, int maximize, int64_t n_samples,
+                              const double* base_samples, double* values, double* d_xq, double* jitter) {
+    int rc = qbatch_check(h, b, q_tot, xq, level_idx, "gpp_acq_qbatch");
+    if (rc != GPP_OK) return rc;
+    if (kind != GPP_QACQ_EI && kind != GPP_QACQ_NEI && kind != GPP_QACQ_UCB) ARG_FAIL("gpp_acq_qbatch: unknown kind");
+    if (kind == GPP_QACQ_NEI ? (n_baseline < 1 || n_baseline >= q_tot) : n_baseline != 0)
+        ARG_FAIL("gpp_acq_qbatch: n_baseline must be in [1, q_tot) for GPP_QACQ_NEI and 0 otherwise");
+    if (n_samples < 1 || n_samples > GPP_MAX_MC_SAMPLES)
+        ARG_FAIL("gpp_acq_qbatch: n_samples must be in [1, GPP_MAX_MC_SAMPLES]");
+    if (!base_samples || !values) ARG_FAIL("gpp_acq_qbatch: base_samples / values missing");
+    if (kind == GPP_QACQ_UCB && !(beta >= 0.0 && beta < INFINITY))
+        ARG_FAIL("gpp_acq_qbatch: beta must be finite and >= 0");
+    if (b == 0) return GPP_OK;
+    QAcqSpec a;
+    memset(&a, 0, sizeof(a));
+    a.kind = kind;
+    a.n_base = kind == GPP_QACQ_NEI ? n_baseline : 0;
+    a.maximize = maximize;
+    a.best_f = best_f;
+    a.cbeta = sqrt(beta * M_PI / 2.0);
+    a.S = n_samples;
+    a.E = base_samples;
+    a.values = values;
+    a.jitter = jitter;
+    QBatchSpec s = qbatch_spec(b, q_tot);
+    s.acq = &a;
+    const bool grad = d_xq && h->dq > 0;
+    s.d_xq = grad ? d_xq : nullptr;
+    return predict_impl(h, qbatch_rows(s), xq, level_idx, noise_idx, mean_idx, include_noise, 0.0, nullptr, nullptr,
+                        nullptr, grad, nullptr, nullptr, nullptr, &s);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -18,6 +18,8 @@ ACQ_HF, ACQ_LF, ACQ_EI = 0, 1, 2
 MAX_DQ, MAX_DZ = 32, 4
 MAX_JOINT = 16384  # GPP_MAX_JOINT: candidates of one gpp_predict_joint / gpp_sample_posterior call
 MAX_QBATCH = 128  # GPP_MAX_QBATCH: points per t-batch of gpp_posterior_qbatch / gpp_posterior_qbatch_grad
+QACQ_EI, QACQ_NEI, QACQ_UCB = 0, 1, 2  # GPP_QACQ_*: utilities of gpp_acq_qbatch
+MAX_MC_SAMPLES = 65536  # GPP_MAX_MC_SAMPLES: base-sample rows of one gpp_acq_qbatch call
 
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libgpplus_b200.so")
 
@@ -25,7 +27,8 @@ EXPORTS = (
     "gpp_version", "gpp_device_count", "gpp_last_error", "gpp_launch_count", "gpp_create", "gpp_destroy", "gpp_pool_clear",
     "gpp_mll_grad",
     "gpp_get_timings", "gpp_get_stats", "gpp_covariance", "gpp_fetch", "gpp_factorize", "gpp_predict", "gpp_predict_grad",
-    "gpp_predict_joint", "gpp_sample_posterior", "gpp_posterior_qbatch", "gpp_posterior_qbatch_grad", "gpp_acq_argmax",
+    "gpp_predict_joint", "gpp_sample_posterior", "gpp_posterior_qbatch", "gpp_posterior_qbatch_grad", "gpp_acq_qbatch",
+    "gpp_acq_argmax",
     "gpp_probe_dgemm", "gpp_probe_i8", "gpp_set_fp64_mode", "gpp_get_fp64_mode", "gpp_set_theta_layout", "gpp_objective", "gpp_objective_enqueue", "gpp_objective_collect",
 )
 
@@ -141,6 +144,10 @@ def load_library():
         lib.gpp_posterior_qbatch_grad.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p,
                                                   C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.gpp_posterior_qbatch_grad.restype = C.c_int
+        lib.gpp_acq_qbatch.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_int, C.c_int, C.c_int32, C.c_double, C.c_double, C.c_int,
+                                       C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.gpp_acq_qbatch.restype = C.c_int
         lib.gpp_acq_argmax.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_double,
                                        C.c_double, C.c_double, C.c_double, C.c_void_p, _dp, C.POINTER(C.c_int64)]
@@ -550,6 +557,38 @@ class Engine:
         if rc != GPP_OK:
             _raise(rc, "gpp_posterior_qbatch_grad")
         return d_xq
+
+    def acquisition_qbatch(self, xq, q_tot, kind, base_samples, best_f: float = 0.0, beta: float = 0.0,
+                           n_baseline: int = 0, maximize: bool = True, want_grad: bool = True, level_idx=None,
+                           noise_idx=None, mean_idx=None, include_noise: bool = False, out_values=None,
+                           out_d_xq=None):
+        """Monte-Carlo batch acquisition of the b t-batches of q_tot consecutive rows of ``xq`` (gpp_acq_qbatch):
+        returns ``(values [b], d_xq [b*q_tot, dq] or None, jitter [b])`` in scaled y units.  ``kind`` is QACQ_EI,
+        QACQ_NEI (the last ``n_baseline`` rows of each t-batch are baseline points) or QACQ_UCB; ``base_samples``
+        [S, q_tot] are shared by every t-batch.  ``d_xq`` is d(sum values)/d xq, computed only when ``want_grad``.
+        Inputs, base samples and output buffers may live on the host or on this engine's GPU, like ``predict``'s."""
+        xq, m, level_idx, noise_idx, mean_idx = self._candidates(xq, level_idx, noise_idx, mean_idx)
+        q_tot = int(q_tot)
+        if q_tot < 1 or m % q_tot:
+            raise ValueError("acquisition_qbatch: %d rows do not split into t-batches of q_tot = %d" % (m, q_tot))
+        b = m // q_tot
+        if isinstance(base_samples, np.ndarray) or not hasattr(base_samples, "data_ptr"):
+            base_samples = _f64(base_samples)
+        if len(base_samples.shape) != 2 or int(base_samples.shape[1]) != q_tot:
+            raise ValueError("acquisition_qbatch: base_samples must have shape [S, %d], got %s"
+                             % (q_tot, tuple(base_samples.shape)))
+        values = np.empty(b) if out_values is None else out_values
+        d_xq = None
+        if want_grad:
+            d_xq = np.empty((m, self.dq)) if out_d_xq is None else out_d_xq
+        jitter = np.empty(b)
+        rc = self._lib.gpp_acq_qbatch(self._h, b, q_tot, _ptr(xq), _ptr(level_idx), _ptr(noise_idx), _ptr(mean_idx),
+                                      1 if include_noise else 0, int(kind), int(n_baseline), float(best_f),
+                                      float(beta), 1 if maximize else 0, int(base_samples.shape[0]),
+                                      _ptr(base_samples), _ptr(values), _ptr(d_xq), _ptr(jitter))
+        if rc != GPP_OK:
+            _raise(rc, "gpp_acq_qbatch")
+        return values, d_xq, jitter
 
     def acq_argmax(self, xq, cost_idx, cost: Sequence[float], kind_by_cost: Sequence[int], best_f: Sequence[float],
                    level_idx=None, mean_idx=None, maximize: bool = True, si: float = 0.0, y_min: float = 0.0,

@@ -478,6 +478,15 @@ class GP_Plus(GPR):
             return super().sample_posterior(Xtest, num_samples=num_samples, include_noise=include_noise,
                                             base_samples=base_samples, generator=generator)
 
+    def acquisition_qbatch(self, X, kind="qEI", best_f=None, X_baseline=None, beta=None, num_samples=512,
+                           base_samples=None, seed=0, maximize=True, observation_noise=False):
+        """Monte-Carlo batch acquisition values of the t-batches of ``X`` [..., q, d] in the original y units
+        (GPR.acquisition_qbatch); differentiable in ``X`` when it requires a gradient, as ``predict_with_grad``."""
+        X = data_type_check(X)
+        return super().acquisition_qbatch(X, kind=kind, best_f=best_f, X_baseline=X_baseline, beta=beta,
+                                          num_samples=num_samples, base_samples=base_samples, seed=seed,
+                                          maximize=maximize, observation_noise=observation_noise)
+
     def noise_value(self):
         return self.likelihood.noise_covar.noise.detach() * self.y_std ** 2
 

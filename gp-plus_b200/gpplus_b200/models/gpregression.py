@@ -137,6 +137,47 @@ class _EngineQBatchPosterior(torch.autograd.Function):
         return gx, None, None, None, None, None
 
 
+_QACQ_KINDS = {"qEI": _engine.QACQ_EI, "qNEI": _engine.QACQ_NEI, "qUCB": _engine.QACQ_UCB}
+
+
+def sobol_normal_samples(num_samples: int, dim: int, seed: int = 0) -> torch.Tensor:
+    """[num_samples, dim] scrambled Sobol points mapped through the normal inverse CDF (botorch's
+    ``draw_sobol_normal_samples``, the base samples of ``SobolQMCNormalSampler``)."""
+    u = torch.quasirandom.SobolEngine(dimension=int(dim), scramble=True, seed=int(seed)).draw(int(num_samples),
+                                                                                            dtype=torch.float64)
+    v = 0.5 + (1.0 - torch.finfo(u.dtype).eps) * (u - 0.5)
+    return torch.erfinv(2.0 * v - 1.0) * math.sqrt(2.0)
+
+
+class _EngineQBatchAcquisition(torch.autograd.Function):
+    """Monte-Carlo batch acquisition values [b] of the t-batches of ``x`` [b, q, d] (gpp_acq_qbatch), differentiable
+    w.r.t. the quantitative columns of ``x``: the forward asks the engine for d(sum values)/dx as well, and the backward
+    scales each t-batch's rows by its upstream gradient.  Categorical and source columns get a zero gradient, the
+    baseline rows and the hyper-parameters none.  First derivatives only: differentiating the backward raises."""
+
+    @staticmethod
+    def forward(ctx, x, eng, xq, q_tot, cols, kwargs):
+        values, d_xq, jitter = eng.acquisition_qbatch(xq, q_tot, want_grad=len(cols) > 0, **kwargs)
+        b, q, d = x.shape
+        dx = torch.zeros(b, q, d, dtype=torch.float64)
+        if len(cols) > 0:
+            dx[:, :, cols] = torch.as_tensor(np.asarray(d_xq)).reshape(b, q_tot, len(cols))[:, :q]
+        ctx.dx = dx
+        ctx.x_meta = (x.dtype, x.device)
+        jitter = torch.as_tensor(np.asarray(jitter))
+        ctx.mark_non_differentiable(jitter)
+        return torch.as_tensor(np.asarray(values)), jitter
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_values, g_jitter):
+        dtype, device = ctx.x_meta
+        if g_values is None:
+            return (torch.zeros(ctx.dx.shape, dtype=dtype, device=device),) + (None,) * 5
+        gx = g_values.double().reshape(-1, 1, 1).cpu() * ctx.dx
+        return (gx.to(dtype=dtype, device=device),) + (None,) * 5
+
+
 class GPR(Module):
     def __init__(
         self,
@@ -507,6 +548,65 @@ class GPR(Module):
         else:
             mean, cov = (torch.from_numpy(np.asarray(a)) for a in eng.posterior_qbatch(xq, q, **kwargs))
         return MultivariateNormal(mean.reshape(*batch, q), cov.reshape(*batch, q, q))
+
+    def acquisition_qbatch(self, X: torch.Tensor, kind: str = "qEI", best_f: Optional[float] = None,
+                           X_baseline: Optional[torch.Tensor] = None, beta: Optional[float] = None,
+                           num_samples: int = 512, base_samples: Optional[torch.Tensor] = None, seed: int = 0,
+                           maximize: bool = True, observation_noise: bool = False) -> torch.Tensor:
+        """Monte-Carlo batch acquisition (botorch's qEI, qNEI, qUCB) of every t-batch of X [..., q, d], in the original
+        y units: values [...] (gpp_acq_qbatch).  All t-batches share the base samples [S, q + n_b], by default
+        ``num_samples`` scrambled Sobol normal draws of ``seed`` (botorch's SobolQMCNormalSampler), so each value is a
+        deterministic function of its own t-batch and L-BFGS-B can optimise it.  qEI needs ``best_f``, qNEI the
+        baseline points ``X_baseline`` [n_b, d] appended to every t-batch (q + n_b <= 128), qUCB ``beta``.  The values
+        are differentiable in the quantitative columns of X when X requires a gradient; a t-batch whose covariance
+        needed jitter raises a NumericalWarning."""
+        if kind not in _QACQ_KINDS:
+            raise ValueError("acquisition_qbatch: kind must be one of %s, got %r" % (sorted(_QACQ_KINDS), kind))
+        if kind == "qEI" and best_f is None:
+            raise ValueError("acquisition_qbatch: qEI needs best_f")
+        if kind == "qNEI" and X_baseline is None:
+            raise ValueError("acquisition_qbatch: qNEI needs X_baseline")
+        if kind == "qUCB" and beta is None:
+            raise ValueError("acquisition_qbatch: qUCB needs beta")
+        if X.dim() < 2:
+            raise ValueError("acquisition_qbatch expects X of shape [..., q, d]")
+        self.eval()
+        batch, q, d = X.shape[:-2], int(X.shape[-2]), int(X.shape[-1])
+        x = X.reshape(-1, q, d)
+        b = x.shape[0]
+        n_b = 0
+        rows = x.detach().double()
+        if kind == "qNEI":
+            Xb = torch.as_tensor(X_baseline).detach().double().reshape(-1, d)
+            n_b = Xb.shape[0]
+            if n_b < 1:
+                raise ValueError("acquisition_qbatch: X_baseline has no rows")
+            rows = torch.cat([rows, Xb.to(rows.device).expand(b, n_b, d)], dim=1)
+        q_tot = q + n_b
+        if q_tot > _engine.MAX_QBATCH:
+            raise ValueError("acquisition_qbatch: q + n_baseline = %d exceeds %d" % (q_tot, _engine.MAX_QBATCH))
+        if base_samples is None:
+            base_samples = sobol_normal_samples(num_samples, q_tot, seed)
+        base = np.ascontiguousarray(torch.as_tensor(base_samples).detach().to("cpu", torch.float64).numpy())
+        if base.ndim != 2 or base.shape[1] != q_tot:
+            raise ValueError("acquisition_qbatch: base_samples must have shape [S, %d], got %s" % (q_tot, base.shape))
+        y_min, y_std = float(self.y_min), float(self.y_std)
+        sgn = 1.0 if maximize else -1.0
+        eng, xq, kwargs = self._joint_request(rows.reshape(-1, d), bool(observation_noise))
+        kwargs.update(kind=_QACQ_KINDS[kind], base_samples=base, n_baseline=n_b, maximize=bool(maximize),
+                      best_f=0.0 if best_f is None else (float(best_f) - y_min) / y_std,
+                      beta=0.0 if beta is None else float(beta))
+        if torch.is_grad_enabled() and X.requires_grad:
+            v, jitter = _EngineQBatchAcquisition.apply(x, eng, xq, q_tot, self._quant_columns(), kwargs)
+        else:
+            values, _, jitter = eng.acquisition_qbatch(xq, q_tot, want_grad=False, **kwargs)
+            v, jitter = torch.as_tensor(np.asarray(values)), torch.as_tensor(np.asarray(jitter))
+        if bool((jitter > 0).any()):
+            warnings.warn("A not p.d., added jitter of %.1e to the diagonal" % float(jitter.max()), NumericalWarning)
+        dtype = self._out_dtype()
+        v = v.to(dtype)
+        out = sgn * y_min + y_std * v if kind == "qUCB" else y_std * v
+        return out.reshape(batch)
 
     def reset_parameters(self) -> None:
         """Reset parameters by sampling from the priors (gpregression.py:168-174)."""

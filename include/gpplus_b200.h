@@ -14,6 +14,8 @@
  *                                 models/gpregression.py:151-166 -> gpp_predict_joint, gpp_sample_posterior
  *   - GPR.posterior on [..., q, d] (botorch's posterior(X) for q-batch acquisition) and its backward
  *                                 models/gpregression.py:151-166 -> gpp_posterior_qbatch, gpp_posterior_qbatch_grad
+ *   - botorch qEI / qNEI / qUCB (MC acquisition on posterior(X).rsample with shared base samples) and their
+ *     gradients in X: GPR.acquisition_qbatch, bayesian_optimizations/qbatch.py -> gpp_acq_qbatch
  *   - AF_*_Engineering + argmax   bayesian_optimizations/AFs.py:102-159,
  *                                 bayesian_optimizations/BO_GP_plus.py:183-194 -> gpp_acq_argmax
  *   - covar_module(x).evaluate()  models/gp_plus.py:472-474      -> gpp_covariance
@@ -229,6 +231,36 @@ int gpp_posterior_qbatch(gpp_handle* h, int64_t b, int32_t q, const double* xq, 
 int gpp_posterior_qbatch_grad(gpp_handle* h, int64_t b, int32_t q, const double* xq, const int32_t* level_idx,
                               const int32_t* noise_idx, const int32_t* mean_idx, int include_noise,
                               const double* g_mean, const double* g_cov, double* d_xq);
+
+/* Monte-Carlo batch acquisition of b t-batches of q_tot rows (botorch's qEI, qNEI, qUCB with base samples shared by
+ * every t-batch), and its gradient in xq.  Pointer conventions as gpp_posterior_qbatch (host or device,
+ * cudaMemcpyDefault).  Per t-batch t, with mu_t and Sigma_t bitwise gpp_posterior_qbatch's (scaled units):
+ *   L_t = chol(Sigma_t + j_t I), j_t the first of 0, 1e-8, 1e-7, 1e-6 whose pivots are all > 0
+ *   y_s = mu_t + L_t e_s for each base-sample row e_s, sigma = +1 when maximize, -1 otherwise
+ *   values[t] = (1/S) sum_s u(y_s) with u
+ *     GPP_QACQ_EI   max(max_i sigma y_si - sigma best_f, 0)                          (n_baseline = 0)
+ *     GPP_QACQ_NEI  max(max_{i<q} sigma y_si - max_{q<=j<q_tot} sigma y_sj, 0)      (the last n_baseline rows of each
+ *                   t-batch are baseline points, q = q_tot - n_baseline, 1 <= n_baseline < q_tot)
+ *     GPP_QACQ_UCB  max_i (sigma mu_i + sqrt(beta pi / 2) |y_si - mu_i|)            (n_baseline = 0, beta >= 0)
+ *   d_xq [b*q_tot*dq] = d(sum_t values[t]) / d xq over all q_tot rows, quantitative inputs only (NULL: values only)
+ *   jitter [b] = j_t (may be NULL)
+ * A t-batch's outputs do not depend on the other t-batches of the call.  The call does not change the factor of K_y,
+ * alpha, gpp_get_stats or gpp_get_timings.  GPP_ERR_NOT_PD when a t-batch fails every rung, GPP_ERR_NAN on NaN.  An
+ * unknown kind, n_baseline out of range for the kind, q_tot outside [1, GPP_MAX_QBATCH], n_samples outside
+ * [1, GPP_MAX_MC_SAMPLES], a missing base_samples or values, or dq > 32 return GPP_ERR_ARG before any allocation.
+ * The base samples (n_samples*q_tot doubles) and one chunk's values and jitters are held on the device from the first
+ * call and freed with the handle. */
+#define GPP_QACQ_EI 0
+#define GPP_QACQ_NEI 1
+#define GPP_QACQ_UCB 2
+#define GPP_MAX_MC_SAMPLES 65536
+int gpp_acq_qbatch(gpp_handle* h, int64_t b, int32_t q_tot, const double* xq, const int32_t* level_idx,
+                   const int32_t* noise_idx, const int32_t* mean_idx, int include_noise,
+                   int kind, int32_t n_baseline, double best_f, double beta, int maximize,
+                   int64_t n_samples, const double* base_samples,   /* [n_samples * q_tot], shared by all t-batches */
+                   double* values,                                  /* [b] */
+                   double* d_xq,                                    /* [b * q_tot * dq] or NULL: values only */
+                   double* jitter);                                 /* [b] or NULL */
 
 /* fused predict + acquisition + argmax over m candidates (BO_GP_plus.py:183-194).
  * y_min/y_std undo the target scaling; cost_idx[m] selects cost[n_cost]; kind_by_cost[n_cost]
