@@ -21,6 +21,7 @@
 #include "objective.h"
 #include "predict.cuh"
 #include "predict_grad.cuh"
+#include "nipv.cuh"
 #include "qacq.cuh"
 #include "qbatch.cuh"
 #include "solve.cuh"
@@ -122,6 +123,19 @@ struct gpp_handle {
     long long a_e_cap = 0, a_chunk_cap = 0;
     double *a_E = nullptr, *a_val = nullptr, *a_jit = nullptr;
     int* a_info = nullptr;
+    // integration set of gpp_nipv_qbatch (gpp_ipv_points; the buffers only grow and are freed with the handle): point
+    // panels of i_m points padded to i_mp rows, U_I = K_I L^-T and V_I = U_I L^-1 [i_mp x Np], a zero vector in the
+    // place of alpha, the mean latent variance, and the factor generation the set was built for
+    long long i_m = 0, i_mp = 0, i_cap = 0, i_gen = -1;
+    double i_vbar = 0.0;
+    double *i_xq = nullptr, *i_xs = nullptr, *i_nrm = nullptr, *i_zpt = nullptr, *i_U = nullptr, *i_V = nullptr;
+    double* i_zero = nullptr;
+    int* i_lvl = nullptr;
+    // gpp_nipv_qbatch chunk buffers (they only grow): C^T [rows x i_mp], one chunk's Gram and A^-1 blocks, and the
+    // gradient partials over the training and the integration column tiles
+    long long n_ccap = 0, n_bcap = 0, n_pcap = 0;
+    double *n_C = nullptr, *n_G = nullptr, *n_Ai = nullptr, *n_pm = nullptr, *n_pv = nullptr;
+    long long fgen = 0;  // bumped whenever the factor (or its hyper-parameters) changes
     double* acq_par = nullptr;  // [cost n_cost | best_f n_cost]
     int* acq_kind = nullptr;
     int acq_cap = 0;
@@ -159,7 +173,7 @@ static const double* hyp_beta(const gpp_handle* h) { return h->hyp + h->dq + zta
 static const double* hyp_sf2(const gpp_handle* h) { return hyp_beta(h) + h->n_mean; }
 static const double* hyp_jitter(const gpp_handle* h) { return hyp_beta(h) + h->n_mean + 1; }
 
-extern "C" int gpp_version(void) { return 110; }
+extern "C" int gpp_version(void) { return 111; }
 
 // process-wide default for handles created afterwards: -1 = by size (INT8-sliced from Np = 4096), 0 = DMMA, 1 = INT8
 static std::atomic<int> g_fp64_mode{-1};
@@ -196,7 +210,9 @@ static void destroy_now(gpp_handle* h) {
                      h->c_blk_best, h->c_blk_idx, h->acq_par, h->acq_kind, h->g_U, h->g_part_m, h->g_part_v,
                      h->g_dmean, h->g_dvar, h->j_xq, h->j_xs, h->j_nrm, h->j_zpt, h->j_U, h->j_S, h->j_Minv,
                      h->j_diag, h->j_mu, h->j_logdet, h->j_E, h->j_Y, h->j_lvl, h->j_noise, h->j_info,
-                     h->q_buf, h->q_gm, h->a_E, h->a_val, h->a_jit, h->a_info};
+                     h->q_buf, h->q_gm, h->a_E, h->a_val, h->a_jit, h->a_info,
+                     h->i_xq, h->i_xs, h->i_nrm, h->i_zpt, h->i_U, h->i_V, h->i_zero, h->i_lvl, h->n_C, h->n_G,
+                     h->n_Ai, h->n_pm, h->n_pv};
     for (void* p : dptrs)
         if (p) cudaFree(p);
     if (h->pinned_slab) cudaFreeHost(h->pinned_slab);
@@ -294,6 +310,8 @@ extern "C" void gpp_destroy(gpp_handle* h) {
         if (g_pool.size() < kPoolMaxHandles && g_pool_bytes + h->slab_bytes <= kPoolMaxBytes) {
             h->layout.set = false;
             h->factorized = false;
+            h->fgen++;
+            h->i_m = 0;
             h->pending = false;
             g_pool.push_back(h);
             g_pool_bytes += h->slab_bytes;
@@ -936,10 +954,12 @@ extern "C" int gpp_mll_grad(gpp_handle* h, const gpp_hyper* hy, int want_grad, g
     if (rc != GPP_OK) return rc;
     CK(cudaSetDevice(h->device));
     h->factorized = false;
+    h->fgen++;
     h->pending = false;
     rc = run_eval(h, hy, want_grad ? 1 : 0);
     if (rc != GPP_OK) return rc;
     h->factorized = true;
+    h->fgen++;
     return collect_mll(h, want_grad, out);
 }
 
@@ -1006,10 +1026,12 @@ extern "C" int gpp_objective(gpp_handle* h, const double* theta, int want_grad, 
     gpp_hyper hy = layout_hyper(h);
     CK(cudaSetDevice(h->device));
     h->factorized = false;
+    h->fgen++;
     h->pending = false;
     int rc = run_eval(h, &hy, want_grad ? 1 : 0);
     if (rc != GPP_OK) return rc;
     h->factorized = true;
+    h->fgen++;
     return finish_objective(h, want_grad, value, grad, detail);
 }
 
@@ -1025,6 +1047,7 @@ extern "C" int gpp_objective_enqueue(gpp_handle* h, const double* theta, int wan
     gpp_hyper hy = layout_hyper(h);
     CK(cudaSetDevice(h->device));
     h->factorized = false;
+    h->fgen++;
     h->stats.evaluations++;
     h->stats.factorizations++;
     const int wg = want_grad ? 1 : 0;
@@ -1064,6 +1087,7 @@ extern "C" int gpp_objective_collect(gpp_handle* h, double* value, double* grad,
         h->last_jitter = kJitter[0];
     }
     h->factorized = true;
+    h->fgen++;
     return finish_objective(h, wg, value, grad, detail);
 }
 
@@ -1085,6 +1109,7 @@ extern "C" int gpp_covariance(gpp_handle* h, const gpp_hyper* hy, double* k_out)
     if (rc != GPP_OK) return rc;
     CK(cudaSetDevice(h->device));
     h->factorized = false;
+    h->fgen++;
     fill_hyper_host(h, hy, 0.0);
     if ((rc = stage_prep(h)) != GPP_OK) return rc;
     CovArgs ca;
@@ -1151,9 +1176,11 @@ extern "C" int gpp_factorize(gpp_handle* h, const gpp_hyper* hy) {
     if (rc != GPP_OK) return rc;
     CK(cudaSetDevice(h->device));
     h->factorized = false;
+    h->fgen++;
     rc = run_eval(h, hy, 0);
     if (rc != GPP_OK) return rc;
     h->factorized = true;
+    h->fgen++;
     return GPP_OK;
 }
 
@@ -1247,6 +1274,12 @@ struct QAcqSpec {
     double* jitter;   // [b] or NULL
 };
 
+// gpp_nipv_qbatch: the per-t-batch outputs (the integration set lives on the handle)
+struct NipvSpec {
+    double* values;  // [b]
+    double* jitter;  // [b] or NULL
+};
+
 // gpp_posterior_qbatch[_grad]: b t-batches of q rows.  Every 128-row tile of the chunk buffers holds qpt = 128 / q whole
 // t-batches followed by padding rows, so chunks (multiples of 128 rows) hold whole t-batches.
 struct QBatchSpec {
@@ -1257,6 +1290,7 @@ struct QBatchSpec {
     const double* g_cov;   // backward: [b*q*q] or NULL
     double* d_xq;          // backward: [b*q*dq]
     const QAcqSpec* acq;   // gpp_acq_qbatch: Monte-Carlo acquisition of every t-batch, or NULL
+    const NipvSpec* ipv;   // gpp_nipv_qbatch: integrated posterior variance against the handle's set, or NULL
 };
 
 // rows of nbat t-batches, from t-batch bt0 of a compact [b*q rows] array, to (into_tiles) or from their tile slots in
@@ -1314,6 +1348,44 @@ static int ensure_acq_buffers(gpp_handle* h, long long e_elems) {
     return GPP_OK;
 }
 
+// rows of one gpp_nipv_qbatch chunk: the C^T buffer [rows x i_mp] holds at most 2^27 doubles (1 GiB)
+static long long nipv_step(const gpp_handle* h) {
+    return std::min(h->g_step, std::max(128LL, ((1LL << 27) / h->i_mp) / 128 * 128));
+}
+
+// C^T of one chunk, its q x q Gram and A^-1 blocks and, with the gradient, the partials of predict_grad_tile_kernel
+// over the T training and i_mp / 128 integration column tiles (leading dimension rows)
+static int ensure_nipv_buffers(gpp_handle* h, long long rows, int q, bool grad) {
+    const long long c = rows * h->i_mp, blk = rows * q;
+    const long long part = grad ? rows * (h->T + h->i_mp / CT) * h->dq : 0;
+    if (c > h->n_ccap) {
+        if (h->n_C) cudaFree(h->n_C);
+        h->n_C = nullptr;
+        h->n_ccap = 0;
+        CK(dev_alloc(&h->n_C, (size_t)c));
+        h->n_ccap = c;
+    }
+    if (blk > h->n_bcap) {
+        if (h->n_G) cudaFree(h->n_G);
+        if (h->n_Ai) cudaFree(h->n_Ai);
+        h->n_G = h->n_Ai = nullptr;
+        h->n_bcap = 0;
+        CK(dev_alloc(&h->n_G, (size_t)blk));
+        CK(dev_alloc(&h->n_Ai, (size_t)blk));
+        h->n_bcap = blk;
+    }
+    if (part > h->n_pcap) {
+        if (h->n_pm) cudaFree(h->n_pm);
+        if (h->n_pv) cudaFree(h->n_pv);
+        h->n_pm = h->n_pv = nullptr;
+        h->n_pcap = 0;
+        CK(dev_alloc(&h->n_pm, (size_t)part));
+        CK(dev_alloc(&h->n_pv, (size_t)part));
+        h->n_pcap = part;
+    }
+    return GPP_OK;
+}
+
 static int predict_impl(gpp_handle* h, long long m, const double* xq, const int32_t* level_idx,
                         const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, double min_var,
                         double* mean, double* var, AcqSpec* acq, bool grad = false, double* d_mean = nullptr,
@@ -1337,6 +1409,13 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
         CK(cudaMemcpyAsync(h->a_E, qa->E, sizeof(double) * qa->S * qb->q, cudaMemcpyDefault, h->st));
         CK(cudaMemsetAsync(h->a_info, 0, sizeof(int), h->st));
     }
+    const NipvSpec* nv = qb ? qb->ipv : nullptr;
+    if (nv) {  // values, jitters and the status word in the acquisition buffers (no base samples)
+        if ((rc = ensure_acq_buffers(h, 0)) != GPP_OK) return rc;
+        if ((rc = ensure_nipv_buffers(h, nipv_step(h), qb->q, grad)) != GPP_OK) return rc;
+        CK(cudaMemsetAsync(h->a_info, 0, sizeof(int), h->st));
+    }
+    const int imt = nv ? (int)(h->i_mp / CT) : 0;  // integration column tiles
     if (acq) {
         if (acq->n_cost <= 0 || !acq->cost || !acq->kind_by_cost || !acq->best_f) ARG_FAIL("acq: cost tables missing");
         if (acq->n_cost > h->acq_cap) {
@@ -1356,7 +1435,7 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
     std::vector<double> hb;
     std::vector<long long> hi;
     const long long MC = h->mc_alloc;  // leading dimension of the chunk buffers
-    const long long step = keep_u ? h->g_step : MC;
+    const long long step = nv ? nipv_step(h) : (keep_u ? h->g_step : MC);
     for (long long base = 0; base < m; base += step) {
         const long long mc = std::min(step, m - base);
         const long long mcp = (mc + 127) / 128 * 128;
@@ -1498,7 +1577,7 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
         predict_finish_kernel<<<nblk, 256, 0, h->st>>>(fa);
         CK(cudaGetLastError());
     count_launch();
-        if (qb && (qa || (!grad && qb->cov))) {  // Sigma_t = K**_t - U_t U_t^T of the chunk's t-batches into q_buf
+        if (qb && (qa || nv || (!grad && qb->cov))) {  // Sigma_t = K**_t - U_t U_t^T of the chunk's t-batches, q_buf
             QSyrkArgs sa;
             memset(&sa, 0, sizeof(sa));
             sa.U = h->g_U;
@@ -1553,6 +1632,72 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             if (qa->jitter)
                 CK(cudaMemcpyAsync(qa->jitter + bt0, h->a_jit, sizeof(double) * nbc, cudaMemcpyDefault, h->st));
         }
+        if (nv) {  // C^T = K(X_chunk, X_I) - U_chunk U_I^T, then per t-batch G_t = C_t^T C_t, A_t's factor, the value
+            CovArgs cc;
+            memset(&cc, 0, sizeof(cc));
+            cc.xs_r = h->c_xs;
+            cc.nrm_r = h->c_nrm;
+            cc.xs_c = h->i_xs;
+            cc.nrm_c = h->i_nrm;
+            cc.out = h->n_C;
+            cc.ld = h->i_mp;
+            cc.n_r = (int)mc;
+            cc.n_c = (int)h->i_m;
+            cc.tiles_r = tiles_r;
+            cc.tiles_c = imt;
+            cc.dqp = h->dqp;
+            cc.dz = h->dz;
+            cc.sf2 = h->sf2;
+            cc.scale = 1.0 / (double)h->n_pass;
+            for (int p = 0; p < h->n_pass; p++) {
+                cc.zpt_r = h->c_zpt + (size_t)p * mcp * ZP;
+                cc.zpt_c = h->i_zpt + (size_t)p * h->i_mp * ZP;
+                cc.accum = p > 0;
+                cc.last = p == h->n_pass - 1;
+                CK(launch_cov(cc, h->kernel, h->st));
+            }
+            GemmOp co = gemm_default();
+            co.A = h->g_U;
+            co.lda = (int)h->np;
+            co.B = h->i_U;
+            co.ldb = (int)h->np;
+            co.C = h->n_C;
+            co.ldc = (int)h->i_mp;
+            co.tiles_m = co.tiles_m_last = tiles_r;
+            co.tiles_n = imt;
+            co.klo_c = 0;
+            co.khi_c = h->T;
+            co.alpha = -1.0;
+            co.beta = 1.0;
+            CK(launch_gemm(co, true, true, 1, h->st));
+            QSyrkArgs ga;
+            memset(&ga, 0, sizeof(ga));
+            ga.U = h->n_C;
+            ga.ldu = h->i_mp;
+            ga.kcols = (int)h->i_m;
+            ga.q = qb->q;
+            ga.qpt = qb->qpt;
+            ga.nb = nbc;
+            ga.cov = h->n_G;
+            CK(launch_qbatch_gram(ga, tiles_r, h->st));
+            NipvArgs na;
+            memset(&na, 0, sizeof(na));
+            na.blk = h->q_buf;
+            na.gram = h->n_G;
+            na.ainv = h->n_Ai;
+            na.q = qb->q;
+            na.nb = nbc;
+            na.inv_m = 1.0 / (double)h->i_m;
+            na.vbar = h->i_vbar;
+            na.grad = grad ? 1 : 0;
+            na.value = h->a_val;
+            na.jitter = h->a_jit;
+            na.info = h->a_info;
+            CK(launch_nipv_block(na, h->st));
+            CK(cudaMemcpyAsync(nv->values + bt0, h->a_val, sizeof(double) * nbc, cudaMemcpyDefault, h->st));
+            if (nv->jitter)
+                CK(cudaMemcpyAsync(nv->jitter + bt0, h->a_jit, sizeof(double) * nbc, cudaMemcpyDefault, h->st));
+        }
         if (grad) {
             // V = U L^-1 = K* K_y^-1 over the K* chunk, which is not read again: B(tj, k) = L^-1[k, tj], k in [tj, T)
             GemmOp vo = gemm_default();
@@ -1573,7 +1718,7 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
                 if (qb->g_cov)  // (the acquisition path has G_t in q_buf and mu_bar in q_gm already)
                     CK(cudaMemcpyAsync(h->q_buf, qb->g_cov + bt0 * qq, sizeof(double) * nbc * qq, cudaMemcpyDefault,
                                        h->st));
-                else if (!qa)
+                else if (!qa && !nv)  // (gpp_nipv_qbatch has A_bar_t there)
                     CK(cudaMemsetAsync(h->q_buf, 0, sizeof(double) * nbc * qq, h->st));
                 if (qb->g_mean && !qa) {
                     CK(cudaMemsetAsync(h->q_gm, 0, sizeof(double) * mcp, h->st));
@@ -1591,6 +1736,34 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
                 qbatch_w_kernel<<<dim3((unsigned)(h->np / QB_KC), (unsigned)tiles_r), QB_THREADS, 0, h->st>>>(wa);
                 CK(cudaGetLastError());
                 count_launch();
+                if (nv) {
+                    // -C_bar^T = blockdiag(-2 A^-1 / M) C^T in place over C^T: each CTA stages the 32-column panel of
+                    // its tile in shared memory before it writes that same panel
+                    QWArgs cw = wa;
+                    cw.V = h->n_C;
+                    cw.ldv = h->i_mp;
+                    cw.G = h->n_Ai;
+                    cw.W = h->n_C;
+                    cw.ldw = h->i_mp;
+                    qbatch_w_kernel<<<dim3((unsigned)(h->i_mp / QB_KC), (unsigned)tiles_r), QB_THREADS, 0, h->st>>>(cw);
+                    CK(cudaGetLastError());
+                    count_launch();
+                    // W += C_bar^T V_I: the K* term that reaches U_t through C_t (finish subtracts W's partials)
+                    GemmOp wo = gemm_default();
+                    wo.A = h->n_C;
+                    wo.lda = (int)h->i_mp;
+                    wo.B = h->i_V;
+                    wo.ldb = (int)h->np;
+                    wo.C = h->g_U;
+                    wo.ldc = (int)h->np;
+                    wo.tiles_m = wo.tiles_m_last = tiles_r;
+                    wo.tiles_n = h->T;
+                    wo.klo_c = 0;
+                    wo.khi_c = imt;
+                    wo.alpha = -1.0;
+                    wo.beta = 1.0;
+                    CK(launch_gemm(wo, true, false, 1, h->st));
+                }
             }
 
             PredGradArgs ga;
@@ -1610,10 +1783,23 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             ga.dqp = h->dqp;
             ga.dz = h->dz;
             ga.n_pass = h->n_pass;
-            ga.part_m = h->g_part_m;
-            ga.part_v = h->g_part_v;
+            ga.part_m = nv ? h->n_pm : h->g_part_m;
+            ga.part_v = nv ? h->n_pv : h->g_part_v;
             ga.ldp = step;
             CK(launch_predict_grad(ga, h->kernel, tiles_r, h->T, h->st));
+            if (nv) {  // K(X_t, X_I) term: integration points as columns, -C_bar^T as V, after the training tiles
+                PredGradArgs gi = ga;
+                gi.xs_c = h->i_xs;
+                gi.zpt_c = h->i_zpt;
+                gi.zs_c = h->i_mp * ZP;
+                gi.alpha = h->i_zero;
+                gi.V = h->n_C;
+                gi.ldv = h->i_mp;
+                gi.n_c = (int)h->i_m;
+                gi.part_m = h->n_pm + (size_t)h->T * h->dq * step;
+                gi.part_v = h->n_pv + (size_t)h->T * h->dq * step;
+                CK(launch_predict_grad(gi, h->kernel, tiles_r, imt, h->st));
+            }
         }
         if (grad && qb) {  // the K**_t term, then d_xq of the chunk's rows (tile layout in g_dvar)
             QInArgs ia;
@@ -1632,10 +1818,10 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             ia.part_k = h->g_dmean;
             CK(launch_qbatch_inbatch_grad(ia, h->kernel, h->st));
             QFinishArgs qf;
-            qf.part_m = h->g_part_m;
-            qf.part_v = h->g_part_v;
+            qf.part_m = nv ? h->n_pm : h->g_part_m;
+            qf.part_v = nv ? h->n_pv : h->g_part_v;
             qf.ldp = step;
-            qf.tiles_c = h->T;
+            qf.tiles_c = h->T + imt;
             qf.part_k = h->g_dmean;
             qf.g_mean = (qb->g_mean || qa) ? h->q_gm : nullptr;
             qf.m = (int)mcp;
@@ -1686,15 +1872,16 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             CK(cudaMemcpyAsync(hi.data(), h->c_blk_idx, sizeof(long long) * nblk, cudaMemcpyDeviceToHost, h->st));
         }
         int qa_info = 0;
-        if (qa) CK(cudaMemcpyAsync(&qa_info, h->a_info, sizeof(int), cudaMemcpyDeviceToHost, h->st));
+        if (qa || nv) CK(cudaMemcpyAsync(&qa_info, h->a_info, sizeof(int), cudaMemcpyDeviceToHost, h->st));
         CK(cudaStreamSynchronize(h->st));
         if (qa_info & 2) {
-            g_err = "gpp_acq_qbatch: NaN in a t-batch posterior or its samples";
+            g_err = nv ? "gpp_nipv_qbatch: NaN in a t-batch posterior or its integrated variance"
+                       : "gpp_acq_qbatch: NaN in a t-batch posterior or its samples";
             return GPP_ERR_NAN;
         }
         if (qa_info & 1) {
-            g_err = "gpp_acq_qbatch: a t-batch posterior covariance is not positive definite after adding jitter up to "
-                    "1e-6";
+            g_err = std::string(nv ? "gpp_nipv_qbatch" : "gpp_acq_qbatch") +
+                    ": a t-batch posterior covariance is not positive definite after adding jitter up to 1e-6";
             return GPP_ERR_NOT_PD;
         }
         if (acq) {
@@ -2123,6 +2310,135 @@ extern "C" int gpp_acq_qbatch(gpp_handle* h, int64_t b, int32_t q_tot, const dou
     s.d_xq = grad ? d_xq : nullptr;
     return predict_impl(h, qbatch_rows(s), xq, level_idx, noise_idx, mean_idx, include_noise, 0.0, nullptr, nullptr,
                         nullptr, grad, nullptr, nullptr, nullptr, &s);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Batch integrated posterior variance (nipv.cuh): gpp_ipv_points keeps the integration set's panels, U_I and V_I on the
+// handle for the current factor; gpp_nipv_qbatch runs the gpp_posterior_qbatch chunk loop with the candidates' noise,
+// forms C^T against the set, and feeds the closed form's adjoint to the q-batch backward in the same chunk.
+static bool ipv_valid(const gpp_handle* h) { return h->factorized && h->i_m > 0 && h->i_gen == h->fgen; }
+
+static int ensure_ipv_buffers(gpp_handle* h, long long mp) {
+    if (mp <= h->i_cap) return GPP_OK;
+    void* olds[] = {h->i_xq, h->i_xs, h->i_nrm, h->i_zpt, h->i_U, h->i_V, h->i_zero, h->i_lvl};
+    CK(cudaStreamSynchronize(h->st));
+    for (void* p : olds)
+        if (p) cudaFree(p);
+    h->i_xq = h->i_xs = h->i_nrm = h->i_zpt = h->i_U = h->i_V = h->i_zero = nullptr;
+    h->i_lvl = nullptr;
+    h->i_cap = 0;
+    const size_t n = (size_t)mp;
+    CK(dev_alloc(&h->i_xq, n * std::max(h->dq, 1)));
+    CK(dev_alloc(&h->i_xs, n * h->dqp));
+    CK(dev_alloc(&h->i_nrm, n));
+    CK(dev_alloc(&h->i_zpt, n * ZP * h->n_pass));
+    CK(dev_alloc(&h->i_U, n * (size_t)h->np));
+    CK(dev_alloc(&h->i_V, n * (size_t)h->np));
+    CK(dev_alloc(&h->i_zero, n));
+    CK(dev_alloc(&h->i_lvl, n));
+    CK(cudaMemsetAsync(h->i_zero, 0, sizeof(double) * n, h->st));
+    h->i_cap = mp;
+    return GPP_OK;
+}
+
+extern "C" int gpp_ipv_points(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx) {
+    const char* why = nullptr;
+    if (!h) why = "null handle";
+    else if (!h->factorized) why = "call gpp_factorize (or gpp_mll_grad) first";
+    else if (m < 1 || m > GPP_MAX_IPV_POINTS) why = "m must be in [1, GPP_MAX_IPV_POINTS]";
+    else if (h->dq > GPP_MAX_DQ) why = "at most GPP_MAX_DQ quantitative inputs";
+    else if (h->dq > 0 && !xq) why = "xq missing";
+    else if (h->dz > 0 && !level_idx) why = "level_idx missing";
+    if (why) {
+        g_err = std::string("gpp_ipv_points: ") + why;
+        return GPP_ERR_ARG;
+    }
+    CK(cudaSetDevice(h->device));
+    h->i_m = 0;  // no valid set until this call has finished
+    const long long mp = round128(m);
+    int rc = ensure_chunk_buffers(h, m);
+    if (rc != GPP_OK || (rc = ensure_ipv_buffers(h, mp)) != GPP_OK) return rc;
+    if (h->dq > 0) CK(cudaMemcpyAsync(h->i_xq, xq, sizeof(double) * m * h->dq, cudaMemcpyDefault, h->st));
+    if (h->dz > 0) CK(cudaMemcpyAsync(h->i_lvl, level_idx, sizeof(int) * m, cudaMemcpyDefault, h->st));
+    PrepArgs pa;
+    pa.xq = h->i_xq;
+    pa.level_idx = h->dz > 0 ? h->i_lvl : nullptr;
+    pa.w = hyp_w(h);
+    pa.centre = h->centre;
+    pa.ztab = hyp_z(h);
+    pa.n = (int)m;
+    pa.np = (int)mp;
+    pa.dq = h->dq;
+    pa.dqp = h->dqp;
+    pa.dz = h->dz;
+    pa.n_combo = h->n_combo;
+    pa.n_pass = h->n_pass;
+    pa.xs = h->i_xs;
+    pa.xst = nullptr;
+    pa.nrm = h->i_nrm;
+    pa.zpt = h->i_zpt;
+    prep_points_kernel<<<(int)((mp + 255) / 256), 256, 0, h->st>>>(pa);
+    CK(cudaGetLastError());
+    count_launch();
+    // U_I through the prediction chunk loop (rows >= m come out zero: K_I is zero there); v_m = sf2 - |U_m|^2
+    // unclamped and without noise
+    JointDest jd;
+    jd.xs = h->i_xs;
+    jd.nrm = h->i_nrm;
+    jd.zpt = h->i_zpt;
+    jd.mp = mp;
+    jd.U = h->i_U;
+    std::vector<double> v((size_t)m);
+    rc = predict_impl(h, m, xq, level_idx, nullptr, nullptr, 0, -INFINITY, nullptr, v.data(), nullptr, false, nullptr,
+                      nullptr, &jd);
+    if (rc != GPP_OK) return rc;
+    if (h->np > h->n)  // columns n .. Np face K_y's identity padding: zero in exact arithmetic, zero here
+        CK(cudaMemset2DAsync(h->i_U + h->n, sizeof(double) * h->np, 0, sizeof(double) * (h->np - h->n), (size_t)mp,
+                             h->st));
+    GemmOp vo = gemm_default();  // V_I = U_I L^-1 = K_I K_y^-1 (the gradient path's product)
+    vo.A = h->i_U;
+    vo.lda = (int)h->np;
+    vo.B = h->M;
+    vo.ldb = (int)h->np;
+    vo.C = h->i_V;
+    vo.ldc = (int)h->np;
+    vo.tiles_m = vo.tiles_m_last = (int)(mp / CT);
+    vo.tiles_n = h->T;
+    vo.klo_sel = KSEL_TJ;
+    vo.klo_c = 0;
+    vo.khi_c = h->T;
+    CK(launch_gemm(vo, true, false, 1, h->st));
+    CK(cudaStreamSynchronize(h->st));
+    double sum = 0.0;
+    for (long long i = 0; i < m; i++) sum += v[(size_t)i];
+    if (std::isnan(sum)) {
+        g_err = "gpp_ipv_points: NaN in the latent variance at the integration points";
+        return GPP_ERR_NAN;
+    }
+    h->i_vbar = sum / (double)m;
+    h->i_m = m;
+    h->i_mp = mp;
+    h->i_gen = h->fgen;
+    return GPP_OK;
+}
+
+extern "C" int gpp_nipv_qbatch(gpp_handle* h, int64_t b, int32_t q, const double* xq, const int32_t* level_idx,
+                               const int32_t* noise_idx, double* values, double* d_xq, double* jitter) {
+    int rc = qbatch_check(h, b, q, xq, level_idx, "gpp_nipv_qbatch");
+    if (rc != GPP_OK) return rc;
+    if (!ipv_valid(h)) ARG_FAIL("gpp_nipv_qbatch: no integration set for the current factor (call gpp_ipv_points)");
+    if (!values) ARG_FAIL("gpp_nipv_qbatch: values missing");
+    if (b == 0) return GPP_OK;
+    NipvSpec v;
+    v.values = values;
+    v.jitter = jitter;
+    QBatchSpec s = qbatch_spec(b, q);
+    s.ipv = &v;
+    const bool grad = d_xq && h->dq > 0;
+    s.d_xq = grad ? d_xq : nullptr;
+    // the candidates are fantasised with their observation noise (include_noise = 1); the mean is not needed
+    return predict_impl(h, qbatch_rows(s), xq, level_idx, noise_idx, nullptr, 1, 0.0, nullptr, nullptr, nullptr, grad,
+                        nullptr, nullptr, nullptr, &s);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -65,8 +65,9 @@ struct QSyrkArgs {
 };
 
 // One CTA per 128-row tile: the lower 8x8 fragments that meet a diagonal block, accumulated on DMMA over the U columns,
-// then Sigma = K** - U U^T written to both triangles (exactly symmetric), the diagonal from the row sums.
-template <int KIND>
+// then Sigma = K** - U U^T written to both triangles (exactly symmetric), the diagonal from the row sums.  GRAM: the
+// blocks of U U^T itself, diagonal included (only U, ldu, kcols, q, qpt, nb and cov are read; KIND is unused).
+template <int KIND, bool GRAM = false>
 __global__ void __launch_bounds__(QB_THREADS) qbatch_syrk_kernel(const QSyrkArgs a) {
     __shared__ double sU[CT * QB_LDS];
     __shared__ unsigned char frag[136][2];
@@ -125,7 +126,9 @@ __global__ void __launch_bounds__(QB_THREADS) qbatch_syrk_kernel(const QSyrkArgs
             const int bt = i / q, li = i - bt * q, lj = j - bt * q;
             const long long gi = (long long)tile * CT + i, gj = (long long)tile * CT + j;
             double v;
-            if (i == j) {  // predict_finish_kernel's unclamped variance, bit for bit
+            if (GRAM) {
+                v = acc[s][e];
+            } else if (i == j) {  // predict_finish_kernel's unclamped variance, bit for bit
                 double qs = 0.0;
                 for (int tc = 0; tc < a.tiles_c; tc++) qs += a.rowsq[(long long)tc * a.ldr + gi];
                 v = a.sf2 - qs;
@@ -289,6 +292,13 @@ inline cudaError_t launch_qbatch_syrk(const QSyrkArgs& a, int kind, int tiles, c
     if (kind == KERNEL_EXPSQ) qbatch_syrk_kernel<KERNEL_EXPSQ><<<tiles, QB_THREADS, 0, st>>>(a);
     else if (kind == KERNEL_MATERN32) qbatch_syrk_kernel<KERNEL_MATERN32><<<tiles, QB_THREADS, 0, st>>>(a);
     else qbatch_syrk_kernel<KERNEL_MATERN52><<<tiles, QB_THREADS, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+// the q x q diagonal blocks of U U^T over columns [0, kcols) (gpp_nipv_qbatch's C_t^T C_t)
+inline cudaError_t launch_qbatch_gram(const QSyrkArgs& a, int tiles, cudaStream_t st) {
+    count_launch();
+    qbatch_syrk_kernel<KERNEL_EXPSQ, true><<<tiles, QB_THREADS, 0, st>>>(a);
     return cudaGetLastError();
 }
 

@@ -20,6 +20,7 @@ MAX_JOINT = 16384  # GPP_MAX_JOINT: candidates of one gpp_predict_joint / gpp_sa
 MAX_QBATCH = 128  # GPP_MAX_QBATCH: points per t-batch of gpp_posterior_qbatch / gpp_posterior_qbatch_grad
 QACQ_EI, QACQ_NEI, QACQ_UCB = 0, 1, 2  # GPP_QACQ_*: utilities of gpp_acq_qbatch
 MAX_MC_SAMPLES = 65536  # GPP_MAX_MC_SAMPLES: base-sample rows of one gpp_acq_qbatch call
+MAX_IPV_POINTS = 16384  # GPP_MAX_IPV_POINTS: integration points of one gpp_ipv_points call
 
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libgpplus_b200.so")
 
@@ -28,7 +29,7 @@ EXPORTS = (
     "gpp_mll_grad",
     "gpp_get_timings", "gpp_get_stats", "gpp_covariance", "gpp_fetch", "gpp_factorize", "gpp_predict", "gpp_predict_grad",
     "gpp_predict_joint", "gpp_sample_posterior", "gpp_posterior_qbatch", "gpp_posterior_qbatch_grad", "gpp_acq_qbatch",
-    "gpp_acq_argmax",
+    "gpp_ipv_points", "gpp_nipv_qbatch", "gpp_acq_argmax",
     "gpp_probe_dgemm", "gpp_probe_i8", "gpp_set_fp64_mode", "gpp_get_fp64_mode", "gpp_set_theta_layout", "gpp_objective", "gpp_objective_enqueue", "gpp_objective_collect",
 )
 
@@ -148,6 +149,11 @@ def load_library():
                                        C.c_void_p, C.c_int, C.c_int, C.c_int32, C.c_double, C.c_double, C.c_int,
                                        C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.gpp_acq_qbatch.restype = C.c_int
+        lib.gpp_ipv_points.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
+        lib.gpp_ipv_points.restype = C.c_int
+        lib.gpp_nipv_qbatch.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.gpp_nipv_qbatch.restype = C.c_int
         lib.gpp_acq_argmax.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_double,
                                        C.c_double, C.c_double, C.c_double, C.c_void_p, _dp, C.POINTER(C.c_int64)]
@@ -588,6 +594,38 @@ class Engine:
                                       _ptr(base_samples), _ptr(values), _ptr(d_xq), _ptr(jitter))
         if rc != GPP_OK:
             _raise(rc, "gpp_acq_qbatch")
+        return values, d_xq, jitter
+
+    def ipv_points(self, xq, level_idx=None):
+        """Stores the integration set of ``nipv_qbatch`` (gpp_ipv_points): the m rows of ``xq`` (and their
+        ``level_idx``), host arrays or tensors on this engine's GPU, 1 <= m <= MAX_IPV_POINTS.  The set belongs to the
+        current factor: after ``factorize`` or ``mll_grad`` it has to be stored again."""
+        xq, m, level_idx, _, _ = self._candidates(xq, level_idx, None, None)
+        rc = self._lib.gpp_ipv_points(self._h, m, _ptr(xq), _ptr(level_idx))
+        if rc != GPP_OK:
+            _raise(rc, "gpp_ipv_points")
+
+    def nipv_qbatch(self, xq, q, want_grad: bool = True, level_idx=None, noise_idx=None, out_values=None,
+                    out_d_xq=None):
+        """Negative integrated posterior variance over the stored integration set of the b t-batches of q consecutive
+        rows of ``xq``, each fantasised with the observation noise of its rows' ``noise_idx`` groups (gpp_nipv_qbatch):
+        returns ``(values [b], d_xq [b*q, dq] or None, jitter [b])`` in scaled y units.  ``d_xq`` is
+        d(sum values)/d xq, computed only when ``want_grad``.  Inputs and output buffers may live on the host or on
+        this engine's GPU, like ``predict``'s."""
+        xq, m, level_idx, noise_idx, _ = self._candidates(xq, level_idx, noise_idx, None)
+        q = int(q)
+        if q < 1 or m % q:
+            raise ValueError("nipv_qbatch: %d rows do not split into t-batches of q = %d" % (m, q))
+        b = m // q
+        values = np.empty(b) if out_values is None else out_values
+        d_xq = None
+        if want_grad:
+            d_xq = np.empty((m, self.dq)) if out_d_xq is None else out_d_xq
+        jitter = np.empty(b)
+        rc = self._lib.gpp_nipv_qbatch(self._h, b, q, _ptr(xq), _ptr(level_idx), _ptr(noise_idx), _ptr(values),
+                                       _ptr(d_xq), _ptr(jitter))
+        if rc != GPP_OK:
+            _raise(rc, "gpp_nipv_qbatch")
         return values, d_xq, jitter
 
     def acq_argmax(self, xq, cost_idx, cost: Sequence[float], kind_by_cost: Sequence[int], best_f: Sequence[float],

@@ -1,6 +1,6 @@
-"""Proposing a batch of q points by maximising a Monte-Carlo batch acquisition (qEI, qNEI, qUCB) of a fitted model:
-Sobol screening of raw t-batches, then one joint L-BFGS-B run over the best restarts with the engine's gradients
-(GPR.acquisition_qbatch / gpp_acq_qbatch)."""
+"""Proposing a batch of q points by maximising a batch acquisition (Monte-Carlo qEI, qNEI, qUCB, or qNIPV) of a
+fitted model: Sobol screening of raw t-batches, then one joint L-BFGS-B run over the best restarts with the engine's
+gradients (GPR.acquisition_qbatch / gpp_acq_qbatch, gpp_nipv_qbatch)."""
 from typing import Dict, Optional, Tuple
 
 import numpy as np
@@ -19,7 +19,7 @@ def optimize_acquisition_qbatch(model, bounds, q: int, kind: str, fixed_columns:
     ``fixed_columns`` ({column: value}, required when the model has such columns).  ``raw_samples`` Sobol t-batches
     inside the bounds are scored in one values-only call; the best ``num_restarts`` (ties broken by index) are
     optimised jointly by one L-BFGS-B run on minus the sum of their values, with the same base samples throughout
-    (drawn once from ``seed`` unless ``base_samples`` is given).  ``options`` go to ``scipy.optimize.minimize``."""
+    (drawn once from ``seed`` unless ``base_samples`` is given; qNIPV, which needs ``mc_points``, draws none).  ``options`` go to ``scipy.optimize.minimize``."""
     q = int(q)
     d = int(model.train_inputs[0].shape[1])
     cols = list(model._quant_columns())
@@ -40,7 +40,7 @@ def optimize_acquisition_qbatch(model, bounds, q: int, kind: str, fixed_columns:
         raise ValueError("optimize_acquisition_qbatch: the model has no quantitative column to optimise")
 
     acq_kwargs = dict(acq_kwargs)
-    if acq_kwargs.get("base_samples") is None:
+    if kind != "qNIPV" and acq_kwargs.get("base_samples") is None:  # qNIPV is exact: no base samples
         n_b = 0
         if acq_kwargs.get("X_baseline") is not None:
             n_b = int(torch.as_tensor(acq_kwargs["X_baseline"]).reshape(-1, d).shape[0])

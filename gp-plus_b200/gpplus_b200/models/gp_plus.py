@@ -479,13 +479,17 @@ class GP_Plus(GPR):
                                             base_samples=base_samples, generator=generator)
 
     def acquisition_qbatch(self, X, kind="qEI", best_f=None, X_baseline=None, beta=None, num_samples=512,
-                           base_samples=None, seed=0, maximize=True, observation_noise=False):
-        """Monte-Carlo batch acquisition values of the t-batches of ``X`` [..., q, d] in the original y units
-        (GPR.acquisition_qbatch); differentiable in ``X`` when it requires a gradient, as ``predict_with_grad``."""
+                           base_samples=None, seed=0, maximize=True, observation_noise=False, mc_points=None):
+        """Batch acquisition values of the t-batches of ``X`` [..., q, d] in the original y units
+        (GPR.acquisition_qbatch: Monte-Carlo qEI / qNEI / qUCB, or qNIPV over ``mc_points``); differentiable in ``X``
+        when it requires a gradient, as ``predict_with_grad``."""
         X = data_type_check(X)
+        if mc_points is not None:
+            mc_points = data_type_check(mc_points)
         return super().acquisition_qbatch(X, kind=kind, best_f=best_f, X_baseline=X_baseline, beta=beta,
                                           num_samples=num_samples, base_samples=base_samples, seed=seed,
-                                          maximize=maximize, observation_noise=observation_noise)
+                                          maximize=maximize, observation_noise=observation_noise,
+                                          mc_points=mc_points)
 
     def noise_value(self):
         return self.likelihood.noise_covar.noise.detach() * self.y_std ** 2

@@ -130,6 +130,7 @@ class _EngineQBatchPosterior(torch.autograd.Function):
         if model._factor_key != key:  # the engine was refactorised since the forward: restore its hyper-parameters
             eng.factorize(hyper)
             model._factor_key = key
+            model._ipv_state = None
         gm, gc = (None if g is None else np.ascontiguousarray(g.detach().double().cpu().numpy()) for g in (g_mean, g_cov))
         d_xq = eng.posterior_qbatch_grad(xq, q, gm, gc, **kwargs)
         gx[:, cols] = torch.as_tensor(np.asarray(d_xq), dtype=torch.float64).reshape(-1, len(cols)).to(dtype=dtype,
@@ -176,6 +177,25 @@ class _EngineQBatchAcquisition(torch.autograd.Function):
             return (torch.zeros(ctx.dx.shape, dtype=dtype, device=device),) + (None,) * 5
         gx = g_values.double().reshape(-1, 1, 1).cpu() * ctx.dx
         return (gx.to(dtype=dtype, device=device),) + (None,) * 5
+
+
+class _EngineNIPV(_EngineQBatchAcquisition):
+    """Negative integrated posterior variances [b] of the t-batches of ``x`` [b, q, d] against the engine's stored
+    integration set (gpp_nipv_qbatch), differentiable w.r.t. the quantitative columns of ``x`` as
+    ``_EngineQBatchAcquisition``, whose backward it shares."""
+
+    @staticmethod
+    def forward(ctx, x, eng, xq, q, cols, kwargs):
+        values, d_xq, jitter = eng.nipv_qbatch(xq, q, want_grad=len(cols) > 0, **kwargs)
+        b, _, d = x.shape
+        dx = torch.zeros(b, q, d, dtype=torch.float64)
+        if len(cols) > 0:
+            dx[:, :, cols] = torch.as_tensor(np.asarray(d_xq)).reshape(b, q, len(cols))
+        ctx.dx = dx
+        ctx.x_meta = (x.dtype, x.device)
+        jitter = torch.as_tensor(np.asarray(jitter))
+        ctx.mark_non_differentiable(jitter)
+        return torch.as_tensor(np.asarray(values)), jitter
 
 
 class GPR(Module):
@@ -245,6 +265,7 @@ class GPR(Module):
         self._engine_device = None
         self._factor_key = None
         self._last_eval = None
+        self._ipv_state = None  # (engine, factor key, integration inputs, levels) of the engine's qNIPV set
 
     # ------------------------------------------------------------------------------------------
     # engine plumbing
@@ -253,6 +274,7 @@ class GPR(Module):
         state["_engine"] = None
         state["_factor_key"] = None
         state["_last_eval"] = None
+        state["_ipv_state"] = None
         return state
 
     def __deepcopy__(self, memo):
@@ -261,7 +283,7 @@ class GPR(Module):
         new = cls.__new__(cls)
         memo[id(self)] = new
         for k, v in self.__dict__.items():
-            if k in ("_engine", "_last_eval"):
+            if k in ("_engine", "_last_eval", "_ipv_state"):
                 new.__dict__[k] = None
             elif k == "_factor_key":
                 new.__dict__[k] = None
@@ -417,6 +439,7 @@ class GPR(Module):
         if self._factor_key != key:
             eng.factorize(hyper)
             self._factor_key = key
+            self._ipv_state = None  # the engine drops its integration set with the old factor
         return eng
 
     # ------------------------------------------------------------------------------------------
@@ -552,16 +575,34 @@ class GPR(Module):
     def acquisition_qbatch(self, X: torch.Tensor, kind: str = "qEI", best_f: Optional[float] = None,
                            X_baseline: Optional[torch.Tensor] = None, beta: Optional[float] = None,
                            num_samples: int = 512, base_samples: Optional[torch.Tensor] = None, seed: int = 0,
-                           maximize: bool = True, observation_noise: bool = False) -> torch.Tensor:
+                           maximize: bool = True, observation_noise: bool = False,
+                           mc_points: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Monte-Carlo batch acquisition (botorch's qEI, qNEI, qUCB) of every t-batch of X [..., q, d], in the original
         y units: values [...] (gpp_acq_qbatch).  All t-batches share the base samples [S, q + n_b], by default
         ``num_samples`` scrambled Sobol normal draws of ``seed`` (botorch's SobolQMCNormalSampler), so each value is a
         deterministic function of its own t-batch and L-BFGS-B can optimise it.  qEI needs ``best_f``, qNEI the
         baseline points ``X_baseline`` [n_b, d] appended to every t-batch (q + n_b <= 128), qUCB ``beta``.  The values
         are differentiable in the quantitative columns of X when X requires a gradient; a t-batch whose covariance
-        needed jitter raises a NumericalWarning."""
+        needed jitter raises a NumericalWarning.
+
+        ``kind="qNIPV"`` (botorch's qNegIntegratedPosteriorVariance) needs ``mc_points`` [M, d], the integration
+        points, and takes none of ``best_f``, ``beta``, ``X_baseline`` or ``base_samples``: the value is minus the mean,
+        over ``mc_points``, of the latent posterior variance after also observing the t-batch with its observation
+        noise, in y units squared.  It is exact (no samples), and the source column of ``mc_points`` selects which
+        fidelity's variance is integrated."""
+        if kind == "qNIPV":
+            given = [k for k, v in (("best_f", best_f), ("beta", beta), ("X_baseline", X_baseline),
+                                    ("base_samples", base_samples)) if v is not None]
+            if given:
+                raise ValueError("acquisition_qbatch: qNIPV takes no %s" % ", ".join(given))
+            if mc_points is None:
+                raise ValueError("acquisition_qbatch: qNIPV needs mc_points")
+            return self._nipv_qbatch(X, mc_points)
+        if mc_points is not None:
+            raise ValueError("acquisition_qbatch: mc_points is for qNIPV only")
         if kind not in _QACQ_KINDS:
-            raise ValueError("acquisition_qbatch: kind must be one of %s, got %r" % (sorted(_QACQ_KINDS), kind))
+            raise ValueError("acquisition_qbatch: kind must be one of %s, got %r"
+                             % (sorted(list(_QACQ_KINDS) + ["qNIPV"]), kind))
         if kind == "qEI" and best_f is None:
             raise ValueError("acquisition_qbatch: qEI needs best_f")
         if kind == "qNEI" and X_baseline is None:
@@ -607,6 +648,45 @@ class GPR(Module):
         v = v.to(dtype)
         out = sgn * y_min + y_std * v if kind == "qUCB" else y_std * v
         return out.reshape(batch)
+
+    def _nipv_qbatch(self, X: torch.Tensor, mc_points) -> torch.Tensor:
+        if X.dim() < 2:
+            raise ValueError("acquisition_qbatch expects X of shape [..., q, d]")
+        self.eval()
+        batch, q, d = X.shape[:-2], int(X.shape[-2]), int(X.shape[-1])
+        if q > _engine.MAX_QBATCH:
+            raise ValueError("acquisition_qbatch: q = %d exceeds %d" % (q, _engine.MAX_QBATCH))
+        x = X.reshape(-1, q, d)
+        n_c = x.shape[0] * q
+        P = torch.as_tensor(mc_points).detach().double()
+        if P.dim() != 2 or P.shape[1] != d:
+            raise ValueError("acquisition_qbatch: mc_points must have shape [M, %d], got %s" % (d, tuple(P.shape)))
+        if not 1 <= P.shape[0] <= _engine.MAX_IPV_POINTS:
+            raise ValueError("acquisition_qbatch: mc_points must have 1 to %d rows" % _engine.MAX_IPV_POINTS)
+        # candidates and integration points are ranked together against the training inputs, as qNEI's baseline
+        rows = torch.cat([x.detach().double().reshape(-1, d), P.to(x.device)])
+        eng, xq, kw = self._joint_request(rows, True)
+        lv, nz = kw["level_idx"], kw["noise_idx"]
+        xq_i = np.ascontiguousarray(xq[n_c:])
+        lv_i = None if lv is None else np.ascontiguousarray(lv[n_c:])
+        st = self._ipv_state
+        if not (st is not None and st[0] is eng and st[1] == self._factor_key and np.array_equal(st[2], xq_i)
+                and (st[3] is None if lv_i is None else (st[3] is not None and np.array_equal(st[3], lv_i)))):
+            self._ipv_state = None
+            eng.ipv_points(xq_i, level_idx=lv_i)
+            self._ipv_state = (eng, self._factor_key, xq_i, lv_i)
+        kwargs = dict(level_idx=None if lv is None else np.ascontiguousarray(lv[:n_c]),
+                      noise_idx=None if nz is None else np.ascontiguousarray(nz[:n_c]))
+        xq_c = np.ascontiguousarray(xq[:n_c])
+        if torch.is_grad_enabled() and X.requires_grad:
+            v, jitter = _EngineNIPV.apply(x, eng, xq_c, q, self._quant_columns(), kwargs)
+        else:
+            values, _, jitter = eng.nipv_qbatch(xq_c, q, want_grad=False, **kwargs)
+            v, jitter = torch.as_tensor(np.asarray(values)), torch.as_tensor(np.asarray(jitter))
+        if bool((jitter > 0).any()):
+            warnings.warn("A not p.d., added jitter of %.1e to the diagonal" % float(jitter.max()), NumericalWarning)
+        y_std = self.y_std.to(self._out_dtype())
+        return (y_std * y_std * v.to(self._out_dtype())).reshape(batch)
 
     def reset_parameters(self) -> None:
         """Reset parameters by sampling from the priors (gpregression.py:168-174)."""

@@ -16,6 +16,8 @@
  *                                 models/gpregression.py:151-166 -> gpp_posterior_qbatch, gpp_posterior_qbatch_grad
  *   - botorch qEI / qNEI / qUCB (MC acquisition on posterior(X).rsample with shared base samples) and their
  *     gradients in X: GPR.acquisition_qbatch, bayesian_optimizations/qbatch.py -> gpp_acq_qbatch
+ *   - botorch qNegIntegratedPosteriorVariance and its gradient in X: GPR.acquisition_qbatch(X, "qNIPV", mc_points)
+ *                                 -> gpp_ipv_points, gpp_nipv_qbatch
  *   - AF_*_Engineering + argmax   bayesian_optimizations/AFs.py:102-159,
  *                                 bayesian_optimizations/BO_GP_plus.py:183-194 -> gpp_acq_argmax
  *   - covar_module(x).evaluate()  models/gp_plus.py:472-474      -> gpp_covariance
@@ -261,6 +263,39 @@ int gpp_acq_qbatch(gpp_handle* h, int64_t b, int32_t q_tot, const double* xq, co
                    double* values,                                  /* [b] */
                    double* d_xq,                                    /* [b * q_tot * dq] or NULL: values only */
                    double* jitter);                                 /* [b] or NULL */
+
+/* Batch integrated posterior variance (botorch's qNegIntegratedPosteriorVariance, acquisition/active_learning.py:
+ * qNegIntegratedPosteriorVariance.forward, which averages posterior(mc_points).variance of
+ * model.fantasize(X_t, observation_noise=True) over the integration points).  The fantasised variance does not depend
+ * on the fantasised y, so the engine evaluates the closed form below; all quantities are in scaled y units.
+ *
+ * gpp_ipv_points stores the integration set X_I of m points (1 <= m <= GPP_MAX_IPV_POINTS) on the handle: its point
+ * panels, U_I = K(X_I, X) L^-T, V_I = U_I L^-1 and vbar = (1/m) sum_m v_m with v_m = sf2 - |U_m|^2 (gpp_predict's
+ * variance without noise or clamp).  Pointer conventions as gpp_predict (host or device, cudaMemcpyDefault).  The set
+ * stays valid until the factor or the hyper-parameters of the handle change (gpp_factorize, gpp_mll_grad, the
+ * gpp_objective calls, gpp_covariance); it then has to be stored again.  It takes [mp x Np] doubles twice (mp = m
+ * rounded up to 128) plus the panels, held from the first call and freed with the handle.
+ *
+ * gpp_nipv_qbatch evaluates b t-batches of q rows against the stored set.  Per t-batch t, with Sigma_t bitwise
+ * gpp_posterior_qbatch's:
+ *   C_t = K(X_I, X_t) - U_I U_t^T                                    [m x q] posterior cross-covariance
+ *   A_t = Sigma_t + diag(noise of each row's group) + j_t I         j_t the first of 0, 1e-8, 1e-7, 1e-6 that factors
+ *   values[t] = -vbar + (1/m) tr(A_t^-1 C_t^T C_t)                   minus the mean posterior variance over X_I after
+ *                                                                    also observing X_t
+ *   d_xq [b*q*dq] = d(sum_t values[t]) / d xq, quantitative inputs only (NULL: values only)
+ *   jitter [b] = j_t (may be NULL)
+ * A t-batch's outputs do not depend on the other t-batches of the call or on how it is split into chunks.  The call
+ * does not change the factor of K_y, alpha, gpp_get_stats or gpp_get_timings.  GPP_ERR_NOT_PD when a t-batch fails
+ * every rung, GPP_ERR_NAN on NaN.  No valid integration set, q outside [1, GPP_MAX_QBATCH], b < 0, a missing values
+ * or dq > 32 return GPP_ERR_ARG before any allocation.  One chunk's C^T (at most 1 GiB), q x q blocks and gradient
+ * partials are held on the device from the first call and freed with the handle. */
+#define GPP_MAX_IPV_POINTS 16384
+int gpp_ipv_points(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx);
+int gpp_nipv_qbatch(gpp_handle* h, int64_t b, int32_t q, const double* xq, const int32_t* level_idx,
+                    const int32_t* noise_idx,
+                    double* values,   /* [b] */
+                    double* d_xq,     /* [b * q * dq] or NULL: values only */
+                    double* jitter);  /* [b] or NULL */
 
 /* fused predict + acquisition + argmax over m candidates (BO_GP_plus.py:183-194).
  * y_min/y_std undo the target scaling; cost_idx[m] selects cost[n_cost]; kind_by_cost[n_cost]
