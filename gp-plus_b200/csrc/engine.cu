@@ -65,6 +65,50 @@ struct CreateConfig {
     OzSchedule oz;         // used when the handle carries an OzCtx
 };
 
+template <typename Tp>
+static cudaError_t dev_alloc(Tp** p, size_t count) {
+    return cudaMalloc((void**)p, std::max<size_t>(count, 1) * sizeof(Tp));
+}
+
+// Grow-only device array of the prediction workspace, allocated on first use.  reserve() keeps the storage when it
+// holds `count` elements already; otherwise it waits for the stream, frees the storage and allocates `count` elements,
+// zero-filled when asked.  The storage is freed with the array, i.e. with the handle.
+template <typename Tp>
+struct DevArray {
+    Tp* p = nullptr;
+    size_t cap = 0;  // elements
+    DevArray() = default;
+    DevArray(const DevArray&) = delete;
+    DevArray& operator=(const DevArray&) = delete;
+    ~DevArray() { release(); }
+    operator Tp*() const { return p; }
+    void release() {
+        if (p) cudaFree(p);
+        p = nullptr;
+        cap = 0;
+    }
+    cudaError_t reserve(long long count, cudaStream_t st, bool zero = false) {
+        if (count <= (long long)cap) return cudaSuccess;
+        cudaError_t e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) return e;
+        release();
+        if ((e = dev_alloc(&p, (size_t)count)) != cudaSuccess) {
+            p = nullptr;
+            return e;
+        }
+        cap = (size_t)count;
+        return zero ? cudaMemsetAsync(p, 0, sizeof(Tp) * (size_t)count, st) : cudaSuccess;
+    }
+};
+
+// Candidate points kept on the handle between calls (the joint set, the integration set): their inputs and prepared
+// panels, m points padded to mp rows, and U = K* L^-T [mp x Np] (load_point_set)
+struct PointSet {
+    long long mp = 0;  // rows of the set last loaded (the panels' leading dimension)
+    DevArray<double> xq, xs, nrm, zpt, U;
+    DevArray<int> lvl;
+};
+
 struct gpp_handle {
     int device = 0;
     cudaStream_t st = nullptr;
@@ -94,51 +138,38 @@ struct gpp_handle {
     double* gz_host = nullptr;   // pinned
     int res_len = 0;
     std::vector<int> level_idx_host;
-    // prediction chunk buffers
+    // prediction workspace (DESIGN.md §3).  Chunk buffers of mc_alloc rows (their leading dimension):
     long long mc_alloc = 0;
-    double *c_xq = nullptr, *c_xs = nullptr, *c_nrm = nullptr, *c_zpt = nullptr, *c_K = nullptr;
-    int *c_lvl = nullptr, *c_noise = nullptr, *c_mean = nullptr, *c_cost = nullptr;
-    double *c_mean_part = nullptr, *c_rowsq = nullptr, *c_mu = nullptr, *c_var = nullptr, *c_score = nullptr;
-    double* c_blk_best = nullptr;
-    long long* c_blk_idx = nullptr;
-    // prediction-gradient buffers (gpp_predict_grad only; allocated on its first call)
-    long long g_alloc = 0;  // mc_alloc they were sized for
-    long long g_step = 0;   // candidates per chunk on that path
-    double *g_U = nullptr, *g_part_m = nullptr, *g_part_v = nullptr, *g_dmean = nullptr, *g_dvar = nullptr;
-    // joint-posterior buffers (gpp_predict_joint / gpp_sample_posterior only; allocated on their first call, they only
-    // grow).  Candidate rows are padded to j_mp; the diagonal-block inverses of L* take a full [j_mp x j_mp] matrix
-    // because potrf_blocked addresses them with the leading dimension of Sigma*.
-    long long j_mp = 0;  // candidate rows the buffers below hold
-    long long j_draw_cap = 0;  // doubles in each of the base-sample / draw chunk buffers (j_E, j_Y)
-    double *j_xq = nullptr, *j_xs = nullptr, *j_nrm = nullptr, *j_zpt = nullptr, *j_U = nullptr, *j_S = nullptr;
-    double *j_Minv = nullptr, *j_diag = nullptr, *j_mu = nullptr, *j_logdet = nullptr, *j_E = nullptr, *j_Y = nullptr;
-    int *j_lvl = nullptr, *j_noise = nullptr, *j_info = nullptr;
-    // t-batch posterior buffers (gpp_posterior_qbatch[_grad] only; allocated on their first call): one chunk's q x q
-    // blocks (Sigma out, or the upstream gradient G in) and its upstream mean gradient in the tile layout
-    long long q_rows = 0;  // g_step they were sized for
-    long long q_cap = 0;   // doubles in q_buf
-    double *q_buf = nullptr, *q_gm = nullptr;
-    // Monte-Carlo acquisition buffers (gpp_acq_qbatch only; allocated on its first call, they only grow): the base
-    // samples of the call, one chunk's values and jitters, and the status word of the call
-    long long a_e_cap = 0, a_chunk_cap = 0;
-    double *a_E = nullptr, *a_val = nullptr, *a_jit = nullptr;
-    int* a_info = nullptr;
-    // integration set of gpp_nipv_qbatch (gpp_ipv_points; the buffers only grow and are freed with the handle): point
-    // panels of i_m points padded to i_mp rows, U_I = K_I L^-T and V_I = U_I L^-1 [i_mp x Np], a zero vector in the
+    DevArray<double> c_xq, c_xs, c_nrm, c_zpt, c_K, c_mean_part, c_rowsq, c_mu, c_var, c_score, c_blk_best;
+    DevArray<int> c_lvl, c_noise, c_mean, c_cost;
+    DevArray<long long> c_blk_idx;
+    DevArray<double> acq_par;  // gpp_acq_argmax: [cost n_cost | best_f n_cost]
+    DevArray<int> acq_kind;
+    // gradient and t-batch paths: chunks of g_step rows with U = K* L^-T stored, the gradient partials and results
+    long long g_step = 0;
+    DevArray<double> g_U, g_part_m, g_part_v, g_dmean, g_dvar;
+    // t-batch paths: one chunk's q x q blocks (Sigma out, or the upstream gradient G in) and its upstream mean gradient
+    DevArray<double> q_buf, q_gm;
+    // gpp_acq_qbatch / gpp_nipv_qbatch: the base samples of the call, one chunk's values and jitters, the status word
+    DevArray<double> a_E, a_val, a_jit;
+    DevArray<int> a_info;
+    // gpp_predict_joint / gpp_sample_posterior: the joint set and, ld the call's mp, Sigma* (then L*), the diagonal-block
+    // inverses of L* (a full [mp x mp] matrix: potrf_blocked addresses them with Sigma*'s leading dimension), the
+    // diagonal additions, mu, the log-determinant partials, the noise groups, the status word, and one chunk of base
+    // samples and draws
+    PointSet jset;
+    DevArray<double> j_S, j_Minv, j_diag, j_mu, j_logdet, j_E, j_Y;
+    DevArray<int> j_noise, j_info;
+    // integration set of gpp_nipv_qbatch (gpp_ipv_points): i_m points, V_I = U_I L^-1 [mp x Np], a zero vector in the
     // place of alpha, the mean latent variance, and the factor generation the set was built for
-    long long i_m = 0, i_mp = 0, i_cap = 0, i_gen = -1;
+    PointSet iset;
+    long long i_m = 0, i_gen = -1;
     double i_vbar = 0.0;
-    double *i_xq = nullptr, *i_xs = nullptr, *i_nrm = nullptr, *i_zpt = nullptr, *i_U = nullptr, *i_V = nullptr;
-    double* i_zero = nullptr;
-    int* i_lvl = nullptr;
-    // gpp_nipv_qbatch chunk buffers (they only grow): C^T [rows x i_mp], one chunk's Gram and A^-1 blocks, and the
-    // gradient partials over the training and the integration column tiles
-    long long n_ccap = 0, n_bcap = 0, n_pcap = 0;
-    double *n_C = nullptr, *n_G = nullptr, *n_Ai = nullptr, *n_pm = nullptr, *n_pv = nullptr;
+    DevArray<double> i_V, i_zero;
+    // gpp_nipv_qbatch chunks: C^T [rows x mp of the set], the Gram and A^-1 blocks, and the gradient partials over the
+    // training and the integration column tiles
+    DevArray<double> n_C, n_G, n_Ai, n_pm, n_pv;
     long long fgen = 0;  // bumped whenever the factor (or its hyper-parameters) changes
-    double* acq_par = nullptr;  // [cost n_cost | best_f n_cost]
-    int* acq_kind = nullptr;
-    int acq_cap = 0;
     bool factorized = false;
     double last_jitter = 0.0;
     cudaEvent_t ev[EV_COUNT];
@@ -196,25 +227,11 @@ extern "C" const char* gpp_last_error(void) { return g_err.c_str(); }
 
 extern "C" long long gpp_launch_count(void) { return g_launches.load(); }
 
-template <typename Tp>
-static cudaError_t dev_alloc(Tp** p, size_t count) {
-    return cudaMalloc((void**)p, std::max<size_t>(count, 1) * sizeof(Tp));
-}
-
 static void destroy_now(gpp_handle* h) {
     if (!h) return;
     cudaSetDevice(h->device);
     if (h->st) cudaStreamSynchronize(h->st);
-    void* dptrs[] = {h->slab, h->c_xq, h->c_xs, h->c_nrm, h->c_zpt, h->c_K, h->c_lvl,
-                     h->c_noise, h->c_mean, h->c_cost, h->c_mean_part, h->c_rowsq, h->c_mu, h->c_var, h->c_score,
-                     h->c_blk_best, h->c_blk_idx, h->acq_par, h->acq_kind, h->g_U, h->g_part_m, h->g_part_v,
-                     h->g_dmean, h->g_dvar, h->j_xq, h->j_xs, h->j_nrm, h->j_zpt, h->j_U, h->j_S, h->j_Minv,
-                     h->j_diag, h->j_mu, h->j_logdet, h->j_E, h->j_Y, h->j_lvl, h->j_noise, h->j_info,
-                     h->q_buf, h->q_gm, h->a_E, h->a_val, h->a_jit, h->a_info,
-                     h->i_xq, h->i_xs, h->i_nrm, h->i_zpt, h->i_U, h->i_V, h->i_zero, h->i_lvl, h->n_C, h->n_G,
-                     h->n_Ai, h->n_pm, h->n_pv};
-    for (void* p : dptrs)
-        if (p) cudaFree(p);
+    if (h->slab) cudaFree(h->slab);
     if (h->pinned_slab) cudaFreeHost(h->pinned_slab);
     for (int i = 0; i < EV_COUNT; i++) cudaEventDestroy(h->ev[i]);
     if (h->ev_info) cudaEventDestroy(h->ev_info);
@@ -303,7 +320,7 @@ extern "C" void gpp_destroy(gpp_handle* h) {
     const char* e = getenv("GPP_POOL");
     const bool pooling = !(e && atoi(e) == 0);
     // a handle that has predicted (chunk or joint buffers allocated) is never parked
-    if (pooling && h->slab_bytes <= kPoolMaxHandleBytes && h->mc_alloc == 0 && h->j_mp == 0) {
+    if (pooling && h->slab_bytes <= kPoolMaxHandleBytes && h->mc_alloc == 0 && h->jset.mp == 0) {
         cudaSetDevice(h->device);
         if (h->st) cudaStreamSynchronize(h->st);
         std::lock_guard<std::mutex> lk(g_pool_mu);
@@ -620,30 +637,74 @@ static void fill_hyper_host(gpp_handle* h, const gpp_hyper* hy, double jitter) {
     h->sf2 = hy->sigma_f2;
 }
 
-// upload the staged hyper-parameters and prepare the per-point panels of the training set
-static int stage_prep(gpp_handle* h) {
-    CK(cudaMemcpyAsync(h->hyp, h->hyp_host, sizeof(double) * h->hyp_len, cudaMemcpyHostToDevice, h->st));
+// point panels of n points (rows np, padding rows zero) from their inputs xq [n x dq] and latent levels (NULL without a
+// latent map) with the current hyper-parameters; xst, the feature-major copy, may be NULL
+static int prep_panels(gpp_handle* h, const double* xq, const int* level_idx, long long n, long long np, double* xs,
+                       double* xst, double* nrm, double* zpt) {
     PrepArgs pa;
-    pa.xq = h->xq;
-    pa.level_idx = h->level_idx;
+    pa.xq = xq;
+    pa.level_idx = level_idx;
     pa.w = hyp_w(h);
     pa.centre = h->centre;
     pa.ztab = hyp_z(h);
-    pa.n = (int)h->n;
-    pa.np = (int)h->np;
+    pa.n = (int)n;
+    pa.np = (int)np;
     pa.dq = h->dq;
     pa.dqp = h->dqp;
     pa.dz = h->dz;
     pa.n_combo = h->n_combo;
     pa.n_pass = h->n_pass;
-    pa.xs = h->xs;
-    pa.xst = h->xst;
-    pa.nrm = h->nrm;
-    pa.zpt = h->zpt;
-    const int nb = (int)((h->np + 255) / 256);
-    prep_points_kernel<<<nb, 256, 0, h->st>>>(pa);
+    pa.xs = xs;
+    pa.xst = xst;
+    pa.nrm = nrm;
+    pa.zpt = zpt;
+    prep_points_kernel<<<(int)((np + 255) / 256), 256, 0, h->st>>>(pa);
     CK(cudaGetLastError());
     count_launch();
+    return GPP_OK;
+}
+
+// prepared panels of a set of points as rows or columns of a covariance block: n points in `tiles` 128-row tiles,
+// xs [tiles*128 x dqp], nrm, and n_pass latent tables of zs doubles each from zpt
+struct Panels {
+    const double *xs, *nrm, *zpt;
+    long long zs;
+    int n, tiles;
+};
+
+static Panels training_panels(const gpp_handle* h) { return {h->xs, h->nrm, h->zpt, h->np * ZP, (int)h->n, h->T}; }
+
+// covariance block of the rows r against the columns c, K = (1/n_pass) sum_p K_p: one launch per latent table.  `ca`
+// carries the block's own options (out, ld, tri, same, pad_identity, sf2_dev, diag_add, alpha, mean_part, ld_part).
+static int launch_cov_passes(const gpp_handle* h, CovArgs ca, const Panels& r, const Panels& c) {
+    ca.xs_r = r.xs;
+    ca.nrm_r = r.nrm;
+    ca.n_r = r.n;
+    ca.tiles_r = r.tiles;
+    ca.xs_c = c.xs;
+    ca.nrm_c = c.nrm;
+    ca.n_c = c.n;
+    ca.tiles_c = c.tiles;
+    ca.dqp = h->dqp;
+    ca.dz = h->dz;
+    ca.sf2 = h->sf2;
+    ca.scale = 1.0 / (double)h->n_pass;
+    for (int p = 0; p < h->n_pass; p++) {
+        ca.zpt_r = r.zpt + (size_t)p * r.zs;
+        ca.zpt_c = c.zpt + (size_t)p * c.zs;
+        ca.accum = p > 0;
+        ca.last = p == h->n_pass - 1;
+        CK(launch_cov(ca, h->kernel, h->st));
+    }
+    return GPP_OK;
+}
+
+// upload the staged hyper-parameters and prepare the per-point panels of the training set
+static int stage_prep(gpp_handle* h) {
+    CK(cudaMemcpyAsync(h->hyp, h->hyp_host, sizeof(double) * h->hyp_len, cudaMemcpyHostToDevice, h->st));
+    int rc = prep_panels(h, h->xq, h->level_idx, h->n, h->np, h->xs, h->xst, h->nrm, h->zpt);
+    if (rc != GPP_OK) return rc;
+    const int nb = (int)((h->np + 255) / 256);
     prep_targets_kernel<<<nb, 256, 0, h->st>>>(h->y, h->mean_idx, hyp_beta(h), h->n_mean, h->noise_idx, hyp_noise(h),
                                                 h->n_noise, 0.0, hyp_jitter(h), (int)h->n, (int)h->np, h->r,
                                                 h->diag_add);
@@ -657,27 +718,15 @@ static int stage_factor(gpp_handle* h) {
     CK(cudaMemsetAsync(h->info, 0, sizeof(int), h->st));
     CovArgs ca;
     memset(&ca, 0, sizeof(ca));
-    ca.xs_r = ca.xs_c = h->xs;
-    ca.nrm_r = ca.nrm_c = h->nrm;
     ca.out = h->A;
     ca.ld = h->np;
-    ca.n_r = ca.n_c = (int)h->n;
-    ca.tiles_r = ca.tiles_c = h->T;
     ca.tri = 1;
     ca.same = 1;
     ca.pad_identity = 1;
-    ca.dqp = h->dqp;
-    ca.dz = h->dz;
-    ca.sf2 = h->sf2;
     ca.sf2_dev = hyp_sf2(h);
     ca.diag_add = h->diag_add;
-    ca.scale = 1.0 / (double)h->n_pass;
-    for (int p = 0; p < h->n_pass; p++) {  // K = (1/k) sum_p K_p: one launch per latent table
-        ca.zpt_r = ca.zpt_c = h->zpt + (size_t)p * h->np * ZP;
-        ca.accum = p > 0;
-        ca.last = p == h->n_pass - 1;
-        CK(launch_cov(ca, h->kernel, h->st));
-    }
+    int rc = launch_cov_passes(h, ca, training_panels(h), training_panels(h));
+    if (rc != GPP_OK) return rc;
     mark(h, EV_COV);
     if (h->cfg.small_block > 0 && h->T <= 16) {
         // small problems: the whole factorisation is one dataflow launch (block_potrf_kernel) instead of a chain of
@@ -1114,25 +1163,10 @@ extern "C" int gpp_covariance(gpp_handle* h, const gpp_hyper* hy, double* k_out)
     if ((rc = stage_prep(h)) != GPP_OK) return rc;
     CovArgs ca;
     memset(&ca, 0, sizeof(ca));
-    ca.xs_r = ca.xs_c = h->xs;
-    ca.nrm_r = ca.nrm_c = h->nrm;
     ca.out = h->S;
     ca.ld = h->np;
-    ca.n_r = ca.n_c = (int)h->n;
-    ca.tiles_r = ca.tiles_c = h->T;
-    ca.tri = 0;
     ca.same = 1;
-    ca.pad_identity = 0;
-    ca.dqp = h->dqp;
-    ca.dz = h->dz;
-    ca.sf2 = h->sf2;
-    ca.scale = 1.0 / (double)h->n_pass;
-    for (int p = 0; p < h->n_pass; p++) {
-        ca.zpt_r = ca.zpt_c = h->zpt + (size_t)p * h->np * ZP;
-        ca.accum = p > 0;
-        ca.last = p == h->n_pass - 1;
-        CK(launch_cov(ca, h->kernel, h->st));
-    }
+    if ((rc = launch_cov_passes(h, ca, training_panels(h), training_panels(h))) != GPP_OK) return rc;
     CK(cudaMemcpy2DAsync(k_out, sizeof(double) * h->n, h->S, sizeof(double) * h->np, sizeof(double) * h->n, h->n,
                          cudaMemcpyDefault, h->st));
     CK(cudaStreamSynchronize(h->st));
@@ -1185,63 +1219,85 @@ extern "C" int gpp_factorize(gpp_handle* h, const gpp_hyper* hy) {
 }
 
 // ---------------------------------------------------------------------------------------------
+// Prediction.  Candidate rows reach mean and variance through the chunk front (K* against the training set, U = K* L^-T,
+// predict_finish_kernel) in chunks of at most mc_alloc rows.  Three caller families each run their own chunk loop and
+// add their own stages:
+//   pointwise  gpp_predict, gpp_predict_grad, gpp_acq_argmax (predict_rows)
+//   point set  J1 of gpp_predict_joint / gpp_sample_posterior, gpp_ipv_points (load_point_set)
+//   t-batch    gpp_posterior_qbatch[_grad], gpp_acq_qbatch, gpp_nipv_qbatch (qbatch_front and the qbatch_* stages)
+static long long round128(long long x) { return (x + 127) / 128 * 128; }
+
+// a call's candidate rows as the caller passed them (host or device; noise_idx and mean_idx may be NULL) and the noise
+// setting and floor of their predictive variance
+struct Rows {
+    const double* xq;
+    const int32_t *level_idx, *noise_idx, *mean_idx;
+    int include_noise;
+    double min_var;
+};
+
+// The argument checks of every entry point that takes candidate rows, in the order they fire: `bad_count` is the entry
+// point's message for a count outside its range, or NULL; xq and level_idx are needed when there are rows.
+static int check_rows(const gpp_handle* h, const char* name, const char* bad_count, long long rows, const double* xq,
+                      const int32_t* level_idx) {
+    const char* why = nullptr;
+    if (!h) why = "null handle";
+    else if (!h->factorized) why = "call gpp_factorize (or gpp_mll_grad) first";
+    else if (bad_count) why = bad_count;
+    else if (h->dq > GPP_MAX_DQ) why = "at most GPP_MAX_DQ quantitative inputs";
+    else if (rows > 0 && h->dq > 0 && !xq) why = "xq missing";
+    else if (rows > 0 && h->dz > 0 && !level_idx) why = "level_idx missing";
+    if (!why) return GPP_OK;
+    g_err = std::string(name) + ": " + why;
+    return GPP_ERR_ARG;
+}
+
+// chunk buffers of mc_alloc rows, their leading dimension: it only grows, and a K* chunk holds at most 2^27 doubles
+// (1 GiB)
 static int ensure_chunk_buffers(gpp_handle* h, long long m) {
-    // K* chunk of at most 2^27 doubles (1 GiB)
-    long long cap = ((1LL << 27) / h->np) / 128 * 128;
-    if (cap < 128) cap = 128;
-    long long want = std::min((m + 127) / 128 * 128, cap);
-    if (want <= h->mc_alloc) return GPP_OK;
-    void* olds[] = {h->c_xq, h->c_xs, h->c_nrm, h->c_zpt, h->c_K, h->c_lvl, h->c_noise, h->c_mean, h->c_cost,
-                    h->c_mean_part, h->c_rowsq, h->c_mu, h->c_var, h->c_score, h->c_blk_best, h->c_blk_idx};
-    for (void* p : olds)
-        if (p) cudaFree(p);
-    h->c_xq = h->c_xs = h->c_nrm = h->c_zpt = h->c_K = nullptr;
-    h->c_lvl = h->c_noise = h->c_mean = h->c_cost = nullptr;
-    h->c_mean_part = h->c_rowsq = h->c_mu = h->c_var = h->c_score = h->c_blk_best = nullptr;
-    h->c_blk_idx = nullptr;
-    h->mc_alloc = 0;
-    const size_t mc = (size_t)want;
-    CK(dev_alloc(&h->c_xq, mc * std::max(h->dq, 1)));
-    CK(dev_alloc(&h->c_xs, mc * h->dqp));
-    CK(dev_alloc(&h->c_nrm, mc));
-    CK(dev_alloc(&h->c_zpt, mc * ZP * h->n_pass));
-    CK(dev_alloc(&h->c_K, mc * (size_t)h->np));
-    CK(dev_alloc(&h->c_lvl, mc));
-    CK(dev_alloc(&h->c_noise, mc));
-    CK(dev_alloc(&h->c_mean, mc));
-    CK(dev_alloc(&h->c_cost, mc));
-    CK(dev_alloc(&h->c_mean_part, mc * (size_t)h->T));
-    CK(dev_alloc(&h->c_rowsq, mc * (size_t)h->T));
-    CK(dev_alloc(&h->c_mu, mc));
-    CK(dev_alloc(&h->c_var, mc));
-    CK(dev_alloc(&h->c_score, mc));
-    CK(dev_alloc(&h->c_blk_best, mc / 256 + 1));
-    CK(dev_alloc(&h->c_blk_idx, mc / 256 + 1));
-    h->mc_alloc = want;
+    const long long cap = std::max(((1LL << 27) / h->np) / 128 * 128, 128LL);
+    const long long mc = std::max(h->mc_alloc, std::min(round128(m), cap));
+    cudaStream_t st = h->st;
+    CK(h->c_xq.reserve(mc * std::max(h->dq, 1), st));
+    CK(h->c_xs.reserve(mc * h->dqp, st));
+    CK(h->c_nrm.reserve(mc, st));
+    CK(h->c_zpt.reserve(mc * ZP * h->n_pass, st));
+    CK(h->c_K.reserve(mc * h->np, st));
+    CK(h->c_lvl.reserve(mc, st));
+    CK(h->c_noise.reserve(mc, st));
+    CK(h->c_mean.reserve(mc, st));
+    CK(h->c_cost.reserve(mc, st));
+    CK(h->c_mean_part.reserve(mc * h->T, st));
+    CK(h->c_rowsq.reserve(mc * h->T, st));
+    CK(h->c_mu.reserve(mc, st));
+    CK(h->c_var.reserve(mc, st));
+    CK(h->c_score.reserve(mc, st));
+    CK(h->c_blk_best.reserve(mc / 256 + 1, st));
+    CK(h->c_blk_idx.reserve(mc / 256 + 1, st));
+    h->mc_alloc = mc;
     return GPP_OK;
 }
 
-// U = K* L^-T of one chunk, the per-column-tile gradient partials and the chunk's gradients (gpp_predict_grad).  The
-// partials take T*dq doubles per candidate each, so this path caps its chunk at 2^24 / (T*dq) candidates (128 MiB per
-// partial buffer; 4096 candidates at N = 16384, dq = 32); mean and variance do not depend on the chunking.
+// U = K* L^-T of one chunk, the per-column-tile gradient partials and the chunk's gradients (gradient and t-batch
+// paths).  The partials take T*dq doubles per candidate each, so these paths cap their chunk at 2^24 / (T*dq)
+// candidates (128 MiB per partial buffer; 4096 candidates at N = 16384, dq = 32); mean and variance do not depend on
+// the chunking.
 static int ensure_grad_buffers(gpp_handle* h) {
-    if (h->g_alloc == h->mc_alloc) return GPP_OK;
-    void* olds[] = {h->g_U, h->g_part_m, h->g_part_v, h->g_dmean, h->g_dvar};
-    for (void* p : olds)
-        if (p) cudaFree(p);
-    h->g_U = h->g_part_m = h->g_part_v = h->g_dmean = h->g_dvar = nullptr;
-    h->g_alloc = h->g_step = 0;
     long long step = ((1LL << 24) / ((long long)h->T * std::max(h->dq, 1))) / 128 * 128;
     step = std::min(std::max(step, 128LL), h->mc_alloc);
-    const size_t sc = (size_t)step;
-    CK(dev_alloc(&h->g_U, sc * (size_t)h->np));
-    CK(dev_alloc(&h->g_part_m, sc * (size_t)h->T * h->dq));
-    CK(dev_alloc(&h->g_part_v, sc * (size_t)h->T * h->dq));
-    CK(dev_alloc(&h->g_dmean, sc * h->dq));
-    CK(dev_alloc(&h->g_dvar, sc * h->dq));
-    h->g_alloc = h->mc_alloc;
+    CK(h->g_U.reserve(step * h->np, h->st));
+    CK(h->g_part_m.reserve(step * h->T * h->dq, h->st));
+    CK(h->g_part_v.reserve(step * h->T * h->dq, h->st));
+    CK(h->g_dmean.reserve(step * h->dq, h->st));
+    CK(h->g_dvar.reserve(step * h->dq, h->st));
     h->g_step = step;
     return GPP_OK;
+}
+
+// prepared panels of the chunk buffers' first mc rows
+static Panels chunk_panels(const gpp_handle* h, long long mc) {
+    const long long mcp = round128(mc);
+    return {h->c_xs, h->c_nrm, h->c_zpt, mcp * ZP, (int)mc, (int)(mcp / CT)};
 }
 
 struct AcqSpec {
@@ -1257,176 +1313,144 @@ struct AcqSpec {
     long long best_index = -1;
 };
 
-// gpp_predict_joint: point panels of all m candidates, prepared once (ld mp), and the destination of U = K* L^-T
-struct JointDest {
-    const double *xs, *nrm, *zpt;  // [mp*dqp], [mp], [n_pass][mp*ZP]
-    long long mp;
-    double* U;                     // [mp x Np]
-};
+// The chunk front: rows [base, base + mc) of the call, their inputs and groups in the chunk buffers, to mean and
+// variance in c_mu / c_var.  `given` holds the rows' prepared panels (a point set), or is NULL: the panels are prepared
+// into c_xs / c_nrm / c_zpt here.  U = K* L^-T goes to U (ld Np) when given, else only its row sums of squares are kept
+// (bitwise the same either way).  `acq` adds the gpp_acq_argmax scores and per-block best.
+static int chunk_front(gpp_handle* h, const Rows& r, long long base, long long mc, const Panels* given, double* U,
+                       const AcqSpec* acq) {
+    const long long MC = h->mc_alloc;
+    const Panels rows = given ? *given : chunk_panels(h, mc);
+    int rc;
+    if (!given && (rc = prep_panels(h, h->c_xq, h->dz > 0 ? h->c_lvl.p : nullptr, mc, round128(mc), h->c_xs, nullptr,
+                                    h->c_nrm, h->c_zpt)) != GPP_OK)
+        return rc;
+    CovArgs ca;
+    memset(&ca, 0, sizeof(ca));
+    ca.out = h->c_K;
+    ca.ld = h->np;
+    ca.alpha = h->alpha;
+    ca.mean_part = h->c_mean_part;
+    ca.ld_part = MC;
+    if ((rc = launch_cov_passes(h, ca, rows, training_panels(h))) != GPP_OK) return rc;
 
-// gpp_acq_qbatch: the utility, its parameters in scaled units and the per-t-batch outputs
-struct QAcqSpec {
-    int kind, n_base, maximize;
-    double best_f, cbeta;
-    long long S;
-    const double* E;  // [S*q] caller's base samples
-    double* values;   // [b]
-    double* jitter;   // [b] or NULL
-};
+    GemmOp op = gemm_default();  // U = K* L^-T: its row sums of squares, and U itself when asked
+    op.A = h->c_K;
+    op.lda = (int)h->np;
+    op.B = h->M;
+    op.ldb = (int)h->np;
+    op.C = U;
+    op.ldc = U ? (int)h->np : 0;
+    op.tiles_m = op.tiles_m_last = rows.tiles;
+    op.tiles_n = h->T;
+    op.klo_c = 0;
+    op.khi_sel = KSEL_TJ;
+    op.khi_c = 1;
+    op.epilogue = U ? EPI_STORE_ROWSQ : EPI_ROWSQ;
+    op.rowsq = h->c_rowsq;
+    op.rowsq_ld = (int)MC;
+    CK(launch_gemm(op, true, true, 1, h->st));
 
-// gpp_nipv_qbatch: the per-t-batch outputs (the integration set lives on the handle)
-struct NipvSpec {
-    double* values;  // [b]
-    double* jitter;  // [b] or NULL
-};
-
-// gpp_posterior_qbatch[_grad]: b t-batches of q rows.  Every 128-row tile of the chunk buffers holds qpt = 128 / q whole
-// t-batches followed by padding rows, so chunks (multiples of 128 rows) hold whole t-batches.
-struct QBatchSpec {
-    long long b;
-    int q, qpt;
-    double* cov;           // forward: [b*q*q] or NULL
-    const double* g_mean;  // backward: [b*q] or NULL
-    const double* g_cov;   // backward: [b*q*q] or NULL
-    double* d_xq;          // backward: [b*q*dq]
-    const QAcqSpec* acq;   // gpp_acq_qbatch: Monte-Carlo acquisition of every t-batch, or NULL
-    const NipvSpec* ipv;   // gpp_nipv_qbatch: integrated posterior variance against the handle's set, or NULL
-};
-
-// rows of nbat t-batches, from t-batch bt0 of a compact [b*q rows] array, to (into_tiles) or from their tile slots in
-// a chunk buffer: one pitched copy for the full tiles, one plain copy for the last, partly filled one
-static cudaError_t qb_copy_rows(const QBatchSpec* qb, void* dst, const void* src, size_t row_bytes, long long bt0,
-                                long long nbat, bool into_tiles, cudaStream_t st) {
-    if (row_bytes == 0 || nbat <= 0) return cudaSuccess;
-    const size_t run = (size_t)qb->qpt * qb->q * row_bytes, tile = (size_t)CT * row_bytes;
-    const size_t off = (size_t)bt0 * qb->q * row_bytes;
-    char* d = (char*)dst + (into_tiles ? 0 : off);
-    const char* s = (const char*)src + (into_tiles ? off : 0);
-    const size_t dp = into_tiles ? tile : run, sp = into_tiles ? run : tile;
-    const long long full = nbat / qb->qpt, rest = nbat % qb->qpt;
-    if (full > 0) {
-        cudaError_t e = cudaMemcpy2DAsync(d, dp, s, sp, run, (size_t)full, cudaMemcpyDefault, st);
-        if (e != cudaSuccess) return e;
-    }
-    if (rest > 0)
-        return cudaMemcpyAsync(d + full * dp, s + full * sp, (size_t)rest * qb->q * row_bytes, cudaMemcpyDefault, st);
-    return cudaSuccess;
-}
-
-static int ensure_qbatch_buffers(gpp_handle* h, int q) {
-    const long long cap = h->g_step * q;
-    if (h->q_rows == h->g_step && cap <= h->q_cap) return GPP_OK;
-    if (h->q_buf) cudaFree(h->q_buf);
-    if (h->q_gm) cudaFree(h->q_gm);
-    h->q_buf = h->q_gm = nullptr;
-    h->q_rows = h->q_cap = 0;
-    CK(dev_alloc(&h->q_buf, (size_t)cap));
-    CK(dev_alloc(&h->q_gm, (size_t)h->g_step));
-    h->q_rows = h->g_step;
-    h->q_cap = cap;
-    return GPP_OK;
-}
-
-static int ensure_acq_buffers(gpp_handle* h, long long e_elems) {
-    if (!h->a_info) CK(dev_alloc(&h->a_info, 1));
-    if (e_elems > h->a_e_cap) {
-        if (h->a_E) cudaFree(h->a_E);
-        h->a_E = nullptr;
-        h->a_e_cap = 0;
-        CK(dev_alloc(&h->a_E, (size_t)e_elems));
-        h->a_e_cap = e_elems;
-    }
-    if (h->g_step > h->a_chunk_cap) {  // a chunk holds at most g_step t-batches
-        if (h->a_val) cudaFree(h->a_val);
-        if (h->a_jit) cudaFree(h->a_jit);
-        h->a_val = h->a_jit = nullptr;
-        h->a_chunk_cap = 0;
-        CK(dev_alloc(&h->a_val, (size_t)h->g_step));
-        CK(dev_alloc(&h->a_jit, (size_t)h->g_step));
-        h->a_chunk_cap = h->g_step;
-    }
-    return GPP_OK;
-}
-
-// rows of one gpp_nipv_qbatch chunk: the C^T buffer [rows x i_mp] holds at most 2^27 doubles (1 GiB)
-static long long nipv_step(const gpp_handle* h) {
-    return std::min(h->g_step, std::max(128LL, ((1LL << 27) / h->i_mp) / 128 * 128));
-}
-
-// C^T of one chunk, its q x q Gram and A^-1 blocks and, with the gradient, the partials of predict_grad_tile_kernel
-// over the T training and i_mp / 128 integration column tiles (leading dimension rows)
-static int ensure_nipv_buffers(gpp_handle* h, long long rows, int q, bool grad) {
-    const long long c = rows * h->i_mp, blk = rows * q;
-    const long long part = grad ? rows * (h->T + h->i_mp / CT) * h->dq : 0;
-    if (c > h->n_ccap) {
-        if (h->n_C) cudaFree(h->n_C);
-        h->n_C = nullptr;
-        h->n_ccap = 0;
-        CK(dev_alloc(&h->n_C, (size_t)c));
-        h->n_ccap = c;
-    }
-    if (blk > h->n_bcap) {
-        if (h->n_G) cudaFree(h->n_G);
-        if (h->n_Ai) cudaFree(h->n_Ai);
-        h->n_G = h->n_Ai = nullptr;
-        h->n_bcap = 0;
-        CK(dev_alloc(&h->n_G, (size_t)blk));
-        CK(dev_alloc(&h->n_Ai, (size_t)blk));
-        h->n_bcap = blk;
-    }
-    if (part > h->n_pcap) {
-        if (h->n_pm) cudaFree(h->n_pm);
-        if (h->n_pv) cudaFree(h->n_pv);
-        h->n_pm = h->n_pv = nullptr;
-        h->n_pcap = 0;
-        CK(dev_alloc(&h->n_pm, (size_t)part));
-        CK(dev_alloc(&h->n_pv, (size_t)part));
-        h->n_pcap = part;
-    }
-    return GPP_OK;
-}
-
-static int predict_impl(gpp_handle* h, long long m, const double* xq, const int32_t* level_idx,
-                        const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, double min_var,
-                        double* mean, double* var, AcqSpec* acq, bool grad = false, double* d_mean = nullptr,
-                        double* d_var = nullptr, const JointDest* jd = nullptr, const QBatchSpec* qb = nullptr) {
-    if (!h->factorized) ARG_FAIL("predict: call gpp_factorize (or gpp_mll_grad) first");
-    if (m <= 0) return GPP_OK;
-    if (h->dq > 0 && !xq) ARG_FAIL("predict: xq missing");
-    if (h->dz > 0 && !level_idx) ARG_FAIL("predict: level_idx missing");
-    CK(cudaSetDevice(h->device));
-    int rc = ensure_chunk_buffers(h, m);
-    if (rc != GPP_OK) return rc;
-    const bool keep_u = grad || qb;  // U = K* L^-T stored per chunk, in chunks of the gradient path
-    if (keep_u) {
-        rc = ensure_grad_buffers(h);
-        if (rc != GPP_OK) return rc;
-    }
-    if (qb && (rc = ensure_qbatch_buffers(h, qb->q)) != GPP_OK) return rc;
-    const QAcqSpec* qa = qb ? qb->acq : nullptr;
-    if (qa) {
-        if ((rc = ensure_acq_buffers(h, qa->S * qb->q)) != GPP_OK) return rc;
-        CK(cudaMemcpyAsync(h->a_E, qa->E, sizeof(double) * qa->S * qb->q, cudaMemcpyDefault, h->st));
-        CK(cudaMemsetAsync(h->a_info, 0, sizeof(int), h->st));
-    }
-    const NipvSpec* nv = qb ? qb->ipv : nullptr;
-    if (nv) {  // values, jitters and the status word in the acquisition buffers (no base samples)
-        if ((rc = ensure_acq_buffers(h, 0)) != GPP_OK) return rc;
-        if ((rc = ensure_nipv_buffers(h, nipv_step(h), qb->q, grad)) != GPP_OK) return rc;
-        CK(cudaMemsetAsync(h->a_info, 0, sizeof(int), h->st));
-    }
-    const int imt = nv ? (int)(h->i_mp / CT) : 0;  // integration column tiles
+    PredFinishArgs fa;
+    memset(&fa, 0, sizeof(fa));
+    fa.mean_part = h->c_mean_part;
+    fa.rowsq = h->c_rowsq;
+    fa.ldp = MC;
+    fa.tiles_c = h->T;
+    fa.m = (int)mc;
+    fa.base = base;
+    fa.sf2 = h->sf2;
+    fa.mean_idx = r.mean_idx ? h->c_mean.p : nullptr;
+    fa.beta = hyp_beta(h);
+    fa.n_mean = h->n_mean;
+    fa.noise_idx = r.noise_idx ? h->c_noise.p : nullptr;
+    fa.noise = hyp_noise(h);
+    fa.n_noise = h->n_noise;
+    fa.include_noise = r.include_noise;
+    fa.min_var = r.min_var;
+    fa.mean_out = h->c_mu;
+    fa.var_out = h->c_var;
     if (acq) {
-        if (acq->n_cost <= 0 || !acq->cost || !acq->kind_by_cost || !acq->best_f) ARG_FAIL("acq: cost tables missing");
-        if (acq->n_cost > h->acq_cap) {
-            if (h->acq_par) cudaFree(h->acq_par);
-            if (h->acq_kind) cudaFree(h->acq_kind);
-            h->acq_par = nullptr;
-            h->acq_kind = nullptr;
-            CK(dev_alloc(&h->acq_par, (size_t)2 * acq->n_cost));
-            CK(dev_alloc(&h->acq_kind, (size_t)acq->n_cost));
-            h->acq_cap = acq->n_cost;
-        }
+        fa.cost_idx = acq->cost_idx ? h->c_cost.p : nullptr;
+        fa.cost = h->acq_par;
+        fa.best_f = h->acq_par + acq->n_cost;
+        fa.kind_by_cost = h->acq_kind;
+        fa.n_cost = acq->n_cost;
+        fa.maximize = acq->maximize;
+        fa.si = acq->si;
+        fa.y_min = acq->y_min;
+        fa.y_std = acq->y_std;
+        fa.score_out = acq->scores ? h->c_score.p : nullptr;
+        fa.blk_best = h->c_blk_best;
+        fa.blk_idx = h->c_blk_idx;
+    }
+    predict_finish_kernel<<<(int)((mc + 255) / 256), 256, 0, h->st>>>(fa);
+    CK(cudaGetLastError());
+    count_launch();
+    return GPP_OK;
+}
+
+// V = U L^-1 = K* K_y^-1 of `tiles` row tiles, U [rows x Np] -> V [rows x Np]: B(tj, k) = L^-1[k, tj], k in [tj, T)
+static int v_gemm(gpp_handle* h, const double* U, double* V, int tiles) {
+    GemmOp vo = gemm_default();
+    vo.A = U;
+    vo.lda = (int)h->np;
+    vo.B = h->M;
+    vo.ldb = (int)h->np;
+    vo.C = V;
+    vo.ldc = (int)h->np;
+    vo.tiles_m = vo.tiles_m_last = tiles;
+    vo.tiles_n = h->T;
+    vo.klo_sel = KSEL_TJ;
+    vo.klo_c = 0;
+    vo.khi_c = h->T;
+    CK(launch_gemm(vo, true, false, 1, h->st));
+    return GPP_OK;
+}
+
+// predict_grad_tile_kernel partials [c.tiles * dq][ldp] of the rows r against the column points c: alpha weighs the
+// mean partials, V [rows x ldv] the variance partials
+static int grad_tiles(gpp_handle* h, const Panels& r, const Panels& c, const double* alpha, const double* V,
+                      long long ldv, double* part_m, double* part_v, long long ldp) {
+    PredGradArgs ga;
+    memset(&ga, 0, sizeof(ga));
+    ga.xs_r = r.xs;
+    ga.zpt_r = r.zpt;
+    ga.zs_r = r.zs;
+    ga.xs_c = c.xs;
+    ga.zpt_c = c.zpt;
+    ga.zs_c = c.zs;
+    ga.alpha = alpha;
+    ga.V = V;
+    ga.ldv = ldv;
+    ga.n_r = r.n;
+    ga.n_c = c.n;
+    ga.dq = h->dq;
+    ga.dqp = h->dqp;
+    ga.dz = h->dz;
+    ga.n_pass = h->n_pass;
+    ga.part_m = part_m;
+    ga.part_v = part_v;
+    ga.ldp = ldp;
+    CK(launch_predict_grad(ga, h->kernel, r.tiles, c.tiles, h->st));
+    return GPP_OK;
+}
+
+// gpp_predict, gpp_predict_grad (d_mean / d_var) and gpp_acq_argmax (acq): m rows in chunks of mc_alloc rows, of g_step
+// rows with the gradient
+static int predict_rows(gpp_handle* h, long long m, const Rows& r, double* mean, double* var, AcqSpec* acq,
+                        double* d_mean, double* d_var) {
+    int rc = check_rows(h, "predict", nullptr, m, r.xq, r.level_idx);
+    if (rc != GPP_OK || m <= 0) return rc;
+    if (acq && (acq->n_cost <= 0 || !acq->cost || !acq->kind_by_cost || !acq->best_f))
+        ARG_FAIL("acq: cost tables missing");
+    const bool grad = d_mean || d_var;
+    CK(cudaSetDevice(h->device));
+    if ((rc = ensure_chunk_buffers(h, m)) != GPP_OK) return rc;
+    if (grad && (rc = ensure_grad_buffers(h)) != GPP_OK) return rc;
+    if (acq) {
+        CK(h->acq_par.reserve(2 * acq->n_cost, h->st));
+        CK(h->acq_kind.reserve(acq->n_cost, h->st));
         CK(cudaMemcpyAsync(h->acq_par, acq->cost, sizeof(double) * acq->n_cost, cudaMemcpyDefault, h->st));
         CK(cudaMemcpyAsync(h->acq_par + acq->n_cost, acq->best_f, sizeof(double) * acq->n_cost, cudaMemcpyDefault,
                            h->st));
@@ -1434,423 +1458,42 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
     }
     std::vector<double> hb;
     std::vector<long long> hi;
-    const long long MC = h->mc_alloc;  // leading dimension of the chunk buffers
-    const long long step = nv ? nipv_step(h) : (keep_u ? h->g_step : MC);
+    const long long step = grad ? h->g_step : h->mc_alloc;
     for (long long base = 0; base < m; base += step) {
         const long long mc = std::min(step, m - base);
-        const long long mcp = (mc + 127) / 128 * 128;
-        const int tiles_r = (int)(mcp / 128);
-        // t-batches of this chunk (t-batch path): [bt0, bt0 + nbc)
-        const long long bt0 = qb ? base / CT * qb->qpt : 0;
-        const long long nbc = qb ? std::min(qb->b, bt0 + (long long)tiles_r * qb->qpt) - bt0 : 0;
-        if (qb) {  // scatter the rows into their tile slots; padding rows are zero points of level, group and mean 0
-            CK(cudaMemsetAsync(h->c_xq, 0, sizeof(double) * mcp * h->dq, h->st));
-            CK(cudaMemsetAsync(h->c_lvl, 0, sizeof(int) * mcp, h->st));
-            CK(cudaMemsetAsync(h->c_noise, 0, sizeof(int) * mcp, h->st));
-            CK(cudaMemsetAsync(h->c_mean, 0, sizeof(int) * mcp, h->st));
-            CK(qb_copy_rows(qb, h->c_xq, xq, sizeof(double) * h->dq, bt0, nbc, true, h->st));
-            if (h->dz > 0) CK(qb_copy_rows(qb, h->c_lvl, level_idx, sizeof(int), bt0, nbc, true, h->st));
-            if (noise_idx) CK(qb_copy_rows(qb, h->c_noise, noise_idx, sizeof(int), bt0, nbc, true, h->st));
-            if (mean_idx) CK(qb_copy_rows(qb, h->c_mean, mean_idx, sizeof(int), bt0, nbc, true, h->st));
-        } else {
-            if (h->dq > 0 && !jd)
-                CK(cudaMemcpyAsync(h->c_xq, xq + base * h->dq, sizeof(double) * mc * h->dq, cudaMemcpyDefault, h->st));
-            if (h->dz > 0 && !jd)
-                CK(cudaMemcpyAsync(h->c_lvl, level_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
-            if (noise_idx)
-                CK(cudaMemcpyAsync(h->c_noise, noise_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
-            if (mean_idx) CK(cudaMemcpyAsync(h->c_mean, mean_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
-        }
+        if (h->dq > 0)
+            CK(cudaMemcpyAsync(h->c_xq, r.xq + base * h->dq, sizeof(double) * mc * h->dq, cudaMemcpyDefault, h->st));
+        if (h->dz > 0) CK(cudaMemcpyAsync(h->c_lvl, r.level_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
+        if (r.noise_idx)
+            CK(cudaMemcpyAsync(h->c_noise, r.noise_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
+        if (r.mean_idx) CK(cudaMemcpyAsync(h->c_mean, r.mean_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
         if (acq && acq->cost_idx)
             CK(cudaMemcpyAsync(h->c_cost, acq->cost_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
-        PrepArgs pa;
-        pa.xq = h->c_xq;
-        pa.level_idx = h->dz > 0 ? h->c_lvl : nullptr;
-        pa.w = hyp_w(h);
-        pa.centre = h->centre;
-        pa.ztab = hyp_z(h);
-        pa.n = (int)mc;
-        pa.np = (int)mcp;
-        pa.dq = h->dq;
-        pa.dqp = h->dqp;
-        pa.dz = h->dz;
-        pa.n_combo = h->n_combo;
-        pa.n_pass = h->n_pass;
-        pa.xs = h->c_xs;
-        pa.xst = nullptr;
-        pa.nrm = h->c_nrm;
-        pa.zpt = h->c_zpt;
-        if (!jd) {
-            prep_points_kernel<<<(int)((mcp + 255) / 256), 256, 0, h->st>>>(pa);
-            CK(cudaGetLastError());
-            count_launch();
-        }
-
-        CovArgs ca;
-        memset(&ca, 0, sizeof(ca));
-        ca.xs_r = jd ? jd->xs + base * h->dqp : h->c_xs;
-        ca.nrm_r = jd ? jd->nrm + base : h->c_nrm;
-        ca.xs_c = h->xs;
-        ca.nrm_c = h->nrm;
-        ca.out = h->c_K;
-        ca.ld = h->np;
-        ca.n_r = (int)mc;
-        ca.n_c = (int)h->n;
-        ca.tiles_r = tiles_r;
-        ca.tiles_c = h->T;
-        ca.dqp = h->dqp;
-        ca.dz = h->dz;
-        ca.sf2 = h->sf2;
-        ca.alpha = h->alpha;
-        ca.mean_part = h->c_mean_part;
-        ca.ld_part = MC;
-        ca.scale = 1.0 / (double)h->n_pass;
-        for (int p = 0; p < h->n_pass; p++) {
-            ca.zpt_r = jd ? jd->zpt + ((size_t)p * jd->mp + base) * ZP : h->c_zpt + (size_t)p * mcp * ZP;
-            ca.zpt_c = h->zpt + (size_t)p * h->np * ZP;
-            ca.accum = p > 0;
-            ca.last = p == h->n_pass - 1;
-            CK(launch_cov(ca, h->kernel, h->st));
-        }
-
-        GemmOp op = gemm_default();  // V = K* L^-T, only its row sums of squares are kept
-        op.A = h->c_K;
-        op.lda = (int)h->np;
-        op.B = h->M;
-        op.ldb = (int)h->np;
-        op.C = nullptr;
-        op.ldc = 0;
-        op.tiles_m = op.tiles_m_last = tiles_r;
-        op.tiles_n = h->T;
-        op.klo_c = 0;
-        op.khi_sel = KSEL_TJ;
-        op.khi_c = 1;
-        op.epilogue = EPI_ROWSQ;
-        op.rowsq = h->c_rowsq;
-        op.rowsq_ld = (int)MC;
-        if (keep_u) {  // the gradient and t-batch passes need U = K* L^-T itself; the row sums come out bitwise the same
-            op.epilogue = EPI_STORE_ROWSQ;
-            op.C = h->g_U;
-            op.ldc = (int)h->np;
-        }
-        if (jd) {  // the joint covariance keeps U of every candidate (rows base .. base + mcp of jd->U)
-            op.epilogue = EPI_STORE_ROWSQ;
-            op.C = jd->U + base * h->np;
-            op.ldc = (int)h->np;
-        }
-        CK(launch_gemm(op, true, true, 1, h->st));
-
-        PredFinishArgs fa;
-        memset(&fa, 0, sizeof(fa));
-        fa.mean_part = h->c_mean_part;
-        fa.rowsq = h->c_rowsq;
-        fa.ldp = MC;
-        fa.tiles_c = h->T;
-        fa.m = (int)mc;
-        fa.base = base;
-        fa.sf2 = h->sf2;
-        fa.mean_idx = mean_idx ? h->c_mean : nullptr;
-        fa.beta = hyp_beta(h);
-        fa.n_mean = h->n_mean;
-        fa.noise_idx = noise_idx ? h->c_noise : nullptr;
-        fa.noise = hyp_noise(h);
-        fa.n_noise = h->n_noise;
-        fa.include_noise = include_noise;
-        fa.min_var = min_var;
-        fa.mean_out = h->c_mu;
-        fa.var_out = h->c_var;
+        if ((rc = chunk_front(h, r, base, mc, nullptr, grad ? h->g_U.p : nullptr, acq)) != GPP_OK) return rc;
         const int nblk = (int)((mc + 255) / 256);
-        if (acq) {
-            fa.cost_idx = acq->cost_idx ? h->c_cost : nullptr;
-            fa.cost = h->acq_par;
-            fa.best_f = h->acq_par + acq->n_cost;
-            fa.kind_by_cost = h->acq_kind;
-            fa.n_cost = acq->n_cost;
-            fa.maximize = acq->maximize;
-            fa.si = acq->si;
-            fa.y_min = acq->y_min;
-            fa.y_std = acq->y_std;
-            fa.score_out = acq->scores ? h->c_score : nullptr;
-            fa.blk_best = h->c_blk_best;
-            fa.blk_idx = h->c_blk_idx;
-        }
-        predict_finish_kernel<<<nblk, 256, 0, h->st>>>(fa);
-        CK(cudaGetLastError());
-    count_launch();
-        if (qb && (qa || nv || (!grad && qb->cov))) {  // Sigma_t = K**_t - U_t U_t^T of the chunk's t-batches, q_buf
-            QSyrkArgs sa;
-            memset(&sa, 0, sizeof(sa));
-            sa.U = h->g_U;
-            sa.ldu = h->np;
-            sa.kcols = (int)h->n;
-            sa.rowsq = h->c_rowsq;
-            sa.ldr = MC;
-            sa.tiles_c = h->T;
-            sa.xs = h->c_xs;
-            sa.zpt = h->c_zpt;
-            sa.zs = mcp * ZP;
-            sa.dq = h->dq;
-            sa.dqp = h->dqp;
-            sa.dz = h->dz;
-            sa.n_pass = h->n_pass;
-            sa.sf2 = h->sf2;
-            sa.noise_idx = noise_idx ? h->c_noise : nullptr;
-            sa.noise = hyp_noise(h);
-            sa.n_noise = h->n_noise;
-            sa.include_noise = include_noise;
-            sa.q = qb->q;
-            sa.qpt = qb->qpt;
-            sa.nb = nbc;
-            sa.cov = h->q_buf;
-            CK(launch_qbatch_syrk(sa, h->kernel, tiles_r, h->st));
-            const size_t qq = (size_t)qb->q * qb->q;
-            if (qb->cov)
-                CK(cudaMemcpyAsync(qb->cov + bt0 * qq, h->q_buf, sizeof(double) * nbc * qq, cudaMemcpyDefault, h->st));
-        }
-        if (qa) {  // values and jitters; with the gradient, G_t over Sigma_t in q_buf and mu_bar into q_gm
-            if (grad) CK(cudaMemsetAsync(h->q_gm, 0, sizeof(double) * mcp, h->st));
-            QAcqArgs aa;
-            memset(&aa, 0, sizeof(aa));
-            aa.blk = h->q_buf;
-            aa.mu = h->c_mu;
-            aa.gm = h->q_gm;
-            aa.E = h->a_E;
-            aa.S = qa->S;
-            aa.q = qb->q;
-            aa.qpt = qb->qpt;
-            aa.n_base = qa->n_base;
-            aa.nb = nbc;
-            aa.sgn = qa->maximize ? 1.0 : -1.0;
-            aa.best_f = qa->best_f;
-            aa.cbeta = qa->cbeta;
-            aa.grad = grad ? 1 : 0;
-            aa.value = h->a_val;
-            aa.jitter = h->a_jit;
-            aa.info = h->a_info;
-            CK(launch_qacq(aa, qa->kind, h->st));
-            CK(cudaMemcpyAsync(qa->values + bt0, h->a_val, sizeof(double) * nbc, cudaMemcpyDefault, h->st));
-            if (qa->jitter)
-                CK(cudaMemcpyAsync(qa->jitter + bt0, h->a_jit, sizeof(double) * nbc, cudaMemcpyDefault, h->st));
-        }
-        if (nv) {  // C^T = K(X_chunk, X_I) - U_chunk U_I^T, then per t-batch G_t = C_t^T C_t, A_t's factor, the value
-            CovArgs cc;
-            memset(&cc, 0, sizeof(cc));
-            cc.xs_r = h->c_xs;
-            cc.nrm_r = h->c_nrm;
-            cc.xs_c = h->i_xs;
-            cc.nrm_c = h->i_nrm;
-            cc.out = h->n_C;
-            cc.ld = h->i_mp;
-            cc.n_r = (int)mc;
-            cc.n_c = (int)h->i_m;
-            cc.tiles_r = tiles_r;
-            cc.tiles_c = imt;
-            cc.dqp = h->dqp;
-            cc.dz = h->dz;
-            cc.sf2 = h->sf2;
-            cc.scale = 1.0 / (double)h->n_pass;
-            for (int p = 0; p < h->n_pass; p++) {
-                cc.zpt_r = h->c_zpt + (size_t)p * mcp * ZP;
-                cc.zpt_c = h->i_zpt + (size_t)p * h->i_mp * ZP;
-                cc.accum = p > 0;
-                cc.last = p == h->n_pass - 1;
-                CK(launch_cov(cc, h->kernel, h->st));
-            }
-            GemmOp co = gemm_default();
-            co.A = h->g_U;
-            co.lda = (int)h->np;
-            co.B = h->i_U;
-            co.ldb = (int)h->np;
-            co.C = h->n_C;
-            co.ldc = (int)h->i_mp;
-            co.tiles_m = co.tiles_m_last = tiles_r;
-            co.tiles_n = imt;
-            co.klo_c = 0;
-            co.khi_c = h->T;
-            co.alpha = -1.0;
-            co.beta = 1.0;
-            CK(launch_gemm(co, true, true, 1, h->st));
-            QSyrkArgs ga;
-            memset(&ga, 0, sizeof(ga));
-            ga.U = h->n_C;
-            ga.ldu = h->i_mp;
-            ga.kcols = (int)h->i_m;
-            ga.q = qb->q;
-            ga.qpt = qb->qpt;
-            ga.nb = nbc;
-            ga.cov = h->n_G;
-            CK(launch_qbatch_gram(ga, tiles_r, h->st));
-            NipvArgs na;
-            memset(&na, 0, sizeof(na));
-            na.blk = h->q_buf;
-            na.gram = h->n_G;
-            na.ainv = h->n_Ai;
-            na.q = qb->q;
-            na.nb = nbc;
-            na.inv_m = 1.0 / (double)h->i_m;
-            na.vbar = h->i_vbar;
-            na.grad = grad ? 1 : 0;
-            na.value = h->a_val;
-            na.jitter = h->a_jit;
-            na.info = h->a_info;
-            CK(launch_nipv_block(na, h->st));
-            CK(cudaMemcpyAsync(nv->values + bt0, h->a_val, sizeof(double) * nbc, cudaMemcpyDefault, h->st));
-            if (nv->jitter)
-                CK(cudaMemcpyAsync(nv->jitter + bt0, h->a_jit, sizeof(double) * nbc, cudaMemcpyDefault, h->st));
-        }
-        if (grad) {
-            // V = U L^-1 = K* K_y^-1 over the K* chunk, which is not read again: B(tj, k) = L^-1[k, tj], k in [tj, T)
-            GemmOp vo = gemm_default();
-            vo.A = h->g_U;
-            vo.lda = (int)h->np;
-            vo.B = h->M;
-            vo.ldb = (int)h->np;
-            vo.C = h->c_K;
-            vo.ldc = (int)h->np;
-            vo.tiles_m = vo.tiles_m_last = tiles_r;
-            vo.tiles_n = h->T;
-            vo.klo_sel = KSEL_TJ;
-            vo.klo_c = 0;
-            vo.khi_c = h->T;
-            CK(launch_gemm(vo, true, false, 1, h->st));
-            if (qb) {  // W = blockdiag(G + G^T) V into g_U (U is not read again), the upstream mean gradient into q_gm
-                const size_t qq = (size_t)qb->q * qb->q;
-                if (qb->g_cov)  // (the acquisition path has G_t in q_buf and mu_bar in q_gm already)
-                    CK(cudaMemcpyAsync(h->q_buf, qb->g_cov + bt0 * qq, sizeof(double) * nbc * qq, cudaMemcpyDefault,
-                                       h->st));
-                else if (!qa && !nv)  // (gpp_nipv_qbatch has A_bar_t there)
-                    CK(cudaMemsetAsync(h->q_buf, 0, sizeof(double) * nbc * qq, h->st));
-                if (qb->g_mean && !qa) {
-                    CK(cudaMemsetAsync(h->q_gm, 0, sizeof(double) * mcp, h->st));
-                    CK(qb_copy_rows(qb, h->q_gm, qb->g_mean, sizeof(double), bt0, nbc, true, h->st));
-                }
-                QWArgs wa;
-                wa.V = h->c_K;
-                wa.ldv = h->np;
-                wa.G = h->q_buf;
-                wa.q = qb->q;
-                wa.qpt = qb->qpt;
-                wa.nb = nbc;
-                wa.W = h->g_U;
-                wa.ldw = h->np;
-                qbatch_w_kernel<<<dim3((unsigned)(h->np / QB_KC), (unsigned)tiles_r), QB_THREADS, 0, h->st>>>(wa);
-                CK(cudaGetLastError());
-                count_launch();
-                if (nv) {
-                    // -C_bar^T = blockdiag(-2 A^-1 / M) C^T in place over C^T: each CTA stages the 32-column panel of
-                    // its tile in shared memory before it writes that same panel
-                    QWArgs cw = wa;
-                    cw.V = h->n_C;
-                    cw.ldv = h->i_mp;
-                    cw.G = h->n_Ai;
-                    cw.W = h->n_C;
-                    cw.ldw = h->i_mp;
-                    qbatch_w_kernel<<<dim3((unsigned)(h->i_mp / QB_KC), (unsigned)tiles_r), QB_THREADS, 0, h->st>>>(cw);
-                    CK(cudaGetLastError());
-                    count_launch();
-                    // W += C_bar^T V_I: the K* term that reaches U_t through C_t (finish subtracts W's partials)
-                    GemmOp wo = gemm_default();
-                    wo.A = h->n_C;
-                    wo.lda = (int)h->i_mp;
-                    wo.B = h->i_V;
-                    wo.ldb = (int)h->np;
-                    wo.C = h->g_U;
-                    wo.ldc = (int)h->np;
-                    wo.tiles_m = wo.tiles_m_last = tiles_r;
-                    wo.tiles_n = h->T;
-                    wo.klo_c = 0;
-                    wo.khi_c = imt;
-                    wo.alpha = -1.0;
-                    wo.beta = 1.0;
-                    CK(launch_gemm(wo, true, false, 1, h->st));
-                }
-            }
-
-            PredGradArgs ga;
-            memset(&ga, 0, sizeof(ga));
-            ga.xs_r = h->c_xs;
-            ga.zpt_r = h->c_zpt;
-            ga.zs_r = mcp * ZP;
-            ga.xs_c = h->xs;
-            ga.zpt_c = h->zpt;
-            ga.zs_c = h->np * ZP;
-            ga.alpha = h->alpha;
-            ga.V = qb ? h->g_U : h->c_K;
-            ga.ldv = h->np;
-            ga.n_r = (int)mc;
-            ga.n_c = (int)h->n;
-            ga.dq = h->dq;
-            ga.dqp = h->dqp;
-            ga.dz = h->dz;
-            ga.n_pass = h->n_pass;
-            ga.part_m = nv ? h->n_pm : h->g_part_m;
-            ga.part_v = nv ? h->n_pv : h->g_part_v;
-            ga.ldp = step;
-            CK(launch_predict_grad(ga, h->kernel, tiles_r, h->T, h->st));
-            if (nv) {  // K(X_t, X_I) term: integration points as columns, -C_bar^T as V, after the training tiles
-                PredGradArgs gi = ga;
-                gi.xs_c = h->i_xs;
-                gi.zpt_c = h->i_zpt;
-                gi.zs_c = h->i_mp * ZP;
-                gi.alpha = h->i_zero;
-                gi.V = h->n_C;
-                gi.ldv = h->i_mp;
-                gi.n_c = (int)h->i_m;
-                gi.part_m = h->n_pm + (size_t)h->T * h->dq * step;
-                gi.part_v = h->n_pv + (size_t)h->T * h->dq * step;
-                CK(launch_predict_grad(gi, h->kernel, tiles_r, imt, h->st));
-            }
-        }
-        if (grad && qb) {  // the K**_t term, then d_xq of the chunk's rows (tile layout in g_dvar)
-            QInArgs ia;
-            ia.xs = h->c_xs;
-            ia.zpt = h->c_zpt;
-            ia.zs = mcp * ZP;
-            ia.dq = h->dq;
-            ia.dqp = h->dqp;
-            ia.dz = h->dz;
-            ia.n_pass = h->n_pass;
-            ia.G = h->q_buf;
-            ia.q = qb->q;
-            ia.qpt = qb->qpt;
-            ia.nb = nbc;
-            ia.rows = (int)mcp;
-            ia.part_k = h->g_dmean;
-            CK(launch_qbatch_inbatch_grad(ia, h->kernel, h->st));
-            QFinishArgs qf;
-            qf.part_m = nv ? h->n_pm : h->g_part_m;
-            qf.part_v = nv ? h->n_pv : h->g_part_v;
-            qf.ldp = step;
-            qf.tiles_c = h->T + imt;
-            qf.part_k = h->g_dmean;
-            qf.g_mean = (qb->g_mean || qa) ? h->q_gm : nullptr;
-            qf.m = (int)mcp;
-            qf.dq = h->dq;
-            qf.w = hyp_w(h);
-            qf.sf2 = h->sf2;
-            qf.d_x = h->g_dvar;
-            qbatch_grad_finish_kernel<<<(int)((mcp + 255) / 256), 256, 0, h->st>>>(qf);
-            CK(cudaGetLastError());
-            count_launch();
-            CK(qb_copy_rows(qb, qb->d_xq, h->g_dvar, sizeof(double) * h->dq, bt0, nbc, false, h->st));
-        } else if (grad) {
+        if (grad) {  // V = U L^-1 over the K* chunk, which is not read again, then the gradient partials and their sums
+            const Panels rows = chunk_panels(h, mc);
+            if ((rc = v_gemm(h, h->g_U, h->c_K, rows.tiles)) != GPP_OK) return rc;
+            if ((rc = grad_tiles(h, rows, training_panels(h), h->alpha, h->c_K, h->np, h->g_part_m, h->g_part_v,
+                                 step)) != GPP_OK)
+                return rc;
             PredGradFinishArgs gf;
             memset(&gf, 0, sizeof(gf));
             gf.part_m = h->g_part_m;
             gf.part_v = h->g_part_v;
             gf.ldp = step;
             gf.rowsq = h->c_rowsq;
-            gf.ldr = MC;
+            gf.ldr = h->mc_alloc;
             gf.tiles_c = h->T;
             gf.m = (int)mc;
             gf.dq = h->dq;
             gf.w = hyp_w(h);
             gf.sf2 = h->sf2;
-            gf.noise_idx = noise_idx ? h->c_noise : nullptr;
+            gf.noise_idx = r.noise_idx ? h->c_noise.p : nullptr;
             gf.noise = hyp_noise(h);
             gf.n_noise = h->n_noise;
-            gf.include_noise = include_noise;
-            gf.min_var = min_var;
+            gf.include_noise = r.include_noise;
+            gf.min_var = r.min_var;
             gf.d_mean = h->g_dmean;
             gf.d_var = h->g_dvar;
             predict_grad_finish_kernel<<<nblk, 256, 0, h->st>>>(gf);
@@ -1860,8 +1503,7 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             if (d_mean) CK(cudaMemcpyAsync(d_mean + base * h->dq, h->g_dmean, gb, cudaMemcpyDefault, h->st));
             if (d_var) CK(cudaMemcpyAsync(d_var + base * h->dq, h->g_dvar, gb, cudaMemcpyDefault, h->st));
         }
-        if (mean && qb) CK(qb_copy_rows(qb, mean, h->c_mu, sizeof(double), bt0, nbc, false, h->st));
-        else if (mean) CK(cudaMemcpyAsync(mean + base, h->c_mu, sizeof(double) * mc, cudaMemcpyDefault, h->st));
+        if (mean) CK(cudaMemcpyAsync(mean + base, h->c_mu, sizeof(double) * mc, cudaMemcpyDefault, h->st));
         if (var) CK(cudaMemcpyAsync(var + base, h->c_var, sizeof(double) * mc, cudaMemcpyDefault, h->st));
         if (acq) {
             if (acq->scores)
@@ -1871,19 +1513,7 @@ static int predict_impl(gpp_handle* h, long long m, const double* xq, const int3
             CK(cudaMemcpyAsync(hb.data(), h->c_blk_best, sizeof(double) * nblk, cudaMemcpyDeviceToHost, h->st));
             CK(cudaMemcpyAsync(hi.data(), h->c_blk_idx, sizeof(long long) * nblk, cudaMemcpyDeviceToHost, h->st));
         }
-        int qa_info = 0;
-        if (qa || nv) CK(cudaMemcpyAsync(&qa_info, h->a_info, sizeof(int), cudaMemcpyDeviceToHost, h->st));
         CK(cudaStreamSynchronize(h->st));
-        if (qa_info & 2) {
-            g_err = nv ? "gpp_nipv_qbatch: NaN in a t-batch posterior or its integrated variance"
-                       : "gpp_acq_qbatch: NaN in a t-batch posterior or its samples";
-            return GPP_ERR_NAN;
-        }
-        if (qa_info & 1) {
-            g_err = std::string(nv ? "gpp_nipv_qbatch" : "gpp_acq_qbatch") +
-                    ": a t-batch posterior covariance is not positive definite after adding jitter up to 1e-6";
-            return GPP_ERR_NOT_PD;
-        }
         if (acq) {
             for (int b = 0; b < nblk; b++) {
                 if (acq->best_index < 0 || hb[b] > acq->best_score ||
@@ -1901,7 +1531,8 @@ extern "C" int gpp_predict(gpp_handle* h, int64_t m, const double* xq, const int
                            const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, double min_var,
                            double* mean, double* var) {
     if (!h) ARG_FAIL("gpp_predict: null handle");
-    return predict_impl(h, m, xq, level_idx, noise_idx, mean_idx, include_noise, min_var, mean, var, nullptr);
+    const Rows r = {xq, level_idx, noise_idx, mean_idx, include_noise, min_var};
+    return predict_rows(h, m, r, mean, var, nullptr, nullptr, nullptr);
 }
 
 extern "C" int gpp_predict_grad(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
@@ -1910,8 +1541,8 @@ extern "C" int gpp_predict_grad(gpp_handle* h, int64_t m, const double* xq, cons
     if (!h) ARG_FAIL("gpp_predict_grad: null handle");
     // no quantitative input (or no gradient asked for): nothing to differentiate, the gpp_predict sequence
     const bool grad = h->dq > 0 && (d_mean || d_var);
-    return predict_impl(h, m, xq, level_idx, noise_idx, mean_idx, include_noise, min_var, mean, var, nullptr, grad,
-                        d_mean, d_var);
+    const Rows r = {xq, level_idx, noise_idx, mean_idx, include_noise, min_var};
+    return predict_rows(h, m, r, mean, var, nullptr, grad ? d_mean : nullptr, grad ? d_var : nullptr);
 }
 
 extern "C" int gpp_acq_argmax(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
@@ -1932,10 +1563,49 @@ extern "C" int gpp_acq_argmax(gpp_handle* h, int64_t m, const double* xq, const 
     a.y_std = y_std;
     a.scores = scores;
     // the reference's candidate-table branch predicts with include_noise=False (BO_GP_plus.py:185-186)
-    int rc = predict_impl(h, m, xq, level_idx, nullptr, mean_idx, 0, min_var, nullptr, nullptr, &a);
+    const Rows r = {xq, level_idx, nullptr, mean_idx, 0, min_var};
+    int rc = predict_rows(h, m, r, nullptr, nullptr, &a, nullptr, nullptr);
     if (rc != GPP_OK) return rc;
     if (best_score) *best_score = a.best_score;
     if (best_index) *best_index = a.best_index;
+    return GPP_OK;
+}
+
+// Loads m points into the set s: their inputs and panels once (ld mp = m padded to 128), then the prediction chunk loop
+// on the set's panels with U = K* L^-T of every row stored in s.U (rows >= m come out zero).  Mean and variance of row
+// i go to mean[i] / var[i] when given, the rows' noise groups to noise_out when the variance includes noise.
+static int load_point_set(gpp_handle* h, PointSet& s, long long m, const Rows& r, int* noise_out, double* mean,
+                          double* var) {
+    const long long mp = round128(m);
+    CK(s.xq.reserve(mp * std::max(h->dq, 1), h->st));
+    CK(s.xs.reserve(mp * h->dqp, h->st));
+    CK(s.nrm.reserve(mp, h->st));
+    CK(s.zpt.reserve(mp * ZP * h->n_pass, h->st));
+    CK(s.U.reserve(mp * h->np, h->st));
+    CK(s.lvl.reserve(mp, h->st));
+    s.mp = mp;
+    if (h->dq > 0) CK(cudaMemcpyAsync(s.xq, r.xq, sizeof(double) * m * h->dq, cudaMemcpyDefault, h->st));
+    if (h->dz > 0) CK(cudaMemcpyAsync(s.lvl, r.level_idx, sizeof(int) * m, cudaMemcpyDefault, h->st));
+    if (noise_out && r.include_noise && r.noise_idx)
+        CK(cudaMemcpyAsync(noise_out, r.noise_idx, sizeof(int) * m, cudaMemcpyDefault, h->st));
+    int rc = prep_panels(h, s.xq, h->dz > 0 ? s.lvl.p : nullptr, m, mp, s.xs, nullptr, s.nrm, s.zpt);
+    if (rc != GPP_OK) return rc;
+    for (long long base = 0; base < m; base += h->mc_alloc) {
+        const long long mc = std::min(h->mc_alloc, m - base);
+        if (r.noise_idx)
+            CK(cudaMemcpyAsync(h->c_noise, r.noise_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
+        if (r.mean_idx) CK(cudaMemcpyAsync(h->c_mean, r.mean_idx + base, sizeof(int) * mc, cudaMemcpyDefault, h->st));
+        const Panels rows = {s.xs + base * h->dqp, s.nrm + base, s.zpt + base * ZP, mp * ZP, (int)mc,
+                             (int)(round128(mc) / CT)};
+        if ((rc = chunk_front(h, r, base, mc, &rows, s.U + base * h->np, nullptr)) != GPP_OK) return rc;
+        if (mean) CK(cudaMemcpyAsync(mean + base, h->c_mu, sizeof(double) * mc, cudaMemcpyDefault, h->st));
+        if (var) CK(cudaMemcpyAsync(var + base, h->c_var, sizeof(double) * mc, cudaMemcpyDefault, h->st));
+        CK(cudaStreamSynchronize(h->st));
+    }
+    // Columns n .. Np of U are K* L^-T against the identity padding of K_y, i.e. zero in exact arithmetic; clear them
+    // so that products over whole 128-blocks of U never depend on how L^-1's padding was produced.
+    if (h->np > h->n)
+        CK(cudaMemset2DAsync(s.U + h->n, sizeof(double) * h->np, 0, sizeof(double) * (h->np - h->n), (size_t)mp, h->st));
     return GPP_OK;
 }
 
@@ -1943,166 +1613,65 @@ extern "C" int gpp_acq_argmax(gpp_handle* h, int64_t m, const double* xq, const 
 // Joint posterior over m candidates: Sigma* = K** - K* K_y^-1 K*^T = K** - U U^T with U = K* L^-T, and draws
 // mu + E L*^T with L* L*^T = Sigma* + jitter I.  Stages (all on h->st, none of them touches A, M, S, alpha or the
 // captured graphs):
-//   J1  panels of all candidates once, then the gpp_predict chunk loop with U stored (mean bitwise gpp_predict's)
+//   J1  the joint set (load_point_set; mean bitwise gpp_predict's)
 //   J2  K** on the lower tiles (+ noise, + jitter), then Sigma* -= U U^T over K range [0, T)  (one DMMA SYRK)
 //   J3  potrf_blocked(Sigma*) in DMMA arithmetic whatever the handle's FP64 mode, psd_safe_cholesky ladder
 //   J4  per chunk of base samples: Y = mu + E L*^T  (one triangular DMMA GEMM)
-static long long round128(long long x) { return (x + 127) / 128 * 128; }
 
+// joint-only buffers for mp rows.  The draw chunk (up to 2 x 1 GiB) is released when the joint set is about to grow,
+// so that it is not held while the larger set is allocated; the next gpp_sample_posterior allocates it again.
 static int ensure_joint_buffers(gpp_handle* h, long long mp) {
-    if (mp <= h->j_mp) return GPP_OK;
-    void* olds[] = {h->j_xq, h->j_xs, h->j_nrm, h->j_zpt, h->j_U, h->j_S, h->j_Minv, h->j_diag, h->j_mu, h->j_logdet,
-                    h->j_lvl, h->j_noise, h->j_info, h->j_E, h->j_Y};
-    CK(cudaStreamSynchronize(h->st));
-    for (void* p : olds)
-        if (p) cudaFree(p);
-    h->j_xq = h->j_xs = h->j_nrm = h->j_zpt = h->j_U = h->j_S = h->j_Minv = h->j_diag = h->j_mu = h->j_logdet = nullptr;
-    h->j_lvl = h->j_noise = h->j_info = nullptr;
-    h->j_E = h->j_Y = nullptr;  // the draw chunk is reallocated by the next gpp_sample_posterior
-    h->j_draw_cap = 0;
-    h->j_mp = 0;
-    const size_t n = (size_t)mp;
-    CK(dev_alloc(&h->j_xq, n * std::max(h->dq, 1)));
-    CK(dev_alloc(&h->j_xs, n * h->dqp));
-    CK(dev_alloc(&h->j_nrm, n));
-    CK(dev_alloc(&h->j_zpt, n * ZP * h->n_pass));
-    CK(dev_alloc(&h->j_U, n * (size_t)h->np));
-    CK(dev_alloc(&h->j_S, n * n));
-    CK(dev_alloc(&h->j_Minv, n * n));
-    CK(dev_alloc(&h->j_diag, n));
-    CK(dev_alloc(&h->j_mu, n));
-    CK(dev_alloc(&h->j_logdet, n / 128));
-    CK(dev_alloc(&h->j_lvl, n));
-    CK(dev_alloc(&h->j_noise, n));
-    CK(dev_alloc(&h->j_info, 1));
-    CK(cudaMemsetAsync(h->j_mu, 0, sizeof(double) * n, h->st));
-    h->j_mp = mp;
+    if (mp > (long long)h->jset.nrm.cap) {  // (nrm holds one double per row of the set)
+        CK(cudaStreamSynchronize(h->st));
+        h->j_E.release();
+        h->j_Y.release();
+    }
+    CK(h->j_S.reserve(mp * mp, h->st));
+    CK(h->j_Minv.reserve(mp * mp, h->st));
+    CK(h->j_diag.reserve(mp, h->st));
+    CK(h->j_mu.reserve(mp, h->st, true));
+    CK(h->j_logdet.reserve(mp / 128, h->st));
+    CK(h->j_noise.reserve(mp, h->st));
+    CK(h->j_info.reserve(1, h->st));
     return GPP_OK;
 }
 
-// base samples and draws of one chunk, `elems` doubles each (rows x mp of the current call)
-static int ensure_draw_buffers(gpp_handle* h, long long elems) {
-    if (elems <= h->j_draw_cap) return GPP_OK;
-    CK(cudaStreamSynchronize(h->st));
-    if (h->j_E) cudaFree(h->j_E);
-    if (h->j_Y) cudaFree(h->j_Y);
-    h->j_E = h->j_Y = nullptr;
-    h->j_draw_cap = 0;
-    CK(dev_alloc(&h->j_E, (size_t)elems));
-    CK(dev_alloc(&h->j_Y, (size_t)elems));
-    CK(cudaMemsetAsync(h->j_E, 0, sizeof(double) * elems, h->st));
-    h->j_draw_cap = elems;
-    return GPP_OK;
+static const char* joint_count_err(long long m) {
+    return (m < 0 || m > GPP_MAX_JOINT) ? "m must be in [0, GPP_MAX_JOINT]" : nullptr;
 }
 
-static int joint_check(gpp_handle* h, long long m, const double* xq, const int32_t* level_idx, const char* name) {
-    if (!h) {
-        g_err = std::string(name) + ": null handle";
-        return GPP_ERR_ARG;
-    }
-    if (!h->factorized) {
-        g_err = std::string(name) + ": call gpp_factorize (or gpp_mll_grad) first";
-        return GPP_ERR_ARG;
-    }
-    if (m < 0 || m > GPP_MAX_JOINT) {
-        g_err = std::string(name) + ": m must be in [0, GPP_MAX_JOINT]";
-        return GPP_ERR_ARG;
-    }
-    if (m > 0 && h->dq > 0 && !xq) {
-        g_err = std::string(name) + ": xq missing";
-        return GPP_ERR_ARG;
-    }
-    if (m > 0 && h->dz > 0 && !level_idx) {
-        g_err = std::string(name) + ": level_idx missing";
-        return GPP_ERR_ARG;
-    }
-    return GPP_OK;
-}
-
-// J1: candidate panels, U = K* L^-T of every candidate into j_U, the predictive mean into j_mu
-static int joint_stage_u(gpp_handle* h, long long m, const double* xq, const int32_t* level_idx,
-                         const int32_t* noise_idx, const int32_t* mean_idx, int include_noise) {
+// J1: the joint set, the predictive mean into j_mu
+static int joint_stage_u(gpp_handle* h, long long m, const Rows& r) {
     CK(cudaSetDevice(h->device));
-    const long long mp = round128(m);
     int rc = ensure_chunk_buffers(h, m);  // before the joint buffers: a handle holding them has mc_alloc > 0
-    if (rc != GPP_OK) return rc;
-    if ((rc = ensure_joint_buffers(h, mp)) != GPP_OK) return rc;
-    if (h->dq > 0) CK(cudaMemcpyAsync(h->j_xq, xq, sizeof(double) * m * h->dq, cudaMemcpyDefault, h->st));
-    if (h->dz > 0) CK(cudaMemcpyAsync(h->j_lvl, level_idx, sizeof(int) * m, cudaMemcpyDefault, h->st));
-    if (include_noise && noise_idx)
-        CK(cudaMemcpyAsync(h->j_noise, noise_idx, sizeof(int) * m, cudaMemcpyDefault, h->st));
-    PrepArgs pa;
-    pa.xq = h->j_xq;
-    pa.level_idx = h->dz > 0 ? h->j_lvl : nullptr;
-    pa.w = hyp_w(h);
-    pa.centre = h->centre;
-    pa.ztab = hyp_z(h);
-    pa.n = (int)m;
-    pa.np = (int)mp;
-    pa.dq = h->dq;
-    pa.dqp = h->dqp;
-    pa.dz = h->dz;
-    pa.n_combo = h->n_combo;
-    pa.n_pass = h->n_pass;
-    pa.xs = h->j_xs;
-    pa.xst = nullptr;
-    pa.nrm = h->j_nrm;
-    pa.zpt = h->j_zpt;
-    prep_points_kernel<<<(int)((mp + 255) / 256), 256, 0, h->st>>>(pa);
-    CK(cudaGetLastError());
-    count_launch();
-    JointDest jd;
-    jd.xs = h->j_xs;
-    jd.nrm = h->j_nrm;
-    jd.zpt = h->j_zpt;
-    jd.mp = mp;
-    jd.U = h->j_U;
-    rc = predict_impl(h, m, xq, level_idx, noise_idx, mean_idx, include_noise, 0.0, h->j_mu, nullptr, nullptr, false,
-                      nullptr, nullptr, &jd);
-    if (rc != GPP_OK) return rc;
-    // Columns n .. Np of U are K* L^-T against the identity padding of K_y, i.e. zero in exact arithmetic; clear them
-    // so that the SYRK, which runs over whole 128-blocks of K, never depends on how L^-1's padding was produced.
-    if (h->np > h->n)
-        CK(cudaMemset2DAsync(h->j_U + h->n, sizeof(double) * h->np, 0, sizeof(double) * (h->np - h->n), (size_t)mp,
-                             h->st));
-    return GPP_OK;
+    if (rc != GPP_OK || (rc = ensure_joint_buffers(h, round128(m))) != GPP_OK) return rc;
+    return load_point_set(h, h->jset, m, r, h->j_noise, h->j_mu, nullptr);
 }
 
 // J2: Sigma* (lower tiles) = K** + diag(noise + jitter) - U U^T into j_S
 static int joint_stage_sigma(gpp_handle* h, long long m, const int32_t* noise_idx, int include_noise, double jitter) {
     const long long mp = round128(m);
     const int mt = (int)(mp / 128);
-    joint_diag_kernel<<<(int)((mp + 255) / 256), 256, 0, h->st>>>(noise_idx ? h->j_noise : nullptr, hyp_noise(h),
+    joint_diag_kernel<<<(int)((mp + 255) / 256), 256, 0, h->st>>>(noise_idx ? h->j_noise.p : nullptr, hyp_noise(h),
                                                                  h->n_noise, include_noise, jitter, (int)m, (int)mp,
                                                                  h->j_diag);
     CK(cudaGetLastError());
     count_launch();
     CovArgs ca;
     memset(&ca, 0, sizeof(ca));
-    ca.xs_r = ca.xs_c = h->j_xs;
-    ca.nrm_r = ca.nrm_c = h->j_nrm;
     ca.out = h->j_S;
     ca.ld = mp;
-    ca.n_r = ca.n_c = (int)m;
-    ca.tiles_r = ca.tiles_c = mt;
     ca.tri = 1;
     ca.same = 1;
     ca.pad_identity = 1;
-    ca.dqp = h->dqp;
-    ca.dz = h->dz;
-    ca.sf2 = h->sf2;
     ca.diag_add = h->j_diag;
-    ca.scale = 1.0 / (double)h->n_pass;
-    for (int p = 0; p < h->n_pass; p++) {
-        ca.zpt_r = ca.zpt_c = h->j_zpt + (size_t)p * mp * ZP;
-        ca.accum = p > 0;
-        ca.last = p == h->n_pass - 1;
-        CK(launch_cov(ca, h->kernel, h->st));
-    }
+    const Panels set = {h->jset.xs, h->jset.nrm, h->jset.zpt, mp * ZP, (int)m, mt};
+    int rc = launch_cov_passes(h, ca, set, set);
+    if (rc != GPP_OK) return rc;
     GemmOp op = gemm_default();  // Sigma* -= U U^T on the lower tiles (the trailing_update op shape)
-    op.A = h->j_U;
+    op.A = h->jset.U;
     op.lda = (int)h->np;
-    op.B = h->j_U;
+    op.B = h->jset.U;
     op.ldb = (int)h->np;
     op.C = h->j_S;
     op.ldc = (int)mp;
@@ -2120,9 +1689,10 @@ static int joint_stage_sigma(gpp_handle* h, long long m, const int32_t* noise_id
 extern "C" int gpp_predict_joint(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
                                  const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, double* mean,
                                  double* cov) {
-    int rc = joint_check(h, m, xq, level_idx, "gpp_predict_joint");
+    int rc = check_rows(h, "gpp_predict_joint", joint_count_err(m), m, xq, level_idx);
     if (rc != GPP_OK || m == 0) return rc;
-    if ((rc = joint_stage_u(h, m, xq, level_idx, noise_idx, mean_idx, include_noise)) != GPP_OK) return rc;
+    const Rows r = {xq, level_idx, noise_idx, mean_idx, include_noise, 0.0};
+    if ((rc = joint_stage_u(h, m, r)) != GPP_OK) return rc;
     if ((rc = joint_stage_sigma(h, m, noise_idx, include_noise, 0.0)) != GPP_OK) return rc;
     const long long mp = round128(m);
     const int nb = (int)(mp / 32);
@@ -2140,7 +1710,7 @@ extern "C" int gpp_predict_joint(gpp_handle* h, int64_t m, const double* xq, con
 extern "C" int gpp_sample_posterior(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
                                     const int32_t* noise_idx, const int32_t* mean_idx, int include_noise,
                                     int64_t n_samples, const double* base_samples, double* samples, double* jitter) {
-    int rc = joint_check(h, m, xq, level_idx, "gpp_sample_posterior");
+    int rc = check_rows(h, "gpp_sample_posterior", joint_count_err(m), m, xq, level_idx);
     if (rc != GPP_OK) return rc;
     if (n_samples < 0) ARG_FAIL("gpp_sample_posterior: n_samples must be >= 0");
     if (m > 0 && n_samples > 0 && (!base_samples || !samples)) ARG_FAIL("gpp_sample_posterior: samples missing");
@@ -2148,7 +1718,8 @@ extern "C" int gpp_sample_posterior(gpp_handle* h, int64_t m, const double* xq, 
         if (jitter) *jitter = 0.0;
         return GPP_OK;
     }
-    if ((rc = joint_stage_u(h, m, xq, level_idx, noise_idx, mean_idx, include_noise)) != GPP_OK) return rc;
+    const Rows r = {xq, level_idx, noise_idx, mean_idx, include_noise, 0.0};
+    if ((rc = joint_stage_u(h, m, r)) != GPP_OK) return rc;
     const long long mp = round128(m);
     const int mt = (int)(mp / 128);
     // The leaf writes only the lower 32 x 32 sub-blocks of each diagonal block of L*^-1, and the TRSM reads the whole
@@ -2185,7 +1756,9 @@ extern "C" int gpp_sample_posterior(gpp_handle* h, int64_t m, const double* xq, 
     long long cap = ((1LL << 27) / mp) / 128 * 128;
     if (cap < 128) cap = 128;
     const long long sc = std::min(round128(n_samples), cap);
-    if ((rc = ensure_draw_buffers(h, sc * mp)) != GPP_OK) return rc;
+    // base samples and draws of one chunk, sc x mp doubles each
+    CK(h->j_E.reserve(sc * mp, h->st, true));
+    CK(h->j_Y.reserve(sc * mp, h->st));
     for (long long s0 = 0; s0 < n_samples; s0 += sc) {
         const long long rows = std::min(sc, n_samples - s0);
         const long long rp = round128(rows);
@@ -2220,69 +1793,306 @@ extern "C" int gpp_sample_posterior(gpp_handle* h, int64_t m, const double* xq, 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Joint posteriors of b independent t-batches of q candidates (qbatch.cuh): the gpp_predict chunk loop on the tile
-// layout of QBatchSpec with U stored, then only the q x q diagonal blocks.  Nothing is kept between the two calls.
-static int qbatch_check(gpp_handle* h, long long b, int q, const double* xq, const int32_t* level_idx,
-                        const char* name) {
-    const char* why = nullptr;
-    if (!h) why = "null handle";
-    else if (!h->factorized) why = "call gpp_factorize (or gpp_mll_grad) first";
-    else if (q < 1 || q > GPP_MAX_QBATCH) why = "q must be in [1, GPP_MAX_QBATCH]";
-    else if (b < 0) why = "b must be >= 0";
-    else if (h->dq > GPP_MAX_DQ) why = "at most GPP_MAX_DQ quantitative inputs";
-    else if (b > 0 && h->dq > 0 && !xq) why = "xq missing";
-    else if (b > 0 && h->dz > 0 && !level_idx) why = "level_idx missing";
-    if (!why) return GPP_OK;
-    g_err = std::string(name) + ": " + why;
-    return GPP_ERR_ARG;
-}
+// Joint posteriors of b independent t-batches of q candidates (qbatch.cuh): chunks of whole t-batches through the
+// chunk front with U stored, then only the q x q diagonal blocks.  Every 128-row tile of the chunk buffers holds
+// qpt = 128 / q whole t-batches followed by padding rows, so chunks (multiples of 128 rows) hold whole t-batches.
+struct QBatchSpec {
+    long long b;
+    int q, qpt;
+};
 
-static QBatchSpec qbatch_spec(long long b, int q) {
-    QBatchSpec s;
-    memset(&s, 0, sizeof(s));
-    s.b = b;
-    s.q = q;
-    s.qpt = CT / q;
-    return s;
-}
+static QBatchSpec qbatch_spec(long long b, int q) { return {b, q, CT / q}; }
 
 static long long qbatch_rows(const QBatchSpec& s) { return (s.b + s.qpt - 1) / s.qpt * CT; }
+
+static const char* qbatch_count_err(long long b, int q) {
+    if (q < 1 || q > GPP_MAX_QBATCH) return "q must be in [1, GPP_MAX_QBATCH]";
+    return b < 0 ? "b must be >= 0" : nullptr;
+}
+
+// one chunk of a t-batch call: rows [base, base + mc), tiles of 128 rows, t-batches [bt0, bt0 + nb)
+struct QChunk {
+    long long base, mc, mcp, bt0, nb;
+    int tiles;
+};
+
+static QChunk qbatch_chunk(const QBatchSpec& s, long long base, long long step) {
+    QChunk c;
+    c.base = base;
+    c.mc = std::min(step, qbatch_rows(s) - base);
+    c.mcp = round128(c.mc);
+    c.tiles = (int)(c.mcp / CT);
+    c.bt0 = base / CT * s.qpt;
+    c.nb = std::min(s.b, c.bt0 + (long long)c.tiles * s.qpt) - c.bt0;
+    return c;
+}
+
+// rows of nbat t-batches, from t-batch bt0 of a compact [b*q rows] array, to (into_tiles) or from their tile slots in
+// a chunk buffer: one pitched copy for the full tiles, one plain copy for the last, partly filled one
+static cudaError_t qb_copy_rows(const QBatchSpec& s, void* dst, const void* src, size_t row_bytes, long long bt0,
+                                long long nbat, bool into_tiles, cudaStream_t st) {
+    if (row_bytes == 0 || nbat <= 0) return cudaSuccess;
+    const size_t run = (size_t)s.qpt * s.q * row_bytes, tile = (size_t)CT * row_bytes;
+    const size_t off = (size_t)bt0 * s.q * row_bytes;
+    char* d = (char*)dst + (into_tiles ? 0 : off);
+    const char* src_c = (const char*)src + (into_tiles ? off : 0);
+    const size_t dp = into_tiles ? tile : run, sp = into_tiles ? run : tile;
+    const long long full = nbat / s.qpt, rest = nbat % s.qpt;
+    if (full > 0) {
+        cudaError_t e = cudaMemcpy2DAsync(d, dp, src_c, sp, run, (size_t)full, cudaMemcpyDefault, st);
+        if (e != cudaSuccess) return e;
+    }
+    if (rest > 0)
+        return cudaMemcpyAsync(d + full * dp, src_c + full * sp, (size_t)rest * s.q * row_bytes, cudaMemcpyDefault,
+                               st);
+    return cudaSuccess;
+}
+
+// chunk, gradient and q x q block buffers of a t-batch call.  q_buf is sized at g_step * q: when g_step has grown since
+// its allocation (q_gm, sized at g_step, shows it) it is allocated afresh rather than kept at an older chunk's size.
+static int qbatch_setup(gpp_handle* h, const QBatchSpec& s) {
+    CK(cudaSetDevice(h->device));
+    int rc = ensure_chunk_buffers(h, qbatch_rows(s));
+    if (rc != GPP_OK || (rc = ensure_grad_buffers(h)) != GPP_OK) return rc;
+    if (h->q_gm.cap < (size_t)h->g_step) h->q_buf.release();
+    CK(h->q_buf.reserve(h->g_step * s.q, h->st));
+    CK(h->q_gm.reserve(h->g_step, h->st));
+    return GPP_OK;
+}
+
+// the rows of the chunk's t-batches into their tile slots (padding rows are zero points of level, group and mean 0),
+// then the chunk front with U stored in g_U
+static int qbatch_front(gpp_handle* h, const QBatchSpec& s, const Rows& r, const QChunk& c) {
+    CK(cudaMemsetAsync(h->c_xq, 0, sizeof(double) * c.mcp * h->dq, h->st));
+    CK(cudaMemsetAsync(h->c_lvl, 0, sizeof(int) * c.mcp, h->st));
+    CK(cudaMemsetAsync(h->c_noise, 0, sizeof(int) * c.mcp, h->st));
+    CK(cudaMemsetAsync(h->c_mean, 0, sizeof(int) * c.mcp, h->st));
+    CK(qb_copy_rows(s, h->c_xq, r.xq, sizeof(double) * h->dq, c.bt0, c.nb, true, h->st));
+    if (h->dz > 0) CK(qb_copy_rows(s, h->c_lvl, r.level_idx, sizeof(int), c.bt0, c.nb, true, h->st));
+    if (r.noise_idx) CK(qb_copy_rows(s, h->c_noise, r.noise_idx, sizeof(int), c.bt0, c.nb, true, h->st));
+    if (r.mean_idx) CK(qb_copy_rows(s, h->c_mean, r.mean_idx, sizeof(int), c.bt0, c.nb, true, h->st));
+    return chunk_front(h, r, c.base, c.mc, nullptr, h->g_U, nullptr);
+}
+
+// Sigma_t = K**_t - U_t U_t^T of the chunk's t-batches into q_buf
+static int qbatch_sigma(gpp_handle* h, const QBatchSpec& s, const Rows& r, const QChunk& c) {
+    QSyrkArgs sa;
+    memset(&sa, 0, sizeof(sa));
+    sa.U = h->g_U;
+    sa.ldu = h->np;
+    sa.kcols = (int)h->n;
+    sa.rowsq = h->c_rowsq;
+    sa.ldr = h->mc_alloc;
+    sa.tiles_c = h->T;
+    sa.xs = h->c_xs;
+    sa.zpt = h->c_zpt;
+    sa.zs = c.mcp * ZP;
+    sa.dq = h->dq;
+    sa.dqp = h->dqp;
+    sa.dz = h->dz;
+    sa.n_pass = h->n_pass;
+    sa.sf2 = h->sf2;
+    sa.noise_idx = r.noise_idx ? h->c_noise.p : nullptr;
+    sa.noise = hyp_noise(h);
+    sa.n_noise = h->n_noise;
+    sa.include_noise = r.include_noise;
+    sa.q = s.q;
+    sa.qpt = s.qpt;
+    sa.nb = c.nb;
+    sa.cov = h->q_buf;
+    CK(launch_qbatch_syrk(sa, h->kernel, c.tiles, h->st));
+    return GPP_OK;
+}
+
+// Backward, first step after V = U L^-1 (in c_K): W = blockdiag(G + G^T) V into g_U (U is not read again), G_t in q_buf
+static int qbatch_w(gpp_handle* h, const QBatchSpec& s, const QChunk& c) {
+    QWArgs wa;
+    wa.V = h->c_K;
+    wa.ldv = h->np;
+    wa.G = h->q_buf;
+    wa.q = s.q;
+    wa.qpt = s.qpt;
+    wa.nb = c.nb;
+    wa.W = h->g_U;
+    wa.ldw = h->np;
+    qbatch_w_kernel<<<dim3((unsigned)(h->np / QB_KC), (unsigned)c.tiles), QB_THREADS, 0, h->st>>>(wa);
+    CK(cudaGetLastError());
+    count_launch();
+    return GPP_OK;
+}
+
+// Backward, last step: the in-batch K**_t term, then d_xq of the chunk's rows from the gradient partials over tiles_c
+// column tiles (tile layout in g_dvar), gathered to the caller's rows; g_mean: the upstream mean gradient in the tile
+// layout, or NULL
+static int qbatch_grad_finish(gpp_handle* h, const QBatchSpec& s, const QChunk& c, const double* part_m,
+                              const double* part_v, long long ldp, int tiles_c, const double* g_mean, double* d_xq) {
+    QInArgs ia;
+    ia.xs = h->c_xs;
+    ia.zpt = h->c_zpt;
+    ia.zs = c.mcp * ZP;
+    ia.dq = h->dq;
+    ia.dqp = h->dqp;
+    ia.dz = h->dz;
+    ia.n_pass = h->n_pass;
+    ia.G = h->q_buf;
+    ia.q = s.q;
+    ia.qpt = s.qpt;
+    ia.nb = c.nb;
+    ia.rows = (int)c.mcp;
+    ia.part_k = h->g_dmean;
+    CK(launch_qbatch_inbatch_grad(ia, h->kernel, h->st));
+    QFinishArgs qf;
+    qf.part_m = part_m;
+    qf.part_v = part_v;
+    qf.ldp = ldp;
+    qf.tiles_c = tiles_c;
+    qf.part_k = h->g_dmean;
+    qf.g_mean = g_mean;
+    qf.m = (int)c.mcp;
+    qf.dq = h->dq;
+    qf.w = hyp_w(h);
+    qf.sf2 = h->sf2;
+    qf.d_x = h->g_dvar;
+    qbatch_grad_finish_kernel<<<(int)((c.mcp + 255) / 256), 256, 0, h->st>>>(qf);
+    CK(cudaGetLastError());
+    count_launch();
+    CK(qb_copy_rows(s, d_xq, h->g_dvar, sizeof(double) * h->dq, c.bt0, c.nb, false, h->st));
+    return GPP_OK;
+}
+
+// the status word of a gpp_acq_qbatch / gpp_nipv_qbatch chunk, once the chunk has finished
+static int qbatch_status(gpp_handle* h, const char* name, const char* nan_msg) {
+    int info = 0;
+    CK(cudaMemcpyAsync(&info, h->a_info, sizeof(int), cudaMemcpyDeviceToHost, h->st));
+    CK(cudaStreamSynchronize(h->st));
+    if (info & 2) {
+        g_err = nan_msg;
+        return GPP_ERR_NAN;
+    }
+    if (info & 1) {
+        g_err = std::string(name) +
+                ": a t-batch posterior covariance is not positive definite after adding jitter up to 1e-6";
+        return GPP_ERR_NOT_PD;
+    }
+    return GPP_OK;
+}
+
+// values, jitters and the status word of gpp_acq_qbatch / gpp_nipv_qbatch (a chunk holds at most g_step t-batches),
+// and the base samples of the call (e_elems doubles)
+static int ensure_acq_buffers(gpp_handle* h, long long e_elems) {
+    CK(h->a_info.reserve(1, h->st));
+    CK(h->a_E.reserve(e_elems, h->st));
+    CK(h->a_val.reserve(h->g_step, h->st));
+    CK(h->a_jit.reserve(h->g_step, h->st));
+    return GPP_OK;
+}
 
 extern "C" int gpp_posterior_qbatch(gpp_handle* h, int64_t b, int32_t q, const double* xq, const int32_t* level_idx,
                                     const int32_t* noise_idx, const int32_t* mean_idx, int include_noise,
                                     double* mean, double* cov) {
-    int rc = qbatch_check(h, b, q, xq, level_idx, "gpp_posterior_qbatch");
+    int rc = check_rows(h, "gpp_posterior_qbatch", qbatch_count_err(b, q), b, xq, level_idx);
     if (rc != GPP_OK || b == 0) return rc;
-    QBatchSpec s = qbatch_spec(b, q);
-    s.cov = cov;
-    return predict_impl(h, qbatch_rows(s), xq, level_idx, noise_idx, mean_idx, include_noise, 0.0, mean, nullptr,
-                        nullptr, false, nullptr, nullptr, nullptr, &s);
+    const QBatchSpec s = qbatch_spec(b, q);
+    const Rows r = {xq, level_idx, noise_idx, mean_idx, include_noise, 0.0};
+    if ((rc = qbatch_setup(h, s)) != GPP_OK) return rc;
+    for (long long base = 0; base < qbatch_rows(s); base += h->g_step) {
+        const QChunk c = qbatch_chunk(s, base, h->g_step);
+        if ((rc = qbatch_front(h, s, r, c)) != GPP_OK) return rc;
+        if (cov) {
+            if ((rc = qbatch_sigma(h, s, r, c)) != GPP_OK) return rc;
+            const size_t qq = (size_t)q * q;
+            CK(cudaMemcpyAsync(cov + c.bt0 * qq, h->q_buf, sizeof(double) * c.nb * qq, cudaMemcpyDefault, h->st));
+        }
+        if (mean) CK(qb_copy_rows(s, mean, h->c_mu, sizeof(double), c.bt0, c.nb, false, h->st));
+        CK(cudaStreamSynchronize(h->st));
+    }
+    return GPP_OK;
 }
 
 extern "C" int gpp_posterior_qbatch_grad(gpp_handle* h, int64_t b, int32_t q, const double* xq,
                                          const int32_t* level_idx, const int32_t* noise_idx, const int32_t* mean_idx,
                                          int include_noise, const double* g_mean, const double* g_cov, double* d_xq) {
-    int rc = qbatch_check(h, b, q, xq, level_idx, "gpp_posterior_qbatch_grad");
+    int rc = check_rows(h, "gpp_posterior_qbatch_grad", qbatch_count_err(b, q), b, xq, level_idx);
     if (rc != GPP_OK) return rc;
     if (b > 0 && h->dq > 0 && !d_xq) ARG_FAIL("gpp_posterior_qbatch_grad: d_xq missing");
     if (b == 0 || h->dq == 0) return GPP_OK;  // no quantitative input: d_xq is empty
-    QBatchSpec s = qbatch_spec(b, q);
-    s.g_mean = g_mean;
-    s.g_cov = g_cov;
-    s.d_xq = d_xq;
-    return predict_impl(h, qbatch_rows(s), xq, level_idx, noise_idx, mean_idx, include_noise, 0.0, nullptr, nullptr,
-                        nullptr, true, nullptr, nullptr, nullptr, &s);
+    const QBatchSpec s = qbatch_spec(b, q);
+    const Rows r = {xq, level_idx, noise_idx, mean_idx, include_noise, 0.0};
+    if ((rc = qbatch_setup(h, s)) != GPP_OK) return rc;
+    const long long step = h->g_step;
+    for (long long base = 0; base < qbatch_rows(s); base += step) {
+        const QChunk c = qbatch_chunk(s, base, step);
+        if ((rc = qbatch_front(h, s, r, c)) != GPP_OK) return rc;
+        if ((rc = v_gemm(h, h->g_U, h->c_K, c.tiles)) != GPP_OK) return rc;
+        const size_t qq = (size_t)q * q;
+        if (g_cov)
+            CK(cudaMemcpyAsync(h->q_buf, g_cov + c.bt0 * qq, sizeof(double) * c.nb * qq, cudaMemcpyDefault, h->st));
+        else
+            CK(cudaMemsetAsync(h->q_buf, 0, sizeof(double) * c.nb * qq, h->st));
+        if (g_mean) {
+            CK(cudaMemsetAsync(h->q_gm, 0, sizeof(double) * c.mcp, h->st));
+            CK(qb_copy_rows(s, h->q_gm, g_mean, sizeof(double), c.bt0, c.nb, true, h->st));
+        }
+        if ((rc = qbatch_w(h, s, c)) != GPP_OK) return rc;
+        if ((rc = grad_tiles(h, chunk_panels(h, c.mc), training_panels(h), h->alpha, h->g_U, h->np, h->g_part_m,
+                             h->g_part_v, step)) != GPP_OK)
+            return rc;
+        if ((rc = qbatch_grad_finish(h, s, c, h->g_part_m, h->g_part_v, step, h->T, g_mean ? h->q_gm.p : nullptr,
+                                     d_xq)) != GPP_OK)
+            return rc;
+        CK(cudaStreamSynchronize(h->st));
+    }
+    return GPP_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
-// Monte-Carlo batch acquisition (qacq.cuh): the gpp_posterior_qbatch chunk loop, then per t-batch the factor, the
-// samples and the utility in one CTA; with d_xq, the utility's adjoint (G_t, mu_bar) feeds the q-batch backward in the
-// same chunk, so no block leaves the device.
+// Monte-Carlo batch acquisition (qacq.cuh): the gpp_posterior_qbatch chunks, then per t-batch the factor, the samples
+// and the utility in one CTA; with d_xq, the utility's adjoint (G_t, mu_bar) feeds the q-batch backward in the same
+// chunk, so no block leaves the device.
+
+// the utility, its parameters in scaled units and the per-t-batch outputs
+struct QAcqSpec {
+    int kind, n_base, maximize;
+    double best_f, cbeta;
+    long long S;
+    const double* E;  // [S*q] caller's base samples
+    double* values;   // [b]
+    double* jitter;   // [b] or NULL
+};
+
+// values and jitters of the chunk's t-batches from Sigma_t in q_buf; with the gradient, G_t over Sigma_t in q_buf and
+// mu_bar into q_gm
+static int qbatch_mc(gpp_handle* h, const QBatchSpec& s, const QAcqSpec& a, const QChunk& c, bool grad) {
+    if (grad) CK(cudaMemsetAsync(h->q_gm, 0, sizeof(double) * c.mcp, h->st));
+    QAcqArgs aa;
+    memset(&aa, 0, sizeof(aa));
+    aa.blk = h->q_buf;
+    aa.mu = h->c_mu;
+    aa.gm = h->q_gm;
+    aa.E = h->a_E;
+    aa.S = a.S;
+    aa.q = s.q;
+    aa.qpt = s.qpt;
+    aa.n_base = a.n_base;
+    aa.nb = c.nb;
+    aa.sgn = a.maximize ? 1.0 : -1.0;
+    aa.best_f = a.best_f;
+    aa.cbeta = a.cbeta;
+    aa.grad = grad ? 1 : 0;
+    aa.value = h->a_val;
+    aa.jitter = h->a_jit;
+    aa.info = h->a_info;
+    CK(launch_qacq(aa, a.kind, h->st));
+    CK(cudaMemcpyAsync(a.values + c.bt0, h->a_val, sizeof(double) * c.nb, cudaMemcpyDefault, h->st));
+    if (a.jitter) CK(cudaMemcpyAsync(a.jitter + c.bt0, h->a_jit, sizeof(double) * c.nb, cudaMemcpyDefault, h->st));
+    return GPP_OK;
+}
+
 extern "C" int gpp_acq_qbatch(gpp_handle* h, int64_t b, int32_t q_tot, const double* xq, const int32_t* level_idx,
                               const int32_t* noise_idx, const int32_t* mean_idx, int include_noise, int kind,
                               int32_t n_baseline, double best_f, double beta, int maximize, int64_t n_samples,
                               const double* base_samples, double* values, double* d_xq, double* jitter) {
-    int rc = qbatch_check(h, b, q_tot, xq, level_idx, "gpp_acq_qbatch");
+    int rc = check_rows(h, "gpp_acq_qbatch", qbatch_count_err(b, q_tot), b, xq, level_idx);
     if (rc != GPP_OK) return rc;
     if (kind != GPP_QACQ_EI && kind != GPP_QACQ_NEI && kind != GPP_QACQ_UCB) ARG_FAIL("gpp_acq_qbatch: unknown kind");
     if (kind == GPP_QACQ_NEI ? (n_baseline < 1 || n_baseline >= q_tot) : n_baseline != 0)
@@ -2304,110 +2114,64 @@ extern "C" int gpp_acq_qbatch(gpp_handle* h, int64_t b, int32_t q_tot, const dou
     a.E = base_samples;
     a.values = values;
     a.jitter = jitter;
-    QBatchSpec s = qbatch_spec(b, q_tot);
-    s.acq = &a;
+    const QBatchSpec s = qbatch_spec(b, q_tot);
+    const Rows r = {xq, level_idx, noise_idx, mean_idx, include_noise, 0.0};
     const bool grad = d_xq && h->dq > 0;
-    s.d_xq = grad ? d_xq : nullptr;
-    return predict_impl(h, qbatch_rows(s), xq, level_idx, noise_idx, mean_idx, include_noise, 0.0, nullptr, nullptr,
-                        nullptr, grad, nullptr, nullptr, nullptr, &s);
+    if ((rc = qbatch_setup(h, s)) != GPP_OK || (rc = ensure_acq_buffers(h, a.S * s.q)) != GPP_OK) return rc;
+    CK(cudaMemcpyAsync(h->a_E, a.E, sizeof(double) * a.S * s.q, cudaMemcpyDefault, h->st));
+    CK(cudaMemsetAsync(h->a_info, 0, sizeof(int), h->st));
+    const long long step = h->g_step;
+    for (long long base = 0; base < qbatch_rows(s); base += step) {
+        const QChunk c = qbatch_chunk(s, base, step);
+        if ((rc = qbatch_front(h, s, r, c)) != GPP_OK || (rc = qbatch_sigma(h, s, r, c)) != GPP_OK ||
+            (rc = qbatch_mc(h, s, a, c, grad)) != GPP_OK)
+            return rc;
+        if (grad) {  // G_t is in q_buf and mu_bar in q_gm already
+            if ((rc = v_gemm(h, h->g_U, h->c_K, c.tiles)) != GPP_OK || (rc = qbatch_w(h, s, c)) != GPP_OK) return rc;
+            if ((rc = grad_tiles(h, chunk_panels(h, c.mc), training_panels(h), h->alpha, h->g_U, h->np, h->g_part_m,
+                                 h->g_part_v, step)) != GPP_OK)
+                return rc;
+            if ((rc = qbatch_grad_finish(h, s, c, h->g_part_m, h->g_part_v, step, h->T, h->q_gm, d_xq)) != GPP_OK)
+                return rc;
+        }
+        if ((rc = qbatch_status(h, "gpp_acq_qbatch", "gpp_acq_qbatch: NaN in a t-batch posterior or its samples")) !=
+            GPP_OK)
+            return rc;
+    }
+    return GPP_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
 // Batch integrated posterior variance (nipv.cuh): gpp_ipv_points keeps the integration set's panels, U_I and V_I on the
-// handle for the current factor; gpp_nipv_qbatch runs the gpp_posterior_qbatch chunk loop with the candidates' noise,
+// handle for the current factor; gpp_nipv_qbatch runs the gpp_posterior_qbatch chunks with the candidates' noise,
 // forms C^T against the set, and feeds the closed form's adjoint to the q-batch backward in the same chunk.
 static bool ipv_valid(const gpp_handle* h) { return h->factorized && h->i_m > 0 && h->i_gen == h->fgen; }
 
-static int ensure_ipv_buffers(gpp_handle* h, long long mp) {
-    if (mp <= h->i_cap) return GPP_OK;
-    void* olds[] = {h->i_xq, h->i_xs, h->i_nrm, h->i_zpt, h->i_U, h->i_V, h->i_zero, h->i_lvl};
-    CK(cudaStreamSynchronize(h->st));
-    for (void* p : olds)
-        if (p) cudaFree(p);
-    h->i_xq = h->i_xs = h->i_nrm = h->i_zpt = h->i_U = h->i_V = h->i_zero = nullptr;
-    h->i_lvl = nullptr;
-    h->i_cap = 0;
-    const size_t n = (size_t)mp;
-    CK(dev_alloc(&h->i_xq, n * std::max(h->dq, 1)));
-    CK(dev_alloc(&h->i_xs, n * h->dqp));
-    CK(dev_alloc(&h->i_nrm, n));
-    CK(dev_alloc(&h->i_zpt, n * ZP * h->n_pass));
-    CK(dev_alloc(&h->i_U, n * (size_t)h->np));
-    CK(dev_alloc(&h->i_V, n * (size_t)h->np));
-    CK(dev_alloc(&h->i_zero, n));
-    CK(dev_alloc(&h->i_lvl, n));
-    CK(cudaMemsetAsync(h->i_zero, 0, sizeof(double) * n, h->st));
-    h->i_cap = mp;
-    return GPP_OK;
+// rows of one gpp_nipv_qbatch chunk: the C^T buffer [rows x mp of the set] holds at most 2^27 doubles (1 GiB)
+static long long nipv_step(const gpp_handle* h) {
+    return std::min(h->g_step, std::max(128LL, ((1LL << 27) / h->iset.mp) / 128 * 128));
+}
+
+static Panels ipv_panels(const gpp_handle* h) {
+    return {h->iset.xs, h->iset.nrm, h->iset.zpt, h->iset.mp * ZP, (int)h->i_m, (int)(h->iset.mp / CT)};
 }
 
 extern "C" int gpp_ipv_points(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx) {
-    const char* why = nullptr;
-    if (!h) why = "null handle";
-    else if (!h->factorized) why = "call gpp_factorize (or gpp_mll_grad) first";
-    else if (m < 1 || m > GPP_MAX_IPV_POINTS) why = "m must be in [1, GPP_MAX_IPV_POINTS]";
-    else if (h->dq > GPP_MAX_DQ) why = "at most GPP_MAX_DQ quantitative inputs";
-    else if (h->dq > 0 && !xq) why = "xq missing";
-    else if (h->dz > 0 && !level_idx) why = "level_idx missing";
-    if (why) {
-        g_err = std::string("gpp_ipv_points: ") + why;
-        return GPP_ERR_ARG;
-    }
+    int rc = check_rows(h, "gpp_ipv_points", (m < 1 || m > GPP_MAX_IPV_POINTS) ? "m must be in [1, GPP_MAX_IPV_POINTS]"
+                                                                               : nullptr,
+                        m, xq, level_idx);
+    if (rc != GPP_OK) return rc;
     CK(cudaSetDevice(h->device));
     h->i_m = 0;  // no valid set until this call has finished
     const long long mp = round128(m);
-    int rc = ensure_chunk_buffers(h, m);
-    if (rc != GPP_OK || (rc = ensure_ipv_buffers(h, mp)) != GPP_OK) return rc;
-    if (h->dq > 0) CK(cudaMemcpyAsync(h->i_xq, xq, sizeof(double) * m * h->dq, cudaMemcpyDefault, h->st));
-    if (h->dz > 0) CK(cudaMemcpyAsync(h->i_lvl, level_idx, sizeof(int) * m, cudaMemcpyDefault, h->st));
-    PrepArgs pa;
-    pa.xq = h->i_xq;
-    pa.level_idx = h->dz > 0 ? h->i_lvl : nullptr;
-    pa.w = hyp_w(h);
-    pa.centre = h->centre;
-    pa.ztab = hyp_z(h);
-    pa.n = (int)m;
-    pa.np = (int)mp;
-    pa.dq = h->dq;
-    pa.dqp = h->dqp;
-    pa.dz = h->dz;
-    pa.n_combo = h->n_combo;
-    pa.n_pass = h->n_pass;
-    pa.xs = h->i_xs;
-    pa.xst = nullptr;
-    pa.nrm = h->i_nrm;
-    pa.zpt = h->i_zpt;
-    prep_points_kernel<<<(int)((mp + 255) / 256), 256, 0, h->st>>>(pa);
-    CK(cudaGetLastError());
-    count_launch();
-    // U_I through the prediction chunk loop (rows >= m come out zero: K_I is zero there); v_m = sf2 - |U_m|^2
-    // unclamped and without noise
-    JointDest jd;
-    jd.xs = h->i_xs;
-    jd.nrm = h->i_nrm;
-    jd.zpt = h->i_zpt;
-    jd.mp = mp;
-    jd.U = h->i_U;
+    if ((rc = ensure_chunk_buffers(h, m)) != GPP_OK) return rc;
+    CK(h->i_V.reserve(mp * h->np, h->st));
+    CK(h->i_zero.reserve(mp, h->st, true));
+    // U_I through the prediction chunk loop; v_m = sf2 - |U_m|^2 unclamped and without noise
     std::vector<double> v((size_t)m);
-    rc = predict_impl(h, m, xq, level_idx, nullptr, nullptr, 0, -INFINITY, nullptr, v.data(), nullptr, false, nullptr,
-                      nullptr, &jd);
-    if (rc != GPP_OK) return rc;
-    if (h->np > h->n)  // columns n .. Np face K_y's identity padding: zero in exact arithmetic, zero here
-        CK(cudaMemset2DAsync(h->i_U + h->n, sizeof(double) * h->np, 0, sizeof(double) * (h->np - h->n), (size_t)mp,
-                             h->st));
-    GemmOp vo = gemm_default();  // V_I = U_I L^-1 = K_I K_y^-1 (the gradient path's product)
-    vo.A = h->i_U;
-    vo.lda = (int)h->np;
-    vo.B = h->M;
-    vo.ldb = (int)h->np;
-    vo.C = h->i_V;
-    vo.ldc = (int)h->np;
-    vo.tiles_m = vo.tiles_m_last = (int)(mp / CT);
-    vo.tiles_n = h->T;
-    vo.klo_sel = KSEL_TJ;
-    vo.klo_c = 0;
-    vo.khi_c = h->T;
-    CK(launch_gemm(vo, true, false, 1, h->st));
+    const Rows r = {xq, level_idx, nullptr, nullptr, 0, -INFINITY};
+    if ((rc = load_point_set(h, h->iset, m, r, nullptr, nullptr, v.data())) != GPP_OK) return rc;
+    if ((rc = v_gemm(h, h->iset.U, h->i_V, (int)(mp / CT))) != GPP_OK) return rc;  // V_I = U_I L^-1 = K_I K_y^-1
     CK(cudaStreamSynchronize(h->st));
     double sum = 0.0;
     for (long long i = 0; i < m; i++) sum += v[(size_t)i];
@@ -2417,28 +2181,140 @@ extern "C" int gpp_ipv_points(gpp_handle* h, int64_t m, const double* xq, const 
     }
     h->i_vbar = sum / (double)m;
     h->i_m = m;
-    h->i_mp = mp;
     h->i_gen = h->fgen;
+    return GPP_OK;
+}
+
+// C^T = K(X_chunk, X_I) - U_chunk U_I^T into n_C, then per t-batch G_t = C_t^T C_t, A_t's factor and the value (A_bar_t
+// over A_t in q_buf and -A_t^-1 / M in n_Ai with the gradient)
+static int nipv_forward(gpp_handle* h, const QBatchSpec& s, const QChunk& c, double* values, double* jitter,
+                        bool grad) {
+    const Panels iset = ipv_panels(h);
+    CovArgs cc;
+    memset(&cc, 0, sizeof(cc));
+    cc.out = h->n_C;
+    cc.ld = h->iset.mp;
+    int rc = launch_cov_passes(h, cc, chunk_panels(h, c.mc), iset);
+    if (rc != GPP_OK) return rc;
+    GemmOp co = gemm_default();
+    co.A = h->g_U;
+    co.lda = (int)h->np;
+    co.B = h->iset.U;
+    co.ldb = (int)h->np;
+    co.C = h->n_C;
+    co.ldc = (int)h->iset.mp;
+    co.tiles_m = co.tiles_m_last = c.tiles;
+    co.tiles_n = iset.tiles;
+    co.klo_c = 0;
+    co.khi_c = h->T;
+    co.alpha = -1.0;
+    co.beta = 1.0;
+    CK(launch_gemm(co, true, true, 1, h->st));
+    QSyrkArgs ga;
+    memset(&ga, 0, sizeof(ga));
+    ga.U = h->n_C;
+    ga.ldu = h->iset.mp;
+    ga.kcols = (int)h->i_m;
+    ga.q = s.q;
+    ga.qpt = s.qpt;
+    ga.nb = c.nb;
+    ga.cov = h->n_G;
+    CK(launch_qbatch_gram(ga, c.tiles, h->st));
+    NipvArgs na;
+    memset(&na, 0, sizeof(na));
+    na.blk = h->q_buf;
+    na.gram = h->n_G;
+    na.ainv = h->n_Ai;
+    na.q = s.q;
+    na.nb = c.nb;
+    na.inv_m = 1.0 / (double)h->i_m;
+    na.vbar = h->i_vbar;
+    na.grad = grad ? 1 : 0;
+    na.value = h->a_val;
+    na.jitter = h->a_jit;
+    na.info = h->a_info;
+    CK(launch_nipv_block(na, h->st));
+    CK(cudaMemcpyAsync(values + c.bt0, h->a_val, sizeof(double) * c.nb, cudaMemcpyDefault, h->st));
+    if (jitter) CK(cudaMemcpyAsync(jitter + c.bt0, h->a_jit, sizeof(double) * c.nb, cudaMemcpyDefault, h->st));
+    return GPP_OK;
+}
+
+// the backward's integration-set terms after W: -C_bar^T = blockdiag(-2 A^-1 / M) C^T in place over C^T, then
+// W += C_bar^T V_I, the K* term that reaches U_t through C_t (the finish subtracts W's partials)
+static int nipv_w_terms(gpp_handle* h, const QBatchSpec& s, const QChunk& c) {
+    // each CTA stages the 32-column panel of its tile in shared memory before it writes that same panel
+    QWArgs cw;
+    cw.V = h->n_C;
+    cw.ldv = h->iset.mp;
+    cw.G = h->n_Ai;
+    cw.q = s.q;
+    cw.qpt = s.qpt;
+    cw.nb = c.nb;
+    cw.W = h->n_C;
+    cw.ldw = h->iset.mp;
+    qbatch_w_kernel<<<dim3((unsigned)(h->iset.mp / QB_KC), (unsigned)c.tiles), QB_THREADS, 0, h->st>>>(cw);
+    CK(cudaGetLastError());
+    count_launch();
+    GemmOp wo = gemm_default();
+    wo.A = h->n_C;
+    wo.lda = (int)h->iset.mp;
+    wo.B = h->i_V;
+    wo.ldb = (int)h->np;
+    wo.C = h->g_U;
+    wo.ldc = (int)h->np;
+    wo.tiles_m = wo.tiles_m_last = c.tiles;
+    wo.tiles_n = h->T;
+    wo.klo_c = 0;
+    wo.khi_c = (int)(h->iset.mp / CT);
+    wo.alpha = -1.0;
+    wo.beta = 1.0;
+    CK(launch_gemm(wo, true, false, 1, h->st));
     return GPP_OK;
 }
 
 extern "C" int gpp_nipv_qbatch(gpp_handle* h, int64_t b, int32_t q, const double* xq, const int32_t* level_idx,
                                const int32_t* noise_idx, double* values, double* d_xq, double* jitter) {
-    int rc = qbatch_check(h, b, q, xq, level_idx, "gpp_nipv_qbatch");
+    int rc = check_rows(h, "gpp_nipv_qbatch", qbatch_count_err(b, q), b, xq, level_idx);
     if (rc != GPP_OK) return rc;
     if (!ipv_valid(h)) ARG_FAIL("gpp_nipv_qbatch: no integration set for the current factor (call gpp_ipv_points)");
     if (!values) ARG_FAIL("gpp_nipv_qbatch: values missing");
     if (b == 0) return GPP_OK;
-    NipvSpec v;
-    v.values = values;
-    v.jitter = jitter;
-    QBatchSpec s = qbatch_spec(b, q);
-    s.ipv = &v;
-    const bool grad = d_xq && h->dq > 0;
-    s.d_xq = grad ? d_xq : nullptr;
+    const QBatchSpec s = qbatch_spec(b, q);
     // the candidates are fantasised with their observation noise (include_noise = 1); the mean is not needed
-    return predict_impl(h, qbatch_rows(s), xq, level_idx, noise_idx, nullptr, 1, 0.0, nullptr, nullptr, nullptr, grad,
-                        nullptr, nullptr, nullptr, &s);
+    const Rows r = {xq, level_idx, noise_idx, nullptr, 1, 0.0};
+    const bool grad = d_xq && h->dq > 0;
+    // values, jitters and the status word in the acquisition buffers (no base samples); C^T of one chunk, its q x q Gram
+    // and A^-1 blocks and, with the gradient, the partials over the T training and the set's column tiles
+    if ((rc = qbatch_setup(h, s)) != GPP_OK || (rc = ensure_acq_buffers(h, 0)) != GPP_OK) return rc;
+    const long long step = nipv_step(h), imt = h->iset.mp / CT;
+    CK(h->n_C.reserve(step * h->iset.mp, h->st));
+    CK(h->n_G.reserve(step * q, h->st));
+    CK(h->n_Ai.reserve(step * q, h->st));
+    CK(h->n_pm.reserve(grad ? step * (h->T + imt) * h->dq : 0, h->st));
+    CK(h->n_pv.reserve(grad ? step * (h->T + imt) * h->dq : 0, h->st));
+    CK(cudaMemsetAsync(h->a_info, 0, sizeof(int), h->st));
+    for (long long base = 0; base < qbatch_rows(s); base += step) {
+        const QChunk c = qbatch_chunk(s, base, step);
+        if ((rc = qbatch_front(h, s, r, c)) != GPP_OK || (rc = qbatch_sigma(h, s, r, c)) != GPP_OK ||
+            (rc = nipv_forward(h, s, c, values, jitter, grad)) != GPP_OK)
+            return rc;
+        if (grad) {  // A_bar_t is in q_buf already
+            const Panels rows = chunk_panels(h, c.mc);
+            double* pm_i = h->n_pm + (size_t)h->T * h->dq * step;  // partials over the set's column tiles
+            double* pv_i = h->n_pv + (size_t)h->T * h->dq * step;
+            if ((rc = v_gemm(h, h->g_U, h->c_K, c.tiles)) != GPP_OK || (rc = qbatch_w(h, s, c)) != GPP_OK ||
+                (rc = nipv_w_terms(h, s, c)) != GPP_OK ||
+                (rc = grad_tiles(h, rows, training_panels(h), h->alpha, h->g_U, h->np, h->n_pm, h->n_pv, step)) !=
+                    GPP_OK ||
+                (rc = grad_tiles(h, rows, ipv_panels(h), h->i_zero, h->n_C, h->iset.mp, pm_i, pv_i, step)) != GPP_OK ||
+                (rc = qbatch_grad_finish(h, s, c, h->n_pm, h->n_pv, step, h->T + (int)imt, nullptr, d_xq)) != GPP_OK)
+                return rc;
+        }
+        if ((rc = qbatch_status(h, "gpp_nipv_qbatch",
+                                "gpp_nipv_qbatch: NaN in a t-batch posterior or its integrated variance")) != GPP_OK)
+            return rc;
+    }
+    return GPP_OK;
 }
 
 // ---------------------------------------------------------------------------------------------

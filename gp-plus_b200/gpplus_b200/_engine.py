@@ -444,12 +444,7 @@ class Engine:
     def predict(self, xq, level_idx=None, noise_idx=None, mean_idx=None, include_noise: bool = False,
                 min_var: float = 1e-10, out_mean=None, out_var=None):
         """xq / index arrays may be numpy (host) or contiguous torch tensors on this engine's GPU."""
-        if isinstance(xq, np.ndarray) or not hasattr(xq, "data_ptr"):
-            xq = _f64(xq)
-            m = xq.shape[0] if xq.ndim == 2 else (xq.size // max(self.dq, 1))
-            level_idx, noise_idx, mean_idx = _i32(level_idx, m), _i32(noise_idx, m), _i32(mean_idx, m)
-        else:
-            m = int(xq.shape[0])
+        xq, m, level_idx, noise_idx, mean_idx = self._candidates(xq, level_idx, noise_idx, mean_idx)
         mean = np.empty(m) if out_mean is None else out_mean
         var = np.empty(m) if out_var is None else out_var
         rc = self._lib.gpp_predict(self._h, m, _ptr(xq), _ptr(level_idx), _ptr(noise_idx), _ptr(mean_idx),
@@ -463,12 +458,7 @@ class Engine:
         """``predict`` plus the derivatives of the scaled mean and of the clamped variance with respect to the
         quantitative inputs: returns ``(mean [m], var [m], d_mean [m, dq], d_var [m, dq])``.  Inputs and output
         buffers as for ``predict``."""
-        if isinstance(xq, np.ndarray) or not hasattr(xq, "data_ptr"):
-            xq = _f64(xq)
-            m = xq.shape[0] if xq.ndim == 2 else (xq.size // max(self.dq, 1))
-            level_idx, noise_idx, mean_idx = _i32(level_idx, m), _i32(noise_idx, m), _i32(mean_idx, m)
-        else:
-            m = int(xq.shape[0])
+        xq, m, level_idx, noise_idx, mean_idx = self._candidates(xq, level_idx, noise_idx, mean_idx)
         mean = np.empty(m) if out_mean is None else out_mean
         var = np.empty(m) if out_var is None else out_var
         d_mean = np.empty((m, self.dq)) if out_d_mean is None else out_d_mean
@@ -521,19 +511,21 @@ class Engine:
             _raise(rc, "gpp_sample_posterior")
         return samples, float(jit.value)
 
-    def _qbatch(self, xq, q, level_idx, noise_idx, mean_idx):
-        xq, m, level_idx, noise_idx, mean_idx = self._candidates(xq, level_idx, noise_idx, mean_idx)
+    @staticmethod
+    def _tbatches(m, q, caller, q_name="q"):
+        """(b, q) of m rows split into t-batches of q consecutive rows; ValueError naming ``caller`` otherwise."""
         q = int(q)
         if q < 1 or m % q:
-            raise ValueError("posterior_qbatch: %d rows do not split into t-batches of q = %d" % (m, q))
-        return xq, m // q, q, level_idx, noise_idx, mean_idx
+            raise ValueError("%s: %d rows do not split into t-batches of %s = %d" % (caller, m, q_name, q))
+        return m // q, q
 
     def posterior_qbatch(self, xq, q, level_idx=None, noise_idx=None, mean_idx=None, include_noise: bool = False,
                          out_mean=None, out_cov=None):
         """Mean [b, q] (bitwise ``predict``'s) and joint covariance [b, q, q] of b t-batches of q consecutive rows of
         ``xq`` in scaled y units (gpp_posterior_qbatch): each block exactly symmetric and not clamped.  Inputs and
         output buffers as for ``predict``; q <= MAX_QBATCH."""
-        xq, b, q, level_idx, noise_idx, mean_idx = self._qbatch(xq, q, level_idx, noise_idx, mean_idx)
+        xq, m, level_idx, noise_idx, mean_idx = self._candidates(xq, level_idx, noise_idx, mean_idx)
+        b, q = self._tbatches(m, q, "posterior_qbatch")
         mean = np.empty((b, q)) if out_mean is None else out_mean
         cov = np.empty((b, q, q)) if out_cov is None else out_cov
         rc = self._lib.gpp_posterior_qbatch(self._h, b, q, _ptr(xq), _ptr(level_idx), _ptr(noise_idx), _ptr(mean_idx),
@@ -547,7 +539,8 @@ class Engine:
         """d_xq [b*q, dq] = d/d xq of sum(g_mean * mean) + sum(g_cov * cov) of ``posterior_qbatch`` at the same
         arguments (gpp_posterior_qbatch_grad).  ``g_mean`` [b, q] and ``g_cov`` [b, q, q] may be None (zero) and live
         on the host or on this engine's GPU, like the other inputs."""
-        xq, b, q, level_idx, noise_idx, mean_idx = self._qbatch(xq, q, level_idx, noise_idx, mean_idx)
+        xq, m, level_idx, noise_idx, mean_idx = self._candidates(xq, level_idx, noise_idx, mean_idx)
+        b, q = self._tbatches(m, q, "posterior_qbatch")
         g = []
         for a, n in ((g_mean, b * q), (g_cov, b * q * q)):
             if a is not None and (isinstance(a, np.ndarray) or not hasattr(a, "data_ptr")):
@@ -574,10 +567,7 @@ class Engine:
         [S, q_tot] are shared by every t-batch.  ``d_xq`` is d(sum values)/d xq, computed only when ``want_grad``.
         Inputs, base samples and output buffers may live on the host or on this engine's GPU, like ``predict``'s."""
         xq, m, level_idx, noise_idx, mean_idx = self._candidates(xq, level_idx, noise_idx, mean_idx)
-        q_tot = int(q_tot)
-        if q_tot < 1 or m % q_tot:
-            raise ValueError("acquisition_qbatch: %d rows do not split into t-batches of q_tot = %d" % (m, q_tot))
-        b = m // q_tot
+        b, q_tot = self._tbatches(m, q_tot, "acquisition_qbatch", "q_tot")
         if isinstance(base_samples, np.ndarray) or not hasattr(base_samples, "data_ptr"):
             base_samples = _f64(base_samples)
         if len(base_samples.shape) != 2 or int(base_samples.shape[1]) != q_tot:
@@ -613,10 +603,7 @@ class Engine:
         d(sum values)/d xq, computed only when ``want_grad``.  Inputs and output buffers may live on the host or on
         this engine's GPU, like ``predict``'s."""
         xq, m, level_idx, noise_idx, _ = self._candidates(xq, level_idx, noise_idx, None)
-        q = int(q)
-        if q < 1 or m % q:
-            raise ValueError("nipv_qbatch: %d rows do not split into t-batches of q = %d" % (m, q))
-        b = m // q
+        b, q = self._tbatches(m, q, "nipv_qbatch")
         values = np.empty(b) if out_values is None else out_values
         d_xq = None
         if want_grad:
