@@ -18,6 +18,7 @@
 #include "chol.cuh"
 #include "cov.cuh"
 #include "joint.cuh"
+#include "kg.cuh"
 #include "objective.h"
 #include "predict.cuh"
 #include "predict_grad.cuh"
@@ -150,7 +151,8 @@ struct gpp_handle {
     DevArray<double> g_U, g_part_m, g_part_v, g_dmean, g_dvar;
     // t-batch paths: one chunk's q x q blocks (Sigma out, or the upstream gradient G in) and its upstream mean gradient
     DevArray<double> q_buf, q_gm;
-    // gpp_acq_qbatch / gpp_nipv_qbatch: the base samples of the call, one chunk's values and jitters, the status word
+    // gpp_acq_qbatch / gpp_nipv_qbatch / gpp_kg_qbatch: the base samples of the call, one chunk's values and jitters,
+    // the status word
     DevArray<double> a_E, a_val, a_jit;
     DevArray<int> a_info;
     // gpp_predict_joint / gpp_sample_posterior: the joint set and, ld the call's mp, Sigma* (then L*), the diagonal-block
@@ -204,7 +206,7 @@ static const double* hyp_beta(const gpp_handle* h) { return h->hyp + h->dq + zta
 static const double* hyp_sf2(const gpp_handle* h) { return hyp_beta(h) + h->n_mean; }
 static const double* hyp_jitter(const gpp_handle* h) { return hyp_beta(h) + h->n_mean + 1; }
 
-extern "C" int gpp_version(void) { return 111; }
+extern "C" int gpp_version(void) { return 112; }
 
 // process-wide default for handles created afterwards: -1 = by size (INT8-sliced from Np = 4096), 0 = DMMA, 1 = INT8
 static std::atomic<int> g_fp64_mode{-1};
@@ -1960,7 +1962,7 @@ static int qbatch_grad_finish(gpp_handle* h, const QBatchSpec& s, const QChunk& 
     return GPP_OK;
 }
 
-// the status word of a gpp_acq_qbatch / gpp_nipv_qbatch chunk, once the chunk has finished
+// the status word of a gpp_acq_qbatch / gpp_nipv_qbatch / gpp_kg_qbatch chunk, once the chunk has finished
 static int qbatch_status(gpp_handle* h, const char* name, const char* nan_msg) {
     int info = 0;
     CK(cudaMemcpyAsync(&info, h->a_info, sizeof(int), cudaMemcpyDeviceToHost, h->st));
@@ -1977,7 +1979,8 @@ static int qbatch_status(gpp_handle* h, const char* name, const char* nan_msg) {
     return GPP_OK;
 }
 
-// values, jitters and the status word of gpp_acq_qbatch / gpp_nipv_qbatch (a chunk holds at most g_step t-batches),
+// values, jitters and the status word of gpp_acq_qbatch / gpp_nipv_qbatch / gpp_kg_qbatch (a chunk holds at most g_step
+// t-batches),
 // and the base samples of the call (e_elems doubles)
 static int ensure_acq_buffers(gpp_handle* h, long long e_elems) {
     CK(h->a_info.reserve(1, h->st));
@@ -2312,6 +2315,68 @@ extern "C" int gpp_nipv_qbatch(gpp_handle* h, int64_t b, int32_t q, const double
         }
         if ((rc = qbatch_status(h, "gpp_nipv_qbatch",
                                 "gpp_nipv_qbatch: NaN in a t-batch posterior or its integrated variance")) != GPP_OK)
+            return rc;
+    }
+    return GPP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// One-shot knowledge gradient (kg.cuh): the gpp_acq_qbatch chunks with every row's observation noise, then per t-batch
+// the factor of the actual rows' block, the F fantasy solves and the value in one CTA; with d_xq, the adjoint
+// (Sigma_bar_t, mu_bar) feeds the q-batch backward in the same chunk, which gives d_xq of the fantasy rows too.
+extern "C" int gpp_kg_qbatch(gpp_handle* h, int64_t b, int32_t q, int32_t n_fantasies, const double* xq,
+                             const int32_t* level_idx, const int32_t* noise_idx, const int32_t* mean_idx, int maximize,
+                             const double* base_samples, double* values, double* d_xq, double* jitter) {
+    const char* bad = nullptr;
+    if (q < 1 || n_fantasies < 1) bad = "q and n_fantasies must be >= 1";
+    else if ((long long)q + n_fantasies > GPP_MAX_QBATCH) bad = "q + n_fantasies must be <= GPP_MAX_QBATCH";
+    else if (b < 0) bad = "b must be >= 0";
+    int rc = check_rows(h, "gpp_kg_qbatch", bad, b, xq, level_idx);
+    if (rc != GPP_OK) return rc;
+    if (!base_samples || !values) ARG_FAIL("gpp_kg_qbatch: base_samples / values missing");
+    if (b == 0) return GPP_OK;
+    const int q_tot = q + n_fantasies;
+    const QBatchSpec s = qbatch_spec(b, q_tot);
+    // the actual rows are fantasised with their observation noise (include_noise = 1, NULL noise_idx: group 0)
+    const Rows r = {xq, level_idx, noise_idx, mean_idx, 1, 0.0};
+    const bool grad = d_xq && h->dq > 0;
+    const long long e_elems = (long long)n_fantasies * q;
+    if ((rc = qbatch_setup(h, s)) != GPP_OK || (rc = ensure_acq_buffers(h, e_elems)) != GPP_OK) return rc;
+    CK(cudaMemcpyAsync(h->a_E, base_samples, sizeof(double) * e_elems, cudaMemcpyDefault, h->st));
+    CK(cudaMemsetAsync(h->a_info, 0, sizeof(int), h->st));
+    KgArgs ka;
+    memset(&ka, 0, sizeof(ka));
+    ka.blk = h->q_buf;
+    ka.mu = h->c_mu;
+    ka.gm = h->q_gm;
+    ka.E = h->a_E;
+    ka.q = q;
+    ka.nf = n_fantasies;
+    ka.qpt = s.qpt;
+    ka.sgn = maximize ? 1.0 : -1.0;
+    ka.grad = grad ? 1 : 0;
+    ka.value = h->a_val;
+    ka.jitter = h->a_jit;
+    ka.info = h->a_info;
+    const long long step = h->g_step;
+    for (long long base = 0; base < qbatch_rows(s); base += step) {
+        const QChunk c = qbatch_chunk(s, base, step);
+        if ((rc = qbatch_front(h, s, r, c)) != GPP_OK || (rc = qbatch_sigma(h, s, r, c)) != GPP_OK) return rc;
+        if (grad) CK(cudaMemsetAsync(h->q_gm, 0, sizeof(double) * c.mcp, h->st));
+        ka.nb = c.nb;
+        CK(launch_kg_block(ka, h->st));
+        CK(cudaMemcpyAsync(values + c.bt0, h->a_val, sizeof(double) * c.nb, cudaMemcpyDefault, h->st));
+        if (jitter) CK(cudaMemcpyAsync(jitter + c.bt0, h->a_jit, sizeof(double) * c.nb, cudaMemcpyDefault, h->st));
+        if (grad) {  // Sigma_bar_t is in q_buf and mu_bar in q_gm already
+            if ((rc = v_gemm(h, h->g_U, h->c_K, c.tiles)) != GPP_OK || (rc = qbatch_w(h, s, c)) != GPP_OK) return rc;
+            if ((rc = grad_tiles(h, chunk_panels(h, c.mc), training_panels(h), h->alpha, h->g_U, h->np, h->g_part_m,
+                                 h->g_part_v, step)) != GPP_OK)
+                return rc;
+            if ((rc = qbatch_grad_finish(h, s, c, h->g_part_m, h->g_part_v, step, h->T, h->q_gm, d_xq)) != GPP_OK)
+                return rc;
+        }
+        if ((rc = qbatch_status(h, "gpp_kg_qbatch",
+                                "gpp_kg_qbatch: NaN in a t-batch posterior or its fantasy means")) != GPP_OK)
             return rc;
     }
     return GPP_OK;

@@ -49,45 +49,15 @@ __global__ void __launch_bounds__(NV_THREADS) nipv_block_kernel(const NipvArgs a
     const double* G = a.gram + t * q * q;
     double* Y = a.ainv + t * q * q;
 
-    // L_t in shared memory; each rung restarts from A_t (qacq_mc_kernel's ladder)
-    double jit = 0.0;
-    for (int rung = 0;; rung++) {
-        jit = rung == 0 ? 0.0 : (rung == 1 ? 1e-8 : (rung == 2 ? 1e-7 : 1e-6));
-        __syncthreads();
-        for (int idx = tid; idx < q * q; idx += NV_THREADS) {
-            const int i = idx / q, j = idx - i * q;
-            if (j <= i) sM[i * lq + j] = blk[idx] + (i == j ? jit : 0.0);
+    // L_t in shared memory (the ladder of block_ladder_chol)
+    const double jit = block_ladder_chol<NV_THREADS>(blk, q, q, sM, lq, &s_fail);
+    if (s_fail) {
+        if (tid == 0) {
+            atomicOr(a.info, s_fail);
+            a.value[t] = 0.0;
+            a.jitter[t] = jit;
         }
-        if (tid == 0) s_fail = 0;
-        __syncthreads();
-        for (int k = 0; k < q; k++) {
-            if (tid == 0) {
-                const double d = sM[k * lq + k];
-                if (isnan(d)) s_fail = 2;
-                else if (!(d > 0.0)) s_fail = 1;
-                else sM[k * lq + k] = sqrt(d);
-            }
-            __syncthreads();
-            if (s_fail) break;
-            const double lkk = sM[k * lq + k];
-            for (int i = k + 1 + tid; i < q; i += NV_THREADS) sM[i * lq + k] /= lkk;
-            __syncthreads();
-            const int m = q - k - 1;
-            for (int idx = tid; idx < m * m; idx += NV_THREADS) {
-                const int i = k + 1 + idx / m, j = k + 1 + idx % m;
-                if (j <= i) sM[i * lq + j] = fma(-sM[i * lq + k], sM[j * lq + k], sM[i * lq + j]);
-            }
-            __syncthreads();
-        }
-        if (!s_fail) break;
-        if (s_fail == 2 || rung == 3) {
-            if (tid == 0) {
-                atomicOr(a.info, s_fail == 2 ? 2 : 1);
-                a.value[t] = 0.0;
-                a.jitter[t] = jit;
-            }
-            return;  // uniform across the CTA
-        }
+        return;  // uniform across the CTA
     }
     // Y = L^-1 (lower) into the scratch block, thread j owns column j:
     // Y_ij = (delta_ij - sum_{j<=k<i} L_ik Y_kj) / L_ii

@@ -69,45 +69,15 @@ __global__ void __launch_bounds__(QA_THREADS) qacq_mc_kernel(const QAcqArgs a) {
         sMu[i] = a.mu[r0 + i];
         if (isnan(sMu[i])) atomicOr(a.info, 2);
     }
-    // L_t in shared memory; each rung restarts from Sigma_t
-    double jit = 0.0;
-    for (int rung = 0;; rung++) {
-        jit = rung == 0 ? 0.0 : (rung == 1 ? 1e-8 : (rung == 2 ? 1e-7 : 1e-6));
-        __syncthreads();
-        for (int idx = tid; idx < q * q; idx += QA_THREADS) {
-            const int i = idx / q, j = idx - i * q;
-            if (j <= i) sL[i * lq + j] = blk[idx] + (i == j ? jit : 0.0);
+    // L_t in shared memory (the ladder of block_ladder_chol)
+    const double jit = block_ladder_chol<QA_THREADS>(blk, q, q, sL, lq, &s_fail);
+    if (s_fail) {
+        if (tid == 0) {
+            atomicOr(a.info, s_fail);
+            a.value[t] = 0.0;
+            a.jitter[t] = jit;
         }
-        if (tid == 0) s_fail = 0;
-        __syncthreads();
-        for (int k = 0; k < q; k++) {
-            if (tid == 0) {
-                const double d = sL[k * lq + k];
-                if (isnan(d)) s_fail = 2;
-                else if (!(d > 0.0)) s_fail = 1;
-                else sL[k * lq + k] = sqrt(d);
-            }
-            __syncthreads();
-            if (s_fail) break;
-            const double lkk = sL[k * lq + k];
-            for (int i = k + 1 + tid; i < q; i += QA_THREADS) sL[i * lq + k] /= lkk;
-            __syncthreads();
-            const int m = q - k - 1;
-            for (int idx = tid; idx < m * m; idx += QA_THREADS) {
-                const int i = k + 1 + idx / m, j = k + 1 + idx % m;
-                if (j <= i) sL[i * lq + j] = fma(-sL[i * lq + k], sL[j * lq + k], sL[i * lq + j]);
-            }
-            __syncthreads();
-        }
-        if (!s_fail) break;
-        if (s_fail == 2 || rung == 3) {
-            if (tid == 0) {
-                atomicOr(a.info, s_fail == 2 ? 2 : 1);
-                a.value[t] = 0.0;
-                a.jitter[t] = jit;
-            }
-            return;  // uniform across the CTA
-        }
+        return;  // uniform across the CTA
     }
     if (a.grad) {  // L_bar accumulates in the block (Sigma_t is no longer needed)
         __syncthreads();
@@ -203,52 +173,7 @@ __global__ void __launch_bounds__(QA_THREADS) qacq_mc_kernel(const QAcqArgs a) {
         for (int r = tid; r < q; r++) blk[r * q + tid] *= inv_s;
     }
     __syncthreads();
-    // M = tril(L^T L_bar), row i from rows k >= i of L_bar, in place in increasing i
-    for (int i = 0; i < q; i++) {
-        double mv = 0.0;
-        if (tid <= i)
-            for (int k = i; k < q; k++) mv = fma(sL[k * lq + i], blk[k * q + tid], mv);
-        __syncthreads();
-        if (tid <= i) blk[i * q + tid] = mv;
-    }
-    __syncthreads();
-    // P = Phi(M) mirrored: P_ij = P_ji = M_ij / 2 (j <= i)
-    for (int idx = tid; idx < q * q; idx += QA_THREADS) {
-        const int i = idx / q, j = idx - i * q;
-        if (j <= i) {
-            const double v = 0.5 * blk[idx];
-            blk[idx] = v;
-            blk[j * q + i] = v;
-        }
-    }
-    __syncthreads();
-    // Z = P L^-1 row by row (Z L = P), in place
-    if (tid < q) {
-        double* zr = blk + tid * q;
-        for (int j = q - 1; j >= 0; j--) {
-            double v = zr[j];
-            for (int k = j + 1; k < q; k++) v = fma(-zr[k], sL[k * lq + j], v);
-            zr[j] = v / sL[j * lq + j];
-        }
-    }
-    __syncthreads();
-    // G = L^-T Z column by column (L^T G = Z), in place
-    if (tid < q) {
-        for (int j = q - 1; j >= 0; j--) {
-            double v = blk[j * q + tid];
-            for (int k = j + 1; k < q; k++) v = fma(-sL[k * lq + j], blk[k * q + tid], v);
-            blk[j * q + tid] = v / sL[j * lq + j];
-        }
-    }
-    __syncthreads();
-    for (int idx = tid; idx < q * q; idx += QA_THREADS) {  // exact symmetry
-        const int i = idx / q, j = idx - i * q;
-        if (j < i) {
-            const double v = 0.5 * (blk[idx] + blk[j * q + i]);
-            blk[idx] = v;
-            blk[j * q + i] = v;
-        }
-    }
+    block_chol_adjoint<QA_THREADS>(blk, q, q, sL, lq);
 }
 
 template <int KIND>

@@ -311,4 +311,101 @@ inline cudaError_t launch_qbatch_inbatch_grad(const QInArgs& a, int kind, cudaSt
     return cudaGetLastError();
 }
 
+// ---- per-t-batch block factor and its adjoint, for kernels that run one CTA of NT threads per t-batch ----
+
+// L = chol(A + j I) of the leading n x n block of A (row-major, leading dimension lda, lower triangle read) into sL
+// [n][lq] in shared memory, j the first rung of 0, 1e-8, 1e-7, 1e-6 whose pivots are all > 0 (dpotrf's test, the
+// psd_safe_cholesky ladder); each rung restarts from A.  Called by every thread of the CTA; returns j with *s_fail
+// (shared) 0 when that rung factored, 1 when every rung failed and 2 on a NaN pivot, the same for all threads.
+template <int NT>
+__device__ __forceinline__ double block_ladder_chol(const double* A, int n, int lda, double* sL, int lq, int* s_fail) {
+    const int tid = threadIdx.x;
+    double jit = 0.0;
+    for (int rung = 0;; rung++) {
+        jit = rung == 0 ? 0.0 : (rung == 1 ? 1e-8 : (rung == 2 ? 1e-7 : 1e-6));
+        __syncthreads();
+        for (int idx = tid; idx < n * n; idx += NT) {
+            const int i = idx / n, j = idx - i * n;
+            if (j <= i) sL[i * lq + j] = A[i * lda + j] + (i == j ? jit : 0.0);
+        }
+        if (tid == 0) *s_fail = 0;
+        __syncthreads();
+        for (int k = 0; k < n; k++) {
+            if (tid == 0) {
+                const double d = sL[k * lq + k];
+                if (isnan(d)) *s_fail = 2;
+                else if (!(d > 0.0)) *s_fail = 1;
+                else sL[k * lq + k] = sqrt(d);
+            }
+            __syncthreads();
+            if (*s_fail) break;
+            const double lkk = sL[k * lq + k];
+            for (int i = k + 1 + tid; i < n; i += NT) sL[i * lq + k] /= lkk;
+            __syncthreads();
+            const int m = n - k - 1;
+            for (int idx = tid; idx < m * m; idx += NT) {
+                const int i = k + 1 + idx / m, j = k + 1 + idx % m;
+                if (j <= i) sL[i * lq + j] = fma(-sL[i * lq + k], sL[j * lq + k], sL[i * lq + j]);
+            }
+            __syncthreads();
+        }
+        if (!*s_fail || *s_fail == 2 || rung == 3) return jit;
+    }
+}
+
+// torch's cholesky backward on the leading n x n block of B (leading dimension ldb), in place: L_bar in its lower
+// triangle in, A_bar = L^-T Phi(L^T L_bar) L^-1 out, exactly symmetric (Phi keeps the lower triangle and halves its
+// diagonal, then mirrors it).  L is block_ladder_chol's factor; n <= NT; called by every thread after a barrier that
+// follows the last write of L_bar.
+template <int NT>
+__device__ __forceinline__ void block_chol_adjoint(double* B, int n, int ldb, const double* sL, int lq) {
+    const int tid = threadIdx.x;
+    // M = tril(L^T L_bar), row i from rows k >= i of L_bar, in place in increasing i
+    for (int i = 0; i < n; i++) {
+        double mv = 0.0;
+        if (tid <= i)
+            for (int k = i; k < n; k++) mv = fma(sL[k * lq + i], B[k * ldb + tid], mv);
+        __syncthreads();
+        if (tid <= i) B[i * ldb + tid] = mv;
+    }
+    __syncthreads();
+    // P = Phi(M) mirrored: P_ij = P_ji = M_ij / 2 (j <= i)
+    for (int idx = tid; idx < n * n; idx += NT) {
+        const int i = idx / n, j = idx - i * n;
+        if (j <= i) {
+            const double v = 0.5 * B[i * ldb + j];
+            B[i * ldb + j] = v;
+            B[j * ldb + i] = v;
+        }
+    }
+    __syncthreads();
+    // Z = P L^-1 row by row (Z L = P), in place
+    if (tid < n) {
+        double* zr = B + tid * ldb;
+        for (int j = n - 1; j >= 0; j--) {
+            double v = zr[j];
+            for (int k = j + 1; k < n; k++) v = fma(-zr[k], sL[k * lq + j], v);
+            zr[j] = v / sL[j * lq + j];
+        }
+    }
+    __syncthreads();
+    // G = L^-T Z column by column (L^T G = Z), in place
+    if (tid < n) {
+        for (int j = n - 1; j >= 0; j--) {
+            double v = B[j * ldb + tid];
+            for (int k = j + 1; k < n; k++) v = fma(-sL[k * lq + j], B[k * ldb + tid], v);
+            B[j * ldb + tid] = v / sL[j * lq + j];
+        }
+    }
+    __syncthreads();
+    for (int idx = tid; idx < n * n; idx += NT) {  // exact symmetry
+        const int i = idx / n, j = idx - i * n;
+        if (j < i) {
+            const double v = 0.5 * (B[i * ldb + j] + B[j * ldb + i]);
+            B[i * ldb + j] = v;
+            B[j * ldb + i] = v;
+        }
+    }
+}
+
 }  // namespace gpp

@@ -29,7 +29,7 @@ EXPORTS = (
     "gpp_mll_grad",
     "gpp_get_timings", "gpp_get_stats", "gpp_covariance", "gpp_fetch", "gpp_factorize", "gpp_predict", "gpp_predict_grad",
     "gpp_predict_joint", "gpp_sample_posterior", "gpp_posterior_qbatch", "gpp_posterior_qbatch_grad", "gpp_acq_qbatch",
-    "gpp_ipv_points", "gpp_nipv_qbatch", "gpp_acq_argmax",
+    "gpp_ipv_points", "gpp_nipv_qbatch", "gpp_kg_qbatch", "gpp_acq_argmax",
     "gpp_probe_dgemm", "gpp_probe_i8", "gpp_set_fp64_mode", "gpp_get_fp64_mode", "gpp_set_theta_layout", "gpp_objective", "gpp_objective_enqueue", "gpp_objective_collect",
 )
 
@@ -154,6 +154,9 @@ def load_library():
         lib.gpp_nipv_qbatch.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.c_void_p, C.c_void_p, C.c_void_p]
         lib.gpp_nipv_qbatch.restype = C.c_int
+        lib.gpp_kg_qbatch.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.gpp_kg_qbatch.restype = C.c_int
         lib.gpp_acq_argmax.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_double,
                                        C.c_double, C.c_double, C.c_double, C.c_void_p, _dp, C.POINTER(C.c_int64)]
@@ -613,6 +616,37 @@ class Engine:
                                        _ptr(d_xq), _ptr(jitter))
         if rc != GPP_OK:
             _raise(rc, "gpp_nipv_qbatch")
+        return values, d_xq, jitter
+
+    def kg_qbatch(self, xq, q, n_fantasies, base_samples, maximize: bool = True, want_grad: bool = True,
+                  level_idx=None, noise_idx=None, mean_idx=None, out_values=None, out_d_xq=None):
+        """One-shot knowledge gradient of the b t-batches of q + n_fantasies consecutive rows of ``xq``, the q actual
+        points followed by the fantasy solutions (gpp_kg_qbatch): returns ``(values [b], d_xq [b*q_tot, dq] or None,
+        jitter [b])`` in scaled y units.  Each value is the mean over the fantasies f of the posterior mean at fantasy
+        solution f after also observing the actual points (with their ``noise_idx`` groups' noise) at their posterior
+        mean plus L e_f; ``base_samples`` [n_fantasies, q] are shared by every t-batch.  ``d_xq`` is
+        d(sum values)/d xq for all rows, computed only when ``want_grad``.  Inputs, base samples and output buffers
+        may live on the host or on this engine's GPU, like ``predict``'s."""
+        xq, m, level_idx, noise_idx, mean_idx = self._candidates(xq, level_idx, noise_idx, mean_idx)
+        q, nf = int(q), int(n_fantasies)
+        if q < 1 or nf < 1:
+            raise ValueError("kg_qbatch: q and n_fantasies must be >= 1, got %d and %d" % (q, nf))
+        b, q_tot = self._tbatches(m, q + nf, "kg_qbatch", "q + n_fantasies")
+        if isinstance(base_samples, np.ndarray) or not hasattr(base_samples, "data_ptr"):
+            base_samples = _f64(base_samples)
+        if tuple(int(n) for n in base_samples.shape) != (nf, q):
+            raise ValueError("kg_qbatch: base_samples must have shape [%d, %d], got %s"
+                             % (nf, q, tuple(base_samples.shape)))
+        values = np.empty(b) if out_values is None else out_values
+        d_xq = None
+        if want_grad:
+            d_xq = np.empty((m, self.dq)) if out_d_xq is None else out_d_xq
+        jitter = np.empty(b)
+        rc = self._lib.gpp_kg_qbatch(self._h, b, q, nf, _ptr(xq), _ptr(level_idx), _ptr(noise_idx), _ptr(mean_idx),
+                                     1 if maximize else 0, _ptr(base_samples), _ptr(values), _ptr(d_xq),
+                                     _ptr(jitter))
+        if rc != GPP_OK:
+            _raise(rc, "gpp_kg_qbatch")
         return values, d_xq, jitter
 
     def acq_argmax(self, xq, cost_idx, cost: Sequence[float], kind_by_cost: Sequence[int], best_f: Sequence[float],

@@ -491,6 +491,15 @@ class GP_Plus(GPR):
                                           maximize=maximize, observation_noise=observation_noise,
                                           mc_points=mc_points)
 
+    def knowledge_gradient(self, X, num_fantasies, base_samples=None, seed=0, maximize=True, current_value=None,
+                           cost_by_source=None):
+        """One-shot knowledge gradient of the t-batches of ``X`` [..., q + num_fantasies, d] in the original y units,
+        optionally net of ``current_value`` and per unit cost of the actual rows' sources (GPR.knowledge_gradient);
+        differentiable in ``X`` when it requires a gradient, as ``predict_with_grad``."""
+        X = data_type_check(X)
+        return super().knowledge_gradient(X, num_fantasies, base_samples=base_samples, seed=seed, maximize=maximize,
+                                          current_value=current_value, cost_by_source=cost_by_source)
+
     def noise_value(self):
         return self.likelihood.noise_covar.noise.detach() * self.y_std ** 2
 

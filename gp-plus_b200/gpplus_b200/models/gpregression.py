@@ -198,6 +198,24 @@ class _EngineNIPV(_EngineQBatchAcquisition):
         return torch.as_tensor(np.asarray(values)), jitter
 
 
+class _EngineKG(_EngineQBatchAcquisition):
+    """One-shot knowledge-gradient values [b] of the t-batches of ``x`` [b, q + F, d] (gpp_kg_qbatch), differentiable
+    w.r.t. the quantitative columns of all q + F rows as ``_EngineQBatchAcquisition``, whose backward it shares."""
+
+    @staticmethod
+    def forward(ctx, x, eng, xq, q, cols, kwargs):
+        b, q_tot, d = x.shape
+        values, d_xq, jitter = eng.kg_qbatch(xq, q, q_tot - q, want_grad=len(cols) > 0, **kwargs)
+        dx = torch.zeros(b, q_tot, d, dtype=torch.float64)
+        if len(cols) > 0:
+            dx[:, :, cols] = torch.as_tensor(np.asarray(d_xq)).reshape(b, q_tot, len(cols))
+        ctx.dx = dx
+        ctx.x_meta = (x.dtype, x.device)
+        jitter = torch.as_tensor(np.asarray(jitter))
+        ctx.mark_non_differentiable(jitter)
+        return torch.as_tensor(np.asarray(values)), jitter
+
+
 class GPR(Module):
     def __init__(
         self,
@@ -687,6 +705,66 @@ class GPR(Module):
             warnings.warn("A not p.d., added jitter of %.1e to the diagonal" % float(jitter.max()), NumericalWarning)
         y_std = self.y_std.to(self._out_dtype())
         return (y_std * y_std * v.to(self._out_dtype())).reshape(batch)
+
+    def knowledge_gradient(self, X: torch.Tensor, num_fantasies: int, base_samples: Optional[torch.Tensor] = None,
+                           seed: int = 0, maximize: bool = True, current_value: Optional[float] = None,
+                           cost_by_source=None) -> torch.Tensor:
+        """One-shot knowledge gradient (botorch's qKnowledgeGradient with the PosteriorMean value function) of every
+        t-batch of X [..., q + F, d] in the original y units: values [...] (gpp_kg_qbatch).  The last F =
+        ``num_fantasies`` rows of each t-batch are the fantasy solutions and the first q the actual points (botorch's
+        X_actual_and_fantasies).  The value is the mean over the fantasies f of sigma times the posterior mean at
+        fantasy solution f after also observing the actual points, each with its observation noise, at y_f = mu + L
+        e_f (sigma = +1 to maximise, -1 to minimise).  All t-batches share the base samples e [F, q], by default
+        ``num_fantasies`` scrambled Sobol normal draws of ``seed``.
+
+        ``current_value`` (original units, times sigma like the values: the best posterior mean, e.g. from
+        ``optimize_posterior_mean``) is subtracted.  ``cost_by_source`` ({source: cost} or a sequence indexed by
+        source; needs ``current_value``) then divides that gain by the summed cost of the q actual rows, whose source
+        is the last column of X: botorch's qMultiFidelityKnowledgeGradient with an InverseCostWeightedUtility of a
+        deterministic per-source cost.  Fixing the fantasy rows' source column at the target source is the
+        multi-fidelity projection.  The values are differentiable in the quantitative columns of all q + F rows when X
+        requires a gradient; a t-batch whose covariance needed jitter raises a NumericalWarning."""
+        if cost_by_source is not None and current_value is None:
+            raise ValueError("knowledge_gradient: cost_by_source needs current_value")
+        if X.dim() < 2:
+            raise ValueError("knowledge_gradient expects X of shape [..., q + num_fantasies, d]")
+        self.eval()
+        nf = int(num_fantasies)
+        batch, q_tot, d = X.shape[:-2], int(X.shape[-2]), int(X.shape[-1])
+        q = q_tot - nf
+        if nf < 1 or q < 1:
+            raise ValueError("knowledge_gradient: X has %d rows per t-batch, which does not leave q >= 1 actual rows "
+                             "besides num_fantasies = %d >= 1" % (q_tot, nf))
+        if q_tot > _engine.MAX_QBATCH:
+            raise ValueError("knowledge_gradient: q + num_fantasies = %d exceeds %d" % (q_tot, _engine.MAX_QBATCH))
+        if base_samples is None:
+            base_samples = sobol_normal_samples(nf, q, seed)
+        base = np.ascontiguousarray(torch.as_tensor(base_samples).detach().to("cpu", torch.float64).numpy())
+        if base.shape != (nf, q):
+            raise ValueError("knowledge_gradient: base_samples must have shape [%d, %d], got %s"
+                             % (nf, q, base.shape))
+        x = X.reshape(-1, q_tot, d)
+        eng, xq, kwargs = self._joint_request(x.detach().double().reshape(-1, d), True)
+        kwargs.pop("include_noise")
+        kwargs.update(base_samples=base, maximize=bool(maximize))
+        if torch.is_grad_enabled() and X.requires_grad:
+            v, jitter = _EngineKG.apply(x, eng, xq, q, self._quant_columns(), kwargs)
+        else:
+            values, _, jitter = eng.kg_qbatch(xq, q, nf, want_grad=False, **kwargs)
+            v, jitter = torch.as_tensor(np.asarray(values)), torch.as_tensor(np.asarray(jitter))
+        if bool((jitter > 0).any()):
+            warnings.warn("A not p.d., added jitter of %.1e to the diagonal" % float(jitter.max()), NumericalWarning)
+        dtype = self._out_dtype()
+        sgn = 1.0 if maximize else -1.0
+        out = sgn * float(self.y_min) + float(self.y_std) * v.to(dtype)
+        if current_value is not None:
+            out = out - float(current_value)
+        if cost_by_source is not None:
+            src = x.detach()[:, :q, -1].cpu().double().round().long()
+            cost = torch.tensor([[float(cost_by_source[int(s_)]) for s_ in row] for row in src.tolist()],
+                                dtype=torch.float64).sum(-1)
+            out = out / cost.to(dtype)
+        return out.reshape(batch)
 
     def reset_parameters(self) -> None:
         """Reset parameters by sampling from the priors (gpregression.py:168-174)."""

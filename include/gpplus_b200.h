@@ -18,6 +18,8 @@
  *     gradients in X: GPR.acquisition_qbatch, bayesian_optimizations/qbatch.py -> gpp_acq_qbatch
  *   - botorch qNegIntegratedPosteriorVariance and its gradient in X: GPR.acquisition_qbatch(X, "qNIPV", mc_points)
  *                                 -> gpp_ipv_points, gpp_nipv_qbatch
+ *   - botorch one-shot qKnowledgeGradient (cost-aware as qMultiFidelityKnowledgeGradient) and its gradient in X:
+ *     GPR.knowledge_gradient, bayesian_optimizations/qbatch.py -> gpp_kg_qbatch
  *   - AF_*_Engineering + argmax   bayesian_optimizations/AFs.py:102-159,
  *                                 bayesian_optimizations/BO_GP_plus.py:183-194 -> gpp_acq_argmax
  *   - covar_module(x).evaluate()  models/gp_plus.py:472-474      -> gpp_covariance
@@ -296,6 +298,30 @@ int gpp_nipv_qbatch(gpp_handle* h, int64_t b, int32_t q, const double* xq, const
                     double* values,   /* [b] */
                     double* d_xq,     /* [b * q * dq] or NULL: values only */
                     double* jitter);  /* [b] or NULL */
+
+/* One-shot knowledge gradient (botorch's qKnowledgeGradient.forward, acquisition/knowledge_gradient.py, with the
+ * PosteriorMean value function and current_value = None).  Each of the b t-batches holds q_tot = q + n_fantasies
+ * consecutive rows of xq: the q actual points X_t, then the F = n_fantasies fantasy solutions x'_f (botorch's
+ * X_actual_and_fantasies layout, _split_fantasy_points).  With mu and Sigma bitwise those of
+ * gpp_posterior_qbatch(..., include_noise = 1) on the same rows (a NULL noise_idx means group 0), in scaled y units:
+ *   A_t = Sigma[0:q, 0:q] + j_t I,  L_t = chol(A_t)   j_t the first of 0, 1e-8, 1e-7, 1e-6 that factors
+ *   c_f = Sigma[0:q, q+f]                             posterior cross-covariance of X_t and x'_f
+ *   values[t] = (1/F) sum_f sigma (mu[q+f] + (L_t^-1 c_f) . e_f)   sigma = +1 to maximise, -1 to minimise
+ * e_f is row f of base_samples [F x q], shared by every t-batch.  Each term is the posterior mean at x'_f of the model
+ * that also observed X_t, each row with its group's noise, at y_f = mu[0:q] + L_t e_f.
+ *   d_xq [b*q_tot*dq] = d(sum_t values[t]) / d xq for all q_tot rows, quantitative inputs only (NULL: values only)
+ *   jitter [b] = j_t (may be NULL)
+ * A t-batch's outputs do not depend on the other t-batches of the call or on how it is split into chunks.  The call
+ * does not change the factor of K_y, alpha, gpp_get_stats or gpp_get_timings.  GPP_ERR_NOT_PD when a t-batch fails
+ * every rung, GPP_ERR_NAN on NaN.  q < 1, n_fantasies < 1, q + n_fantasies > GPP_MAX_QBATCH, b < 0, a missing
+ * base_samples or values, or dq > 32 return GPP_ERR_ARG before any allocation.  It uses the buffers of gpp_acq_qbatch
+ * and allocates none of its own. */
+int gpp_kg_qbatch(gpp_handle* h, int64_t b, int32_t q, int32_t n_fantasies, const double* xq,
+                  const int32_t* level_idx, const int32_t* noise_idx, const int32_t* mean_idx, int maximize,
+                  const double* base_samples,  /* [n_fantasies * q], shared by all t-batches */
+                  double* values,              /* [b] */
+                  double* d_xq,                /* [b * (q + n_fantasies) * dq] or NULL: values only */
+                  double* jitter);             /* [b] or NULL */
 
 /* fused predict + acquisition + argmax over m candidates (BO_GP_plus.py:183-194).
  * y_min/y_std undo the target scaling; cost_idx[m] selects cost[n_cost]; kind_by_cost[n_cost]
