@@ -17,6 +17,7 @@
 
 #include "chol.cuh"
 #include "cov.cuh"
+#include "gibbon.cuh"
 #include "joint.cuh"
 #include "kg.cuh"
 #include "objective.h"
@@ -151,10 +152,14 @@ struct gpp_handle {
     DevArray<double> g_U, g_part_m, g_part_v, g_dmean, g_dvar;
     // t-batch paths: one chunk's q x q blocks (Sigma out, or the upstream gradient G in) and its upstream mean gradient
     DevArray<double> q_buf, q_gm;
-    // gpp_acq_qbatch / gpp_nipv_qbatch / gpp_kg_qbatch: the base samples of the call, one chunk's values and jitters,
-    // the status word
+    // gpp_acq_qbatch / gpp_nipv_qbatch / gpp_kg_qbatch / gpp_gibbon_qbatch: the base samples (max values) of the call,
+    // one chunk's values and jitters, the status word
     DevArray<double> a_E, a_val, a_jit;
     DevArray<int> a_info;
+    // gpp_max_value_quartiles: the m marginal means and variances, the per-block partials, the bracket state and the
+    // NaN flag
+    DevArray<double> v_mu, v_var, v_part, v_state;
+    DevArray<int> v_nan;
     // gpp_predict_joint / gpp_sample_posterior: the joint set and, ld the call's mp, Sigma* (then L*), the diagonal-block
     // inverses of L* (a full [mp x mp] matrix: potrf_blocked addresses them with Sigma*'s leading dimension), the
     // diagonal additions, mu, the log-determinant partials, the noise groups, the status word, and one chunk of base
@@ -206,7 +211,7 @@ static const double* hyp_beta(const gpp_handle* h) { return h->hyp + h->dq + zta
 static const double* hyp_sf2(const gpp_handle* h) { return hyp_beta(h) + h->n_mean; }
 static const double* hyp_jitter(const gpp_handle* h) { return hyp_beta(h) + h->n_mean + 1; }
 
-extern "C" int gpp_version(void) { return 112; }
+extern "C" int gpp_version(void) { return 113; }
 
 // process-wide default for handles created afterwards: -1 = by size (INT8-sliced from Np = 4096), 0 = DMMA, 1 = INT8
 static std::atomic<int> g_fp64_mode{-1};
@@ -1962,7 +1967,8 @@ static int qbatch_grad_finish(gpp_handle* h, const QBatchSpec& s, const QChunk& 
     return GPP_OK;
 }
 
-// the status word of a gpp_acq_qbatch / gpp_nipv_qbatch / gpp_kg_qbatch chunk, once the chunk has finished
+// the status word of a gpp_acq_qbatch / gpp_nipv_qbatch / gpp_kg_qbatch / gpp_gibbon_qbatch chunk, once the chunk has
+// finished
 static int qbatch_status(gpp_handle* h, const char* name, const char* nan_msg) {
     int info = 0;
     CK(cudaMemcpyAsync(&info, h->a_info, sizeof(int), cudaMemcpyDeviceToHost, h->st));
@@ -1979,9 +1985,8 @@ static int qbatch_status(gpp_handle* h, const char* name, const char* nan_msg) {
     return GPP_OK;
 }
 
-// values, jitters and the status word of gpp_acq_qbatch / gpp_nipv_qbatch / gpp_kg_qbatch (a chunk holds at most g_step
-// t-batches),
-// and the base samples of the call (e_elems doubles)
+// values, jitters and the status word of gpp_acq_qbatch / gpp_nipv_qbatch / gpp_kg_qbatch / gpp_gibbon_qbatch (a chunk
+// holds at most g_step t-batches), and the base samples (max values) of the call (e_elems doubles)
 static int ensure_acq_buffers(gpp_handle* h, long long e_elems) {
     CK(h->a_info.reserve(1, h->st));
     CK(h->a_E.reserve(e_elems, h->st));
@@ -2379,6 +2384,144 @@ extern "C" int gpp_kg_qbatch(gpp_handle* h, int64_t b, int32_t q, int32_t n_fant
                                 "gpp_kg_qbatch: NaN in a t-batch posterior or its fantasy means")) != GPP_OK)
             return rc;
     }
+    return GPP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// GIBBON (gibbon.cuh): the gpp_acq_qbatch chunks with the latent block (no noise), then per t-batch the noise of the
+// actual rows, the factor of their block, the diversity and quality terms and the value in one CTA; with d_xq, the
+// adjoint (Sigma_bar_t, mu_bar) feeds the q-batch backward in the same chunk, which gives d_xq of the target rows too.
+extern "C" int gpp_gibbon_qbatch(gpp_handle* h, int64_t b, int32_t q, int32_t projected, const double* xq,
+                                 const int32_t* level_idx, const int32_t* noise_idx, const int32_t* mean_idx,
+                                 int maximize, int64_t n_max_values, const double* max_values, double* values,
+                                 double* d_xq, double* jitter) {
+    const char* bad = nullptr;
+    if (q < 1) bad = "q must be >= 1";
+    else if (projected != 0 && projected != 1) bad = "projected must be 0 or 1";
+    else if ((long long)q * (1 + projected) > GPP_MAX_QBATCH) bad = "q * (1 + projected) must be <= GPP_MAX_QBATCH";
+    else if (b < 0) bad = "b must be >= 0";
+    int rc = check_rows(h, "gpp_gibbon_qbatch", bad, b, xq, level_idx);
+    if (rc != GPP_OK) return rc;
+    if (n_max_values < 1 || n_max_values > GPP_MAX_MC_SAMPLES)
+        ARG_FAIL("gpp_gibbon_qbatch: n_max_values must be in [1, GPP_MAX_MC_SAMPLES]");
+    if (!max_values || !values) ARG_FAIL("gpp_gibbon_qbatch: max_values / values missing");
+    if (b == 0) return GPP_OK;
+    const int q_tot = q * (1 + projected);
+    const QBatchSpec s = qbatch_spec(b, q_tot);
+    // the latent block: the actual rows' noise is added inside gibbon_block_kernel, the target rows stay noiseless
+    const Rows r = {xq, level_idx, noise_idx, mean_idx, 0, 0.0};
+    const bool grad = d_xq && h->dq > 0;
+    if ((rc = qbatch_setup(h, s)) != GPP_OK || (rc = ensure_acq_buffers(h, n_max_values)) != GPP_OK) return rc;
+    CK(cudaMemcpyAsync(h->a_E, max_values, sizeof(double) * n_max_values, cudaMemcpyDefault, h->st));
+    CK(cudaMemsetAsync(h->a_info, 0, sizeof(int), h->st));
+    GibbonArgs ga;
+    memset(&ga, 0, sizeof(ga));
+    ga.blk = h->q_buf;
+    ga.mu = h->c_mu;
+    ga.gm = h->q_gm;
+    ga.noise_idx = noise_idx ? h->c_noise.p : nullptr;
+    ga.noise = hyp_noise(h);
+    ga.n_noise = h->n_noise;
+    ga.mv = h->a_E;
+    ga.K = (int)n_max_values;
+    ga.q = q;
+    ga.q_tot = q_tot;
+    ga.qpt = s.qpt;
+    ga.sgn = maximize ? 1.0 : -1.0;
+    ga.grad = grad ? 1 : 0;
+    ga.value = h->a_val;
+    ga.jitter = h->a_jit;
+    ga.info = h->a_info;
+    const long long step = h->g_step;
+    for (long long base = 0; base < qbatch_rows(s); base += step) {
+        const QChunk c = qbatch_chunk(s, base, step);
+        if ((rc = qbatch_front(h, s, r, c)) != GPP_OK || (rc = qbatch_sigma(h, s, r, c)) != GPP_OK) return rc;
+        if (grad) CK(cudaMemsetAsync(h->q_gm, 0, sizeof(double) * c.mcp, h->st));
+        ga.nb = c.nb;
+        CK(launch_gibbon_block(ga, h->st));
+        CK(cudaMemcpyAsync(values + c.bt0, h->a_val, sizeof(double) * c.nb, cudaMemcpyDefault, h->st));
+        if (jitter) CK(cudaMemcpyAsync(jitter + c.bt0, h->a_jit, sizeof(double) * c.nb, cudaMemcpyDefault, h->st));
+        if (grad) {  // Sigma_bar_t is in q_buf and mu_bar in q_gm already
+            if ((rc = v_gemm(h, h->g_U, h->c_K, c.tiles)) != GPP_OK || (rc = qbatch_w(h, s, c)) != GPP_OK) return rc;
+            if ((rc = grad_tiles(h, chunk_panels(h, c.mc), training_panels(h), h->alpha, h->g_U, h->np, h->g_part_m,
+                                 h->g_part_v, step)) != GPP_OK)
+                return rc;
+            if ((rc = qbatch_grad_finish(h, s, c, h->g_part_m, h->g_part_v, step, h->T, h->q_gm, d_xq)) != GPP_OK)
+                return rc;
+        }
+        if ((rc = qbatch_status(h, "gpp_gibbon_qbatch",
+                                "gpp_gibbon_qbatch: NaN in a t-batch posterior or its GIBBON value")) != GPP_OK)
+            return rc;
+    }
+    return GPP_OK;
+}
+
+// Max-value quartiles (gibbon.cuh): the marginals by the pointwise family into v_mu / v_var (bitwise gpp_predict's at
+// include_noise = 0, min_var = 1e-8), the bracket, its widening (one host check per step) and 40 bisection steps of
+// the three brackets on the device
+extern "C" int gpp_max_value_quartiles(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
+                                       const int32_t* mean_idx, int maximize, double* quartiles) {
+    int rc = check_rows(h, "gpp_max_value_quartiles", m < 1 ? "m must be >= 1" : nullptr, m, xq, level_idx);
+    if (rc != GPP_OK) return rc;
+    if (!quartiles) ARG_FAIL("gpp_max_value_quartiles: quartiles missing");
+    CK(cudaSetDevice(h->device));
+    const int nblk = mv_blocks(m);
+    CK(h->v_mu.reserve(m, h->st));
+    CK(h->v_var.reserve(m, h->st));
+    CK(h->v_part.reserve((size_t)nblk * 4, h->st));
+    CK(h->v_state.reserve(MV_STATE, h->st));
+    CK(h->v_nan.reserve(1, h->st));
+    const Rows r = {xq, level_idx, nullptr, mean_idx, 0, 1e-8};
+    if ((rc = predict_rows(h, m, r, h->v_mu, h->v_var, nullptr, nullptr, nullptr)) != GPP_OK) return rc;
+    const double sgn = maximize ? 1.0 : -1.0;
+    mv_range_kernel<<<nblk, MV_THREADS, 0, h->st>>>(h->v_mu, h->v_var, m, sgn, h->v_part);
+    CK(cudaGetLastError());
+    mv_range_finish_kernel<<<1, 32, 0, h->st>>>(h->v_part, nblk, h->v_state, h->v_nan);
+    CK(cudaGetLastError());
+    count_launch();
+    count_launch();
+    int nan = 0;
+    CK(cudaMemcpyAsync(&nan, h->v_nan, sizeof(int), cudaMemcpyDeviceToHost, h->st));
+    CK(cudaStreamSynchronize(h->st));
+    if (nan) {
+        g_err = "gpp_max_value_quartiles: NaN or infinity in a candidate's posterior mean or variance";
+        return GPP_ERR_NAN;
+    }
+    auto step = [&](int widen) -> cudaError_t {
+        mv_loglik_kernel<<<nblk, MV_THREADS, 0, h->st>>>(h->v_mu, h->v_var, m, sgn, h->v_state, widen ? 1 : MV_PTS,
+                                                         h->v_part);
+        mv_step_kernel<<<1, 32, 0, h->st>>>(h->v_part, nblk, h->v_state, widen);
+        count_launch();
+        count_launch();
+        return cudaGetLastError();
+    };
+    // widen hi until l(hi) >= log 3/4: for m >~ 1e6 the first bracket misses the upper quartile.  With finite marginals
+    // one doubling puts every term at z >= 15, where log Phi(15) = -3.7e-51, so a second check always passes; the
+    // bound only keeps the loop finite.
+    for (int it = 0;; it++) {
+        if (it == 8) {
+            g_err = "gpp_max_value_quartiles: l(hi) stays below log 3/4 after 8 doublings of the bracket";
+            return GPP_ERR_NAN;
+        }
+        CK(step(1));
+        double flag = 0.0;
+        CK(cudaMemcpyAsync(&flag, h->v_state.p + 11, sizeof(double), cudaMemcpyDeviceToHost, h->st));
+        CK(cudaStreamSynchronize(h->st));
+        if (flag == 0.0) break;
+    }
+    // 40 halvings leave each quartile within 2^-41 (hi - lo) < 1e-12 (hi - lo) of the midpoint returned
+    for (int it = 0; it < 40; it++) CK(step(0));
+    double state[MV_STATE];
+    CK(cudaMemcpyAsync(state, h->v_state, sizeof(double) * MV_STATE, cudaMemcpyDeviceToHost, h->st));
+    CK(cudaStreamSynchronize(h->st));
+    for (int p = 0; p < MV_PTS; p++) {
+        if (!std::isfinite(state[8 + p])) {
+            g_err = "gpp_max_value_quartiles: a quartile is not finite";
+            return GPP_ERR_NAN;
+        }
+    }
+    CK(cudaMemcpyAsync(quartiles, h->v_state.p + 8, sizeof(double) * MV_PTS, cudaMemcpyDefault, h->st));
+    CK(cudaStreamSynchronize(h->st));
     return GPP_OK;
 }
 

@@ -29,7 +29,8 @@ EXPORTS = (
     "gpp_mll_grad",
     "gpp_get_timings", "gpp_get_stats", "gpp_covariance", "gpp_fetch", "gpp_factorize", "gpp_predict", "gpp_predict_grad",
     "gpp_predict_joint", "gpp_sample_posterior", "gpp_posterior_qbatch", "gpp_posterior_qbatch_grad", "gpp_acq_qbatch",
-    "gpp_ipv_points", "gpp_nipv_qbatch", "gpp_kg_qbatch", "gpp_acq_argmax",
+    "gpp_ipv_points", "gpp_nipv_qbatch", "gpp_kg_qbatch", "gpp_gibbon_qbatch", "gpp_max_value_quartiles",
+    "gpp_acq_argmax",
     "gpp_probe_dgemm", "gpp_probe_i8", "gpp_set_fp64_mode", "gpp_get_fp64_mode", "gpp_set_theta_layout", "gpp_objective", "gpp_objective_enqueue", "gpp_objective_collect",
 )
 
@@ -157,6 +158,13 @@ def load_library():
         lib.gpp_kg_qbatch.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                       C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.gpp_kg_qbatch.restype = C.c_int
+        lib.gpp_gibbon_qbatch.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                          C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p,
+                                          C.c_void_p, C.c_void_p]
+        lib.gpp_gibbon_qbatch.restype = C.c_int
+        lib.gpp_max_value_quartiles.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                                C.c_void_p]
+        lib.gpp_max_value_quartiles.restype = C.c_int
         lib.gpp_acq_argmax.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_double,
                                        C.c_double, C.c_double, C.c_double, C.c_void_p, _dp, C.POINTER(C.c_int64)]
@@ -648,6 +656,49 @@ class Engine:
         if rc != GPP_OK:
             _raise(rc, "gpp_kg_qbatch")
         return values, d_xq, jitter
+
+    def gibbon_qbatch(self, xq, q, max_values, projected: bool = False, maximize: bool = True,
+                      want_grad: bool = True, level_idx=None, noise_idx=None, mean_idx=None, out_values=None,
+                      out_d_xq=None):
+        """GIBBON values of the b t-batches of q_tot consecutive rows of ``xq`` (gpp_gibbon_qbatch): the q actual points,
+        then with ``projected`` their copies at the target fidelity (q_tot = 2q; otherwise q_tot = q).  Returns
+        ``(values [b], d_xq [b*q_tot, dq] or None, jitter [b])``, values in nats.  ``max_values`` [K] are samples of
+        the maximum of sigma f in scaled y units, shared by every t-batch; the actual rows are observed with their
+        ``noise_idx`` groups' noise.  ``d_xq`` is d(sum values)/d xq for all rows, computed only when ``want_grad``.
+        Inputs, max values and output buffers may live on the host or on this engine's GPU, like ``predict``'s."""
+        xq, m, level_idx, noise_idx, mean_idx = self._candidates(xq, level_idx, noise_idx, mean_idx)
+        q = int(q)
+        if q < 1:
+            raise ValueError("gibbon_qbatch: q must be >= 1, got %d" % q)
+        b, q_tot = self._tbatches(m, 2 * q if projected else q, "gibbon_qbatch", "q_tot")
+        if isinstance(max_values, np.ndarray) or not hasattr(max_values, "data_ptr"):
+            max_values = _f64(max_values).reshape(-1)
+        if len(max_values.shape) != 1:
+            raise ValueError("gibbon_qbatch: max_values must be one-dimensional, got %s" % (tuple(max_values.shape),))
+        values = np.empty(b) if out_values is None else out_values
+        d_xq = None
+        if want_grad:
+            d_xq = np.empty((m, self.dq)) if out_d_xq is None else out_d_xq
+        jitter = np.empty(b)
+        rc = self._lib.gpp_gibbon_qbatch(self._h, b, q, 1 if projected else 0, _ptr(xq), _ptr(level_idx),
+                                         _ptr(noise_idx), _ptr(mean_idx), 1 if maximize else 0,
+                                         int(max_values.shape[0]), _ptr(max_values), _ptr(values), _ptr(d_xq),
+                                         _ptr(jitter))
+        if rc != GPP_OK:
+            _raise(rc, "gpp_gibbon_qbatch")
+        return values, d_xq, jitter
+
+    def max_value_quartiles(self, xq, level_idx=None, mean_idx=None, maximize: bool = True, out=None):
+        """Quartiles [3] (p = 1/4, 1/2, 3/4) of the maximum of sigma f over the m rows of ``xq`` under their
+        independent posterior marginals (``predict`` at min_var = 1e-8), in scaled y units
+        (gpp_max_value_quartiles).  Inputs and the output buffer may live on the host or on this engine's GPU."""
+        xq, m, level_idx, _, mean_idx = self._candidates(xq, level_idx, None, mean_idx)
+        quartiles = np.empty(3) if out is None else out
+        rc = self._lib.gpp_max_value_quartiles(self._h, m, _ptr(xq), _ptr(level_idx), _ptr(mean_idx),
+                                               1 if maximize else 0, _ptr(quartiles))
+        if rc != GPP_OK:
+            _raise(rc, "gpp_max_value_quartiles")
+        return quartiles
 
     def acq_argmax(self, xq, cost_idx, cost: Sequence[float], kind_by_cost: Sequence[int], best_f: Sequence[float],
                    level_idx=None, mean_idx=None, maximize: bool = True, si: float = 0.0, y_min: float = 0.0,

@@ -1,8 +1,8 @@
-"""Proposing a batch of q points by maximising a batch acquisition (Monte-Carlo qEI, qNEI, qUCB, qNIPV, or the one-shot
-knowledge gradient) of a fitted model: Sobol screening of raw t-batches, then one joint L-BFGS-B run over the best
-restarts with the engine's gradients (GPR.acquisition_qbatch / gpp_acq_qbatch, gpp_nipv_qbatch;
-GPR.knowledge_gradient / gpp_kg_qbatch), and the maximiser of the posterior mean that cost-aware knowledge gradient
-is measured against (GPR.predict / gpp_predict_grad)."""
+"""Proposing a batch of q points by maximising a batch acquisition (Monte-Carlo qEI, qNEI, qUCB, qNIPV, the one-shot
+knowledge gradient, or GIBBON) of a fitted model: Sobol screening of raw t-batches, then one joint L-BFGS-B run over
+the best restarts with the engine's gradients (GPR.acquisition_qbatch / gpp_acq_qbatch, gpp_nipv_qbatch;
+GPR.knowledge_gradient / gpp_kg_qbatch; GPR.gibbon / gpp_gibbon_qbatch), and the maximiser of the posterior mean that
+cost-aware knowledge gradient is measured against (GPR.predict / gpp_predict_grad)."""
 from typing import Dict, Optional, Tuple
 
 import numpy as np
@@ -166,3 +166,69 @@ def optimize_posterior_mean(model, bounds, fixed_columns: Optional[Dict[int, flo
     if v_raw > v:
         X, v = X_raw, v_raw
     return X[0], v
+
+
+def optimize_gibbon(model, bounds, q: int, max_values, fixed_columns: Optional[Dict[int, float]] = None,
+                    target_fixed_columns: Optional[Dict[int, float]] = None, cost_by_source=None, sources=None,
+                    sequential: bool = True, num_restarts: int = 8, raw_samples: int = 256,
+                    options: Optional[dict] = None, seed: int = 0, maximize: bool = True) -> Tuple[torch.Tensor, float]:
+    """Batch ``X`` [q, d] chosen by GIBBON (``model.gibbon`` with ``max_values``, ``maximize``,
+    ``target_fixed_columns`` and ``cost_by_source``), and ``model.gibbon`` of that batch (per unit cost when costs are
+    given).
+
+    ``sequential=True`` is botorch's recommended greedy mode: q steps, each a one-row screening and L-BFGS-B run (as
+    ``optimize_acquisition_qbatch``, seed ``seed + step``) on the gain over the earlier picks, passed as ``X_pending``.
+    ``sources`` (sequential only) runs one such search per listed value of the source column (the last column) at
+    every step and keeps the pick with the highest gain per unit cost; ties go to the first listed source.
+    ``sequential=False`` optimises the q rows jointly in one run.  ``bounds`` and ``fixed_columns`` are those of
+    ``optimize_acquisition_qbatch``; a search's best screened row replaces its optimised one when it scores higher."""
+    q = int(q)
+    if q < 1:
+        raise ValueError("optimize_gibbon: q must be >= 1, got %d" % q)
+    fixed_columns = dict(fixed_columns or {})
+    if sources is not None:
+        if not sequential:
+            raise ValueError("optimize_gibbon: sources needs sequential=True")
+        if len(sources) == 0:
+            raise ValueError("optimize_gibbon: sources is empty")
+        last = int(model.train_inputs[0].shape[1]) - 1
+        if last in model._quant_columns():
+            raise ValueError("optimize_gibbon: sources needs a source column (the last), not a quantitative one")
+        fixed_columns.setdefault(last, float(sources[0]))  # the source column is set per search
+    d, cols, lo, hi, fixed = _columns(model, bounds, fixed_columns, "optimize_gibbon")
+    kw = dict(maximize=maximize, target_fixed_columns=target_fixed_columns, cost_by_source=cost_by_source)
+
+    def full_with(fx: Dict[int, float], rows: int):
+        def full(z: torch.Tensor) -> torch.Tensor:  # quantitative inputs [k, rows, dq] -> model inputs [k, rows, d]
+            X = torch.zeros(z.shape[0], rows, d, dtype=torch.float64)
+            X[:, :, cols] = z
+            for c, v in fx.items():
+                X[:, :, c] = float(v)
+            return X
+        return full
+
+    def search(fx: Dict[int, float], rows: int, pending: Optional[torch.Tensor], step_seed: int):
+        X, v, X_raw, v_raw = _multistart(lambda X: model.gibbon(X, max_values, X_pending=pending, **kw),
+                                         full_with(fx, rows), cols, lo, hi, rows, num_restarts, raw_samples, options,
+                                         step_seed)
+        return (X_raw, v_raw) if v_raw > v else (X, v)
+
+    if sequential:
+        picks = []
+        for step in range(q):
+            pending = torch.stack(picks) if picks else None
+            best = None
+            for src in (sources if sources is not None else [None]):
+                fx = dict(fixed)
+                if src is not None:
+                    fx[d - 1] = float(src)
+                X1, v1 = search(fx, 1, pending, int(seed) + step)
+                if best is None or v1 > best[1]:
+                    best = (X1[0], v1)
+            picks.append(best[0])
+        X = torch.stack(picks)
+    else:
+        X, _ = search(fixed, q, None, int(seed))
+    with torch.no_grad():
+        v = float(model.gibbon(X[None], max_values, **kw)[0])
+    return X, v

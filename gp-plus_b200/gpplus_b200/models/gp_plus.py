@@ -500,6 +500,20 @@ class GP_Plus(GPR):
         return super().knowledge_gradient(X, num_fantasies, base_samples=base_samples, seed=seed, maximize=maximize,
                                           current_value=current_value, cost_by_source=cost_by_source)
 
+    def gibbon(self, X, max_values, maximize=True, target_fixed_columns=None, X_pending=None, cost_by_source=None):
+        """GIBBON values of the t-batches of ``X`` [..., q, d] in nats, optionally against the target rows of
+        ``target_fixed_columns``, net of ``X_pending`` and per unit cost of the rows' sources (GPR.gibbon);
+        differentiable in ``X`` when it requires a gradient, as ``predict_with_grad``."""
+        X = data_type_check(X)
+        return super().gibbon(X, max_values, maximize=maximize, target_fixed_columns=target_fixed_columns,
+                              X_pending=X_pending, cost_by_source=cost_by_source)
+
+    def sample_max_values(self, candidate_set, num_samples=10, method="gumbel", maximize=True, seed=0):
+        """Samples of the optimum of f over ``candidate_set`` [M, d] in the original y units (GPR.sample_max_values)."""
+        candidate_set = data_type_check(candidate_set)
+        return super().sample_max_values(candidate_set, num_samples=num_samples, method=method, maximize=maximize,
+                                         seed=seed)
+
     def noise_value(self):
         return self.likelihood.noise_covar.noise.detach() * self.y_std ** 2
 

@@ -216,6 +216,33 @@ class _EngineKG(_EngineQBatchAcquisition):
         return torch.as_tensor(np.asarray(values)), jitter
 
 
+class _EngineGIBBON(_EngineQBatchAcquisition):
+    """GIBBON values [b] of the t-batches of ``x`` [b, q, d] (gpp_gibbon_qbatch), differentiable w.r.t. the
+    quantitative columns of ``x`` as ``_EngineQBatchAcquisition``, whose backward it shares.  The engine's t-batches
+    hold the q rows of ``x``, then the pending rows, then (projected) the target copies of both.  ``layout`` is
+    (q_eff, held): q_eff rows per half, and the columns the target rows hold at a fixed value.  A target row copies
+    every other quantitative column of its actual row, so row i's gradient in column c is d_xq[i, c] +
+    d_xq[q_eff + i, c], and d_xq[i, c] alone for a held column.  Pending rows get none."""
+
+    @staticmethod
+    def forward(ctx, x, eng, xq, layout, cols, kwargs):
+        b, q, d = x.shape
+        q_eff, held = layout
+        values, d_xq, jitter = eng.gibbon_qbatch(xq, q_eff, want_grad=len(cols) > 0, **kwargs)
+        dx = torch.zeros(b, q, d, dtype=torch.float64)
+        if len(cols) > 0:
+            g = torch.as_tensor(np.asarray(d_xq)).reshape(b, -1, len(cols))
+            if kwargs["projected"]:
+                copied = torch.tensor([c not in held for c in cols], dtype=torch.float64)
+                g = g[:, :q_eff] + g[:, q_eff:] * copied
+            dx[:, :, cols] = g[:, :q]
+        ctx.dx = dx
+        ctx.x_meta = (x.dtype, x.device)
+        jitter = torch.as_tensor(np.asarray(jitter))
+        ctx.mark_non_differentiable(jitter)
+        return torch.as_tensor(np.asarray(values)), jitter
+
+
 class GPR(Module):
     def __init__(
         self,
@@ -764,6 +791,118 @@ class GPR(Module):
             cost = torch.tensor([[float(cost_by_source[int(s_)]) for s_ in row] for row in src.tolist()],
                                 dtype=torch.float64).sum(-1)
             out = out / cost.to(dtype)
+        return out.reshape(batch)
+
+    def sample_max_values(self, candidate_set: torch.Tensor, num_samples: int = 10, method: str = "gumbel",
+                          maximize: bool = True, seed: int = 0) -> torch.Tensor:
+        """``num_samples`` samples [K] of the optimum of f over ``candidate_set`` [M, d] in the original y units: the
+        maximum when ``maximize``, else the minimum (botorch's max-value samplers for max-value entropy search; for
+        multi-fidelity pass the candidates at the target fidelity).
+
+        ``method="gumbel"`` is botorch's _sample_max_value_Gumbel: the engine finds the quartiles of the maximum under
+        the candidates' independent marginals (gpp_max_value_quartiles, the marginals never leave the GPU), a Gumbel
+        distribution is fitted to them and sampled at ``num_samples`` uniforms.  ``method="thompson"`` takes the
+        optimum over the candidates of each joint posterior draw (``sample_posterior``, M <= MAX_JOINT).  The uniforms
+        or normals come from a ``torch.Generator`` seeded with ``seed``."""
+        if method not in ("gumbel", "thompson"):
+            raise ValueError("sample_max_values: method must be 'gumbel' or 'thompson', got %r" % (method,))
+        k = int(num_samples)
+        if k < 1:
+            raise ValueError("sample_max_values: num_samples must be >= 1, got %d" % k)
+        if candidate_set.dim() != 2:
+            raise ValueError("sample_max_values expects candidate_set of shape [M, d]")
+        gen = torch.Generator().manual_seed(int(seed))
+        sgn = 1.0 if maximize else -1.0
+        dtype = self._out_dtype()
+        with torch.no_grad():
+            if method == "thompson":
+                if candidate_set.shape[0] > _engine.MAX_JOINT:
+                    raise ValueError("sample_max_values: Thompson sampling takes at most %d candidates, got %d"
+                                     % (_engine.MAX_JOINT, candidate_set.shape[0]))
+                base = torch.randn(k, int(candidate_set.shape[0]), generator=gen, dtype=torch.float64)
+                draws = self.sample_posterior(candidate_set, k, base_samples=base)
+                return draws.amax(-1) if maximize else draws.amin(-1)
+            eng, xq, kwargs = self._joint_request(candidate_set, False)
+            y1, y2, y3 = (float(v) for v in np.asarray(eng.max_value_quartiles(
+                xq, level_idx=kwargs["level_idx"], mean_idx=kwargs["mean_idx"], maximize=bool(maximize))))
+            beta = (y1 - y3) / (math.log(math.log(4.0 / 3.0)) - math.log(math.log(4.0)))
+            alpha = y2 + beta * math.log(math.log(2.0))
+            u = torch.rand(k, generator=gen, dtype=torch.float64)
+            m_sc = alpha - beta * torch.log(-torch.log(u))
+            return float(self.y_min) + sgn * float(self.y_std) * m_sc.to(dtype)
+
+    def gibbon(self, X: torch.Tensor, max_values, maximize: bool = True, target_fixed_columns=None, X_pending=None,
+               cost_by_source=None) -> torch.Tensor:
+        """GIBBON (botorch's qLowerBoundMaxValueEntropy; with ``target_fixed_columns``,
+        qMultiFidelityLowerBoundMaxValueEntropy) of every t-batch of X [..., q, d]: values [...] in nats
+        (gpp_gibbon_qbatch).  The value is the diversity of the batch (1/2 log det of the correlation matrix of its
+        noisy observations) plus, per row, 1/2 log of the variance of its observation over that variance given that
+        f at the row (at its target-fidelity copy) stays below the optimum, averaged over ``max_values`` [K] (samples
+        of the optimum in the original y units, e.g. from ``sample_max_values``).
+
+        ``target_fixed_columns`` ({column: value}, e.g. the source column at the target fidelity, or a continuous
+        fidelity column at its target value) gives the target rows: X with those columns overwritten, so a held
+        quantitative column passes no gradient through the target rows.  ``X_pending`` [p, d] is appended to every t-batch and the value
+        becomes the gain alpha([X_t, X_pending]) - alpha(X_pending).  ``cost_by_source`` ({source: cost} or a
+        sequence indexed by source) then divides that gain by the summed cost of X_t's rows, whose source is the last
+        column.  The values are differentiable in the quantitative columns of X when it requires a gradient; a
+        t-batch whose covariance needed jitter raises a NumericalWarning."""
+        if X.dim() < 2:
+            raise ValueError("gibbon expects X of shape [..., q, d]")
+        self.eval()
+        batch, q, d = X.shape[:-2], int(X.shape[-2]), int(X.shape[-1])
+        mv = torch.as_tensor(max_values).detach().to("cpu", torch.float64).reshape(-1)
+        if not 1 <= mv.numel() <= _engine.MAX_MC_SAMPLES:
+            raise ValueError("gibbon: between 1 and %d max values, got %d" % (_engine.MAX_MC_SAMPLES, mv.numel()))
+        sgn = 1.0 if maximize else -1.0
+        m_sc = np.ascontiguousarray((sgn * (mv - float(self.y_min)) / float(self.y_std)).numpy())
+        pend = None
+        if X_pending is not None:
+            pend = torch.as_tensor(X_pending).detach().to("cpu", torch.float64).reshape(-1, d)
+        q_eff = q + (0 if pend is None else int(pend.shape[0]))
+        proj = target_fixed_columns is not None
+        if q < 1 or q_eff * (2 if proj else 1) > _engine.MAX_QBATCH:
+            raise ValueError("gibbon: %d rows per t-batch (with pending and target rows) is outside [1, %d]"
+                             % (q_eff * (2 if proj else 1), _engine.MAX_QBATCH))
+
+        def rows(xa: torch.Tensor) -> torch.Tensor:  # [b, r, d] -> the engine's t-batches [b, r or 2r, d]
+            if not proj:
+                return xa
+            xt = xa.clone()
+            for c, v in target_fixed_columns.items():
+                xt[:, :, int(c)] = float(v)
+            return torch.cat([xa, xt], 1)
+
+        def request(xa: torch.Tensor):
+            x_all = rows(xa)
+            eng, xq, kwargs = self._joint_request(x_all.reshape(-1, d), True)
+            kwargs.pop("include_noise")
+            kwargs.update(max_values=m_sc, projected=proj, maximize=bool(maximize))
+            return eng, xq, kwargs
+
+        x = X.reshape(-1, q, d)
+        xd = x.detach().to("cpu", torch.float64)
+        xa = xd if pend is None else torch.cat([xd, pend.expand(xd.shape[0], -1, -1)], 1)
+        eng, xq, kwargs = request(xa)
+        if torch.is_grad_enabled() and X.requires_grad:
+            held = tuple(int(c) for c in target_fixed_columns) if proj else ()
+            v, jitter = _EngineGIBBON.apply(x, eng, xq, (q_eff, held), self._quant_columns(), kwargs)
+        else:
+            values, _, jitter = eng.gibbon_qbatch(xq, q_eff, want_grad=False, **kwargs)
+            v, jitter = torch.as_tensor(np.asarray(values)), torch.as_tensor(np.asarray(jitter))
+        if pend is not None:
+            eng, xq, kwargs = request(pend[None])
+            base, _, jit_p = eng.gibbon_qbatch(xq, int(pend.shape[0]), want_grad=False, **kwargs)
+            v = v - float(np.asarray(base)[0])
+            jitter = torch.cat([jitter, torch.as_tensor(np.asarray(jit_p))])
+        if bool((jitter > 0).any()):
+            warnings.warn("A not p.d., added jitter of %.1e to the diagonal" % float(jitter.max()), NumericalWarning)
+        out = v.to(self._out_dtype())
+        if cost_by_source is not None:
+            src = xd[:, :, -1].round().long()
+            cost = torch.tensor([[float(cost_by_source[int(s_)]) for s_ in row] for row in src.tolist()],
+                                dtype=torch.float64).sum(-1)
+            out = out / cost.to(out.dtype)
         return out.reshape(batch)
 
     def reset_parameters(self) -> None:

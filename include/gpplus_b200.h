@@ -20,6 +20,9 @@
  *                                 -> gpp_ipv_points, gpp_nipv_qbatch
  *   - botorch one-shot qKnowledgeGradient (cost-aware as qMultiFidelityKnowledgeGradient) and its gradient in X:
  *     GPR.knowledge_gradient, bayesian_optimizations/qbatch.py -> gpp_kg_qbatch
+ *   - botorch qLowerBoundMaxValueEntropy / qMultiFidelityLowerBoundMaxValueEntropy (GIBBON) and its gradient in X, and
+ *     the max-value samples of _sample_max_value_Gumbel: GPR.gibbon, GPR.sample_max_values,
+ *     bayesian_optimizations/qbatch.py -> gpp_gibbon_qbatch, gpp_max_value_quartiles
  *   - AF_*_Engineering + argmax   bayesian_optimizations/AFs.py:102-159,
  *                                 bayesian_optimizations/BO_GP_plus.py:183-194 -> gpp_acq_argmax
  *   - covar_module(x).evaluate()  models/gp_plus.py:472-474      -> gpp_covariance
@@ -322,6 +325,44 @@ int gpp_kg_qbatch(gpp_handle* h, int64_t b, int32_t q, int32_t n_fantasies, cons
                   double* values,              /* [b] */
                   double* d_xq,                /* [b * (q + n_fantasies) * dq] or NULL: values only */
                   double* jitter);             /* [b] or NULL */
+
+/* GIBBON, the lower bound of max-value entropy search (botorch's qLowerBoundMaxValueEntropy and, with target rows,
+ * qMultiFidelityLowerBoundMaxValueEntropy, acquisition/max_value_entropy_search.py; Moss et al., 2021).  Each of the b
+ * t-batches holds q_tot consecutive rows of xq: the q actual points x_1..x_q, then with projected = 1 their copies
+ * g_1..g_q at the target fidelity (tau(i) = q + i, q_tot = 2q; projected = 0: tau(i) = i, q_tot = q).  With mu and
+ * Sigma bitwise those of gpp_posterior_qbatch(..., include_noise = 0) on the same rows, n_i the noise of row i's group
+ * (a NULL noise_idx means group 0), eps = 1e-8, sigma = +1 to maximise and -1 to minimise, in scaled y units:
+ *   V = Sigma[0:q, 0:q] + diag(n_i),  L L^T = V + j_t I   j_t the first of 0, 1e-8, 1e-7, 1e-6 that factors
+ *   v_i = max(V_ii, eps)  s_i^2 = max(Sigma_tau(i)tau(i), eps)  c_i = Sigma_i,tau(i)  rho_i^2 = c_i^2 / (v_i s_i^2)
+ *   gamma_ik = (m_k - sigma mu_tau(i)) / s_i,  r_ik = phi(gamma_ik) / max(Phi(gamma_ik), eps)
+ *   Q_i = -(1/2K) sum_k log max(1 - rho_i^2 r_ik (gamma_ik + r_ik), eps)      quality of row i
+ *   D   = sum_i (log L_ii - 1/2 log (V + j_t I)_ii)                            diversity
+ *   values[t] = D + sum_i Q_i   (nats)
+ * m_k = max_values[k], K = n_max_values samples of max sigma f in scaled units, shared by every t-batch.
+ *   d_xq [b*q_tot*dq] = d(sum_t values[t]) / d xq for all q_tot rows, quantitative inputs only (NULL: values only)
+ *   jitter [b] = j_t (may be NULL)
+ * A t-batch's outputs do not depend on the other t-batches of the call or on how it is split into chunks.  The call
+ * does not change the factor of K_y, alpha, gpp_get_stats or gpp_get_timings.  GPP_ERR_NOT_PD when a t-batch fails
+ * every rung, GPP_ERR_NAN on NaN.  q < 1, projected not 0 or 1, q_tot > GPP_MAX_QBATCH, b < 0, n_max_values outside
+ * [1, GPP_MAX_MC_SAMPLES], a missing max_values or values, or dq > 32 return GPP_ERR_ARG before any allocation.  It
+ * uses the buffers of gpp_acq_qbatch (the max values in its base-sample buffer) and allocates none of its own. */
+int gpp_gibbon_qbatch(gpp_handle* h, int64_t b, int32_t q, int32_t projected, const double* xq,
+                      const int32_t* level_idx, const int32_t* noise_idx, const int32_t* mean_idx, int maximize,
+                      int64_t n_max_values, const double* max_values, /* [K] samples of max sigma f, scaled units */
+                      double* values,                               /* [b] */
+                      double* d_xq,                                 /* [b * q_tot * dq] or NULL: values only */
+                      double* jitter);                              /* [b] or NULL */
+
+/* Quartiles of the maximum of sigma f over m candidates under independent marginals (botorch's
+ * _sample_max_value_Gumbel, acquisition/max_value_entropy_search.py, without the marginals leaving the device).  The
+ * marginals mu_j, s_j^2 are gpp_predict's at include_noise = 0, min_var = 1e-8 (bitwise), held in two buffers of m
+ * doubles on the handle.  quartiles[0..2] solve l(y) = sum_j log Phi((y - sigma mu_j) / s_j) = log p for p = 1/4, 1/2,
+ * 3/4 by bisection, each to within 1e-12 (hi - lo) of the bracket: lo = min sigma mu - 5 max s, hi = max sigma mu +
+ * 5 max s, hi doubled away from lo while l(hi) < log 3/4.  The sums run in an order that depends only on m.  GPP_ERR_NAN
+ * on a NaN or infinite marginal; m < 1, a missing quartiles, xq or level_idx, or dq > 32 return GPP_ERR_ARG.  quartiles may be
+ * host or device memory. */
+int gpp_max_value_quartiles(gpp_handle* h, int64_t m, const double* xq, const int32_t* level_idx,
+                            const int32_t* mean_idx, int maximize, double* quartiles /* [3], scaled units */);
 
 /* fused predict + acquisition + argmax over m candidates (BO_GP_plus.py:183-194).
  * y_min/y_std undo the target scaling; cost_idx[m] selects cost[n_cost]; kind_by_cost[n_cost]
